@@ -16,7 +16,10 @@ north-star step (10-D ARD, n = 4096, 1 000 000 candidates x 100 000 MC points). 
 `extras` of every line: cfg-1 (N = 1), cfg-3 (whole 1 024-point conditional-entropy design from 250 000 candidates) and
 cfg-4 (512-point MI design; pool 40 000 / 80 000 / 120 000 / 200 000 on 1 / 2 / 4 / 8 GPUs).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
+
+--dump-outputs DIR writes what the last timed step returned to its caller as float64 .npy files (see dump_step_outputs);
+the inputs are seeded, so two builds run with the same arguments can be compared output for output.
 
 --impl reference times the UNMODIFIED reference (baseline/_ref/gpExp, staged by __graft_entry__.build(); the line-by-line
 oracle port if it is absent) on the host cores: costFunctionGP_IVAR.evaluate (experimentalDesign.py:79-117 ->
@@ -54,6 +57,31 @@ def make_inputs():
     cand = rng.uniform(-1.0, 1.0, (CFG["C"], CFG["d"]))
     mc = rng.uniform(-1.0, 1.0, (CFG["M"], CFG["d"]))
     return cand, mc
+
+
+def dump_step_outputs(out_dir, eng, n_points, total_c, torch, dist, world, rank):
+    """What a caller of the timed step `eng.run(256)` receives, taken after the last timed step (restore() resets only the
+    running variances, so these still hold that step's results): the 256 design indices (exact in float64), the cost of
+    each pick, the pivot var_D(p) + noise of each pick, and the cost of every one of the candidates at design size 255.
+    0.8 MB in all at cfg-2 size.  With N > 1 the candidate costs of the ranks' contiguous blocks are gathered in global
+    order and rank 0 writes."""
+    scores = eng.scores[: eng.cand.n]
+    if world > 1:
+        from gpexp_b200.engine import Shard
+        width = -(-total_c // world)
+        mine = torch.zeros(width, dtype=torch.float64, device=scores.device)
+        mine[: scores.numel()] = scores
+        parts = [torch.empty_like(mine) for _ in range(world)]
+        dist.all_gather(parts, mine)
+        sizes = [hi - lo for lo, hi in (Shard.split(total_c, world, r) for r in range(world))]
+        scores = torch.cat([p[:s] for p, s in zip(parts, sizes)])
+    if rank != 0:
+        return
+    os.makedirs(out_dir, exist_ok=True)
+    out = {"indices": eng.picks[:n_points], "pick_scores": eng.pick_scores[:n_points], "pivots": eng.pick_pivots[:n_points],
+           "scores": scores}
+    for name, t in out.items():
+        np.save(os.path.join(out_dir, name + ".npy"), t.cpu().numpy().astype(np.float64))
 
 
 # ---------------------------------------------------------------------------------------------
@@ -530,6 +558,8 @@ def run_ours(args):
     launches = dev.launches - launches0
     ms = ev[0].elapsed_time(ev[1])
     clk = clocks.stop() if clocks else None
+    if args.dump_outputs:
+        dump_step_outputs(args.dump_outputs, eng, N, cand_all.shape[0], torch, dist, world, rank)
     # the dominant kernel alone, on the same state (its CUDA-event time is what the roofline is computed from)
     kev = [(torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)) for _ in range(args.steps)]
     for s in range(args.steps):
@@ -837,7 +867,11 @@ def main():
     ap.add_argument("--no-configs", action="store_true", help="skip extras.cfg3 / extras.cfg4 (the other BASELINE configurations)")
     ap.add_argument("--quick-design", action="store_true",
                     help="profiling aid: load a random 255-point design instead of running the 255 greedy steps")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the outputs of the last timed step to DIR/<name>.npy (float64) for output-for-output comparison")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
     if args.impl == "reference":
         run_reference(args)

@@ -1,9 +1,12 @@
-"""CPU-side checks of the driver contract: build() is callable, and the reference arm of bench.py prints exactly one
-JSON line with the keys the driver reads (the GPU arm needs a B200 and is exercised by the driver itself)."""
+"""Checks of the benchmark's interface: build() is callable, the reference arm of bench.py prints exactly one JSON line
+with the keys a reader of the result expects, and (on a GPU) --dump-outputs writes the results of the timed step."""
 import json
 import os
 import subprocess
 import sys
+
+import numpy as np
+import pytest
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
@@ -54,3 +57,19 @@ def test_cpu_legs_of_the_other_configs_print_one_json_line():
     assert d["kind"] == "reference" and d["cores"] >= 1
     for cfg in ("cfg1", "cfg3", "cfg4"):
         assert d[cfg]["candidates_per_s_per_step"] > 0 and d[cfg]["seconds"] < 120 and d[cfg]["sample"]
+
+
+@pytest.mark.gpu
+def test_dump_outputs_of_the_timed_step(tmp_path):
+    """--dump-outputs: the 256 picks of the timed step, their costs and pivots, and the cost of every candidate, as float64;
+    the last pick is the arg-min of those costs.  --quick-design keeps the run short (same state shape, random design)."""
+    out = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--steps", "1", "--quick-design", "--no-cpu",
+                          "--no-configs", "--dump-outputs", str(tmp_path)], capture_output=True, text=True, timeout=900, cwd=ROOT)
+    assert out.returncode == 0, out.stderr[-2000:]
+    assert json.loads(out.stdout.strip().splitlines()[-1])["steps"] == 1
+    z = {n: np.load(tmp_path / f"{n}.npy") for n in ("indices", "pick_scores", "pivots", "scores")}
+    assert all(a.dtype == np.float64 for a in z.values())
+    assert z["indices"].shape == z["pick_scores"].shape == z["pivots"].shape == (256,) and z["scores"].shape == (100_000,)
+    last = int(z["indices"][-1])
+    assert z["scores"][last] == z["scores"].min() == z["pick_scores"][-1]
+    assert np.all(np.isfinite(z["scores"])) and z["pivots"][-1] > 0

@@ -709,12 +709,12 @@ def test_ivar_gradient_matches_finite_differences(gx):
 
 @pytest.fixture(scope="module")
 def patched_ref(gx):
-    """The UNMODIFIED reference package from baseline/_ref (copied there by __graft_entry__.build(); git-ignored, shipped to
-    the GPU box), with its hot methods rebound by gpexp_b200.install_as_gpExp: its own constructors and optimiser loops run
+    """The UNMODIFIED reference package from baseline/_ref (copied there by __graft_entry__.build() from $GPEXP_REFERENCE;
+    git-ignored), with its hot methods rebound by gpexp_b200.install_as_gpExp: its own constructors and optimiser loops run
     on the device path."""
     path = os.path.join(ROOT, "baseline", "_ref")
     if not os.path.isdir(os.path.join(path, "gpExp")):
-        pytest.skip("baseline/_ref/gpExp is not present (run __graft_entry__.build() where /root/reference exists)")
+        pytest.skip("baseline/_ref/gpExp is not present (set GPEXP_REFERENCE and run __graft_entry__.build() to stage it)")
     import gpexp_b200
     ref = gpexp_b200.install_as_gpExp(path)
     import importlib
