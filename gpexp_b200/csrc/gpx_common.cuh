@@ -198,12 +198,35 @@ __device__ __forceinline__ void gpx_append_two_columns(const KParams& kp, const 
 }
 
 // 2^(j/256): table-driven exp used by the covariance prologue of the hot kernel and by the Gram kernel.  exp(x) = 2^k * T[j] * e^r with
-// n = rint(x * 256/ln2) = 256 k + j and |r| <= ln2/512, e^r - 1 by a degree-4 polynomial: 9 FP64-pipe
-// operations and one shared-memory lookup per value, <= 1 ulp (libdevice exp: 19 FP64 + 26 other instructions).
+// n = rint(x * 256/ln2) = 256 k + j and |r| <= ln2/512, e^r - 1 by a degree-4 polynomial: 9 FP64-pipe operations, one
+// compare and one shared-memory lookup per value (libdevice exp: 19 FP64 + 26 other instructions).
+// The callers fold the signal variance (and a sign) into the table, tab[j] = s * 2^(j/256), so the result is s * exp(x)
+// for any normal s; its exponent is assembled in the high word as (biased exponent of tab[j] e^r) + k.
+//   accuracy  <= 2 ulp of s * exp(x) for an exact argument (measured over every table slot and |x| <= 700: the entry,
+//             the polynomial and the final product each round once); the rounding of x itself adds |x| eps relative.
+//   flush     a result below 2^-1022 (biased exponent <= 0) is returned as 0 -- no subnormals; so is every x below
+//             -2^19 ln2/256 ~ -1453, where k << 20 would leave the int range (and, below -5.8e6, n its 32 bits).
+//   OVF       a result above DBL_MAX (biased exponent > 2046), and every x above +1453, saturates to +-inf with the
+//             sign of the table.  Only the Mehler exponent can be large and positive (x ~ y, kernels.py:282-285); the
+//             SE and Matern exponents are <= 0 up to cancellation error, so their instantiations leave it out.
 static __device__ const double gpx_exp2_tab[256] = {
 #include "gpx_exp_table.inc"
 };
 
+// 2^k * res for a table value res = tab[j] e^r, with the flush / saturation rules above; nf = n exactly (as a double)
+template <bool OVF>
+__device__ __forceinline__ double gpx_exp_tab_scale(double res, int n, double nf) {
+    const int hi = __double2hiint(res);
+    const int k = n >> 8;
+    const int e = ((hi >> 20) & 0x7ff) + k;                     // biased exponent of the result
+    // |nf| > 2^19 first: there k (and beyond 2^31 n itself) has wrapped, so e means nothing
+    if (nf < -0x1p19) return 0.0;
+    if (OVF && (nf > 0x1p19 || e > 2046)) return __hiloint2double((hi & 0x80000000) | 0x7ff00000, 0);
+    if (e <= 0) return 0.0;
+    return __hiloint2double(hi + (k << 20), __double2loint(res));
+}
+
+template <bool OVF = false>
 __device__ __forceinline__ double gpx_exp_tab(double x, const double* __restrict__ tab) {
     const double MAGIC = 6755399441055744.0;                    // 1.5 * 2^52
     const double t = fma(x, 0x1.71547652b82fep+8, MAGIC);       // x * 256/ln2, rounded to an integer in the low word
@@ -216,14 +239,12 @@ __device__ __forceinline__ double gpx_exp_tab(double x, const double* __restrict
     p = fma(p, r, 1.0);
     const double q = p * r;                                     // e^r - 1
     const double tj = tab[n & 255];
-    double res = fma(tj, q, tj);
-    res = __hiloint2double(__double2hiint(res) + ((n >> 8) << 20), __double2loint(res));  // * 2^k
-    return n < -261632 ? 0.0 : res;                             // below 2^-1022: flush (x < -708.4)
+    return gpx_exp_tab_scale<OVF>(fma(tj, q, tj), n, nf);
 }
 
 // exp(-S * ln2/256) for an exponent that was accumulated ALREADY SCALED by 256/ln2 (S >= 0): the SE Gram kernel folds
 // sqrt(a_q/2 * 256/ln2) into its coordinates, so that S = sum ((x_q - y_q) w_q)^2 costs two FP64 operations per dimension
-// and the argument scaling of gpx_exp_tab disappears.  Same table, same polynomial.
+// and the argument scaling of gpx_exp_tab disappears.  Same table, same polynomial, same flush rule (S > 2^19 gives 0).
 __device__ __forceinline__ double gpx_exp_tab_scaled(double S, const double* __restrict__ tab) {
     const double MAGIC = 6755399441055744.0;                    // 1.5 * 2^52
     const double t = MAGIC - S;                                 // -rint(S) in the low word
@@ -235,9 +256,7 @@ __device__ __forceinline__ double gpx_exp_tab_scaled(double S, const double* __r
     p = fma(p, r, 1.0);
     const double q = p * r;                                     // e^r - 1
     const double tj = tab[n & 255];
-    double res = fma(tj, q, tj);
-    res = __hiloint2double(__double2hiint(res) + ((n >> 8) << 20), __double2loint(res));  // * 2^k
-    return n < -261632 ? 0.0 : res;                             // below 2^-1022: flush
+    return gpx_exp_tab_scale<false>(fma(tj, q, tj), n, nf);
 }
 
 // difference-form finish with the table exp; `tab` already carries the signal variance (tab[j] = signal * 2^(j/256))
@@ -248,7 +267,7 @@ __device__ __forceinline__ double kfinish_tab(double acc, const KParams& kp, con
         const double t = kp.c0 * sqrt(acc);
         return (1.0 + t) * gpx_exp_tab(-t, tab);
     }
-    return gpx_exp_tab(-acc, tab);
+    return gpx_exp_tab<true>(-acc, tab);
 }
 
 // Expanded form used by the tensor-core prologue:  k = kexpand(alpha(x) + beta(y) + sum_i u_i(x) v_i(y)).

@@ -47,7 +47,7 @@ __device__ __forceinline__ double neg_kexpand_tab(double e, const KParams& kp, c
         const double t = kp.c0 * sqrt(fmax(e, 0.0));
         return (1.0 + t) * gpx_exp_tab(-t, ntab);
     }
-    return gpx_exp_tab(e, ntab);
+    return gpx_exp_tab<FAM == GPX_MEHLER>(e, ntab);
 }
 
 constexpr int BN = 128;
