@@ -14,6 +14,7 @@ LIB_PATH = os.environ.get("GPX_LIB") or os.path.join(HERE, "lib", "libgpexp_b200
 GPX_VERSION = 200
 GPX_MAX_DIM = 16
 GPX_KROWS = 16
+GPX_I8_MAX_N = 16384  # largest design size the INT8 IVAR core runs
 GPX_PIVOT_HDR = 3 + GPX_MAX_DIM
 GPX_COMM_ID_BYTES = 128
 SE, MATERN32, MEHLER = 0, 1, 2
@@ -87,6 +88,9 @@ SIGNATURES = {
     "gpx_argreduce": [_p, _p, _p, _p, _i64, _int, _p, _p, _p],
     "gpx_sum": [_p, _p, _i64, _p, _p],
     "gpx_set_ivar_ring": [_p, _int],
+    "gpx_set_ivar_core": [_p, _int],
+    "gpx_ivar_scratch_bytes": [_p, _i64, _i64, _i64],
+    "gpx_set_ivar_scratch": [_p, _p, _i64],
     "gpx_score_ivar_workspace": [_p, _i64, _i64],
     "gpx_score_ivar": [_p, _int, _p, _i64, _p, _p, _i64, _p, _i64, _p, _p, _i64, _i64, _dbl, _dbl, _p, _p, _p, _p, _p, _p],
     "gpx_cov_segments": [_i64, _i64],
@@ -131,7 +135,7 @@ SIGNATURES = {
     "gpx_bench_dmma": [_p, _i64, _p, _p],
     "gpx_bench_dfma": [_p, _i64, _p, _p],
 }
-_RESTYPES = {"gpx_last_error": C.c_char_p, "gpx_score_ivar_workspace": _i64, "gpx_mi_prec_column_workspace": _i64,
+_RESTYPES = {"gpx_last_error": C.c_char_p, "gpx_score_ivar_workspace": _i64, "gpx_ivar_scratch_bytes": _i64, "gpx_mi_prec_column_workspace": _i64,
              "gpx_state_bytes": _i64, "gpx_launch_count": _i64, "gpx_se_loglike_grad_workspace": _i64,
              "gpx_gram_matvec_workspace": _i64}
 

@@ -80,6 +80,8 @@ extern "C" int gpx_create(int device, gpx_handle* out) {
     {
         const char* e = getenv("GPX_IVAR_RING");
         c->ivar_ring = (e && e[0] >= '0' && e[0] <= '2' && e[1] == 0) ? (e[0] - '0') : GPX_DEFAULT_IVAR_RING;
+        const char* k = getenv("GPX_IVAR_CORE");
+        c->ivar_core = (k && strcmp(k, "dmma") == 0) ? GPX_CORE_DMMA : GPX_CORE_I8;
     }
     bool ok = cudaMalloc(&c->red_val, GPX_RED_SLOTS * sizeof(double)) == cudaSuccess &&
               cudaMalloc(&c->red_idx, GPX_RED_SLOTS * sizeof(int64_t)) == cudaSuccess &&

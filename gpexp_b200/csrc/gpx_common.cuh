@@ -52,6 +52,9 @@ struct gpx_context {
     void* nccl_comm;
     int comm_rank, comm_size;
     int ivar_ring;            // ring geometry of ivar_ws_kernel (gpx_set_ivar_ring)
+    int ivar_core;            // GPX_CORE_DMMA | GPX_CORE_I8 (gpx_set_ivar_core)
+    void* i8_scratch;         // caller memory for the INT8 core's operand slices (gpx_set_ivar_scratch)
+    int64_t i8_scratch_bytes;
 };
 
 #ifndef GPX_DEFAULT_IVAR_RING

@@ -994,11 +994,368 @@ int prologue_rows(gpx_handle h, int prologue) {
     return -1;
 }
 
+// ---------------------------------------------------------------------------------------------
+// INT8 tensor-core IVAR core (tcgen05.mma .kind::i8): the contraction S = W_M^T W_C emulated exactly by fixed-point
+// slicing (Ozaki-style).  Each column x = W[:, c] gets a power-of-two scale 2^e_c > max_i |x_i| and the integer
+//     Y[i, c] = rint(x_i * 2^(54 - e_c)),   |Y| <= 2^54,
+// written as I8_L = 7 balanced base-256 digits  Y = sum_p a_p 256^(6-p),  a_1..a_6 in [-128, 127],  |a_0| <= 64.
+// Then  sum_i Y_M Y_C = sum_t D_t 256^(12-t),  D_t = sum_{p+q=t} sum_i a_p(m) b_q(c),  and the kernel keeps the
+// diagonals t = 0..6 (28 int8 products per K step): one exact int32 TMEM accumulator per diagonal
+// (|D_t| <= (t+1) K 2^14 < 2^31 for K <= 16384).
+// Error of one pair, in units u = 2^(e_m + e_c - 54) (so u <= 4 * 2^-54 * max|W_M[:,m]| max|W_C[:,c]|):
+//     rounding of the operands     |x~ - x| <= 2^(e - 55) and |x| < 2^e per side: <= K u (1 + 2^-56)
+//     dropped diagonals t = 7..12  <= K 2^14 sum_{t>=7} (13 - t) 256^(12 - t) / 2^54 < 6.03 K u
+//     the FP64 recombination       one rounding of S (relative 2^-53)
+// i.e. |S_i8 - S| <= 7.04 K u + |S| 2^-53, against the FP64 DMMA bound ~ K eps sum_i |W_M[i,m]| |W_C[i,c]|.
+// L = 7 is the smallest L for which the bound stays at the FP64 level (L = 6 is 256 times coarser); L = 8 would add
+// 8 products per K step and an eighth accumulator (8 x 64 TMEM columns: no room for anything else) for accuracy the
+// FP64 epilogue cannot use.  tests/test_ivar_int8_core.py checks the model against exact integer arithmetic.
+//
+// Slices live K-major ([p][column][k], ldk = roundup(n, 64) bytes) in caller scratch (gpx_set_ivar_scratch) and are
+// rebuilt from the FP64 factors on every scoring call by ivar_slice_kernel: one streaming pass over W (0.75 ms of the
+// 107.8 ms cfg-2 call at n = 255 on a B200, DESIGN.md section 5), so no other producer of W has to know about them.
+//
+// ivar_i8_kernel: 128 (integration points) x 64 (candidates) tiles, K in 64-byte chunks (SWIZZLE_64B, 2 stages).
+//   warp 8    TMA producer: one 3-D tensor-map load per operand and chunk brings all 7 slices.
+//   warp 9    MMA issuer (one lane): 56 tcgen05.mma per chunk into the 7 accumulators (7 x 64 of the 512 TMEM columns).
+//   warps 0-7 epilogue: warp w reads TMEM lanes 32 (w % 4).. (its integration points) for columns 32 (w / 4)..; per pair
+//             it recombines S in int64 + FP64, evaluates k with the same prologue arithmetic as the DMMA kernels and
+//             adds (S - k)^2 to a per-thread column sum kept across the CTA's M tiles.
+// Determinism: fixed M-split grid and rasterisation as ivar_ws_kernel; per-column summation order independent of the
+// candidate's position in its tile.
+// ---------------------------------------------------------------------------------------------
+constexpr int I8_L = 7;
+constexpr int I8_BM = 128;
+constexpr int I8_BN = 64;
+constexpr int I8_BK = 64;                                  // bytes of K per chunk = the 64-byte swizzle span
+constexpr int I8_A_BYTES = I8_L * I8_BM * I8_BK;           // 57344
+constexpr int I8_B_BYTES = I8_L * I8_BN * I8_BK;           // 28672
+constexpr int I8_STAGE = I8_A_BYTES + I8_B_BYTES;          // multiple of 1024
+constexpr int I8_STAGES = 2;
+constexpr int I8_EPI_WARPS = 8;
+constexpr int I8_THREADS = (I8_EPI_WARPS + 2) * 32;
+constexpr int I8_KMAX = GPX_I8_MAX_N;
+// smem: ring | neg. exp table | column prologue rows | column scales | reduction | barriers | tmem address
+constexpr size_t I8_SMEM_BYTES =
+    1024 + (size_t)I8_STAGES * I8_STAGE + 256 * 8 + GPX_KROWS * I8_BN * 8 + I8_BN * 8 + 4 * I8_BN * 8 + 16 * 8 + 16;
+
+struct I8Maps {
+    CUtensorMap a, b;
+};
+
+struct I8Args {
+    const double* Ap;  // prologue rows of the integration points (ld lda) and of the candidates (ld ldb)
+    const double* Bp;
+    const double* fa;  // per-column scales 2^(e - 30)
+    const double* fb;
+    double* out;
+    int64_t lda, ldb, ldo;
+    int64_t I, J;
+    int K;
+    int np;            // prologue rows read: EXPANDED d + 2, DIFF d
+    int tiles_per_cta, group_w, splits;
+};
+
+__device__ __forceinline__ void tma_load_3d(void* dst, const CUtensorMap* tm, int c0, int c1, int c2, uint64_t* bar) {
+    asm volatile(
+        "cp.async.bulk.tensor.3d.shared::cluster.global.tile.mbarrier::complete_tx::bytes [%0], [%1, {%2, %3, %4}], [%5];\n" ::"r"(
+            smem_u32(dst)),
+        "l"(reinterpret_cast<uint64_t>(tm)), "r"(c0), "r"(c1), "r"(c2), "r"(smem_u32(bar))
+        : "memory");
+}
+
+// K-major operand, 64-byte swizzle: 8-row core groups 512 bytes apart (SBO), LBO unused, descriptor version 1
+__device__ __forceinline__ uint64_t i8_desc(uint32_t saddr) {
+    return (uint64_t)((saddr & 0x3FFFF) >> 4) | ((uint64_t)1 << 16) | ((uint64_t)(512 >> 4) << 32) | ((uint64_t)1 << 46) |
+           ((uint64_t)4 << 61);
+}
+// kind::i8: D s32, A and B signed, both K-major, N = 64, M = 128
+constexpr uint32_t I8_IDESC = (2u << 4) | (1u << 7) | (1u << 10) | ((uint32_t)(I8_BN >> 3) << 17) | ((uint32_t)(I8_BM >> 4) << 24);
+
+__device__ __forceinline__ void i8_mma(uint32_t dtm, uint64_t ad, uint64_t bd, uint32_t acc) {
+    asm volatile(
+        "{\n.reg .pred p;\nsetp.ne.b32 p, %4, 0;\n"
+        "tcgen05.mma.cta_group::1.kind::i8 [%0], %1, %2, %3, p;\n}\n" ::"r"(dtm),
+        "l"(ad), "l"(bd), "r"(I8_IDESC), "r"(acc)
+        : "memory");
+}
+__device__ __forceinline__ void tc_commit(uint64_t* bar) {
+    asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];\n" ::"r"(smem_u32(bar)) : "memory");
+}
+__device__ __forceinline__ void tc_fence_after() { asm volatile("tcgen05.fence::after_thread_sync;\n" ::: "memory"); }
+__device__ __forceinline__ void tc_fence_before() { asm volatile("tcgen05.fence::before_thread_sync;\n" ::: "memory"); }
+__device__ __forceinline__ void tmem_ld4(uint32_t taddr, int (&v)[4]) {
+    asm volatile("tcgen05.ld.sync.aligned.32x32b.x4.b32 {%0, %1, %2, %3}, [%4];\n"
+                 : "=r"(v[0]), "=r"(v[1]), "=r"(v[2]), "=r"(v[3])
+                 : "r"(taddr));
+}
+__device__ __forceinline__ void tmem_wait_ld() { asm volatile("tcgen05.wait::ld.sync.aligned;\n" ::: "memory"); }
+
+// |v| < 2^51 -> exact double without the conversion unit
+__device__ __forceinline__ double i64_to_f64(int64_t v) {
+    return __longlong_as_double(0x4338000000000000LL + v) - 6755399441055744.0;
+}
+
+template <int FAM, int PRO>
+__global__ void __launch_bounds__(I8_THREADS, 1) ivar_i8_kernel(const __grid_constant__ I8Args a, const __grid_constant__ KParams kp,
+                                                                const __grid_constant__ I8Maps maps) {
+    extern __shared__ __align__(128) unsigned char smem_raw[];
+    unsigned char* ring = reinterpret_cast<unsigned char*>(((uintptr_t)smem_raw + 1023) & ~(uintptr_t)1023);
+    double* s_tab = reinterpret_cast<double*>(ring + I8_STAGES * I8_STAGE);
+    double* s_colp = s_tab + 256;               // [GPX_KROWS][I8_BN]
+    double* s_fb = s_colp + GPX_KROWS * I8_BN;  // [I8_BN]
+    double* s_red = s_fb + I8_BN;               // [4][I8_BN]
+    uint64_t* full = reinterpret_cast<uint64_t*>(s_red + 4 * I8_BN);
+    uint64_t* empty = full + I8_STAGES;
+    uint64_t* acc_full = empty + I8_STAGES;
+    uint64_t* acc_empty = acc_full + 1;
+    uint32_t* s_tmem = reinterpret_cast<uint32_t*>(acc_empty + 1);
+
+    const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+    // rasterisation of ivar_ws_kernel: j-group -> M-split -> tile
+    const int64_t jtiles = (a.J + I8_BN - 1) / I8_BN;
+    const int64_t gw = a.group_w;
+    const int64_t per_group = gw * a.splits;
+    const int64_t jg = blockIdx.x / per_group;
+    const int64_t rem = blockIdx.x - jg * per_group;
+    const int64_t gsz = (jtiles - jg * gw) < gw ? (jtiles - jg * gw) : gw;
+    const int64_t split = rem / gsz;
+    const int64_t jt = jg * gw + rem % gsz;
+    if (split >= a.splits) return;
+    const int64_t j0 = jt * I8_BN;
+    const int64_t itiles = (a.I + I8_BM - 1) / I8_BM;
+    const int64_t it_begin = split * a.tiles_per_cta;
+    int64_t it_end = it_begin + a.tiles_per_cta;
+    if (it_end > itiles) it_end = itiles;
+    const int ntiles = it_end > it_begin ? (int)(it_end - it_begin) : 0;
+    const int kch = (a.K + I8_BK - 1) / I8_BK;
+
+    if (tid == 0) {
+        for (int s = 0; s < I8_STAGES; ++s) {
+            mbar_init(full + s, 1);
+            mbar_init(empty + s, 1);
+        }
+        mbar_init(acc_full, 1);
+        mbar_init(acc_empty, I8_EPI_WARPS);
+        asm volatile("fence.mbarrier_init.release.cluster;\n" ::: "memory");
+    }
+    if (warp == 9) {
+        asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], 512;\n" ::"r"(smem_u32(s_tmem)) : "memory");
+        asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;\n" ::: "memory");
+    }
+    if (tid < 256) s_tab[tid] = -kp.signal * gpx_exp2_tab[tid];
+    for (int i = tid; i < a.np * I8_BN; i += I8_THREADS) {
+        const int q = i / I8_BN, c = i - q * I8_BN;
+        s_colp[i] = j0 + c < a.J ? a.Bp[(int64_t)q * a.ldb + j0 + c] : 0.0;
+    }
+    if (tid < I8_BN) s_fb[tid] = j0 + tid < a.J ? a.fb[j0 + tid] : 0.0;
+    tc_fence_before();
+    __syncthreads();
+    tc_fence_after();
+    const uint32_t tmem = *s_tmem;
+
+    if (warp == 8) {
+        // ---- TMA producer ----
+        if (lane == 0) {
+            int g = 0;
+            for (int tl = 0; tl < ntiles; ++tl) {
+                const int i0 = (int)((it_begin + tl) * I8_BM);
+                for (int kc = 0; kc < kch; ++kc, ++g) {
+                    const int s = g % I8_STAGES;
+                    mbar_wait(empty + s, ((unsigned)(g / I8_STAGES) & 1u) ^ 1u);
+                    mbar_arrive_expect_tx(full + s, (unsigned)I8_STAGE);
+                    unsigned char* st = ring + s * I8_STAGE;
+                    tma_load_3d(st, &maps.a, kc * I8_BK, i0, 0, full + s);
+                    tma_load_3d(st + I8_A_BYTES, &maps.b, kc * I8_BK, (int)j0, 0, full + s);
+                }
+            }
+        }
+    } else if (warp == 9) {
+        // ---- MMA issuer ----
+        if (lane == 0) {
+            const uint32_t ring_s = smem_u32(ring);
+            int g = 0;
+            for (int tl = 0; tl < ntiles; ++tl) {
+                if (tl > 0) {
+                    mbar_wait(acc_empty, (unsigned)(tl - 1) & 1u);  // the epilogue has read the previous tile
+                    tc_fence_after();
+                }
+                for (int kc = 0; kc < kch; ++kc, ++g) {
+                    const int s = g % I8_STAGES;
+                    mbar_wait(full + s, (unsigned)(g / I8_STAGES) & 1u);
+                    tc_fence_after();
+                    const uint32_t sa = ring_s + s * I8_STAGE, sb = sa + I8_A_BYTES;
+#pragma unroll
+                    for (int t = 0; t < I8_L; ++t)
+#pragma unroll
+                        for (int p = 0; p <= t; ++p)
+#pragma unroll
+                            for (int kk = 0; kk < I8_BK / 32; ++kk)
+                                i8_mma(tmem + t * I8_BN, i8_desc(sa + p * (I8_BM * I8_BK) + kk * 32),
+                                       i8_desc(sb + (t - p) * (I8_BN * I8_BK) + kk * 32), (kc | p | kk) != 0);
+                    tc_commit(empty + s);
+                }
+                tc_commit(acc_full);
+            }
+        }
+    } else {
+        // ---- epilogue ----
+        const int quad = warp & 3, chalf = warp >> 2;
+        const uint32_t trow = tmem + ((uint32_t)(quad * 32) << 16) + chalf * 32;
+        double p[32];
+#pragma unroll
+        for (int j = 0; j < 32; ++j) p[j] = 0.0;
+        for (int tl = 0; tl < ntiles; ++tl) {
+            const int64_t m = (it_begin + tl) * I8_BM + quad * 32 + lane;
+            const bool mok = m < a.I;
+            const double fm = mok ? a.fa[m] : 0.0;
+            mbar_wait(acc_full, (unsigned)tl & 1u);
+            tc_fence_after();
+#pragma unroll
+            for (int cb = 0; cb < 32; cb += 4) {
+                int d[I8_L][4];
+#pragma unroll
+                for (int t = 0; t < I8_L; ++t) tmem_ld4(trow + t * I8_BN + cb, d[t]);
+                tmem_wait_ld();
+                if (cb == 28) {
+                    // every accumulator of this tile is in registers: hand TMEM back to the MMA issuer
+                    tc_fence_before();
+                    __syncwarp();
+                    if (lane == 0) mbar_arrive(acc_empty);
+                }
+                const int c0 = chalf * 32 + cb;
+                double e[4];
+#pragma unroll
+                for (int j = 0; j < 4; ++j) e[j] = 0.0;
+                for (int q = 0; q < a.np; ++q) {
+                    const double x = mok ? a.Ap[(int64_t)q * a.lda + m] : 0.0;
+                    const double* y = s_colp + q * I8_BN + c0;
+#pragma unroll
+                    for (int j = 0; j < 4; ++j) {
+                        if (PRO == PRO_EXPANDED) e[j] = fma(x, y[j], e[j]);
+                        else kacc_dim<FAM>(e[j], kp, q, x, y[j]);
+                    }
+                }
+#pragma unroll
+                for (int j = 0; j < 4; ++j) {
+                    const double negk = PRO == PRO_EXPANDED ? neg_kexpand_tab<FAM>(e[j], kp, s_tab) : kfinish_tab<FAM>(e[j], kp, s_tab);
+                    const int64_t hi = ((int64_t)d[0][j] << 24) + ((int64_t)d[1][j] << 16) + ((int64_t)d[2][j] << 8) + d[3][j];
+                    const int64_t lo = ((int64_t)d[4][j] << 16) + ((int64_t)d[5][j] << 8) + d[6][j];
+                    const double S = fma(i64_to_f64(hi), 0x1p24, i64_to_f64(lo)) * (fm * s_fb[c0 + j]);
+                    const double v = mok ? S + negk : 0.0;
+                    p[cb + j] = fma(v, v, p[cb + j]);
+                }
+            }
+        }
+        // column sums over the warp's 32 rows: reduce-scatter, lane l ends with column chalf*32 + l
+#pragma unroll
+        for (int st = 0; st < 5; ++st) {
+            const int off = 16 >> st;
+            const bool up = (lane & off) != 0;
+#pragma unroll
+            for (int j = 0; j < off; ++j) {
+                const double keep = up ? p[j + off] : p[j];
+                const double send = up ? p[j] : p[j + off];
+                p[j] = keep + __shfl_xor_sync(0xffffffffu, send, off);
+            }
+        }
+        s_red[quad * I8_BN + chalf * 32 + lane] = p[0];
+    }
+    tc_fence_before();
+    __syncthreads();
+    if (warp == 9) {
+        tc_fence_after();
+        asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, 512;\n" ::"r"(tmem) : "memory");
+    }
+    if (tid < I8_BN && j0 + tid < a.J) {
+        const double r = ((s_red[tid] + s_red[I8_BN + tid]) + s_red[2 * I8_BN + tid]) + s_red[3 * I8_BN + tid];
+        a.out[split * a.ldo + j0 + tid] = r;
+    }
+}
+
+// digits of one side: S[p][c][k] (int8, ldk bytes per column, slice stride sstride) and f[c] = 2^(e_c - 30)
+// block: 32 columns x 8 row lanes
+__global__ void __launch_bounds__(256) ivar_slice_kernel(const double* __restrict__ W, int64_t ldw, int n, int64_t ncols,
+                                                         int8_t* __restrict__ S, int64_t ldk, int64_t sstride,
+                                                         double* __restrict__ f) {
+    __shared__ double s_mx[8][32];
+    __shared__ __align__(16) int8_t s_dig[I8_L][32][64];
+    const int tx = threadIdx.x & 31, ty = threadIdx.x >> 5;
+    const int64_t c = (int64_t)blockIdx.x * 32 + tx;
+    const bool cok = c < ncols;
+    double mx = 0.0;
+    if (cok)
+        for (int i = ty; i < n; i += 8) mx = fmax(mx, fabs(W[(int64_t)i * ldw + c]));
+    s_mx[ty][tx] = mx;
+    __syncthreads();
+    mx = s_mx[0][tx];
+#pragma unroll
+    for (int r = 1; r < 8; ++r) mx = fmax(mx, s_mx[r][tx]);
+    int e = 0;
+    if (mx > 0.0) frexp(mx, &e);  // mx < 2^e
+    if (ty == 0 && cok) f[c] = ldexp(1.0, e - 30);
+    const int kpad = (n + 63) & ~63;
+    for (int i0 = 0; i0 < kpad; i0 += 64) {
+        __syncthreads();
+#pragma unroll
+        for (int r = 0; r < 8; ++r) {
+            const int i = i0 + ty + 8 * r;
+            long long Y = 0;
+            if (cok && i < n) Y = llrint(ldexp(W[(int64_t)i * ldw + c], 54 - e));
+#pragma unroll
+            for (int pp = I8_L - 1; pp > 0; --pp) {
+                const int dg = (int)((Y + 128) & 255) - 128;
+                s_dig[pp][tx][ty + 8 * r] = (int8_t)dg;
+                Y = (Y - dg) >> 8;
+            }
+            s_dig[0][tx][ty + 8 * r] = (int8_t)Y;
+        }
+        __syncthreads();
+        // 7 x 32 runs of 64 bytes -> 16-byte stores
+        for (int v = threadIdx.x; v < I8_L * 32 * 4; v += 256) {
+            const int pp = v / 128, col = (v / 4) & 31, part = v & 3;
+            const int64_t cc = (int64_t)blockIdx.x * 32 + col;
+            if (cc < ncols)
+                *reinterpret_cast<int4*>(S + pp * sstride + cc * ldk + i0 + part * 16) =
+                    *reinterpret_cast<const int4*>(&s_dig[pp][col][part * 16]);
+        }
+    }
+}
+
+// 3-D map over the slices of one side: dims {n (K bytes), ncols, 7}, box {64, rows, 7}, 64-byte swizzle
+int make_i8_map(CUtensorMap* m, const int8_t* base, int64_t ldk, int64_t n, int64_t ncols, int64_t sstride, int box_rows) {
+    EncodeTiledFn enc = encode_tiled();
+    if (!enc) {
+        gpx_set_error("ivar_i8: cuTensorMapEncodeTiled is not available from this driver");
+        return GPX_EINVAL;
+    }
+    const cuuint64_t dims[3] = {(cuuint64_t)n, (cuuint64_t)ncols, (cuuint64_t)I8_L};
+    const cuuint64_t strides[2] = {(cuuint64_t)ldk, (cuuint64_t)sstride};
+    const cuuint32_t box[3] = {(cuuint32_t)I8_BK, (cuuint32_t)box_rows, (cuuint32_t)I8_L};
+    const cuuint32_t estr[3] = {1, 1, 1};
+    CUresult r = enc(m, CU_TENSOR_MAP_DATA_TYPE_UINT8, 3, const_cast<int8_t*>(base), dims, strides, box, estr,
+                     CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_64B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
+                     CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
+    if (r != CUDA_SUCCESS) {
+        gpx_set_error("ivar_i8: cuTensorMapEncodeTiled failed with CUresult %d", (int)r);
+        return GPX_EINVAL;
+    }
+    return GPX_OK;
+}
+
+// scratch layout for one call: [slices of M][slices of C][fa][fb]; returns the bytes needed
+int64_t i8_layout(int64_t M, int64_t C, int64_t n, int64_t* ldk, int64_t* sm, int64_t* sc) {
+    *ldk = (n + 63) & ~(int64_t)63;
+    *sm = ((M + I8_BM - 1) / I8_BM * I8_BM) * *ldk;
+    *sc = ((C + I8_BM - 1) / I8_BM * I8_BM) * *ldk;
+    return I8_L * (*sm + *sc) + 8 * (((M + 1) & ~(int64_t)1) + ((C + 1) & ~(int64_t)1)) + 256;
+}
+
 }  // namespace
 
 // number of i-splits for the IVAR grid: fill the machine in whole waves
-static int ivar_splits_for(gpx_handle h, int64_t M, int64_t C, int bm) {
-    const int64_t jt = (C + BN - 1) / BN;
+static int ivar_splits_for(gpx_handle h, int64_t M, int64_t C, int bm, int bn = BN) {
+    const int64_t jt = (C + bn - 1) / bn;
     const int64_t itl = (M + bm - 1) / bm;
     const int sms = h->sm_count > 0 ? h->sm_count : 148;
     int best = 1;
@@ -1020,6 +1377,61 @@ static int ivar_splits_for(gpx_handle h, int64_t M, int64_t C, int bm) {
 }
 int gpx_ivar_splits(gpx_handle, int64_t, int64_t) { return 32; }  // workspace bound: never more than 32 splits
 
+// INT8 core: slice both factors into the handle's scratch, then one ivar_i8_kernel launch (same workspace contract as
+// ivar_ws_kernel: partial column sums per M-split)
+static int launch_ivar_i8(gpx_handle h, int prologue, const double* Wm, int64_t ldm, const double* Ma_rows, int64_t M,
+                          const double* Wc, int64_t ldc, const double* Cb_rows, int64_t C, int64_t n, double* partial,
+                          int64_t ldp, int* nsplit_out, cudaStream_t st) {
+    int64_t ldk, sm, sc;
+    i8_layout(M, C, n, &ldk, &sm, &sc);
+    int8_t* Sm = reinterpret_cast<int8_t*>(((uintptr_t)h->i8_scratch + 127) & ~(uintptr_t)127);
+    int8_t* Sc = Sm + I8_L * sm;
+    double* fa = reinterpret_cast<double*>(Sc + I8_L * sc);
+    double* fb = fa + ((M + 1) & ~(int64_t)1);
+    ivar_slice_kernel<<<(unsigned)((M + 31) / 32), 256, 0, st>>>(Wm, ldm, (int)n, M, Sm, ldk, sm, fa);
+    int rc = gpx_check_launch("ivar_slice");
+    if (rc) return rc;
+    ivar_slice_kernel<<<(unsigned)((C + 31) / 32), 256, 0, st>>>(Wc, ldc, (int)n, C, Sc, ldk, sc, fb);
+    if ((rc = gpx_check_launch("ivar_slice"))) return rc;
+    I8Maps maps;
+    memset(&maps, 0, sizeof(maps));
+    if ((rc = make_i8_map(&maps.a, Sm, ldk, n, M, sm, I8_BM))) return rc;
+    if ((rc = make_i8_map(&maps.b, Sc, ldk, n, C, sc, I8_BN))) return rc;
+    const int splits = ivar_splits_for(h, M, C, I8_BM, I8_BN);
+    const int64_t itl = (M + I8_BM - 1) / I8_BM;
+    const int64_t jt = (C + I8_BN - 1) / I8_BN;
+    I8Args a;
+    a.Ap = Ma_rows;
+    a.Bp = Cb_rows;
+    a.fa = fa;
+    a.fb = fb;
+    a.out = partial;
+    a.lda = ldm;
+    a.ldb = ldc;
+    a.ldo = ldp;
+    a.I = M;
+    a.J = C;
+    a.K = (int)n;
+    a.np = prologue == PRO_DIFF ? h->kp.d : h->kp.d + 2;
+    a.tiles_per_cta = (int)((itl + splits - 1) / splits);
+    a.group_w = h->sm_count > 0 ? h->sm_count : 148;
+    a.splits = splits;
+    *nsplit_out = splits;
+    const dim3 grid((unsigned)(jt * splits), 1u);
+#define GPX_I8_LAUNCH(F, P)                                                                                        \
+    do {                                                                                                           \
+        if ((rc = gpx_ensure_smem(h, (const void*)ivar_i8_kernel<F, P>, I8_SMEM_BYTES, "ivar_i8"))) return rc;    \
+        ivar_i8_kernel<F, P><<<grid, I8_THREADS, I8_SMEM_BYTES, st>>>(a, h->kp, maps);                            \
+    } while (0)
+    if (prologue == PRO_DIFF) {
+        GPX_DISPATCH_FAMILY(h->kp.family, GPX_I8_LAUNCH(FAM, PRO_DIFF));
+    } else {
+        GPX_DISPATCH_FAMILY(h->kp.family, GPX_I8_LAUNCH(FAM, PRO_EXPANDED));
+    }
+#undef GPX_I8_LAUNCH
+    return gpx_check_launch("ivar_i8");
+}
+
 int gpx_launch_core_ivar(gpx_handle h, int prologue, const double* Wm, int64_t ldm, const double* Ma_rows, int64_t M,
                          const double* Wc, int64_t ldc, const double* Cb_rows, int64_t C, int64_t n, double* partial,
                          int64_t ldp, int* nsplit_out, cudaStream_t st) {
@@ -1036,6 +1448,11 @@ int gpx_launch_core_ivar(gpx_handle h, int prologue, const double* Wm, int64_t l
     // anything else goes through the predicated cp.async core
     const bool tma = (ldm % WS_BM) == 0 && (ldc % BN) == 0 && ldm >= (M + WS_BM - 1) / WS_BM * WS_BM &&
                      ldc >= (C + BN - 1) / BN * BN;
+    if (tma && h->ivar_core == GPX_CORE_I8 && n > 0 && n <= I8_KMAX) {
+        int64_t ldk, sm, sc;
+        if (i8_layout(M, C, n, &ldk, &sm, &sc) <= h->i8_scratch_bytes)
+            return launch_ivar_i8(h, prologue, Wm, ldm, Ma_rows, M, Wc, ldc, Cb_rows, C, n, partial, ldp, nsplit_out, st);
+    }
     const int bm = tma ? WS_BM : Cfg::BM;
     const int splits = ivar_splits_for(h, M, C, bm);
     const int64_t itl = (M + bm - 1) / bm;
@@ -1312,6 +1729,26 @@ static int ivar_finalize_argmin(gpx_handle h, const double* partial, int nsplit,
 extern "C" int gpx_set_ivar_ring(gpx_handle h, int ring) {
     GPX_REQUIRE(h != nullptr && ring >= 0 && ring <= 2, GPX_EINVAL, "ring must be 0, 1 or 2");
     h->ivar_ring = ring;
+    return GPX_OK;
+}
+
+extern "C" int gpx_set_ivar_core(gpx_handle h, int core) {
+    GPX_REQUIRE(h != nullptr && (core == GPX_CORE_DMMA || core == GPX_CORE_I8), GPX_EINVAL,
+                "core must be GPX_CORE_DMMA or GPX_CORE_I8");
+    h->ivar_core = core;
+    return GPX_OK;
+}
+
+extern "C" int64_t gpx_ivar_scratch_bytes(gpx_handle h, int64_t M, int64_t C, int64_t n_max) {
+    if (!h || M < 0 || C < 0 || n_max < 0) return 0;
+    int64_t ldk, sm, sc;
+    return i8_layout(M, C, n_max, &ldk, &sm, &sc);
+}
+
+extern "C" int gpx_set_ivar_scratch(gpx_handle h, void* scratch, int64_t bytes) {
+    GPX_REQUIRE(h != nullptr && bytes >= 0 && (scratch != nullptr || bytes == 0), GPX_EINVAL, "bad scratch");
+    h->i8_scratch = scratch;
+    h->i8_scratch_bytes = bytes;
     return GPX_OK;
 }
 

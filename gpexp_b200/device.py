@@ -97,6 +97,16 @@ class Device:
         self._kernel_key = None
         self._center = None
         self.force_diff_form = False  # tests / A-B runs: never use the expanded-form prologue
+        self._ivar_scratch = None
+
+    def reserve_ivar_scratch(self, M: int, C: int, n_max: int) -> None:
+        """Grow the handle's scratch for the INT8 IVAR core to cover M integration points, C candidates and designs of
+        up to n_max points.  The device keeps the buffer for its lifetime, so every engine on the handle can use it."""
+        need = int(lib.gpx_ivar_scratch_bytes(self.h, M, C, n_max))
+        if self._ivar_scratch is not None and self._ivar_scratch.numel() >= need:
+            return
+        self._ivar_scratch = torch.empty(need, dtype=torch.uint8, device=self.torch_device)
+        check(lib.gpx_set_ivar_scratch(self.h, self._ivar_scratch.data_ptr(), need), "gpx_set_ivar_scratch")
 
     @property
     def launches(self) -> int:

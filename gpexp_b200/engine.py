@@ -542,6 +542,8 @@ class GreedyIVAREngine(_Pivoting):
         # partial column sums: M-splits of the contraction, or row segments of the resident update
         ws = max(int(lib.gpx_score_ivar_workspace(dev.h, mc.n, cand.n)), self.nseg * self.ldp)
         self.workspace = dev.zeros(max(ws, 1))
+        if not self.resident and ncap <= _lib.GPX_I8_MAX_N:  # only the contraction of the INT8 core reads it
+            dev.reserve_ivar_scratch(mc.n, cand.n, ncap)
         self.scores = dev.zeros(cand.ld)
         self.score_trace = None
         self.cov = None

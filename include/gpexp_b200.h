@@ -199,6 +199,26 @@ int gpx_sum(gpx_handle h, const double* v, int64_t n, double* out, void* stream)
  * 2 = 24-row chunks x 4 stages, two chunks ahead, tensor-map loads. */
 int gpx_set_ivar_ring(gpx_handle h, int ring);
 
+/* Arithmetic of the IVAR contraction on padded operands (leading dimensions covering whole 128-wide tiles):
+ *     GPX_CORE_I8    (default) W_M^T W_C emulated exactly enough on the INT8 tensor cores: 7 fixed-point 8-bit slices
+ *                    per factor entry, 28 slice products, error <= 7.04 n 2^-52 max|W_M[:,m]| max|W_C[:,c]| per pair
+ *                    plus one FP64 rounding (DESIGN.md section 5).  Needs the scratch of gpx_set_ivar_scratch and
+ *                    1 <= n <= GPX_I8_MAX_N; otherwise the call uses the FP64 core.
+ *     GPX_CORE_DMMA  the FP64 DMMA kernel (ring per gpx_set_ivar_ring).
+ * Unpadded operands always use the FP64 generic core.  The GPX_IVAR_CORE environment variable (dmma | i8) sets the
+ * default of new handles. */
+#define GPX_CORE_DMMA 1
+#define GPX_CORE_I8 2
+#define GPX_I8_MAX_N 16384 /* largest design size the INT8 core runs */
+int gpx_set_ivar_core(gpx_handle h, int core);
+
+/* Bytes of scratch the INT8 core needs for M integration points, C candidates and designs up to n_max points. */
+int64_t gpx_ivar_scratch_bytes(gpx_handle h, int64_t M, int64_t C, int64_t n_max);
+
+/* Caller memory (any alignment; NULL, 0 to detach) the INT8 core re-slices the factors into on every scoring call.
+ * The handle only keeps the pointer; calls on the handle's stream use it in order. */
+int gpx_set_ivar_scratch(gpx_handle h, void* scratch, int64_t bytes);
+
 /* Workspace (doubles) gpx_score_ivar needs for C candidates. */
 int64_t gpx_score_ivar_workspace(gpx_handle h, int64_t M, int64_t C);
 
