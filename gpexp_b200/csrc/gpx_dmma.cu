@@ -1013,14 +1013,19 @@ int prologue_rows(gpx_handle h, int prologue) {
 //
 // Slices live K-major ([p][column][k], ldk = roundup(n, 64) bytes) in caller scratch (gpx_set_ivar_scratch) and are
 // rebuilt from the FP64 factors on every scoring call by ivar_slice_kernel: one streaming pass over W (0.75 ms of the
-// 107.8 ms cfg-2 call at n = 255 on a B200, DESIGN.md section 5), so no other producer of W has to know about them.
+// 90.7 ms cfg-2 call at n = 255 on a B200, DESIGN.md section 5), so no other producer of W has to know about them.
 //
 // ivar_i8_kernel: 128 (integration points) x 64 (candidates) tiles, K in 64-byte chunks (SWIZZLE_64B, 2 stages).
-//   warp 8    TMA producer: one 3-D tensor-map load per operand and chunk brings all 7 slices.
-//   warp 9    MMA issuer (one lane): 56 tcgen05.mma per chunk into the 7 accumulators (7 x 64 of the 512 TMEM columns).
-//   warps 0-7 epilogue: warp w reads TMEM lanes 32 (w % 4).. (its integration points) for columns 32 (w / 4)..; per pair
-//             it recombines S in int64 + FP64, evaluates k with the same prologue arithmetic as the DMMA kernels and
-//             adds (S - k)^2 to a per-thread column sum kept across the CTA's M tiles.
+//   warp 16    TMA producer: one 3-D tensor-map load per operand and chunk brings all 7 slices.
+//   warp 17    MMA issuer (one lane): 56 tcgen05.mma per chunk into the 7 accumulators (7 x 64 of the 512 TMEM columns).
+//   warps 0-15 epilogue: warp w owns TMEM lanes 32 (w % 4).. (its integration points) and columns 16 (w / 4)..
+//             Per tile it first evaluates -k for its 16 pairs (same prologue arithmetic as the DMMA kernels), then
+//             waits for the accumulators, drains them two columns at a time (int64 recombination, one FP64 fma with
+//             the scales and -k) into per-thread column sums of (S - k)^2 kept across the CTA's M tiles, and hands
+//             TMEM back as soon as the last load has landed.  The 7 accumulators leave no room for a second TMEM
+//             buffer, so this is the overlap there is: the next tile's MMAs run under the -k work of that tile.
+//   At 18 warps the register file allows 96 registers a thread; 16 epilogue warps beat 8 (168 registers) because
+//   the -k work is latency bound (cfg-2 n = 255 call on a B200 at 1000 W: 92.2 ms against 97.7 ms, DESIGN.md 5).
 // Determinism: fixed M-split grid and rasterisation as ivar_ws_kernel; per-column summation order independent of the
 // candidate's position in its tile.
 // ---------------------------------------------------------------------------------------------
@@ -1032,7 +1037,8 @@ constexpr int I8_A_BYTES = I8_L * I8_BM * I8_BK;           // 57344
 constexpr int I8_B_BYTES = I8_L * I8_BN * I8_BK;           // 28672
 constexpr int I8_STAGE = I8_A_BYTES + I8_B_BYTES;          // multiple of 1024
 constexpr int I8_STAGES = 2;
-constexpr int I8_EPI_WARPS = 8;
+constexpr int I8_EPI_WARPS = 16;                        // 4 per TMEM lane quarter
+constexpr int I8_EPI_COLS = 4 * I8_BN / I8_EPI_WARPS;  // columns per epilogue thread
 constexpr int I8_THREADS = (I8_EPI_WARPS + 2) * 32;
 constexpr int I8_KMAX = GPX_I8_MAX_N;
 // smem: ring | neg. exp table | column prologue rows | column scales | reduction | barriers | tmem address
@@ -1084,10 +1090,8 @@ __device__ __forceinline__ void tc_commit(uint64_t* bar) {
 }
 __device__ __forceinline__ void tc_fence_after() { asm volatile("tcgen05.fence::after_thread_sync;\n" ::: "memory"); }
 __device__ __forceinline__ void tc_fence_before() { asm volatile("tcgen05.fence::before_thread_sync;\n" ::: "memory"); }
-__device__ __forceinline__ void tmem_ld4(uint32_t taddr, int (&v)[4]) {
-    asm volatile("tcgen05.ld.sync.aligned.32x32b.x4.b32 {%0, %1, %2, %3}, [%4];\n"
-                 : "=r"(v[0]), "=r"(v[1]), "=r"(v[2]), "=r"(v[3])
-                 : "r"(taddr));
+__device__ __forceinline__ void tmem_ld2(uint32_t taddr, int (&v)[2]) {
+    asm volatile("tcgen05.ld.sync.aligned.32x32b.x2.b32 {%0, %1}, [%2];\n" : "=r"(v[0]), "=r"(v[1]) : "r"(taddr));
 }
 __device__ __forceinline__ void tmem_wait_ld() { asm volatile("tcgen05.wait::ld.sync.aligned;\n" ::: "memory"); }
 
@@ -1139,7 +1143,7 @@ __global__ void __launch_bounds__(I8_THREADS, 1) ivar_i8_kernel(const __grid_con
         mbar_init(acc_empty, I8_EPI_WARPS);
         asm volatile("fence.mbarrier_init.release.cluster;\n" ::: "memory");
     }
-    if (warp == 9) {
+    if (warp == I8_EPI_WARPS + 1) {
         asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], 512;\n" ::"r"(smem_u32(s_tmem)) : "memory");
         asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;\n" ::: "memory");
     }
@@ -1154,7 +1158,7 @@ __global__ void __launch_bounds__(I8_THREADS, 1) ivar_i8_kernel(const __grid_con
     tc_fence_after();
     const uint32_t tmem = *s_tmem;
 
-    if (warp == 8) {
+    if (warp == I8_EPI_WARPS) {
         // ---- TMA producer ----
         if (lane == 0) {
             int g = 0;
@@ -1170,7 +1174,7 @@ __global__ void __launch_bounds__(I8_THREADS, 1) ivar_i8_kernel(const __grid_con
                 }
             }
         }
-    } else if (warp == 9) {
+    } else if (warp == I8_EPI_WARPS + 1) {
         // ---- MMA issuer ----
         if (lane == 0) {
             const uint32_t ring_s = smem_u32(ring);
@@ -1200,57 +1204,67 @@ __global__ void __launch_bounds__(I8_THREADS, 1) ivar_i8_kernel(const __grid_con
         }
     } else {
         // ---- epilogue ----
-        const int quad = warp & 3, chalf = warp >> 2;
-        const uint32_t trow = tmem + ((uint32_t)(quad * 32) << 16) + chalf * 32;
-        double p[32];
+        const int quad = warp & 3, c00 = (warp >> 2) * I8_EPI_COLS;
+        const uint32_t trow = tmem + ((uint32_t)(quad * 32) << 16) + c00;
+        double p[I8_EPI_COLS];
 #pragma unroll
-        for (int j = 0; j < 32; ++j) p[j] = 0.0;
+        for (int j = 0; j < I8_EPI_COLS; ++j) p[j] = 0.0;
         for (int tl = 0; tl < ntiles; ++tl) {
             const int64_t m = (it_begin + tl) * I8_BM + quad * 32 + lane;
             const bool mok = m < a.I;
+            // -k of the thread's pairs, evaluated while the tensor cores work on this tile (and, from the second tile
+            // on, right after the previous tile's accumulators were handed back)
+            double nk[I8_EPI_COLS];
+#pragma unroll
+            for (int j = 0; j < I8_EPI_COLS; ++j) nk[j] = 0.0;
+            for (int q = 0; q < a.np; ++q) {
+                const double x = mok ? a.Ap[(int64_t)q * a.lda + m] : 0.0;
+                const double* y = s_colp + q * I8_BN + c00;
+#pragma unroll
+                for (int j = 0; j < I8_EPI_COLS; ++j) {
+                    if (PRO == PRO_EXPANDED) nk[j] = fma(x, y[j], nk[j]);
+                    else kacc_dim<FAM>(nk[j], kp, q, x, y[j]);
+                }
+            }
+#pragma unroll
+            for (int j = 0; j < I8_EPI_COLS; ++j)
+                nk[j] = PRO == PRO_EXPANDED ? neg_kexpand_tab<FAM>(nk[j], kp, s_tab) : kfinish_tab<FAM>(nk[j], kp, s_tab);
             const double fm = mok ? a.fa[m] : 0.0;
             mbar_wait(acc_full, (unsigned)tl & 1u);
             tc_fence_after();
 #pragma unroll
-            for (int cb = 0; cb < 32; cb += 4) {
-                int d[I8_L][4];
+            for (int cb = 0; cb < I8_EPI_COLS; cb += 2) {
+                int d[I8_L][2];
 #pragma unroll
-                for (int t = 0; t < I8_L; ++t) tmem_ld4(trow + t * I8_BN + cb, d[t]);
+                for (int t = 0; t < I8_L; ++t) tmem_ld2(trow + t * I8_BN + cb, d[t]);
                 tmem_wait_ld();
-                if (cb == 28) {
+                if (cb == I8_EPI_COLS - 2) {
                     // every accumulator of this tile is in registers: hand TMEM back to the MMA issuer
                     tc_fence_before();
                     __syncwarp();
                     if (lane == 0) mbar_arrive(acc_empty);
                 }
-                const int c0 = chalf * 32 + cb;
-                double e[4];
 #pragma unroll
-                for (int j = 0; j < 4; ++j) e[j] = 0.0;
-                for (int q = 0; q < a.np; ++q) {
-                    const double x = mok ? a.Ap[(int64_t)q * a.lda + m] : 0.0;
-                    const double* y = s_colp + q * I8_BN + c0;
-#pragma unroll
-                    for (int j = 0; j < 4; ++j) {
-                        if (PRO == PRO_EXPANDED) e[j] = fma(x, y[j], e[j]);
-                        else kacc_dim<FAM>(e[j], kp, q, x, y[j]);
-                    }
-                }
-#pragma unroll
-                for (int j = 0; j < 4; ++j) {
-                    const double negk = PRO == PRO_EXPANDED ? neg_kexpand_tab<FAM>(e[j], kp, s_tab) : kfinish_tab<FAM>(e[j], kp, s_tab);
+                for (int j = 0; j < 2; ++j) {
                     const int64_t hi = ((int64_t)d[0][j] << 24) + ((int64_t)d[1][j] << 16) + ((int64_t)d[2][j] << 8) + d[3][j];
                     const int64_t lo = ((int64_t)d[4][j] << 16) + ((int64_t)d[5][j] << 8) + d[6][j];
-                    const double S = fma(i64_to_f64(hi), 0x1p24, i64_to_f64(lo)) * (fm * s_fb[c0 + j]);
-                    const double v = mok ? S + negk : 0.0;
+                    // S - k with S = (D_0..3 2^24 + D_4..6) (fm fb): the scale product inside one fma with -k
+                    const double R = fma(i64_to_f64(hi), 0x1p24, i64_to_f64(lo));
+                    const double v = mok ? __fma_rn(R, __dmul_rn(fm, s_fb[c00 + cb + j]), nk[cb + j]) : 0.0;
                     p[cb + j] = fma(v, v, p[cb + j]);
                 }
             }
         }
-        // column sums over the warp's 32 rows: reduce-scatter, lane l ends with column chalf*32 + l
+        // column sums over the warp's 32 rows, pairing lanes 16, 8, 4, 2, 1 apart: a reduce-scatter that leaves
+        // lane l with column c00 + l % I8_EPI_COLS (lanes 16 apart hold the same sum when a warp has 16 columns)
 #pragma unroll
         for (int st = 0; st < 5; ++st) {
             const int off = 16 >> st;
+            if (off >= I8_EPI_COLS) {
+#pragma unroll
+                for (int j = 0; j < I8_EPI_COLS; ++j) p[j] += __shfl_xor_sync(0xffffffffu, p[j], off);
+                continue;
+            }
             const bool up = (lane & off) != 0;
 #pragma unroll
             for (int j = 0; j < off; ++j) {
@@ -1259,11 +1273,11 @@ __global__ void __launch_bounds__(I8_THREADS, 1) ivar_i8_kernel(const __grid_con
                 p[j] = keep + __shfl_xor_sync(0xffffffffu, send, off);
             }
         }
-        s_red[quad * I8_BN + chalf * 32 + lane] = p[0];
+        if (lane < I8_EPI_COLS) s_red[quad * I8_BN + c00 + lane] = p[0];
     }
     tc_fence_before();
     __syncthreads();
-    if (warp == 9) {
+    if (warp == I8_EPI_WARPS + 1) {
         tc_fence_after();
         asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, 512;\n" ::"r"(tmem) : "memory");
     }
