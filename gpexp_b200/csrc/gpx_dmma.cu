@@ -1015,9 +1015,11 @@ int prologue_rows(gpx_handle h, int prologue) {
 // rebuilt from the FP64 factors on every scoring call by ivar_slice_kernel: one streaming pass over W (0.75 ms of the
 // 90.7 ms cfg-2 call at n = 255 on a B200, DESIGN.md section 5), so no other producer of W has to know about them.
 //
-// ivar_i8_kernel: 128 (integration points) x 64 (candidates) tiles, K in 64-byte chunks (SWIZZLE_64B, 2 stages).
+// ivar_i8_kernel: 128 (integration points) x 64 (candidates) tiles, K in 32-byte chunks (SWIZZLE_32B, 4 stages of 42 KB).
 //   warp 16    TMA producer: one 3-D tensor-map load per operand and chunk brings all 7 slices.
-//   warp 17    MMA issuer (one lane): 56 tcgen05.mma per chunk into the 7 accumulators (7 x 64 of the 512 TMEM columns).
+//   warp 17    MMA issuer (one lane): 10 tcgen05.mma per chunk into the 7 accumulators (7 x 64 of the 512 TMEM columns):
+//             each A slice meets a stack of adjacent B slices (N up to 256) and writes several diagonals at once, so a
+//             chunk reads 96 KB of operands from smem instead of the 168 KB of 28 separate N = 64 products.
 //   warps 0-15 epilogue: warp w owns TMEM lanes 32 (w % 4).. (its integration points) and columns 16 (w / 4)..
 //             Per tile it first evaluates -k for its 16 pairs (same prologue arithmetic as the DMMA kernels), then
 //             waits for the accumulators, drains them two columns at a time (int64 recombination, one FP64 fma with
@@ -1026,17 +1028,21 @@ int prologue_rows(gpx_handle h, int prologue) {
 //             buffer, so this is the overlap there is: the next tile's MMAs run under the -k work of that tile.
 //   At 18 warps the register file allows 96 registers a thread; 16 epilogue warps beat 8 (168 registers) because
 //   the -k work is latency bound (cfg-2 n = 255 call on a B200 at 1000 W: 92.2 ms against 97.7 ms, DESIGN.md 5).
+//   Kernel time at cfg-2 n = 255 (B200, 1000 W, 1965 MHz; DESIGN.md 5): 89.9 ms with 28 MMAs per K step and 64-byte
+//   chunks x 2, 68.0 ms now.  The MMA/TMA stream alone (epilogue handing TMEM back at once) takes 47.9 ms and TMA alone
+//   46.5 ms: 32-byte boxes cost the TMA more than 64-byte ones (29.8 ms), but the 64-byte ring fits only 2 stages
+//   (69.8 ms).  What is left above the stream is the TMEM drain, during which the MMAs wait.
 // Determinism: fixed M-split grid and rasterisation as ivar_ws_kernel; per-column summation order independent of the
 // candidate's position in its tile.
 // ---------------------------------------------------------------------------------------------
 constexpr int I8_L = 7;
 constexpr int I8_BM = 128;
 constexpr int I8_BN = 64;
-constexpr int I8_BK = 64;                                  // bytes of K per chunk = the 64-byte swizzle span
-constexpr int I8_A_BYTES = I8_L * I8_BM * I8_BK;           // 57344
-constexpr int I8_B_BYTES = I8_L * I8_BN * I8_BK;           // 28672
+constexpr int I8_BK = 32;                                  // bytes of K per chunk = one MMA K step = the swizzle span
+constexpr int I8_A_BYTES = I8_L * I8_BM * I8_BK;           // 28672
+constexpr int I8_B_BYTES = I8_L * I8_BN * I8_BK;           // 14336
 constexpr int I8_STAGE = I8_A_BYTES + I8_B_BYTES;          // multiple of 1024
-constexpr int I8_STAGES = 2;
+constexpr int I8_STAGES = 4;
 constexpr int I8_EPI_WARPS = 16;                        // 4 per TMEM lane quarter
 constexpr int I8_EPI_COLS = 4 * I8_BN / I8_EPI_WARPS;  // columns per epilogue thread
 constexpr int I8_THREADS = (I8_EPI_WARPS + 2) * 32;
@@ -1070,20 +1076,43 @@ __device__ __forceinline__ void tma_load_3d(void* dst, const CUtensorMap* tm, in
         : "memory");
 }
 
-// K-major operand, 64-byte swizzle: 8-row core groups 512 bytes apart (SBO), LBO unused, descriptor version 1
+// K-major operand, 32-byte swizzle: 8-row core groups 256 bytes apart (SBO), LBO unused, descriptor version 1,
+// layout type 6
 __device__ __forceinline__ uint64_t i8_desc(uint32_t saddr) {
-    return (uint64_t)((saddr & 0x3FFFF) >> 4) | ((uint64_t)1 << 16) | ((uint64_t)(512 >> 4) << 32) | ((uint64_t)1 << 46) |
-           ((uint64_t)4 << 61);
+    return (uint64_t)((saddr & 0x3FFFF) >> 4) | ((uint64_t)1 << 16) | ((uint64_t)(256 >> 4) << 32) | ((uint64_t)1 << 46) |
+           ((uint64_t)6 << 61);
 }
-// kind::i8: D s32, A and B signed, both K-major, N = 64, M = 128
-constexpr uint32_t I8_IDESC = (2u << 4) | (1u << 7) | (1u << 10) | ((uint32_t)(I8_BN >> 3) << 17) | ((uint32_t)(I8_BM >> 4) << 24);
-
+// kind::i8: D s32, A and B signed, both K-major, M = 128, N = 64 nq
+template <int NQ>
 __device__ __forceinline__ void i8_mma(uint32_t dtm, uint64_t ad, uint64_t bd, uint32_t acc) {
+    constexpr uint32_t idesc =
+        (2u << 4) | (1u << 7) | (1u << 10) | ((uint32_t)(NQ * I8_BN >> 3) << 17) | ((uint32_t)(I8_BM >> 4) << 24);
     asm volatile(
         "{\n.reg .pred p;\nsetp.ne.b32 p, %4, 0;\n"
         "tcgen05.mma.cta_group::1.kind::i8 [%0], %1, %2, %3, p;\n}\n" ::"r"(dtm),
-        "l"(ad), "l"(bd), "r"(I8_IDESC), "r"(acc)
+        "l"(ad), "l"(bd), "r"(idesc), "r"(acc)
         : "memory");
+}
+// One K step of the 7 diagonals: A slice p against the stack of B slices q0 .. q0 + nq - 1 (adjacent in smem with the
+// uniform core-group stride, so one operand of N = 64 nq) writes a_p^T b_q into D_{p+q}, which sit 64 TMEM columns
+// apart.  N <= 256 splits the 28 slice products into these 10 MMAs; the p = 0 pair covers all 448 columns and comes
+// first, so it alone carries the tile's first-step overwrite.
+template <int P, int Q0, int NQ>
+__device__ __forceinline__ void i8_mma_stack(uint32_t tmem, uint32_t sa, uint32_t sb, uint32_t first) {
+    i8_mma<NQ>(tmem + (P + Q0) * I8_BN, i8_desc(sa + P * (I8_BM * I8_BK)), i8_desc(sb + Q0 * (I8_BN * I8_BK)),
+               P != 0 || !first);
+}
+__device__ __forceinline__ void i8_mma_kstep(uint32_t tmem, uint32_t sa, uint32_t sb, uint32_t first) {
+    i8_mma_stack<0, 0, 4>(tmem, sa, sb, first);
+    i8_mma_stack<0, 4, 3>(tmem, sa, sb, first);
+    i8_mma_stack<1, 0, 4>(tmem, sa, sb, first);
+    i8_mma_stack<1, 4, 2>(tmem, sa, sb, first);
+    i8_mma_stack<2, 0, 4>(tmem, sa, sb, first);
+    i8_mma_stack<2, 4, 1>(tmem, sa, sb, first);
+    i8_mma_stack<3, 0, 4>(tmem, sa, sb, first);
+    i8_mma_stack<4, 0, 3>(tmem, sa, sb, first);
+    i8_mma_stack<5, 0, 2>(tmem, sa, sb, first);
+    i8_mma_stack<6, 0, 1>(tmem, sa, sb, first);
 }
 __device__ __forceinline__ void tc_commit(uint64_t* bar) {
     asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];\n" ::"r"(smem_u32(bar)) : "memory");
@@ -1161,12 +1190,12 @@ __global__ void __launch_bounds__(I8_THREADS, 1) ivar_i8_kernel(const __grid_con
     if (warp == I8_EPI_WARPS) {
         // ---- TMA producer ----
         if (lane == 0) {
-            int g = 0;
+            int s = 0;
+            unsigned ph = 0;
             for (int tl = 0; tl < ntiles; ++tl) {
                 const int i0 = (int)((it_begin + tl) * I8_BM);
-                for (int kc = 0; kc < kch; ++kc, ++g) {
-                    const int s = g % I8_STAGES;
-                    mbar_wait(empty + s, ((unsigned)(g / I8_STAGES) & 1u) ^ 1u);
+                for (int kc = 0; kc < kch; ++kc, s = s + 1 == I8_STAGES ? 0 : s + 1, ph ^= s == 0) {
+                    mbar_wait(empty + s, ph ^ 1u);
                     mbar_arrive_expect_tx(full + s, (unsigned)I8_STAGE);
                     unsigned char* st = ring + s * I8_STAGE;
                     tma_load_3d(st, &maps.a, kc * I8_BK, i0, 0, full + s);
@@ -1178,25 +1207,18 @@ __global__ void __launch_bounds__(I8_THREADS, 1) ivar_i8_kernel(const __grid_con
         // ---- MMA issuer ----
         if (lane == 0) {
             const uint32_t ring_s = smem_u32(ring);
-            int g = 0;
+            int s = 0;
+            unsigned ph = 0;
             for (int tl = 0; tl < ntiles; ++tl) {
                 if (tl > 0) {
                     mbar_wait(acc_empty, (unsigned)(tl - 1) & 1u);  // the epilogue has read the previous tile
                     tc_fence_after();
                 }
-                for (int kc = 0; kc < kch; ++kc, ++g) {
-                    const int s = g % I8_STAGES;
-                    mbar_wait(full + s, (unsigned)(g / I8_STAGES) & 1u);
+                for (int kc = 0; kc < kch; ++kc, s = s + 1 == I8_STAGES ? 0 : s + 1, ph ^= s == 0) {
+                    mbar_wait(full + s, ph);
                     tc_fence_after();
                     const uint32_t sa = ring_s + s * I8_STAGE, sb = sa + I8_A_BYTES;
-#pragma unroll
-                    for (int t = 0; t < I8_L; ++t)
-#pragma unroll
-                        for (int p = 0; p <= t; ++p)
-#pragma unroll
-                            for (int kk = 0; kk < I8_BK / 32; ++kk)
-                                i8_mma(tmem + t * I8_BN, i8_desc(sa + p * (I8_BM * I8_BK) + kk * 32),
-                                       i8_desc(sb + (t - p) * (I8_BN * I8_BK) + kk * 32), (kc | p | kk) != 0);
+                    i8_mma_kstep(tmem, sa, sb, kc == 0);
                     tc_commit(empty + s);
                 }
                 tc_commit(acc_full);
@@ -1336,7 +1358,7 @@ __global__ void __launch_bounds__(256) ivar_slice_kernel(const double* __restric
     }
 }
 
-// 3-D map over the slices of one side: dims {n (K bytes), ncols, 7}, box {64, rows, 7}, 64-byte swizzle
+// 3-D map over the slices of one side: dims {n (K bytes), ncols, 7}, box {32, rows, 7}, 32-byte swizzle
 int make_i8_map(CUtensorMap* m, const int8_t* base, int64_t ldk, int64_t n, int64_t ncols, int64_t sstride, int box_rows) {
     EncodeTiledFn enc = encode_tiled();
     if (!enc) {
@@ -1348,7 +1370,7 @@ int make_i8_map(CUtensorMap* m, const int8_t* base, int64_t ldk, int64_t n, int6
     const cuuint32_t box[3] = {(cuuint32_t)I8_BK, (cuuint32_t)box_rows, (cuuint32_t)I8_L};
     const cuuint32_t estr[3] = {1, 1, 1};
     CUresult r = enc(m, CU_TENSOR_MAP_DATA_TYPE_UINT8, 3, const_cast<int8_t*>(base), dims, strides, box, estr,
-                     CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_64B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
+                     CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_32B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
                      CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
     if (r != CUDA_SUCCESS) {
         gpx_set_error("ivar_i8: cuTensorMapEncodeTiled failed with CUresult %d", (int)r);
