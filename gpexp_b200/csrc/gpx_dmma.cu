@@ -1009,7 +1009,10 @@ int prologue_rows(gpx_handle h, int prologue) {
 // i.e. |S_i8 - S| <= 7.04 K u + |S| 2^-53, against the FP64 DMMA bound ~ K eps sum_i |W_M[i,m]| |W_C[i,c]|.
 // L = 7 is the smallest L for which the bound stays at the FP64 level (L = 6 is 256 times coarser); L = 8 would add
 // 8 products per K step and an eighth accumulator (8 x 64 TMEM columns: no room for anything else) for accuracy the
-// FP64 epilogue cannot use.  tests/test_ivar_int8_core.py checks the model against exact integer arithmetic.
+// FP64 epilogue cannot use.  tests/test_ivar_int8_core.py checks the model against exact integer arithmetic, and
+// tests/test_ivar_contraction_exact.py checks this kernel against the model bit for bit, pair by pair.
+// Domain of the bound: both column maxima >= 2^-1044 (2^(e - 30) > 0) and 2^(e_m + e_c - 60) normal; outside it S_i8
+// flushes to 0, which in IVAR (|W| <= sqrt(k) < 2^512) only happens where |S| < 2^-517 and S^2 is not a normal number.
 //
 // Slices live K-major ([p][column][k], ldk = roundup(n, 64) bytes) in caller scratch (gpx_set_ivar_scratch) and are
 // rebuilt from the FP64 factors on every scoring call by ivar_slice_kernel: one streaming pass over W (0.75 ms of the

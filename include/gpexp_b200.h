@@ -227,7 +227,9 @@ int64_t gpx_score_ivar_workspace(gpx_handle h, int64_t M, int64_t C);
  *         r[c]     = sum_m ( k(m,c) - sum_{i<n} Wm[i,m] Wc[i,c] )^2            FP64 DMMA contraction
  *         cost[c]  = | sum(varM)/M - (r[c] / (varC[c] + noise)) / M |           (reduction = 0 if the
  *                    denominator is numerically zero: the pinv null-direction rule, SURVEY.md section 7)
- *     then arg-min with lowest-index tie-break into best/idx (a NaN score wins, as in np.argmin).
+ *     then arg-min with lowest-index tie-break into best/idx (a NaN score wins, as in np.argmin).  mask (nullable):
+ *     candidates with mask[c] != 0 are skipped by the arg-min (their scores are still written); if all are masked,
+ *     best[0] = 0.0 and idx[0] = -1.
  *     Ma_rows : integration points, Cb_rows : candidates -- per `prologue` the prepared sides (GPX_SIDE_A / GPX_SIDE_B)
  *     or the raw coordinates; leading dimensions ldm / ldc. */
 int gpx_score_ivar(gpx_handle h, int prologue, const double* Wm, int64_t ldm, const double* varM, const double* Ma_rows,

@@ -28,8 +28,8 @@ def slice_column(x):
     return dig, e
 
 
-def i8_dot(xm, xc):
-    """S as the kernel forms it: int32 diagonals t = 0..6, int64 hi/lo, one FP64 rounding, scales 2^(e-30)."""
+def i8_parts(xm, xc):
+    """(D, hi, lo, e_m, e_c) of one pair: the int32 diagonals t = 0..6 and their int64 recombination."""
     am, em = slice_column(xm)
     bc, ec = slice_column(xc)
     D = [sum(int(np.dot(am[p], bc[t - p])) for p in range(t + 1)) for t in range(L)]
@@ -37,6 +37,12 @@ def i8_dot(xm, xc):
     hi = (D[0] << 24) + (D[1] << 16) + (D[2] << 8) + D[3]
     lo = (D[4] << 16) + (D[5] << 8) + D[6]
     assert abs(hi) < 2 ** 51 and abs(lo) < 2 ** 51
+    return D, hi, lo, em, ec
+
+
+def i8_dot(xm, xc):
+    """S as the kernel forms it: int32 diagonals t = 0..6, int64 hi/lo, one FP64 rounding, scales 2^(e-30)."""
+    _, hi, lo, em, ec = i8_parts(xm, xc)
     return float((hi << 24) + lo) * (np.ldexp(1.0, em - 30) * np.ldexp(1.0, ec - 30)), em, ec
 
 
