@@ -7,7 +7,7 @@ host reads the picked indices back once at the end.  Layouts (all float64):
     X      d x ld        dimension-major coordinates of a point set (ld = roundup(n, 128))
     W      ncap x ld     row i = i-th row of L^-1 K(D, .) for every point of the set (K-major for DMMA)
     var    ld            running posterior variance of every point
-    rec    19 + ncap     pivot record: score, global index, var_p + noise, x_p[16], W[0:n, p]
+    rec    19 + ncap     pivot record: score, global index, var_p + noise (or + nu(p)), x_p[16], W[0:n, p]
 
 Candidates shard across ranks (one process per GPU): each rank owns a contiguous block of the pool,
 the integration points are replicated, and the only exchange per step is one NCCL all-gather of the
@@ -140,7 +140,7 @@ class _Pivoting:
         return self.picks[: self.n].cpu().numpy()
 
     def pivots(self) -> np.ndarray:
-        """var_D(p) + noise of every pick, in pick order."""
+        """var_D(p) + noise of the pick, for every pick in pick order (noise = nu(p) for a per-candidate noise)."""
         return self.pick_pivots[: self.n].cpu().numpy()
 
     def ill_conditioned_from(self, scale: float):
@@ -520,13 +520,26 @@ class GreedyIVAREngine(_Pivoting):
     ONE_KERNEL_PAIRS = int(os.environ.get("GPX_ONE_KERNEL_PAIRS", ONE_KERNEL_DEFAULT))
 
     def __init__(self, dev: Device, cand: PointSet, mc: PointSet, n_max: int, noise: float, zero_scale: float,
-                 shard=None, index_offset: int = 0, resident: bool = False):
+                 shard=None, index_offset: int = 0, resident: bool = False, cand_noise=None):
         """resident=True keeps the posterior covariance cov_D(m, c) (8*M*C bytes) in HBM and replaces the per-step
         O(M n C) contraction by one rank-1 update pass (16*M*C bytes of traffic per step, independent of n) -- the
-        better algorithm for a greedy LOOP whenever the matrix fits; scoring a GIVEN design still takes the contraction."""
+        better algorithm for a greedy LOOP whenever the matrix fits; scoring a GIVEN design still takes the contraction.
+
+        cand_noise: host vector nu of a heteroscedastic noise function at the local candidates (noise must be 0.0 then).
+        The candidate running variance is then kept noise-inclusive, varC[c] = var_D(c) + nu(c): every kernel sees the
+        noise only as varC + noise, the append's (var + nu) - w^2 is the same update, and the pivot var_D(p) + nu(p)
+        makes U the factor of K_DD + diag(nu(D)).  Integration points carry no noise."""
         self.cand, self.mc = cand, mc
         self.resident = bool(resident)
         self.noise = float(noise)
+        self.cand_noise = None
+        if cand_noise is not None:
+            nu = np.asarray(cand_noise, dtype=np.float64).ravel()
+            if self.noise != 0.0:
+                raise ValueError("cand_noise replaces the scalar noise: pass noise=0.0 with it")
+            if nu.size != cand.n:
+                raise ValueError(f"cand_noise has {nu.size} values for {cand.n} candidates")
+            self.cand_noise = dev.upload(nu)
         self.zero_tol = ZERO_VAR_TOL * float(zero_scale)
         ncap = max(int(n_max), 1)
         self._init_pivot(dev, ncap, n_max, shard, index_offset)
@@ -536,6 +549,7 @@ class GreedyIVAREngine(_Pivoting):
         self.varM = dev.zeros(mc.ld)
         self.U = dev.zeros(ncap, roundup(ncap))
         check(lib.gpx_prior_diag(dev.h, ptr(cand.X), cand.n, cand.ld, ptr(self.varC), dev.stream), "gpx_prior_diag")
+        self._add_cand_noise()
         check(lib.gpx_prior_diag(dev.h, ptr(mc.X), mc.n, mc.ld, ptr(self.varM), dev.stream), "gpx_prior_diag")
         self.nseg = int(lib.gpx_cov_segments(mc.n, cand.n))
         self.ldp = (cand.n + 1) & ~1
@@ -557,6 +571,12 @@ class GreedyIVAREngine(_Pivoting):
 
     def _local_count(self):
         return self.cand.n
+
+    def _add_cand_noise(self):
+        """varC += nu: called wherever varC is (re)built from the prior or from a factor."""
+        if self.cand_noise is not None:
+            check(lib.gpx_axpby(self.dev.h, self.cand.n, 1.0, ptr(self.cand_noise), 1.0, ptr(self.varC), self.dev.stream),
+                  "gpx_axpby")
 
     def _cov_pass(self, a, b):
         dev, cand, mc = self.dev, self.cand, self.mc
@@ -628,6 +648,7 @@ class GreedyIVAREngine(_Pivoting):
         prior = dev.zeros(cand.ld)
         check(lib.gpx_prior_diag(dev.h, ptr(cand.X), cand.n, cand.ld, ptr(prior), dev.stream), "gpx_prior_diag")
         check(lib.gpx_colsumsq(dev.h, ptr(self.Wc), self.n, cand.n, cand.ld, ptr(prior), ptr(self.varC), dev.stream), "colsumsq")
+        self._add_cand_noise()
         prior = dev.zeros(mc.ld)
         check(lib.gpx_prior_diag(dev.h, ptr(mc.X), mc.n, mc.ld, ptr(prior), dev.stream), "gpx_prior_diag")
         check(lib.gpx_colsumsq(dev.h, ptr(self.Wm), self.n, mc.n, mc.ld, ptr(prior), ptr(self.varM), dev.stream), "colsumsq")
@@ -639,6 +660,7 @@ class GreedyIVAREngine(_Pivoting):
         _, vC = factor.solve_gram(self.cand, W=self.Wc)
         _, vM = factor.solve_gram(self.mc, W=self.Wm)
         self.varC.copy_(vC)
+        self._add_cand_noise()
         self.varM.copy_(vM)
         if self.resident:
             dev, cand, mc = self.dev, self.cand, self.mc

@@ -225,6 +225,18 @@ def performGreedyVarExperimentalDesign(kernel, mcPoints, nPoints, dimension, wei
     return mcPoints[indKeep, :]
 
 
+def _noise_values(noiseFunc, points):
+    """noiseFunc(points) as one float64 nugget per point; the noise function is user code, so its output is checked."""
+    nu = np.asarray(noiseFunc(points), dtype=np.float64).ravel()
+    if nu.size != points.shape[0]:
+        raise ValueError(f"noise function returned {nu.size} values for {points.shape[0]} points (one per point expected)")
+    if not np.all(np.isfinite(nu)):
+        raise ValueError("noise function returned a value that is not finite")
+    if np.any(nu < 0.0):
+        raise ValueError("noise function returned a negative value")
+    return nu
+
+
 def beginGreedyIVARExperimentalDesign(costFuncIVAR, candidates, nPoints, shard=None, resident=None):
     """The greedy-IVAR design as a steppable object (a gpexp_b200.engine.GreedyIVAREngine): `.run(n)` grows the design to n
     points (one C call for all steps), `.indices()`, `.pick_scores`, `.snapshot()` / `.restore()` re-time a step.
@@ -233,18 +245,25 @@ def beginGreedyIVARExperimentalDesign(costFuncIVAR, candidates, nPoints, shard=N
     scores its own contiguous block.
     resident : keep the M x C posterior covariance in HBM and update it by one rank-1 pass per step instead of
     re-contracting (identical picks, 16*M*C bytes per step instead of 2*M*n*C flop).  None = automatic: on when
-    the matrix takes less than half of the free device memory."""
+    the matrix takes less than half of the free device memory.
+
+    With a heteroscedastic `costFuncIVAR.space.noiseFunc`, the cost of design + [c] uses the nugget noiseFunc(design + [c])
+    as costFunctionGP_IVAR.evaluate does, and gp.noise is not used.  The noise function must be pointwise and
+    deterministic: it is evaluated once on this rank's candidates (the reference re-evaluates it on every design + [c]).
+    It must return one finite value >= 0 per point, else ValueError."""
     gp = costFuncIVAR.gaussianProcess
-    if costFuncIVAR.space.noiseFunc is not None:
-        raise NotImplementedError("greedy IVAR with a heteroscedastic noise function is not on the device path")
-    noise = _nugget_arg(gp.noise)
-    if isinstance(noise, np.ndarray):
-        raise NotImplementedError("greedy IVAR needs a scalar noise")
-    dev = gp.kernel._bind()
-    fam, d, params = gp.kernel._gpx_spec()
     lo, hi = 0, candidates.shape[0]
     if shard is not None:
         lo, hi = Shard.split(candidates.shape[0], shard.world, shard.rank)
+    if costFuncIVAR.space.noiseFunc is not None:
+        noise, cand_noise = 0.0, _noise_values(costFuncIVAR.space.noiseFunc, candidates[lo:hi])
+    else:
+        noise, cand_noise = _nugget_arg(gp.noise), None
+        if isinstance(noise, np.ndarray):
+            raise NotImplementedError("greedy IVAR needs a scalar noise")
+        noise = float(noise)
+    dev = gp.kernel._bind()
+    fam, d, params = gp.kernel._gpx_spec()
     cand = dev.points(candidates[lo:hi])
     mc = _ivar_mc_points(costFuncIVAR, dev)
     if resident is None:
@@ -255,8 +274,8 @@ def beginGreedyIVARExperimentalDesign(costFuncIVAR, candidates, nPoints, shard=N
             flag = torch.tensor([1 if resident else 0], device=dev.torch_device)
             shard.dist.all_reduce(flag, op=shard.dist.ReduceOp.MIN, group=shard.group)
             resident = bool(flag.item())
-    return GreedyIVAREngine(dev, cand, mc, nPoints, float(noise), prior_scale(fam, params), shard=shard, index_offset=lo,
-                            resident=bool(resident))
+    return GreedyIVAREngine(dev, cand, mc, nPoints, noise, prior_scale(fam, params), shard=shard, index_offset=lo,
+                            resident=bool(resident), cand_noise=cand_noise)
 
 
 def performGreedyIVARExperimentalDesign(costFuncIVAR, candidates, nPoints, returnIndices=False, shard=None, resident=None):
@@ -280,20 +299,28 @@ def performGreedyIVARExperimentalDesign(costFuncIVAR, candidates, nPoints, retur
 def scoreCandidatesIVAR(costFuncIVAR, design, candidates, shard=None):
     """One stateless IVAR scoring pass from HOST buffers: cost of design + [c] for every candidate c.
     Returns (costs, argmin index).  With `shard` every rank passes the full candidate array, scores its own contiguous
-    block and returns (costs of its block, GLOBAL arg-min index).  This is the end-to-end call bench.py times (`e2e`)."""
+    block and returns (costs of its block, GLOBAL arg-min index).  This is the end-to-end call bench.py times (`e2e`).
+    A heteroscedastic `costFuncIVAR.space.noiseFunc` is honoured as in beginGreedyIVARExperimentalDesign: the design
+    Gram gets the nugget noiseFunc(design) and candidate c the noise noiseFunc(c)."""
     gp = costFuncIVAR.gaussianProcess
-    noise = _nugget_arg(gp.noise)
-    dev = gp.kernel._bind()
-    fam, d, params = gp.kernel._gpx_spec()
+    noiseFunc = costFuncIVAR.space.noiseFunc
     lo, hi = 0, candidates.shape[0]
     if shard is not None:
         lo, hi = Shard.split(candidates.shape[0], shard.world, shard.rank)
+    n = design.shape[0]
+    if noiseFunc is None:
+        noise = nugget = float(_nugget_arg(gp.noise))
+        cand_noise = None
+    else:
+        noise, cand_noise = 0.0, _noise_values(noiseFunc, candidates[lo:hi])
+        nugget = _noise_values(noiseFunc, design) if n else None
+    dev = gp.kernel._bind()
+    fam, d, params = gp.kernel._gpx_spec()
     cand = dev.points(candidates[lo:hi])
     mc = dev.points(costFuncIVAR.mcPoints)
-    n = design.shape[0]
-    eng = GreedyIVAREngine(dev, cand, mc, max(n, 1), float(noise), prior_scale(fam, params))
+    eng = GreedyIVAREngine(dev, cand, mc, max(n, 1), noise, prior_scale(fam, params), cand_noise=cand_noise)
     if n:
-        eng.load_design(DesignFactor(dev, dev.points(design), float(noise)))
+        eng.load_design(DesignFactor(dev, dev.points(design), nugget))
     eng.score()
     costs = eng.scores[: cand.n].cpu().numpy()
     best = int(eng.idx.item())

@@ -1,5 +1,6 @@
 """Multi-GPU parity check (run under torch.distributed.run, one rank per GPU):
-sharded greedy IVAR and greedy max-variance must pick exactly the indices of the single-process CPU oracle."""
+sharded greedy IVAR (scalar noise and a heteroscedastic noise function) and greedy max-variance must pick exactly the
+indices of the single-process CPU oracle."""
 import os
 import sys
 
@@ -30,6 +31,12 @@ def main():
     kern = kernels.KernelSquaredExponential([0.2, 0.3], 1.0, 2)
     cf = ed.costFunctionGP_IVAR(gp.GP(kern, 1e-6), 1, Space(2, None, None), mcPoints=mc)
     idx = ed.performGreedyIVARExperimentalDesign(cf, cand, 12, returnIndices=True, shard=shard)
+
+    # --- the same with a noise function: each rank evaluates it on its own block, nu(p) travels in the pivot record -----
+    def nu(p):
+        return 1e-4 + 1e-3 * p[:, 0] ** 2
+    cfh = ed.costFunctionGP_IVAR(gp.GP(kern, 1e-6), 1, Space(2, None, None, noise=nu), mcPoints=mc)
+    hidx = ed.performGreedyIVARExperimentalDesign(cfh, cand, 12, returnIndices=True, shard=shard)
     # --- greedy max variance, pool sharded ----------------------------------------------------------
     pool = rng.uniform(-1, 1, (10007, 5))
     mk = kernels.KernelIsoMatern(1.0, 1.0, 5)
@@ -54,13 +61,21 @@ def main():
             print("ref mi", mref, "got", [int(i) for i in midx], "info", minfo)
         ref, _ = orc.fast_greedy_ivar(orc.KernelSpec.se([0.2, 0.3], 1.0, 2), cand, mc, 12, 1e-6)
         vref, _ = orc.fast_greedy_var(orc.KernelSpec.matern32(1.0, 1.0, 5), pool, 25)
-        ok = [int(i) for i in idx] == ref and [int(i) for i in vidx] == vref and mi_ok
+        from tests.hetero_oracle import fast_greedy_ivar_nu
+        href, _ = fast_greedy_ivar_nu(orc.KernelSpec.se([0.2, 0.3], 1.0, 2), cand, mc, 12, nu(cand))
+        h_ok = [int(i) for i in hidx] == href
+        print("multigpu_check world=%d hetero ivar=%s -> %s" % (world, [int(i) for i in hidx][:6], "OK" if h_ok else "MISMATCH"),
+              flush=True)
+        if not h_ok:
+            print("ref hetero ivar", href, "got", [int(i) for i in hidx])
+        ok = [int(i) for i in idx] == ref and [int(i) for i in vidx] == vref and mi_ok and h_ok
         print("multigpu_check world=%d ivar=%s var=%s -> %s" % (world, [int(i) for i in idx][:6], [int(i) for i in vidx][:6],
                                                                  "OK" if ok else "MISMATCH"), flush=True)
         if not ok:
             print("ref ivar", ref, "got", [int(i) for i in idx]); print("ref var", vref, "got", [int(i) for i in vidx])
     # every rank must hold the same picks
-    t = torch.tensor([int(i) for i in idx] + [int(i) for i in vidx] + [int(i) for i in midx], device="cuda")
+    t = torch.tensor([int(i) for i in idx] + [int(i) for i in hidx] + [int(i) for i in vidx] + [int(i) for i in midx],
+                     device="cuda")
     g = [torch.zeros_like(t) for _ in range(world)]
     dist.all_gather(g, t)
     same = all(bool((x == t).all()) for x in g)
