@@ -396,7 +396,8 @@ extern "C" int gpx_chol_append(gpx_handle h, double* U, int64_t n, int64_t ld, c
     GPX_REQUIRE(knew || n == 0, GPX_EINVAL, "knew is NULL");
     const size_t smem = (size_t)n * sizeof(double);
     GPX_REQUIRE(smem <= 200 * 1024, GPX_ESIZE, "design size exceeds the shared-memory buffer (25600)");
-    if (smem > 48 * 1024) {
+    // the kernel's static reduction buffer (red[32]) counts against the 48 KB a launch gets without the opt-in
+    if (smem + 32 * sizeof(double) > 48 * 1024) {
         int rc = gpx_ensure_smem(h, (const void*)chol_append_kernel, 200 * 1024, "gpx_chol_append");
         if (rc) return rc;
     }

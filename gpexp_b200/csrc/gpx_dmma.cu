@@ -86,7 +86,7 @@ struct CoreArgs {
     int K;
     int prows;         // prologue rows to stage: EXPANDED roundup(d+2, 4), DIFF d
     int tiles_per_cta; // IVAR: i-tiles each CTA walks
-    int upper_only;    // SUB: skip tiles below the diagonal ; ivar_ws_kernel: candidate tiles per wave group
+    int upper_only;    // SUB: update only j >= i (strictly-lower entries untouched) ; ivar_ws_kernel: candidate tiles per wave group
     int ldo_splits;    // ivar_ws_kernel: number of M-splits
     // sub_ws_kernel: operand B is this rank's column slice of a LOWER-triangular matrix distributed block-cyclically
     // (local column j = block j / tri_blk of this rank = global block (j / tri_blk) * tri_world + tri_rank): rows above the
@@ -421,6 +421,9 @@ __global__ void __launch_bounds__(Cfg::NT, 2)
                                 } else {
                                     dst[0] = -v0;
                                 }
+                            } else if (a.upper_only && j < i) {
+                                // symmetric update of a diagonal-straddling tile: the strictly-lower part is left untouched
+                                if (j + 1 == i && j + 1 < a.J) dst[1] -= v1;
                             } else {
                                 if (j + 1 < a.J) {
                                     double2 c = *reinterpret_cast<double2*>(dst);
@@ -890,7 +893,10 @@ __global__ void __launch_bounds__(256, 1) sub_ws_kernel(const __grid_constant__ 
                 if (j >= a.J) continue;
                 double* dst = a.out + i * a.ldo + j;
                 const double v0 = acc[t][u2 * 2][e], v1 = acc[t][u2 * 2 + 1][e];
-                if (j + 1 < a.J) {
+                if (a.upper_only && j < i) {
+                    // symmetric update of a diagonal-straddling tile: the strictly-lower part is left untouched
+                    if (j + 1 == i && j + 1 < a.J) dst[1] -= v1;
+                } else if (j + 1 < a.J) {
                     double2 c = *reinterpret_cast<double2*>(dst);
                     c.x -= v0;
                     c.y -= v1;

@@ -145,8 +145,8 @@ int gpx_trsm_back(gpx_handle h, const double* Ut, int64_t n, int64_t ldu, double
  * diag((K+noise I)^-1) = column sums of squares of Y, columns of the precision come from gpx_mi_prec_column. */
 int gpx_trtri_t(gpx_handle h, const double* U, int64_t n, int64_t ldu, double* Y, int64_t ldy, void* stream);
 
-/* C[i,j] -= sum_k A[k*lda+i] * B[k*ldb+j]   (i<I, j<J, k<K), FP64 DMMA.  upper_only != 0 skips tiles
- * strictly below the diagonal (symmetric rank-k update of the Cholesky trailing matrix). */
+/* C[i,j] -= sum_k A[k*lda+i] * B[k*ldb+j]   (i<I, j<J, k<K), FP64 DMMA.  upper_only != 0 updates only the entries
+ * j >= i and leaves the strictly-lower ones untouched (symmetric rank-k update of the Cholesky trailing matrix). */
 int gpx_dgemm_tn_sub(gpx_handle h, const double* A, int64_t lda, const double* B, int64_t ldb, double* C,
                      int64_t ldc, int64_t I, int64_t J, int64_t K, int upper_only, void* stream);
 
