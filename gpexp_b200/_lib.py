@@ -83,6 +83,7 @@ SIGNATURES = {
     "gpx_dgemm_tn_sub": [_p, _p, _i64, _p, _i64, _p, _i64, _i64, _i64, _i64, _int, _p],
     "gpx_dgemm_tn_sub_padded": [_p, _p, _i64, _p, _i64, _p, _i64, _i64, _i64, _i64, _int, _p],
     "gpx_gather_pivot": [_p, _p, _i64, _i64, _p, _p, _i64, _p, _p, _i64, _p, _dbl, _p, _p],
+    "gpx_gather_pivot_nu": [_p, _p, _i64, _i64, _p, _p, _i64, _p, _p, _i64, _p, _p, _dbl, _p, _p],
     "gpx_select_pivot": [_p, _p, _int, _i64, _i64, _int, _p, _p],
     "gpx_append_row": [_p, _int, _p, _p, _p, _i64, _i64, _p, _i64, _i64, _p, _p],
     "gpx_argreduce": [_p, _p, _p, _p, _i64, _int, _p, _p, _p],
@@ -98,12 +99,14 @@ SIGNATURES = {
     "gpx_cov_from_factors": [_p, _int, _p, _i64, _p, _i64, _p, _i64, _p, _i64, _i64, _p, _i64, _p],
     "gpx_score_ivar_partials": [_p, _p, _int, _i64, _p, _i64, _p, _i64, _dbl, _dbl, _p, _p, _p, _p, _p],
     "gpx_score_mi": [_p, _p, _p, _dbl, _p, _i64, _p, _p, _p, _p],
+    "gpx_score_mi_nu": [_p, _p, _p, _p, _dbl, _p, _i64, _p, _p, _p, _p],
     "gpx_mi_prec_column_workspace": [_i64, _i64],
     "gpx_mi_prec_column": [_p, _p, _i64, _i64, _i64, _i64, _i64, _i64, _p, _p, _p, _p, _p],
     "gpx_gather_column": [_p, _p, _i64, _i64, _p, _p, _p, _p],
     "gpx_local_index": [_p, _p, _i64, _i64, _p, _p],
     "gpx_local_index_cyclic": [_p, _p, _i64, _i64, _i64, _i64, _p, _p],
     "gpx_add_at_rows": [_p, _p, _i64, _p, _i64, _dbl, _p],
+    "gpx_add_at_rows_vec": [_p, _p, _i64, _p, _i64, _p, _dbl, _p],
     "gpx_dgemm_tn_sub_lower": [_p, _p, _i64, _p, _i64, _p, _i64, _i64, _i64, _i64, _int, _int, _int, _p],
     "gpx_colsumsq": [_p, _p, _i64, _i64, _i64, _p, _p, _p],
     "gpx_transpose": [_p, _p, _i64, _i64, _i64, _p, _i64, _p],

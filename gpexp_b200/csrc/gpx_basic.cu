@@ -441,7 +441,8 @@ __global__ void __launch_bounds__(256) gather_pivot_kernel(const double* __restr
                                                             const double* __restrict__ var, const double* __restrict__ X,
                                                             int64_t ldx, int d, const double* __restrict__ score,
                                                             const int64_t* __restrict__ idx, int64_t offset,
-                                                            const int64_t* __restrict__ index_map, double noise,
+                                                            const int64_t* __restrict__ index_map,
+                                                            const double* __restrict__ nu, double noise,
                                                             double* __restrict__ rec) {
     const int64_t p = idx[0];
     if (p < 0) {
@@ -456,24 +457,38 @@ __global__ void __launch_bounds__(256) gather_pivot_kernel(const double* __restr
         if (threadIdx.x == 0) {
             rec[0] = score ? score[0] : 0.0;
             rec[1] = (double)(index_map ? index_map[p] : p + offset);
-            rec[2] = var[p] + noise;
+            rec[2] = var[p] + (nu ? nu[p] : noise);
         }
         if (threadIdx.x < GPX_MAX_DIM) rec[3 + threadIdx.x] = threadIdx.x < d ? X[threadIdx.x * ldx + p] : 0.0;
     }
     for (int i = blockIdx.x * 256 + threadIdx.x; i < n; i += gridDim.x * 256) rec[GPX_PIVOT_HDR + i] = W[(int64_t)i * ldw + p];
 }
 
-extern "C" int gpx_gather_pivot(gpx_handle h, const double* W, int64_t ldw, int64_t n, const double* var, const double* X,
-                                int64_t ldx, const double* score_dev, const int64_t* idx_dev, int64_t index_offset,
-                                const int64_t* index_map, double noise, double* rec, void* stream) {
+static int gather_pivot_impl(gpx_handle h, const double* W, int64_t ldw, int64_t n, const double* var, const double* X,
+                             int64_t ldx, const double* score_dev, const int64_t* idx_dev, int64_t index_offset,
+                             const int64_t* index_map, const double* nu, double noise, double* rec, void* stream) {
     GPX_NEED_KERNEL(h);
     GPX_REQUIRE(n >= 0 && var && X && idx_dev && rec && (W || n == 0), GPX_EINVAL, "bad arguments");
     unsigned grid = (unsigned)((n + 255) / 256);
     if (grid < 1) grid = 1;
     if (grid > 64) grid = 64;
     gather_pivot_kernel<<<grid, 256, 0, (cudaStream_t)stream>>>(W, ldw, (int)n, var, X, ldx, h->kp.d, score_dev, idx_dev,
-                                                              index_offset, index_map, noise, rec);
+                                                              index_offset, index_map, nu, noise, rec);
     return gpx_check_launch("gpx_gather_pivot");
+}
+
+extern "C" int gpx_gather_pivot(gpx_handle h, const double* W, int64_t ldw, int64_t n, const double* var, const double* X,
+                                int64_t ldx, const double* score_dev, const int64_t* idx_dev, int64_t index_offset,
+                                const int64_t* index_map, double noise, double* rec, void* stream) {
+    return gather_pivot_impl(h, W, ldw, n, var, X, ldx, score_dev, idx_dev, index_offset, index_map, nullptr, noise, rec,
+                             stream);
+}
+
+extern "C" int gpx_gather_pivot_nu(gpx_handle h, const double* W, int64_t ldw, int64_t n, const double* var,
+                                   const double* X, int64_t ldx, const double* score_dev, const int64_t* idx_dev,
+                                   int64_t index_offset, const int64_t* index_map, const double* nu, double noise,
+                                   double* rec, void* stream) {
+    return gather_pivot_impl(h, W, ldw, n, var, X, ldx, score_dev, idx_dev, index_offset, index_map, nu, noise, rec, stream);
 }
 
 __global__ void __launch_bounds__(256) select_pivot_kernel(const double* __restrict__ recs, int nrec, int64_t stride, int n,
@@ -619,7 +634,8 @@ extern "C" int gpx_transpose(gpx_handle h, const double* in, int64_t rows, int64
 // K6  mutual-information helpers
 // ---------------------------------------------------------------------------------------------
 __global__ void __launch_bounds__(256) score_mi_kernel(const double* __restrict__ num, const double* __restrict__ pd,
-                                                        double noise, const uint8_t* __restrict__ mask, int64_t n,
+                                                        const double* __restrict__ nu, double noise,
+                                                        const uint8_t* __restrict__ mask, int64_t n,
                                                         double* __restrict__ score) {
     const int64_t j = (int64_t)blockIdx.x * 256 + threadIdx.x;
     if (j >= n) return;
@@ -627,18 +643,29 @@ __global__ void __launch_bounds__(256) score_mi_kernel(const double* __restrict_
         score[j] = -INFINITY;
         return;
     }
-    const double den = 1.0 / pd[j] - noise;  // var(y | V minus A minus y)   experimentalDesign.py:277-281
-    score[j] = num[j] / den;                 // :284
+    const double den = 1.0 / pd[j] - (nu ? nu[j] : noise);  // var(y | V minus A minus y)   experimentalDesign.py:277-281
+    score[j] = num[j] / den;                                 // :284
+}
+
+static int score_mi_impl(gpx_handle h, const double* num_var, const double* prec_diag, const double* nu, double noise,
+                         const uint8_t* mask, int64_t n, double* score_out, double* best, int64_t* idx, void* stream) {
+    GPX_REQUIRE(h && num_var && prec_diag && score_out && best && idx && n >= 1, GPX_EINVAL, "bad arguments");
+    cudaStream_t st = (cudaStream_t)stream;
+    score_mi_kernel<<<(unsigned)((n + 255) / 256), 256, 0, st>>>(num_var, prec_diag, nu, noise, mask, n, score_out);
+    int rc = gpx_check_launch("gpx_score_mi");
+    if (rc) return rc;
+    return gpx_argreduce_impl(h, score_out, nullptr, mask, n, 0, best, idx, st);
 }
 
 extern "C" int gpx_score_mi(gpx_handle h, const double* num_var, const double* prec_diag, double noise,
                             const uint8_t* mask, int64_t n, double* score_out, double* best, int64_t* idx, void* stream) {
-    GPX_REQUIRE(h && num_var && prec_diag && score_out && best && idx && n >= 1, GPX_EINVAL, "bad arguments");
-    cudaStream_t st = (cudaStream_t)stream;
-    score_mi_kernel<<<(unsigned)((n + 255) / 256), 256, 0, st>>>(num_var, prec_diag, noise, mask, n, score_out);
-    int rc = gpx_check_launch("gpx_score_mi");
-    if (rc) return rc;
-    return gpx_argreduce_impl(h, score_out, nullptr, mask, n, 0, best, idx, st);
+    return score_mi_impl(h, num_var, prec_diag, nullptr, noise, mask, n, score_out, best, idx, stream);
+}
+
+extern "C" int gpx_score_mi_nu(gpx_handle h, const double* num_var, const double* prec_diag, const double* nu,
+                               double noise, const uint8_t* mask, int64_t n, double* score_out, double* best, int64_t* idx,
+                               void* stream) {
+    return score_mi_impl(h, num_var, prec_diag, nu, noise, mask, n, score_out, best, idx, stream);
 }
 
 // out[i] = sum_{k >= max(i,p)} Y[k,i] * Y[k,p]   (Y lower triangular, row-major).  Reads ~4 n^2 bytes.
@@ -794,19 +821,30 @@ extern "C" int gpx_local_index_cyclic(gpx_handle h, const double* rec, int64_t b
     return gpx_check_launch("gpx_local_index_cyclic");
 }
 
-// A[rows[j] * ld + j] += value for j < n : the diagonal of a matrix whose columns are a scattered subset of a square one
+// A[rows[j] * ld + j] += vals ? vals[j] : value for j < n : the diagonal of a matrix whose columns are a scattered subset
+// of a square one
 __global__ void __launch_bounds__(256) add_at_rows_kernel(double* __restrict__ A, int64_t ld, const int64_t* __restrict__ rows,
-                                                           int64_t n, double value) {
+                                                           int64_t n, const double* __restrict__ vals, double value) {
     const int64_t j = (int64_t)blockIdx.x * 256 + threadIdx.x;
-    if (j < n) A[rows[j] * ld + j] += value;
+    if (j < n) A[rows[j] * ld + j] += vals ? vals[j] : value;
 }
 
-extern "C" int gpx_add_at_rows(gpx_handle h, double* A, int64_t ld, const int64_t* rows, int64_t n, double value, void* stream) {
+static int add_at_rows_impl(gpx_handle h, double* A, int64_t ld, const int64_t* rows, int64_t n, const double* vals,
+                            double value, void* stream) {
     GPX_REQUIRE(h && n >= 0, GPX_EINVAL, "bad arguments");
     if (n == 0) return GPX_OK;
     GPX_REQUIRE(A && rows && ld >= n, GPX_EINVAL, "bad arguments");
-    add_at_rows_kernel<<<(unsigned)((n + 255) / 256), 256, 0, (cudaStream_t)stream>>>(A, ld, rows, n, value);
+    add_at_rows_kernel<<<(unsigned)((n + 255) / 256), 256, 0, (cudaStream_t)stream>>>(A, ld, rows, n, vals, value);
     return gpx_check_launch("gpx_add_at_rows");
+}
+
+extern "C" int gpx_add_at_rows(gpx_handle h, double* A, int64_t ld, const int64_t* rows, int64_t n, double value, void* stream) {
+    return add_at_rows_impl(h, A, ld, rows, n, nullptr, value, stream);
+}
+
+extern "C" int gpx_add_at_rows_vec(gpx_handle h, double* A, int64_t ld, const int64_t* rows, int64_t n, const double* vals,
+                                   double value, void* stream) {
+    return add_at_rows_impl(h, A, ld, rows, n, vals, value, stream);
 }
 
 

@@ -77,6 +77,18 @@ class Shard:
         return True
 
 
+def _noise_vector(name: str, nu, noise: float, n: int, what: str):
+    """A per-point noise vector for an engine (None stays None): it replaces the scalar noise, one value per point."""
+    if nu is None:
+        return None
+    nu = np.asarray(nu, dtype=np.float64).ravel()
+    if noise != 0.0:
+        raise ValueError(f"{name} replaces the scalar noise: pass noise=0.0 with it")
+    if nu.size != n:
+        raise ValueError(f"{name} has {nu.size} values for {n} {what}")
+    return nu
+
+
 def prior_scale(family: int, params) -> float:
     """k(0,0): the magnitude against which 'numerically zero variance' is judged."""
     params = np.asarray(params, dtype=np.float64)
@@ -111,11 +123,12 @@ class _Pivoting:
             self.rec_all = None
             self.rec_win = self.rec
 
-    def _gather(self, W, ld, var, X: PointSet, noise: float, minimize: bool):
+    def _gather(self, W, ld, var, X: PointSet, noise: float, minimize: bool, nu=None):
+        """Local pivot record with rec[2] = var[p] + noise, or var[p] + nu[p] when a per-point noise vector is given."""
         dev = self.dev
-        check(lib.gpx_gather_pivot(dev.h, ptr(W), ld, self.n, ptr(var), ptr(X.X), X.ld, ptr(self.best), ptr(self.idx),
-                                   self.index_offset, ptr(getattr(self, "index_map", None)), noise, ptr(self.rec), dev.stream),
-              "gpx_gather_pivot")
+        check(lib.gpx_gather_pivot_nu(dev.h, ptr(W), ld, self.n, ptr(var), ptr(X.X), X.ld, ptr(self.best), ptr(self.idx),
+                                      self.index_offset, ptr(getattr(self, "index_map", None)), ptr(nu), noise, ptr(self.rec),
+                                      dev.stream), "gpx_gather_pivot_nu")
         if self.rec_all is not None:
             self.shard.all_gather(self.rec_all, self.rec)
             check(lib.gpx_select_pivot(dev.h, ptr(self.rec_all), self.shard.world, self.reclen, self.n,
@@ -532,14 +545,8 @@ class GreedyIVAREngine(_Pivoting):
         self.cand, self.mc = cand, mc
         self.resident = bool(resident)
         self.noise = float(noise)
-        self.cand_noise = None
-        if cand_noise is not None:
-            nu = np.asarray(cand_noise, dtype=np.float64).ravel()
-            if self.noise != 0.0:
-                raise ValueError("cand_noise replaces the scalar noise: pass noise=0.0 with it")
-            if nu.size != cand.n:
-                raise ValueError(f"cand_noise has {nu.size} values for {cand.n} candidates")
-            self.cand_noise = dev.upload(nu)
+        nu = _noise_vector("cand_noise", cand_noise, self.noise, cand.n, "candidates")
+        self.cand_noise = None if nu is None else dev.upload(nu)
         self.zero_tol = ZERO_VAR_TOL * float(zero_scale)
         ncap = max(int(n_max), 1)
         self._init_pivot(dev, ncap, n_max, shard, index_offset)
@@ -721,19 +728,25 @@ class GreedyMIEngine(_Pivoting):
     numerator = running posterior variance given A (nugget = noise); denominator from the diagonal of
     the precision of V minus A, kept current by lazy rank-1 downdates."""
 
-    def __init__(self, dev: Device, pool: PointSet, n_max: int, noise: float):
+    def __init__(self, dev: Device, pool: PointSet, n_max: int, noise: float, pool_noise=None):
+        """pool_noise: host vector nu of a per-point noise at the pool points (noise must be 0.0 then).  It replaces the
+        scalar noise in the three places the noise enters: the set-up factors K_VV + diag(nu), the append divides by
+        sqrt(num_p + nu_p), and the score's denominator is 1/pd_j - nu_j."""
         self.pool = pool
         self.noise = float(noise)
+        nu = _noise_vector("pool_noise", pool_noise, self.noise, pool.n, "pool points")
+        self.nu = None if nu is None else dev.upload(nu)
         ncap = max(int(n_max), 1)
         self._init_pivot(dev, ncap, n_max, None, 0)
         v, ld = pool.n, pool.ld
         self.W = dev.zeros(ncap, ld)          # numerator factor rows
         self.num = dev.zeros(ld)
         check(lib.gpx_prior_diag(dev.h, ptr(pool.X), v, ld, ptr(self.num), dev.stream), "gpx_prior_diag")
-        # set-up: K_VV + noise I = U^T U ; Y = U^-T ; pd = diag(P) = colsumsq(Y)
+        # set-up: K_VV + diag(noise) = U^T U ; Y = U^-T ; pd = diag(P) = colsumsq(Y)
         K = dev.zeros(v, ld)
         info = dev.zeros(1, dtype=torch.int32)
-        check(lib.gpx_gram(dev.h, ptr(pool.X), v, ld, ptr(pool.X), v, ld, ptr(K), ld, 1, None, self.noise, dev.stream), "gpx_gram")
+        check(lib.gpx_gram(dev.h, ptr(pool.X), v, ld, ptr(pool.X), v, ld, ptr(K), ld, 1, ptr(self.nu), self.noise, dev.stream),
+              "gpx_gram")
         self.cov = K.clone()
         check(lib.gpx_potrf(dev.h, ptr(K), v, ld, ptr(info), dev.stream), "gpx_potrf")
         self.U = K
@@ -757,7 +770,7 @@ class GreedyMIEngine(_Pivoting):
         """Move the point in self.idx from S = V minus A into A."""
         dev, pool = self.dev, self.pool
         v, ld = pool.n, pool.ld
-        self._gather(self.W, ld, self.num, pool, self.noise, minimize=False)
+        self._gather(self.W, ld, self.num, pool, self.noise, minimize=False, nu=self.nu)
         check(lib.gpx_append_row(dev.h, _lib.ROW_KERNEL, ptr(self.rec), None, ptr(pool.X), v, ld, ptr(self.W), ld, self.n,
                                  ptr(self.num), dev.stream), "gpx_append_row")
         check(lib.gpx_mi_prec_column(dev.h, ptr(self.Y), v, v, ld, 0, 0, 1, ptr(self.idx), None, ptr(self.pws), ptr(self.pcol),
@@ -776,8 +789,8 @@ class GreedyMIEngine(_Pivoting):
 
     def score(self):
         dev = self.dev
-        check(lib.gpx_score_mi(dev.h, ptr(self.num), ptr(self.pd), self.noise, ptr(self.mask), self.pool.n, ptr(self.scores),
-                               ptr(self.best), ptr(self.idx), dev.stream), "gpx_score_mi")
+        check(lib.gpx_score_mi_nu(dev.h, ptr(self.num), ptr(self.pd), ptr(self.nu), self.noise, ptr(self.mask), self.pool.n,
+                                  ptr(self.scores), ptr(self.best), ptr(self.idx), dev.stream), "gpx_score_mi_nu")
 
     def step(self):
         self.score()
@@ -816,7 +829,10 @@ class ShardedMIEngine(_Pivoting):
     # 2 GPUs, |V| = 80 000: 512 -> 5.81 s, 1024 -> 5.64 s (round 1, contiguous ranges, no zero skipping: 10.65 s)
     BLK = 1024
 
-    def __init__(self, dev: Device, pool_host: np.ndarray, n_max: int, noise: float, shard=None):
+    def __init__(self, dev: Device, pool_host: np.ndarray, n_max: int, noise: float, shard=None, pool_noise=None):
+        """pool_noise: host vector nu of a per-point noise at ALL |V| pool points (noise must be 0.0 then), as in
+        GreedyMIEngine.  Each rank keeps nu at its own columns; the owner of a pivot p sends num_p + nu_p to the other
+        ranks in the pivot record's divisor rec[2]."""
         import os
         self.BLK = int(os.environ.get("GPX_MI_BLK", self.BLK))
         if self.BLK < 256 or self.BLK & (self.BLK - 1):
@@ -830,6 +846,7 @@ class ShardedMIEngine(_Pivoting):
         self.world, self.rank = world, rank
         V = pool_host.shape[0]
         self.V = V
+        nu = _noise_vector("pool_noise", pool_noise, self.noise, V, "pool points")
         # keep a few elimination blocks per rank on small pools
         while self.BLK > 256 and (V + self.BLK - 1) // self.BLK < 4 * world:
             self.BLK //= 2
@@ -847,13 +864,15 @@ class ShardedMIEngine(_Pivoting):
         ld = self.pool.ld
         self.ld = ld
         self.index_map = dev.upload(self.gcols, dtype=torch.int64) if nloc else dev.zeros(1, dtype=torch.int64)
+        self.nu = dev.upload(nu[gcols]) if nu is not None and nloc else None   # nu at the local columns
         st = dev.stream
-        # ---- local columns of K_VV + noise I and of the identity (all V rows: only rows <= column are read)
+        # ---- local columns of K_VV + diag(noise) and of the identity (all V rows: only rows <= column are read)
         A = dev.zeros(V, ld)
         Y = dev.zeros(V, ld)
         if nloc > 0:
             check(lib.gpx_gram(dev.h, ptr(allpts.X), V, allpts.ld, ptr(self.pool.X), nloc, ld, ptr(A), ld, 0, None, 0.0, st), "gpx_gram")
-            check(lib.gpx_add_at_rows(dev.h, ptr(A), ld, ptr(self.index_map), nloc, self.noise, st), "gpx_add_at_rows")
+            check(lib.gpx_add_at_rows_vec(dev.h, ptr(A), ld, ptr(self.index_map), nloc, ptr(self.nu), self.noise, st),
+                  "gpx_add_at_rows_vec")
             check(lib.gpx_add_at_rows(dev.h, ptr(Y), ld, ptr(self.index_map), nloc, 1.0, st), "gpx_add_at_rows")
         del allpts
         panel = dev.zeros(V, B)
@@ -966,14 +985,14 @@ class ShardedMIEngine(_Pivoting):
             self.idx.fill_(-1)
             self.best.zero_()
             return
-        check(lib.gpx_score_mi(dev.h, ptr(self.num), ptr(self.pd), self.noise, ptr(self.mask), nloc, ptr(self.scores),
-                               ptr(self.best), ptr(self.idx), dev.stream), "gpx_score_mi")
+        check(lib.gpx_score_mi_nu(dev.h, ptr(self.num), ptr(self.pd), ptr(self.nu), self.noise, ptr(self.mask), nloc,
+                                  ptr(self.scores), ptr(self.best), ptr(self.idx), dev.stream), "gpx_score_mi_nu")
 
     def take(self):
         dev, pool, ld, V = self.dev, self.pool, self.ld, self.V
         nloc = self.nloc
         st = dev.stream
-        self._gather(self.W, ld, self.num, pool, self.noise, minimize=False)
+        self._gather(self.W, ld, self.num, pool, self.noise, minimize=False, nu=self.nu)
         check(lib.gpx_append_row(dev.h, _lib.ROW_KERNEL, ptr(self.rec_win), None, ptr(pool.X), nloc, ld, ptr(self.W), ld,
                                  self.n, ptr(self.num), st), "gpx_append_row")
         check(lib.gpx_local_index_cyclic(dev.h, ptr(self.rec_win), self.BLK, self.world, self.rank, nloc, ptr(self.loc2), st),

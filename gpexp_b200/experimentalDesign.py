@@ -15,6 +15,7 @@ wrappers, experimentalDesign.py:296-751) are deliberately not re-typed here: wit
 module, and its optimiser loops then drive the device path unchanged.
 """
 import copy
+import hashlib
 import itertools
 
 import numpy as np
@@ -80,14 +81,21 @@ def _ivar_derivative(self, inputPoints):
 
 
 # ---- costFunctionGP_MI ----------------------------------------------------------------------------------------------------
-def _mi_new_engine(self, n_max):
-    gp = self.gaussianProcess
-    noise = _nugget_arg(gp.noise)
+def _mi_noise(self):
+    """(scalar noise, per-point noise vector or None) of the cost function's GP: an ndarray gp.noise is the noise at
+    each pool point, checked to hold one finite value >= 0 per point."""
+    noise = _nugget_arg(self.gaussianProcess.noise)
     if isinstance(noise, np.ndarray):
-        raise NotImplementedError("MI with per-point noise is not supported on the device path")
+        return 0.0, _checked_noise(noise, len(self.mcPoints), "gp.noise has")
+    return float(noise), None
+
+
+def _mi_new_engine(self, n_max, shard=None):
+    gp = self.gaussianProcess
+    noise, nu = _mi_noise(self)
     # left-looking blocked set-up (measured faster than a right-looking dense engine on one GPU as well:
     # |V| = 40 000: 2.33 s vs 2.97 s)
-    return ShardedMIEngine(gp.kernel._bind(), self.mcPoints, n_max, float(noise))
+    return ShardedMIEngine(gp.kernel._bind(), self.mcPoints, n_max, noise, shard=shard, pool_noise=nu)
 
 
 def _mi_evaluate(self, index, indexAdded):
@@ -100,7 +108,9 @@ def _mi_evaluate(self, index, indexAdded):
     added = [int(i) for i in indexAdded]
     gp = self.gaussianProcess
     fam, _, params = gp.kernel._gpx_spec()
-    key = (fam, tuple(np.ravel(params)), float(_nugget_arg(gp.noise)), id(self.mcPoints), len(self.mcPoints))
+    noise, nu = _mi_noise(self)
+    noise_key = noise if nu is None else hashlib.sha256(nu.tobytes()).hexdigest()
+    key = (fam, tuple(np.ravel(params)), noise_key, id(self.mcPoints), len(self.mcPoints))
     st = self.__dict__.setdefault("_mi_cache", {})
     eng = st.get("engine")
     if eng is None or st.get("key") != key:
@@ -143,7 +153,11 @@ class costFunctionGP_IVAR(costFunctionBase):
 class costFunctionGP_MI(costFunctionBase):
     """Krause-Guestrin mutual-information ratio var(y|A) / var(y|V minus A minus y) over a candidate pool (:223-285).
     The GP passed in is used directly, not copied (:227); pool = mcpoints[nmc], a 10 x 10 grid (square=True, 2-D) or 200
-    samples of the space."""
+    samples of the space.
+
+    gp.noise is a scalar nugget or an ndarray nu with one finite value >= 0 per pool point (aligned with mcPoints): each
+    subset's Gram then takes diag(nu) on that subset, K_AA + diag nu_A and K_S'S' + diag nu_S'.  space.noiseFunc is not
+    used, as in the reference; a caller with a noise function passes gp.noise = noiseFunc(pool)."""
 
     def __init__(self, gaussianProcess, nInputs, space, nmc=None, mcpoints=None, square=False):
         costFunctionBase.__init__(self, nInputs, space)
@@ -180,16 +194,10 @@ class costFunctionGP_MI(costFunctionBase):
 def performGreedyMIExperimentalDesign(costFuncMI, nPoints, start=0, shard=None):
     """Greedy MI design over the cost function's pool (experimentalDesign.py:753-785).
     Returns the chosen POINTS (as the reference does); the indices are left in
-    `costFuncMI.lastIndices`.  With `shard` (gpexp_b200.engine.Shard, every rank passing the same pool) the
-    |V| x |V| factorisation is column-sharded over the ranks (ShardedMIEngine) -- required above |V| ~ 9e4."""
-    if shard is not None:
-        gp = costFuncMI.gaussianProcess
-        noise = _nugget_arg(gp.noise)
-        if isinstance(noise, np.ndarray):
-            raise NotImplementedError("MI with per-point noise is not supported on the device path")
-        eng = ShardedMIEngine(gp.kernel._bind(), costFuncMI.mcPoints, nPoints, float(noise), shard=shard)
-    else:
-        eng = _mi_new_engine(costFuncMI, nPoints)
+    `costFuncMI.lastIndices`.  With `shard` (gpexp_b200.engine.Shard, every rank passing the same pool and the same
+    gp.noise) the |V| x |V| factorisation is column-sharded over the ranks (ShardedMIEngine) -- required above |V| ~ 9e4.
+    A per-point gp.noise works as in costFunctionGP_MI.evaluate (one finite value >= 0 per pool point, else ValueError)."""
+    eng = _mi_new_engine(costFuncMI, nPoints, shard=shard)
     idx = eng.run(nPoints, start=start)
     costFuncMI.lastIndices = idx
     costFuncMI.lastEngine = eng
@@ -225,16 +233,22 @@ def performGreedyVarExperimentalDesign(kernel, mcPoints, nPoints, dimension, wei
     return mcPoints[indKeep, :]
 
 
+def _checked_noise(values, n, source):
+    """`values` as one float64 nugget per point for n points; `source` ("noise function returned", "gp.noise has") starts
+    the message of the ValueError raised unless there is exactly one finite value >= 0 per point."""
+    nu = np.asarray(values, dtype=np.float64).ravel()
+    if nu.size != n:
+        raise ValueError(f"{source} {nu.size} values for {n} points (one per point expected)")
+    if not np.all(np.isfinite(nu)):
+        raise ValueError(f"{source} a value that is not finite")
+    if np.any(nu < 0.0):
+        raise ValueError(f"{source} a negative value")
+    return nu
+
+
 def _noise_values(noiseFunc, points):
     """noiseFunc(points) as one float64 nugget per point; the noise function is user code, so its output is checked."""
-    nu = np.asarray(noiseFunc(points), dtype=np.float64).ravel()
-    if nu.size != points.shape[0]:
-        raise ValueError(f"noise function returned {nu.size} values for {points.shape[0]} points (one per point expected)")
-    if not np.all(np.isfinite(nu)):
-        raise ValueError("noise function returned a value that is not finite")
-    if np.any(nu < 0.0):
-        raise ValueError("noise function returned a negative value")
-    return nu
+    return _checked_noise(noiseFunc(points), points.shape[0], "noise function returned")
 
 
 def beginGreedyIVARExperimentalDesign(costFuncIVAR, candidates, nPoints, shard=None, resident=None):

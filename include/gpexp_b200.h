@@ -173,6 +173,10 @@ int gpx_dgemm_tn_sub_lower(gpx_handle h, const double* A, int64_t lda, const dou
 int gpx_gather_pivot(gpx_handle h, const double* W, int64_t ldw, int64_t n, const double* var, const double* X,
                      int64_t ldx, const double* score_dev, const int64_t* idx_dev, int64_t index_offset,
                      const int64_t* index_map, double noise, double* rec, void* stream);
+/* The same with a per-point noise: rec[2] = var[p] + (nu ? nu[p] : noise), nu indexed like var (by the local index). */
+int gpx_gather_pivot_nu(gpx_handle h, const double* W, int64_t ldw, int64_t n, const double* var, const double* X,
+                        int64_t ldx, const double* score_dev, const int64_t* idx_dev, int64_t index_offset,
+                        const int64_t* index_map, const double* nu, double noise, double* rec, void* stream);
 
 /* Pick the winning record among `nrec` records spaced `stride` doubles apart (NCCL all-gather output):
  * lowest score if minimize else highest, ties -> lowest global index (np.argmax / np.argmin order). */
@@ -257,6 +261,10 @@ int gpx_score_ivar_partials(gpx_handle h, const double* partial, int nseg, int64
  *     (experimentalDesign.py:259-285 restated: denominator = 1/[(K_SS+noise I)^-1]_yy - noise). */
 int gpx_score_mi(gpx_handle h, const double* num_var, const double* prec_diag, double noise, const uint8_t* mask,
                  int64_t n, double* score_out, double* best, int64_t* idx, void* stream);
+/* The same with a per-point noise: score = num_var[j] / (1/prec_diag[j] - (nu ? nu[j] : noise)), the denominator
+ *     1/[(K_SS + diag nu_S)^-1]_yy - nu_y. */
+int gpx_score_mi_nu(gpx_handle h, const double* num_var, const double* prec_diag, const double* nu, double noise,
+                    const uint8_t* mask, int64_t n, double* score_out, double* best, int64_t* idx, void* stream);
 
 /* K6  column p of P = Y^T Y for the lower-triangular Y = U^-T:  out[i] = sum_{k >= max(i,p)} Y[k,i] Y[k,p].
  *     Y is nrows x ncols (row-major): the whole matrix (col_offset = 0, ncols = nrows, ycol = NULL) or the column slice
@@ -282,6 +290,9 @@ int gpx_local_index_cyclic(gpx_handle h, const double* rec, int64_t blk, int64_t
                            int64_t* out2, void* stream);
 /* A[rows[j] * ld + j] += value, j < n (nugget / identity on the diagonal of a scattered column subset) */
 int gpx_add_at_rows(gpx_handle h, double* A, int64_t ld, const int64_t* rows, int64_t n, double value, void* stream);
+/* A[rows[j] * ld + j] += vals ? vals[j] : value (a per-point nugget on the scattered diagonal) */
+int gpx_add_at_rows_vec(gpx_handle h, double* A, int64_t ld, const int64_t* rows, int64_t n, const double* vals, double value,
+                        void* stream);
 
 /* Column sums of squares: out[j] = sum_{i<n} W[i,j]^2 (optionally out[j] = base[j] - that). */
 int gpx_colsumsq(gpx_handle h, const double* W, int64_t n, int64_t ncols, int64_t ldw, const double* base,

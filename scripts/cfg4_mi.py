@@ -1,7 +1,9 @@
 """BASELINE cfg-4: 3-D Mehler kernel, greedy mutual-information design of 512 points from |V| = 200 000 candidates,
 the |V| x |V| factor and its inverse-transpose sharded by column blocks over the ranks.
 
-    python -m torch.distributed.run --nproc-per-node 8 ... scripts/cfg4_mi.py [--V 200000] [--N 512] [--compare-dense]
+    python -m torch.distributed.run --nproc-per-node 8 ... scripts/cfg4_mi.py [--V 200000] [--N 512] [--compare-dense] [--nu]
+
+--nu replaces the scalar noise 1e-2 by the per-point noise nu(x) = 1e-2 (1 + |x|^2 / 3) at every pool point.
 """
 import argparse
 import json
@@ -20,6 +22,7 @@ ap = argparse.ArgumentParser()
 ap.add_argument("--V", type=int, default=200_000)
 ap.add_argument("--N", type=int, default=512)
 ap.add_argument("--compare-dense", action="store_true", help="rank 0 also runs the single-GPU dense engine (small V only)")
+ap.add_argument("--nu", action="store_true", help="per-point noise nu(x) = 1e-2 (1 + |x|^2 / 3) instead of the scalar 1e-2")
 args = ap.parse_args()
 
 world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -35,6 +38,7 @@ from gpexp_b200.engine import GreedyMIEngine, Shard, ShardedMIEngine  # noqa: E4
 
 V, N, noise = args.V, args.N, 1e-2
 pool = np.random.default_rng(4).standard_normal((V, 3))
+nu = 1e-2 * (1.0 + np.sum(pool * pool, axis=1) / 3.0) if args.nu else None
 dev = Device.get(local)
 kern = kernels.KernelMehlerND([0.9, 0.9, 0.9], 3)
 kern._bind(dev)
@@ -50,7 +54,7 @@ def sync():
 
 sync()
 t0 = time.perf_counter()
-eng = ShardedMIEngine(dev, pool, N, noise, shard=shard)
+eng = ShardedMIEngine(dev, pool, N, 0.0 if args.nu else noise, shard=shard, pool_noise=nu)
 sync()
 setup_s = time.perf_counter() - t0
 t0 = time.perf_counter()
@@ -60,7 +64,8 @@ design_s = time.perf_counter() - t0
 info = int(eng.info.item())
 scores = eng.pick_scores[:N].cpu().numpy()
 if rank == 0:
-    out = {"workload": "cfg-4: 3-D Mehler t=0.9, greedy MI design of %d points from |V|=%d, noise 1e-2" % (N, V),
+    out = {"workload": "cfg-4: 3-D Mehler t=0.9, greedy MI design of %d points from |V|=%d, noise %s"
+                       % (N, V, "1e-2 (1 + |x|^2 / 3)" if args.nu else "1e-2"),
            "n_gpus": world, "setup_s": setup_s, "setup_useful_tflops_total": (2.0 * V ** 3 / 3.0) / setup_s / 1e12,
            "setup_tflops_per_gpu": (2.0 * V ** 3 / 3.0 / world) / setup_s / 1e12,
            "design_s": design_s, "ms_per_step": 1e3 * design_s / (N - 1), "candidates_per_s_per_step": (N - 1) * V / design_s,
@@ -69,7 +74,7 @@ if rank == 0:
            "hbm_per_gpu_gb": 2 * 8.0 * V * max(eng.ncols_per_rank) / 1e9, "blk": eng.BLK,
            "distribution": "block-cyclic column blocks, structural zeros of Y skipped in-kernel"}
     if args.compare_dense:
-        dense = GreedyMIEngine(dev, dev.points(pool), N, noise)
+        dense = GreedyMIEngine(dev, dev.points(pool), N, 0.0 if args.nu else noise, pool_noise=nu)
         didx = dense.run(N, start=0)
         out["indices_equal_dense_single_gpu_engine"] = [int(i) for i in didx] == [int(i) for i in idx]
     print(json.dumps(out), flush=True)

@@ -1,6 +1,6 @@
 """Multi-GPU parity check (run under torch.distributed.run, one rank per GPU):
-sharded greedy IVAR (scalar noise and a heteroscedastic noise function) and greedy max-variance must pick exactly the
-indices of the single-process CPU oracle."""
+sharded greedy IVAR (scalar noise and a heteroscedastic noise function), greedy max-variance and greedy MI (scalar and
+per-point noise) must pick exactly the indices of the single-process CPU oracle."""
 import os
 import sys
 
@@ -51,14 +51,28 @@ def main():
     meng = ShardedMIEngine(dev, vpool, 14, 1e-2, shard=shard)
     midx = meng.run(14, start=0)
     minfo = int(meng.info.item())
+    # --- the same with a per-point noise (public API): each rank keeps nu at its own columns, nu(p) travels in rec[2] ----
+    vnu = 1e-2 * (1.0 + np.sum(vpool * vpool, axis=1) / 3.0)
+    cfm = ed.costFunctionGP_MI(gp.GP(hk, vnu), 14, Space(3, None, None), nmc=len(vpool), mcpoints=vpool)
+    ed.performGreedyMIExperimentalDesign(cfm, 14, start=0, shard=shard)
+    hmidx, hminfo = [int(i) for i in cfm.lastIndices], int(cfm.lastEngine.info.item())
     torch.cuda.synchronize()
     if rank == 0:
         from oracle import gpexp_oracle as orc
+        from tests.hetero_mi_oracle import fast_greedy_mi_nu
         mref, _ = orc.fast_greedy_mi(orc.KernelSpec.mehler([0.9, 0.9, 0.9], 3), vpool, 1e-2, 14, start=0)
         mi_ok = [int(i) for i in midx] == mref and minfo == 0
         print("multigpu_check world=%d mi=%s -> %s" % (world, [int(i) for i in midx][:8], "OK" if mi_ok else "MISMATCH"), flush=True)
         if not mi_ok:
             print("ref mi", mref, "got", [int(i) for i in midx], "info", minfo)
+        hmref, _, _ = fast_greedy_mi_nu(orc.KernelSpec.mehler([0.9, 0.9, 0.9], 3), vpool, vnu, 14, start=0)
+        ed.performGreedyMIExperimentalDesign(cfm, 14, start=0)   # the same design on this GPU alone
+        hm_one = [int(i) for i in cfm.lastIndices]
+        hm_ok = hmidx == hmref == hm_one and hminfo == 0
+        print("multigpu_check world=%d hetero mi=%s -> %s" % (world, hmidx[:8], "OK" if hm_ok else "MISMATCH"), flush=True)
+        if not hm_ok:
+            print("ref hetero mi", hmref, "got", hmidx, "one gpu", hm_one, "info", hminfo)
+        mi_ok = mi_ok and hm_ok
         ref, _ = orc.fast_greedy_ivar(orc.KernelSpec.se([0.2, 0.3], 1.0, 2), cand, mc, 12, 1e-6)
         vref, _ = orc.fast_greedy_var(orc.KernelSpec.matern32(1.0, 1.0, 5), pool, 25)
         from tests.hetero_oracle import fast_greedy_ivar_nu
@@ -74,7 +88,7 @@ def main():
         if not ok:
             print("ref ivar", ref, "got", [int(i) for i in idx]); print("ref var", vref, "got", [int(i) for i in vidx])
     # every rank must hold the same picks
-    t = torch.tensor([int(i) for i in idx] + [int(i) for i in hidx] + [int(i) for i in vidx] + [int(i) for i in midx],
+    t = torch.tensor([int(i) for i in idx] + [int(i) for i in hidx] + [int(i) for i in vidx] + [int(i) for i in midx] + hmidx,
                      device="cuda")
     g = [torch.zeros_like(t) for _ in range(world)]
     dist.all_gather(g, t)
