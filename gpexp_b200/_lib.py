@@ -50,7 +50,7 @@ class IvarState(C.Structure):
                 ("workspace", _p), ("scores", _p), ("best", _p), ("idx", _p),
                 ("rec", _p), ("rec_all", _p), ("rec_win", _p),
                 ("U", _p), ("ldu", _i64), ("picks", _p), ("pick_scores", _p), ("pick_pivots", _p),
-                ("cov", _p), ("ldcov", _i64), ("ldp", _i64)]
+                ("cov", _p), ("ldcov", _i64), ("ldp", _i64), ("wM", _p)]
 
 
 class VarState(C.Structure):
@@ -88,16 +88,21 @@ SIGNATURES = {
     "gpx_append_row": [_p, _int, _p, _p, _p, _i64, _i64, _p, _i64, _i64, _p, _p],
     "gpx_argreduce": [_p, _p, _p, _p, _i64, _int, _p, _p, _p],
     "gpx_sum": [_p, _p, _i64, _p, _p],
+    "gpx_sum_w": [_p, _p, _p, _i64, _p, _p],
     "gpx_set_ivar_ring": [_p, _int],
     "gpx_set_ivar_core": [_p, _int],
     "gpx_ivar_scratch_bytes": [_p, _i64, _i64, _i64],
     "gpx_set_ivar_scratch": [_p, _p, _i64],
     "gpx_score_ivar_workspace": [_p, _i64, _i64],
     "gpx_score_ivar": [_p, _int, _p, _i64, _p, _p, _i64, _p, _i64, _p, _p, _i64, _i64, _dbl, _dbl, _p, _p, _p, _p, _p, _p],
+    "gpx_score_ivar_w": [_p, _int, _p, _i64, _p, _p, _i64, _p, _i64, _p, _p, _i64, _i64, _dbl, _dbl, _p, _p, _p, _p, _p, _p,
+                         _p],
     "gpx_cov_segments": [_i64, _i64],
     "gpx_cov_update": [_p, _p, _i64, _i64, _i64, _p, _p, _p, _i64, _p],
+    "gpx_cov_update_w": [_p, _p, _i64, _i64, _i64, _p, _p, _p, _p, _i64, _p],
     "gpx_cov_from_factors": [_p, _int, _p, _i64, _p, _i64, _p, _i64, _p, _i64, _i64, _p, _i64, _p],
     "gpx_score_ivar_partials": [_p, _p, _int, _i64, _p, _i64, _p, _i64, _dbl, _dbl, _p, _p, _p, _p, _p],
+    "gpx_score_ivar_partials_w": [_p, _p, _int, _i64, _p, _i64, _p, _i64, _dbl, _dbl, _p, _p, _p, _p, _p, _p],
     "gpx_score_mi": [_p, _p, _p, _dbl, _p, _i64, _p, _p, _p, _p],
     "gpx_score_mi_nu": [_p, _p, _p, _p, _dbl, _p, _i64, _p, _p, _p, _p],
     "gpx_mi_prec_column_workspace": [_i64, _i64],
@@ -134,6 +139,7 @@ SIGNATURES = {
     "gpx_axpby": [_p, _i64, _dbl, _p, _dbl, _p, _p],
     "gpx_coldot": [_p, _p, _p, _i64, _i64, _i64, _p, _p, _p],
     "gpx_rowsum": [_p, _p, _i64, _i64, _i64, _dbl, _p, _p],
+    "gpx_rowsum_w": [_p, _p, _i64, _i64, _i64, _p, _p, _p],
     "gpx_logdet_chol": [_p, _p, _i64, _i64, _p, _p],
     "gpx_bench_dmma": [_p, _i64, _p, _p],
     "gpx_bench_dfma": [_p, _i64, _p, _p],

@@ -343,12 +343,17 @@ __device__ __forceinline__ double gpx_block_sum(double s, double* sm) {
     return t;  // valid in warp 0
 }
 
-__global__ void __launch_bounds__(256) sum_kernel(const double* __restrict__ v, int64_t n, double* red_val,
-                                                   unsigned int* counter, double* out) {
+// WT: out = sum_j w[j] v[j] in the same tree (one fma per term in place of the add)
+template <bool WT>
+__global__ void __launch_bounds__(256) sum_kernel(const double* __restrict__ v, const double* __restrict__ w, int64_t n,
+                                                   double* red_val, unsigned int* counter, double* out) {
     __shared__ double sm[8];
     __shared__ bool last;
     double s = 0.0;
-    for (int64_t j = (int64_t)blockIdx.x * 256 + threadIdx.x; j < n; j += (int64_t)gridDim.x * 256) s += v[j];
+    for (int64_t j = (int64_t)blockIdx.x * 256 + threadIdx.x; j < n; j += (int64_t)gridDim.x * 256) {
+        if (WT) s = fma(w[j], v[j], s);
+        else s += v[j];
+    }
     s = gpx_block_sum(s, sm);
     if (threadIdx.x == 0) {
         red_val[blockIdx.x] = s;
@@ -367,18 +372,24 @@ __global__ void __launch_bounds__(256) sum_kernel(const double* __restrict__ v, 
     }
 }
 
-int gpx_sum_impl(gpx_handle h, const double* v, int64_t n, double* out, cudaStream_t st) {
+int gpx_sum_impl(gpx_handle h, const double* v, const double* w, int64_t n, double* out, cudaStream_t st) {
     int64_t blocks = (n + 4095) / 4096;
     if (blocks < 1) blocks = 1;
     if (blocks > 1024) blocks = 1024;
     // slots [1024, 2048) of the scratch and ticket 1, so that a sum can sit next to an arg-reduce
-    sum_kernel<<<(unsigned)blocks, 256, 0, st>>>(v, n, h->red_val + 1024, h->red_counter + 1, out);
+    if (w) sum_kernel<true><<<(unsigned)blocks, 256, 0, st>>>(v, w, n, h->red_val + 1024, h->red_counter + 1, out);
+    else sum_kernel<false><<<(unsigned)blocks, 256, 0, st>>>(v, w, n, h->red_val + 1024, h->red_counter + 1, out);
     return gpx_check_launch("gpx_sum");
 }
 
 extern "C" int gpx_sum(gpx_handle h, const double* v, int64_t n, double* out, void* stream) {
     GPX_REQUIRE(h != nullptr && out && n >= 0 && (v || n == 0), GPX_EINVAL, "bad arguments");
-    return gpx_sum_impl(h, v, n, out, (cudaStream_t)stream);
+    return gpx_sum_impl(h, v, nullptr, n, out, (cudaStream_t)stream);
+}
+
+extern "C" int gpx_sum_w(gpx_handle h, const double* v, const double* w, int64_t n, double* out, void* stream) {
+    GPX_REQUIRE(h != nullptr && out && n >= 0 && (v || n == 0), GPX_EINVAL, "bad arguments");
+    return gpx_sum_impl(h, v, w, n, out, (cudaStream_t)stream);
 }
 
 // ---------------------------------------------------------------------------------------------
@@ -854,12 +865,15 @@ extern "C" int gpx_add_at_rows_vec(gpx_handle h, double* A, int64_t ld, const in
 //     cov -= a b^T   (a = the new row of W_M, b = the new row of W_C)  while accumulating  r[c] = sum_m cov[m,c]^2
 // in the same pass: 16 bytes of HBM traffic per (m,c) pair and step, independent of the design size n.
 // Block = 512 columns (16-byte accesses) x one row segment; per-segment partial sums are added in a fixed order.
+// WT: weighted integration points, r[c] = sum_m fma(wM[m] cov[m,c], cov[m,c], r) (w = 2^-k scales r exactly).
 // ---------------------------------------------------------------------------------------------
 #define COV_MAX_SEG 160
 
+template <bool WT>
 __global__ void __launch_bounds__(256) cov_update_kernel(double* __restrict__ cov, int64_t ldc, int64_t M, int64_t C,
                                                           const double* __restrict__ a, const double* __restrict__ b,
-                                                          int64_t rows_per_seg, double* __restrict__ part, int64_t ldp) {
+                                                          const double* __restrict__ wM, int64_t rows_per_seg,
+                                                          double* __restrict__ part, int64_t ldp) {
     const int64_t c = ((int64_t)blockIdx.x * 256 + threadIdx.x) * 2;
     if (c >= C) return;
     const int64_t m0 = (int64_t)blockIdx.y * rows_per_seg;
@@ -890,8 +904,14 @@ __global__ void __launch_bounds__(256) cov_update_kernel(double* __restrict__ co
         }
 #pragma unroll
         for (int u = 0; u < 8; ++u) {
-            r0 = fma(v[u].x, v[u].x, r0);
-            r1 = fma(v[u].y, v[u].y, r1);
+            if (WT) {
+                const double wm = __ldg(wM + m + u);
+                r0 = fma(wm * v[u].x, v[u].x, r0);
+                r1 = fma(wm * v[u].y, v[u].y, r1);
+            } else {
+                r0 = fma(v[u].x, v[u].x, r0);
+                r1 = fma(v[u].y, v[u].y, r1);
+            }
         }
         p += 8 * ldc;
     }
@@ -903,8 +923,14 @@ __global__ void __launch_bounds__(256) cov_update_kernel(double* __restrict__ co
             v.y = fma(-am, b1, v.y);
             __stcs(reinterpret_cast<double2*>(p), v);
         }
-        r0 = fma(v.x, v.x, r0);
-        r1 = fma(v.y, v.y, r1);
+        if (WT) {
+            const double wm = __ldg(wM + m);
+            r0 = fma(wm * v.x, v.x, r0);
+            r1 = fma(wm * v.y, v.y, r1);
+        } else {
+            r0 = fma(v.x, v.x, r0);
+            r1 = fma(v.y, v.y, r1);
+        }
         p += ldc;
     }
     double* dst = part + (int64_t)blockIdx.y * ldp + c;
@@ -927,8 +953,8 @@ extern "C" int gpx_cov_segments(int64_t M, int64_t C) {
     return (int)s;
 }
 
-extern "C" int gpx_cov_update(gpx_handle h, double* cov, int64_t ldc, int64_t M, int64_t C, const double* a, const double* b,
-                              double* partial, int64_t ldp, void* stream) {
+extern "C" int gpx_cov_update_w(gpx_handle h, double* cov, int64_t ldc, int64_t M, int64_t C, const double* a, const double* b,
+                                const double* wM, double* partial, int64_t ldp, void* stream) {
     GPX_REQUIRE(h && cov && partial && M >= 1 && C >= 1, GPX_EINVAL, "bad arguments");
     GPX_REQUIRE((a == nullptr) == (b == nullptr), GPX_EINVAL, "a and b must both be given or both be NULL");
     GPX_REQUIRE((ldc % 2) == 0 && ldc >= C + (C & 1) && gpx_aligned16(cov), GPX_EALIGN,
@@ -938,6 +964,12 @@ extern "C" int gpx_cov_update(gpx_handle h, double* cov, int64_t ldc, int64_t M,
     const int seg = gpx_cov_segments(M, C);
     const int64_t rows = (M + seg - 1) / seg;
     dim3 grid((unsigned)((C + 511) / 512), (unsigned)seg);
-    cov_update_kernel<<<grid, 256, 0, (cudaStream_t)stream>>>(cov, ldc, M, C, a, b, rows, partial, ldp);
+    if (wM) cov_update_kernel<true><<<grid, 256, 0, (cudaStream_t)stream>>>(cov, ldc, M, C, a, b, wM, rows, partial, ldp);
+    else cov_update_kernel<false><<<grid, 256, 0, (cudaStream_t)stream>>>(cov, ldc, M, C, a, b, wM, rows, partial, ldp);
     return gpx_check_launch("gpx_cov_update");
+}
+
+extern "C" int gpx_cov_update(gpx_handle h, double* cov, int64_t ldc, int64_t M, int64_t C, const double* a, const double* b,
+                              double* partial, int64_t ldp, void* stream) {
+    return gpx_cov_update_w(h, cov, ldc, M, C, a, b, nullptr, partial, ldp, stream);
 }

@@ -340,12 +340,12 @@ __device__ __forceinline__ void gpx_warp_argreduce(double& v, int64_t& i, bool m
 
 // internal launchers shared between translation units
 int gpx_launch_core_ivar(gpx_handle h, int prologue, const double* Wm, int64_t ldm, const double* Ma_rows, int64_t M,
-                         const double* Wc, int64_t ldc, const double* Cb_rows, int64_t C, int64_t n, double* partial,
-                         int64_t ldp, int* nsplit_out, cudaStream_t st);
+                         const double* Wc, int64_t ldc, const double* Cb_rows, int64_t C, int64_t n, const double* wM,
+                         double* partial, int64_t ldp, int* nsplit_out, cudaStream_t st);
 int gpx_launch_core_store(gpx_handle h, int prologue, const double* A, int64_t lda, const double* Ap, int64_t I,
                           const double* B, int64_t ldb, const double* Bp, int64_t J, int64_t K, double* out, int64_t ldo,
                           cudaStream_t st);
 int gpx_ivar_splits(gpx_handle h, int64_t M, int64_t C);
 int gpx_argreduce_impl(gpx_handle h, const double* v, const double* weights, const uint8_t* mask, int64_t n,
                        int minimize, double* best, int64_t* idx, cudaStream_t st);
-int gpx_sum_impl(gpx_handle h, const double* v, int64_t n, double* out, cudaStream_t st);
+int gpx_sum_impl(gpx_handle h, const double* v, const double* w, int64_t n, double* out, cudaStream_t st);

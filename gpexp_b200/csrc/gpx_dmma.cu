@@ -5,6 +5,7 @@
 // with an optional *prologue* that evaluates the covariance k(x_i, y_j) inside the same kernel, and three epilogues:
 //
 //   EPI_IVAR   r[j] += sum_i (k(i,j) - T[i,j])^2          K5: IVAR scoring, experimentalDesign.py:105-117 restated
+//              (weighted integration points, template flag WT: r[j] += sum_i fma(w_i v, v, .) with v = k - T)
 //   EPI_STORE  out[i,j] = k(i,j) - T[i,j]                  K1+K3: block row of the left-looking TRSM
 //   EPI_SUB    C[i,j]  -= T[i,j]                           K2: Cholesky trailing update / materialised TRSM / MI set-up
 //
@@ -92,6 +93,7 @@ struct CoreArgs {
     // (local column j = block j / tri_blk of this rank = global block (j / tri_blk) * tri_world + tri_rank): rows above the
     // first global column of a tile are structurally zero and are skipped.  tri_blk = 0: dense operand.
     int tri_blk, tri_world, tri_rank;
+    const double* wM;  // IVAR kernels instantiated with WT: one weight per integration point (row i), length I
 };
 
 __device__ __forceinline__ void cp_async16(double* dst, const double* src, bool ok) {
@@ -177,31 +179,37 @@ __device__ __forceinline__ void diff_prologue(double (&acc)[4][8][2], const KPar
 }
 
 // squares of the warp's accumulator block summed over its 32 rows: butterfly reduce-scatter over the 8 lanes that
-// share q4; lane g4 ends up owning columns u = g4, e = 0, 1
+// share q4; lane g4 ends up owning columns u = g4, e = 0, 1.  WT: row i's square is weighted, fma(wM[i] v, v, .); the
+// lane's 4 rows of the tile take one weight load each.
+template <bool WT>
 __device__ __forceinline__ void column_squares(const double (&acc)[4][8][2], bool full, int64_t i_first, int64_t I, int lane,
-                                               double (&rs)[2]) {
+                                               const double* __restrict__ wM, double (&rs)[2]) {
     const int g4 = lane >> 2;
     double p[8][2];
 #pragma unroll
     for (int u = 0; u < 8; ++u) p[u][0] = p[u][1] = 0.0;
     if (full) {  // every row of the tile is a real integration point: no masking
 #pragma unroll
-        for (int t = 0; t < 4; ++t)
+        for (int t = 0; t < 4; ++t) {
+            const double w = WT ? __ldg(wM + i_first + (t >> 1) * 16 + g4 * 2 + (t & 1)) : 1.0;
 #pragma unroll
             for (int u = 0; u < 8; ++u)
 #pragma unroll
-                for (int e = 0; e < 2; ++e) p[u][e] = fma(acc[t][u][e], acc[t][u][e], p[u][e]);
+                for (int e = 0; e < 2; ++e)
+                    p[u][e] = fma(WT ? w * acc[t][u][e] : acc[t][u][e], acc[t][u][e], p[u][e]);
+        }
     } else {
 #pragma unroll
         for (int t = 0; t < 4; ++t) {
             const int64_t i = i_first + (t >> 1) * 16 + g4 * 2 + (t & 1);
             const bool ok = i < I;
+            const double w = WT ? (ok ? __ldg(wM + i) : 0.0) : 1.0;
 #pragma unroll
             for (int u = 0; u < 8; ++u)
 #pragma unroll
                 for (int e = 0; e < 2; ++e) {
                     const double v = ok ? acc[t][u][e] : 0.0;
-                    p[u][e] = fma(v, v, p[u][e]);
+                    p[u][e] = fma(WT ? w * v : v, v, p[u][e]);
                 }
         }
     }
@@ -231,7 +239,7 @@ __device__ __forceinline__ void column_squares(const double (&acc)[4][8][2], boo
     }
 }
 
-template <int FAM, int EPI, int PRO>
+template <int FAM, int EPI, int PRO, bool WT = false>
 __global__ void __launch_bounds__(Cfg::NT, 2)
     dmma_core_kernel(const __grid_constant__ CoreArgs a, const __grid_constant__ KParams kp) {
     using C = Cfg;
@@ -401,7 +409,7 @@ __global__ void __launch_bounds__(Cfg::NT, 2)
         if (ch == T - 1) {
             // ---- tile epilogue ---------------------------------------------------------------------
             if (EPI == EPI_IVAR) {
-                column_squares(acc, i0 + BM <= a.I, i0 + wm * 32, a.I, lane, rs);
+                column_squares<WT>(acc, i0 + BM <= a.I, i0 + wm * 32, a.I, lane, a.wM, rs);
             } else {
 #pragma unroll
                 for (int t = 0; t < 4; ++t) {
@@ -566,7 +574,7 @@ __device__ __forceinline__ void load_frags_ws(double (&af)[4], double (&bf)[8], 
     }
 }
 
-template <int FAM, int PRO, class RING, bool TMAP>
+template <int FAM, int PRO, class RING, bool TMAP, bool WT>
 __global__ void __launch_bounds__(256, 1) ivar_ws_kernel(const __grid_constant__ CoreArgs a, const __grid_constant__ KParams kp,
                                                          const __grid_constant__ TmaMaps maps) {
     constexpr int BM = WS_BM, LD = WS_LD, NW = 8;
@@ -741,7 +749,7 @@ __global__ void __launch_bounds__(256, 1) ivar_ws_kernel(const __grid_constant__
             if (lane == 0) mbar_arrive(empty + s);
 
             if (ch == T - 1) {
-                column_squares(acc, i0 + BM <= a.I, i0 + wm * 32, a.I, lane, rs);
+                column_squares<WT>(acc, i0 + BM <= a.I, i0 + wm * 32, a.I, lane, a.wM, rs);
                 ch = 0;
                 ++tl;
             } else {
@@ -946,7 +954,7 @@ int make_map(CUtensorMap* m, const double* base, int64_t ld, int64_t rows, int b
     return GPX_OK;
 }
 
-template <int FAM, int PRO, class RING, bool TMAP>
+template <int FAM, int PRO, class RING, bool TMAP, bool WT>
 int launch_ivar_ws_ring(gpx_handle h, const CoreArgs& a, dim3 grid, cudaStream_t st) {
     TmaMaps maps;
     memset(&maps, 0, sizeof(maps));
@@ -960,28 +968,28 @@ int launch_ivar_ws_ring(gpx_handle h, const CoreArgs& a, dim3 grid, cudaStream_t
         if ((rc = make_map(&maps.a_pro, a.Ap, a.lda, a.prows, a.prows))) return rc;
         if ((rc = make_map(&maps.b_pro, a.Bp, a.ldb, a.prows, a.prows))) return rc;
     }
-    rc = gpx_ensure_smem(h, (const void*)ivar_ws_kernel<FAM, PRO, RING, TMAP>, RING::SMEM_BYTES, "ivar_ws");
+    rc = gpx_ensure_smem(h, (const void*)ivar_ws_kernel<FAM, PRO, RING, TMAP, WT>, RING::SMEM_BYTES, "ivar_ws");
     if (rc) return rc;
-    ivar_ws_kernel<FAM, PRO, RING, TMAP><<<grid, 256, RING::SMEM_BYTES, st>>>(a, h->kp, maps);
+    ivar_ws_kernel<FAM, PRO, RING, TMAP, WT><<<grid, 256, RING::SMEM_BYTES, st>>>(a, h->kp, maps);
     return gpx_check_launch("ivar_ws");
 }
 
-template <int FAM, int PRO>
+template <int FAM, int PRO, bool WT>
 int launch_ivar_ws(gpx_handle h, const CoreArgs& a, dim3 grid, cudaStream_t st) {
     // every prologue fits one chunk of every ring (EXPANDED <= 16 rows, DIFF <= 16 coordinates, chunks >= 24 rows)
     switch (h->ivar_ring) {
-        case 1: return launch_ivar_ws_ring<FAM, PRO, RingSync, true>(h, a, grid, st);
-        case 2: return launch_ivar_ws_ring<FAM, PRO, RingDeep, true>(h, a, grid, st);
-        default: return launch_ivar_ws_ring<FAM, PRO, RingSync, false>(h, a, grid, st);
+        case 1: return launch_ivar_ws_ring<FAM, PRO, RingSync, true, WT>(h, a, grid, st);
+        case 2: return launch_ivar_ws_ring<FAM, PRO, RingDeep, true, WT>(h, a, grid, st);
+        default: return launch_ivar_ws_ring<FAM, PRO, RingSync, false, WT>(h, a, grid, st);
     }
 }
 
-template <int FAM, int EPI, int PRO>
+template <int FAM, int EPI, int PRO, bool WT = false>
 int launch_core(gpx_handle h, const CoreArgs& a, int64_t jt, int64_t it_or_splits, cudaStream_t st) {
     dim3 grid((unsigned)jt, (unsigned)it_or_splits);
-    int rc = gpx_ensure_smem(h, (const void*)dmma_core_kernel<FAM, EPI, PRO>, Cfg::SMEM_BYTES, "dmma core");
+    int rc = gpx_ensure_smem(h, (const void*)dmma_core_kernel<FAM, EPI, PRO, WT>, Cfg::SMEM_BYTES, "dmma core");
     if (rc) return rc;
-    dmma_core_kernel<FAM, EPI, PRO><<<grid, Cfg::NT, Cfg::SMEM_BYTES, st>>>(a, h->kp);
+    dmma_core_kernel<FAM, EPI, PRO, WT><<<grid, Cfg::NT, Cfg::SMEM_BYTES, st>>>(a, h->kp);
     return gpx_check_launch("dmma core");
 }
 
@@ -1075,6 +1083,7 @@ struct I8Args {
     int K;
     int np;            // prologue rows read: EXPANDED d + 2, DIFF d
     int tiles_per_cta, group_w, splits;
+    const double* wM;  // WT: one weight per integration point
 };
 
 __device__ __forceinline__ void tma_load_3d(void* dst, const CUtensorMap* tm, int c0, int c1, int c2, uint64_t* bar) {
@@ -1138,7 +1147,7 @@ __device__ __forceinline__ double i64_to_f64(int64_t v) {
     return __longlong_as_double(0x4338000000000000LL + v) - 6755399441055744.0;
 }
 
-template <int FAM, int PRO>
+template <int FAM, int PRO, bool WT>
 __global__ void __launch_bounds__(I8_THREADS, 1) ivar_i8_kernel(const __grid_constant__ I8Args a, const __grid_constant__ KParams kp,
                                                                 const __grid_constant__ I8Maps maps) {
     extern __shared__ __align__(128) unsigned char smem_raw[];
@@ -1261,6 +1270,7 @@ __global__ void __launch_bounds__(I8_THREADS, 1) ivar_i8_kernel(const __grid_con
             for (int j = 0; j < I8_EPI_COLS; ++j)
                 nk[j] = PRO == PRO_EXPANDED ? neg_kexpand_tab<FAM>(nk[j], kp, s_tab) : kfinish_tab<FAM>(nk[j], kp, s_tab);
             const double fm = mok ? a.fa[m] : 0.0;
+            const double wm = WT ? (mok ? a.wM[m] : 0.0) : 1.0;  // the thread's row m carries one weight per tile
             mbar_wait(acc_full, (unsigned)tl & 1u);
             tc_fence_after();
 #pragma unroll
@@ -1282,7 +1292,7 @@ __global__ void __launch_bounds__(I8_THREADS, 1) ivar_i8_kernel(const __grid_con
                     // S - k with S = (D_0..3 2^24 + D_4..6) (fm fb): the scale product inside one fma with -k
                     const double R = fma(i64_to_f64(hi), 0x1p24, i64_to_f64(lo));
                     const double v = mok ? __fma_rn(R, __dmul_rn(fm, s_fb[c00 + cb + j]), nk[cb + j]) : 0.0;
-                    p[cb + j] = fma(v, v, p[cb + j]);
+                    p[cb + j] = fma(WT ? wm * v : v, v, p[cb + j]);
                 }
             }
         }
@@ -1425,8 +1435,8 @@ int gpx_ivar_splits(gpx_handle, int64_t, int64_t) { return 32; }  // workspace b
 // INT8 core: slice both factors into the handle's scratch, then one ivar_i8_kernel launch (same workspace contract as
 // ivar_ws_kernel: partial column sums per M-split)
 static int launch_ivar_i8(gpx_handle h, int prologue, const double* Wm, int64_t ldm, const double* Ma_rows, int64_t M,
-                          const double* Wc, int64_t ldc, const double* Cb_rows, int64_t C, int64_t n, double* partial,
-                          int64_t ldp, int* nsplit_out, cudaStream_t st) {
+                          const double* Wc, int64_t ldc, const double* Cb_rows, int64_t C, int64_t n, const double* wM,
+                          double* partial, int64_t ldp, int* nsplit_out, cudaStream_t st) {
     int64_t ldk, sm, sc;
     i8_layout(M, C, n, &ldk, &sm, &sc);
     int8_t* Sm = reinterpret_cast<int8_t*>(((uintptr_t)h->i8_scratch + 127) & ~(uintptr_t)127);
@@ -1461,25 +1471,28 @@ static int launch_ivar_i8(gpx_handle h, int prologue, const double* Wm, int64_t 
     a.tiles_per_cta = (int)((itl + splits - 1) / splits);
     a.group_w = h->sm_count > 0 ? h->sm_count : 148;
     a.splits = splits;
+    a.wM = wM;
     *nsplit_out = splits;
     const dim3 grid((unsigned)(jt * splits), 1u);
-#define GPX_I8_LAUNCH(F, P)                                                                                        \
+#define GPX_I8_LAUNCH(F, P, W)                                                                                     \
     do {                                                                                                           \
-        if ((rc = gpx_ensure_smem(h, (const void*)ivar_i8_kernel<F, P>, I8_SMEM_BYTES, "ivar_i8"))) return rc;    \
-        ivar_i8_kernel<F, P><<<grid, I8_THREADS, I8_SMEM_BYTES, st>>>(a, h->kp, maps);                            \
+        if ((rc = gpx_ensure_smem(h, (const void*)ivar_i8_kernel<F, P, W>, I8_SMEM_BYTES, "ivar_i8"))) return rc; \
+        ivar_i8_kernel<F, P, W><<<grid, I8_THREADS, I8_SMEM_BYTES, st>>>(a, h->kp, maps);                         \
     } while (0)
     if (prologue == PRO_DIFF) {
-        GPX_DISPATCH_FAMILY(h->kp.family, GPX_I8_LAUNCH(FAM, PRO_DIFF));
+        if (wM) GPX_DISPATCH_FAMILY(h->kp.family, GPX_I8_LAUNCH(FAM, PRO_DIFF, true));
+        else GPX_DISPATCH_FAMILY(h->kp.family, GPX_I8_LAUNCH(FAM, PRO_DIFF, false));
     } else {
-        GPX_DISPATCH_FAMILY(h->kp.family, GPX_I8_LAUNCH(FAM, PRO_EXPANDED));
+        if (wM) GPX_DISPATCH_FAMILY(h->kp.family, GPX_I8_LAUNCH(FAM, PRO_EXPANDED, true));
+        else GPX_DISPATCH_FAMILY(h->kp.family, GPX_I8_LAUNCH(FAM, PRO_EXPANDED, false));
     }
 #undef GPX_I8_LAUNCH
     return gpx_check_launch("ivar_i8");
 }
 
 int gpx_launch_core_ivar(gpx_handle h, int prologue, const double* Wm, int64_t ldm, const double* Ma_rows, int64_t M,
-                         const double* Wc, int64_t ldc, const double* Cb_rows, int64_t C, int64_t n, double* partial,
-                         int64_t ldp, int* nsplit_out, cudaStream_t st) {
+                         const double* Wc, int64_t ldc, const double* Cb_rows, int64_t C, int64_t n, const double* wM,
+                         double* partial, int64_t ldp, int* nsplit_out, cudaStream_t st) {
     int rc;
     const int prows = prologue_rows(h, prologue);
     GPX_REQUIRE(prows >= 0, GPX_ESIZE, "prologue must be GPX_PRO_DIFF, or GPX_PRO_EXPANDED with d <= GPX_KROWS - 2");
@@ -1496,7 +1509,7 @@ int gpx_launch_core_ivar(gpx_handle h, int prologue, const double* Wm, int64_t l
     if (tma && h->ivar_core == GPX_CORE_I8 && n > 0 && n <= I8_KMAX) {
         int64_t ldk, sm, sc;
         if (i8_layout(M, C, n, &ldk, &sm, &sc) <= h->i8_scratch_bytes)
-            return launch_ivar_i8(h, prologue, Wm, ldm, Ma_rows, M, Wc, ldc, Cb_rows, C, n, partial, ldp, nsplit_out, st);
+            return launch_ivar_i8(h, prologue, Wm, ldm, Ma_rows, M, Wc, ldc, Cb_rows, C, n, wM, partial, ldp, nsplit_out, st);
     }
     const int bm = tma ? WS_BM : Cfg::BM;
     const int splits = ivar_splits_for(h, M, C, bm);
@@ -1518,6 +1531,7 @@ int gpx_launch_core_ivar(gpx_handle h, int prologue, const double* Wm, int64_t l
     a.upper_only = 0;
     a.ldo_splits = 0;
     a.tri_blk = a.tri_world = a.tri_rank = 0;
+    a.wM = wM;
     *nsplit_out = splits;
     if (tma) {
         const int64_t jt = (C + BN - 1) / BN;
@@ -1532,16 +1546,21 @@ int gpx_launch_core_ivar(gpx_handle h, int prologue, const double* Wm, int64_t l
         (void)groups;
         dim3 grid((unsigned)(jt * splits), 1u);
         if (prologue == PRO_DIFF) {
-            GPX_DISPATCH_FAMILY(h->kp.family, rc = (launch_ivar_ws<FAM, PRO_DIFF>(h, a, grid, st)));
+            if (wM) GPX_DISPATCH_FAMILY(h->kp.family, rc = (launch_ivar_ws<FAM, PRO_DIFF, true>(h, a, grid, st)));
+            else GPX_DISPATCH_FAMILY(h->kp.family, rc = (launch_ivar_ws<FAM, PRO_DIFF, false>(h, a, grid, st)));
         } else {
-            GPX_DISPATCH_FAMILY(h->kp.family, rc = (launch_ivar_ws<FAM, PRO_EXPANDED>(h, a, grid, st)));
+            if (wM) GPX_DISPATCH_FAMILY(h->kp.family, rc = (launch_ivar_ws<FAM, PRO_EXPANDED, true>(h, a, grid, st)));
+            else GPX_DISPATCH_FAMILY(h->kp.family, rc = (launch_ivar_ws<FAM, PRO_EXPANDED, false>(h, a, grid, st)));
         }
         return rc;
     }
+    const int64_t jt = (C + BN - 1) / BN;
     if (prologue == PRO_DIFF) {
-        GPX_DISPATCH_FAMILY(h->kp.family, rc = (launch_core<FAM, EPI_IVAR, PRO_DIFF>(h, a, (C + BN - 1) / BN, splits, st)));
+        if (wM) GPX_DISPATCH_FAMILY(h->kp.family, rc = (launch_core<FAM, EPI_IVAR, PRO_DIFF, true>(h, a, jt, splits, st)));
+        else GPX_DISPATCH_FAMILY(h->kp.family, rc = (launch_core<FAM, EPI_IVAR, PRO_DIFF>(h, a, jt, splits, st)));
     } else {
-        GPX_DISPATCH_FAMILY(h->kp.family, rc = (launch_core<FAM, EPI_IVAR, PRO_EXPANDED>(h, a, (C + BN - 1) / BN, splits, st)));
+        if (wM) GPX_DISPATCH_FAMILY(h->kp.family, rc = (launch_core<FAM, EPI_IVAR, PRO_EXPANDED, true>(h, a, jt, splits, st)));
+        else GPX_DISPATCH_FAMILY(h->kp.family, rc = (launch_core<FAM, EPI_IVAR, PRO_EXPANDED>(h, a, jt, splits, st)));
     }
     return rc;
 }
@@ -1681,7 +1700,9 @@ extern "C" int gpx_dgemm_tn_sub_lower(gpx_handle h, const double* A, int64_t lda
 // K5 + K7: IVAR scores of every candidate and their arg-min.  The finalisation (sum the M-splits, apply the
 // pinv null-direction rule, |base - reduction|) and the first level of the arg-min share one kernel; the last block
 // to finish reduces the per-block winners (np.argmin order: lowest index wins ties).
+// WT: weighted integration points -- sumVarM and the partials already carry the weights, nothing is divided by M.
 // ---------------------------------------------------------------------------------------------
+template <bool WT>
 __global__ void __launch_bounds__(256) ivar_finalize_argmin_kernel(const double* __restrict__ partial, int nsplit, int64_t ldp,
                                                                     const double* __restrict__ varC,
                                                                     const double* __restrict__ sumVarM, int64_t M, int64_t C,
@@ -1692,14 +1713,14 @@ __global__ void __launch_bounds__(256) ivar_finalize_argmin_kernel(const double*
     __shared__ double sv[8];
     __shared__ int64_t si[8];
     __shared__ bool last;
-    const double base = sumVarM[0] / (double)M;            // (1/nMC) sum varMC   experimentalDesign.py:109
+    const double base = WT ? sumVarM[0] : sumVarM[0] / (double)M;  // (1/nMC) sum varMC   experimentalDesign.py:109
     double bv = 0.0;
     int64_t bi = -1;
     for (int64_t c = (int64_t)blockIdx.x * 256 + threadIdx.x; c < C; c += (int64_t)gridDim.x * 256) {
         double r = 0.0;
         for (int s = 0; s < nsplit; ++s) r += partial[(int64_t)s * ldp + c];
         const double den = varC[c] + noise;
-        const double red = (den <= zero_tol) ? 0.0 : (r / den) / (double)M;
+        const double red = (den <= zero_tol) ? 0.0 : (WT ? r / den : (r / den) / (double)M);
         const double sc = fabs(base - red);                // np.abs(cost)        experimentalDesign.py:117
         score[c] = sc;
         if (!(mask && mask[c]) && gpx_better(sc, c, bv, bi, true)) {
@@ -1757,14 +1778,19 @@ __global__ void __launch_bounds__(256) ivar_finalize_argmin_kernel(const double*
 }
 
 static int ivar_finalize_argmin(gpx_handle h, const double* partial, int nsplit, int64_t ldp, const double* varC, int64_t M,
-                                int64_t C, double noise, double zero_tol, const uint8_t* mask, double* score_out, double* best,
-                                int64_t* idx, cudaStream_t st) {
+                                int64_t C, double noise, double zero_tol, bool weighted, const uint8_t* mask, double* score_out,
+                                double* best, int64_t* idx, cudaStream_t st) {
     int64_t blocks = (C + 255) / 256;
     if (blocks > 1024) blocks = 1024;
     // slots [0, 1024) and ticket 0 of the handle scratch, like gpx_argreduce (never concurrent on one handle)
-    ivar_finalize_argmin_kernel<<<(unsigned)blocks, 256, 0, st>>>(partial, nsplit, ldp, varC, h->scal, M, C, noise, zero_tol,
-                                                                 mask, score_out, h->red_val, h->red_idx, h->red_counter, best,
-                                                                 idx);
+    if (weighted)
+        ivar_finalize_argmin_kernel<true><<<(unsigned)blocks, 256, 0, st>>>(partial, nsplit, ldp, varC, h->scal, M, C, noise,
+                                                                            zero_tol, mask, score_out, h->red_val, h->red_idx,
+                                                                            h->red_counter, best, idx);
+    else
+        ivar_finalize_argmin_kernel<false><<<(unsigned)blocks, 256, 0, st>>>(partial, nsplit, ldp, varC, h->scal, M, C, noise,
+                                                                             zero_tol, mask, score_out, h->red_val, h->red_idx,
+                                                                             h->red_counter, best, idx);
     return gpx_check_launch("gpx_score_ivar finalize");
 }
 
@@ -1803,34 +1829,53 @@ extern "C" int64_t gpx_score_ivar_workspace(gpx_handle h, int64_t M, int64_t C) 
     return (int64_t)gpx_ivar_splits(h, M, C) * ldp;
 }
 
-extern "C" int gpx_score_ivar(gpx_handle h, int prologue, const double* Wm, int64_t ldm, const double* varM,
-                              const double* Ma_rows, int64_t M, const double* Wc, int64_t ldc, const double* varC,
-                              const double* Cb_rows, int64_t C, int64_t n, double noise, double zero_tol, const uint8_t* mask,
-                              double* workspace, double* score_out, double* best, int64_t* idx, void* stream) {
+extern "C" int gpx_score_ivar_w(gpx_handle h, int prologue, const double* Wm, int64_t ldm, const double* varM,
+                                const double* Ma_rows, int64_t M, const double* Wc, int64_t ldc, const double* varC,
+                                const double* Cb_rows, int64_t C, int64_t n, double noise, double zero_tol, const double* wM,
+                                const uint8_t* mask, double* workspace, double* score_out, double* best, int64_t* idx,
+                                void* stream) {
     GPX_NEED_KERNEL(h);
     GPX_REQUIRE(M >= 1 && C >= 1 && n >= 0, GPX_EINVAL, "bad sizes");
     GPX_REQUIRE(varM && Ma_rows && varC && Cb_rows && workspace && score_out && best && idx, GPX_EINVAL, "NULL pointer");
     GPX_REQUIRE(n == 0 || (Wm && Wc), GPX_EINVAL, "W is NULL");
     cudaStream_t st = (cudaStream_t)stream;
-    int rc = gpx_sum_impl(h, varM, M, h->scal, st);
+    int rc = gpx_sum_impl(h, varM, wM, M, h->scal, st);
     if (rc) return rc;
     const int64_t ldp = (C + 1) & ~(int64_t)1;
     int nsplit = 1;
-    rc = gpx_launch_core_ivar(h, prologue, Wm, ldm, Ma_rows, M, Wc, ldc, Cb_rows, C, n, workspace, ldp, &nsplit, st);
+    rc = gpx_launch_core_ivar(h, prologue, Wm, ldm, Ma_rows, M, Wc, ldc, Cb_rows, C, n, wM, workspace, ldp, &nsplit, st);
     if (rc) return rc;
-    return ivar_finalize_argmin(h, workspace, nsplit, ldp, varC, M, C, noise, zero_tol, mask, score_out, best, idx, st);
+    return ivar_finalize_argmin(h, workspace, nsplit, ldp, varC, M, C, noise, zero_tol, wM != nullptr, mask, score_out, best,
+                                idx, st);
+}
+
+extern "C" int gpx_score_ivar(gpx_handle h, int prologue, const double* Wm, int64_t ldm, const double* varM,
+                              const double* Ma_rows, int64_t M, const double* Wc, int64_t ldc, const double* varC,
+                              const double* Cb_rows, int64_t C, int64_t n, double noise, double zero_tol, const uint8_t* mask,
+                              double* workspace, double* score_out, double* best, int64_t* idx, void* stream) {
+    return gpx_score_ivar_w(h, prologue, Wm, ldm, varM, Ma_rows, M, Wc, ldc, varC, Cb_rows, C, n, noise, zero_tol, nullptr,
+                            mask, workspace, score_out, best, idx, stream);
 }
 
 // IVAR scores from per-segment column sums of squares (resident-covariance mode): same finalisation + arg-min
-extern "C" int gpx_score_ivar_partials(gpx_handle h, const double* partial, int nseg, int64_t ldp, const double* varM, int64_t M,
-                                       const double* varC, int64_t C, double noise, double zero_tol, const uint8_t* mask,
-                                       double* score_out, double* best, int64_t* idx, void* stream) {
+extern "C" int gpx_score_ivar_partials_w(gpx_handle h, const double* partial, int nseg, int64_t ldp, const double* varM,
+                                         int64_t M, const double* varC, int64_t C, double noise, double zero_tol,
+                                         const double* wM, const uint8_t* mask, double* score_out, double* best, int64_t* idx,
+                                         void* stream) {
     GPX_REQUIRE(h && partial && varM && varC && score_out && best && idx && nseg >= 1 && M >= 1 && C >= 1, GPX_EINVAL,
                 "bad arguments");
     cudaStream_t st = (cudaStream_t)stream;
-    int rc = gpx_sum_impl(h, varM, M, h->scal, st);
+    int rc = gpx_sum_impl(h, varM, wM, M, h->scal, st);
     if (rc) return rc;
-    return ivar_finalize_argmin(h, partial, nseg, ldp, varC, M, C, noise, zero_tol, mask, score_out, best, idx, st);
+    return ivar_finalize_argmin(h, partial, nseg, ldp, varC, M, C, noise, zero_tol, wM != nullptr, mask, score_out, best, idx,
+                                st);
+}
+
+extern "C" int gpx_score_ivar_partials(gpx_handle h, const double* partial, int nseg, int64_t ldp, const double* varM, int64_t M,
+                                       const double* varC, int64_t C, double noise, double zero_tol, const uint8_t* mask,
+                                       double* score_out, double* best, int64_t* idx, void* stream) {
+    return gpx_score_ivar_partials_w(h, partial, nseg, ldp, varM, M, varC, C, noise, zero_tol, nullptr, mask, score_out, best,
+                                     idx, stream);
 }
 
 // cov[m,c] = k(m,c) - sum_{i<n} Wm[i,m] Wc[i,c] for a GIVEN design (DMMA contraction with the Gram prologue, stored)

@@ -83,13 +83,17 @@ extern "C" int gpx_se_var_grad(gpx_handle h, const double* P, int64_t n, int64_t
     return gpx_check_launch("gpx_se_var_grad");
 }
 
-// out[r] = scale * sum_c A[r, c]  (one block per row, fixed summation order)
+// out[r] = scale * sum_c A[r, c]  (one block per row, fixed summation order); WT: sum_c w[c] A[r, c] in the same order
+template <bool WT>
 __global__ void __launch_bounds__(256) rowsum_kernel(const double* __restrict__ A, int64_t cols, int64_t ld, double scale,
-                                                      double* __restrict__ out) {
+                                                      const double* __restrict__ w, double* __restrict__ out) {
     __shared__ double sm[8];
     const double* row = A + (int64_t)blockIdx.x * ld;
     double s = 0.0;
-    for (int64_t c = threadIdx.x; c < cols; c += 256) s += row[c];
+    for (int64_t c = threadIdx.x; c < cols; c += 256) {
+        if (WT) s = fma(w[c], row[c], s);
+        else s += row[c];
+    }
 #pragma unroll
     for (int off = 16; off > 0; off >>= 1) s += __shfl_xor_sync(0xffffffffu, s, off);
     if ((threadIdx.x & 31) == 0) sm[threadIdx.x >> 5] = s;
@@ -106,8 +110,17 @@ extern "C" int gpx_rowsum(gpx_handle h, const double* A, int64_t rows, int64_t c
     GPX_REQUIRE(h && rows >= 0 && cols >= 0, GPX_EINVAL, "bad arguments");
     if (rows == 0) return GPX_OK;
     GPX_REQUIRE(A && out && rows <= 2147483647LL, GPX_EINVAL, "bad arguments");
-    rowsum_kernel<<<(unsigned)rows, 256, 0, (cudaStream_t)stream>>>(A, cols, ld, scale, out);
+    rowsum_kernel<false><<<(unsigned)rows, 256, 0, (cudaStream_t)stream>>>(A, cols, ld, scale, nullptr, out);
     return gpx_check_launch("gpx_rowsum");
+}
+
+extern "C" int gpx_rowsum_w(gpx_handle h, const double* A, int64_t rows, int64_t cols, int64_t ld, const double* w, double* out,
+                            void* stream) {
+    GPX_REQUIRE(h && rows >= 0 && cols >= 0, GPX_EINVAL, "bad arguments");
+    if (rows == 0) return GPX_OK;
+    GPX_REQUIRE(A && out && w && rows <= 2147483647LL, GPX_EINVAL, "bad arguments");
+    rowsum_kernel<true><<<(unsigned)rows, 256, 0, (cudaStream_t)stream>>>(A, cols, ld, 1.0, w, out);
+    return gpx_check_launch("gpx_rowsum_w");
 }
 
 // out[0] = log det(U^T U) = 2 sum_i log U[i,i]          (np.linalg.slogdet at gp.py:432 for a PD matrix)

@@ -301,6 +301,7 @@ int exchange(gpx_handle h, const double* rec, double* rec_all, double* rec_win, 
 // State conventions at entry and exit are those of the resident engine (cov current, partial sums valid), so the two
 // paths can be mixed.  The winner's pivot var_D(p) + noise travels with the block results: it must be read before any
 // block starts updating the variances in phase B.
+// WT: weighted integration points (s.wM): sum w varM and the weighted column sums, in the same trees; nothing / M.
 // ---------------------------------------------------------------------------------------------
 namespace {
 namespace cg = cooperative_groups;
@@ -353,7 +354,7 @@ __device__ __forceinline__ void small_block_argmin(double& v, int64_t& i, double
         }
 }
 
-template <int FAM>
+template <int FAM, bool WT>
 __global__ void __launch_bounds__(256, 2) ivar_small_greedy_kernel(const __grid_constant__ KParams kp, const gpx_ivar_state s,
                                                                  int n_begin, int n_end, double* __restrict__ blk_val,
                                                                  int64_t* __restrict__ blk_idx, double* __restrict__ blk_piv,
@@ -369,11 +370,14 @@ __global__ void __launch_bounds__(256, 2) ivar_small_greedy_kernel(const __grid_
     const int64_t cgroups = (C + 31) / 32;
     // sum of var_M for the first step (every block, same order); later steps get it from the blocks' phase-B partials
     double part = 0.0;
-    for (int64_t m = tid; m < M; m += 256) part += s.varM[m];
+    for (int64_t m = tid; m < M; m += 256) {
+        if (WT) part = fma(s.wM[m], s.varM[m], part);
+        else part += s.varM[m];
+    }
     double base_sum = small_block_sum(part, sm);
     for (int n = n_begin; n < n_end; ++n) {
         // ---- phase A: scores of my candidate groups (32 candidates x 8 warps over the row segments), block arg-min ------
-        const double base = base_sum / (double)M;                      // (1/nMC) sum varMC   experimentalDesign.py:109
+        const double base = WT ? base_sum : base_sum / (double)M;     // (1/nMC) sum varMC   experimentalDesign.py:109
         double bv = 0.0, bp = 1.0;
         int64_t bi = -1;
         for (int64_t grp = b; grp < cgroups; grp += nb) {
@@ -406,7 +410,7 @@ __global__ void __launch_bounds__(256, 2) ivar_small_greedy_kernel(const __grid_
                 double r = 0.0;
 #pragma unroll
                 for (int w = 0; w < 8; ++w) r += s_part[w][lane];
-                const double red = (den <= s.zero_tol) ? 0.0 : (r / den) / (double)M;
+                const double red = (den <= s.zero_tol) ? 0.0 : (WT ? r / den : (r / den) / (double)M);
                 const double sc = fabs(base - red);                     // np.abs(cost)        experimentalDesign.py:117
                 s.scores[c] = sc;
                 if (gpx_better(sc, c, bv, bi, true)) {
@@ -512,7 +516,10 @@ __global__ void __launch_bounds__(256, 2) ivar_small_greedy_kernel(const __grid_
             W[(int64_t)n * ld + col] = w;
             const double nv = var_old - w * w;
             var[col] = nv;
-            if (!cside) vpart += nv;
+            if (!cside) {
+                if (WT) vpart = fma(s.wM[col], nv, vpart);
+                else vpart += nv;
+            }
         }
         const double vsum = small_block_sum(vpart, sm);
         if (tid == 0) blk_base[b] = vsum;
@@ -545,8 +552,9 @@ __global__ void __launch_bounds__(256, 2) ivar_small_greedy_kernel(const __grid_
                     v[u].x = fma(-a, bb.x, v[u].x);
                     v[u].y = fma(-a, bb.y, v[u].y);
                     *reinterpret_cast<double2*>(cp + (int64_t)u * s.ldcov) = v[u];
-                    r0 = fma(v[u].x, v[u].x, r0);
-                    r1 = fma(v[u].y, v[u].y, r1);
+                    const double w = WT ? s.wM[m + u] : 1.0;
+                    r0 = fma(WT ? w * v[u].x : v[u].x, v[u].x, r0);
+                    r1 = fma(WT ? w * v[u].y : v[u].y, v[u].y, r1);
                 }
                 cp += 8 * s.ldcov;
             }
@@ -556,8 +564,9 @@ __global__ void __launch_bounds__(256, 2) ivar_small_greedy_kernel(const __grid_
                 v.x = fma(-a, bb.x, v.x);
                 v.y = fma(-a, bb.y, v.y);
                 *reinterpret_cast<double2*>(cp) = v;
-                r0 = fma(v.x, v.x, r0);
-                r1 = fma(v.y, v.y, r1);
+                const double w = WT ? s.wM[m] : 1.0;
+                r0 = fma(WT ? w * v.x : v.x, v.x, r0);
+                r1 = fma(WT ? w * v.y : v.y, v.y, r1);
             }
             double* dst = s.workspace + seg * s.ldp + c;
             dst[0] = r0;
@@ -589,9 +598,9 @@ extern "C" int gpx_ivar_greedy_small(gpx_handle h, const gpx_ivar_state* s, int6
     if (n_end == n_begin) return GPX_OK;
     int per_sm = 0;
     cudaError_t e;
-#define GPX_SMALL_LAUNCH(F)                                                                                              \
+#define GPX_SMALL_LAUNCH(F, W)                                                                                           \
     do {                                                                                                                 \
-        e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, ivar_small_greedy_kernel<F>, 256, 0);                 \
+        e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, ivar_small_greedy_kernel<F, W>, 256, 0);              \
         if (e == cudaSuccess) {                                                                                          \
             if (per_sm > 2) per_sm = 2;                                                                                  \
             int blocks = per_sm * (h->sm_count > 0 ? h->sm_count : 148);                                                 \
@@ -604,12 +613,13 @@ extern "C" int gpx_ivar_greedy_small(gpx_handle h, const gpx_ivar_state* s, int6
             double* bp = h->red_val + 512;                                                                               \
             double* bb = h->red_val + 1024;                                                                              \
             void* args[] = {&kp, &st, &nb0, &ne0, &bv, &bi, &bp, &bb};                                                   \
-            e = blocks > 0 ? cudaLaunchCooperativeKernel((const void*)ivar_small_greedy_kernel<F>, dim3(blocks), dim3(256), \
+            e = blocks > 0 ? cudaLaunchCooperativeKernel((const void*)ivar_small_greedy_kernel<F, W>, dim3(blocks), dim3(256), \
                                                          args, 0, (cudaStream_t)stream)                                  \
                            : cudaErrorLaunchOutOfResources;                                                              \
         }                                                                                                                \
     } while (0)
-    GPX_DISPATCH_FAMILY(h->kp.family, GPX_SMALL_LAUNCH(FAM));
+    if (s->wM) GPX_DISPATCH_FAMILY(h->kp.family, GPX_SMALL_LAUNCH(FAM, true));
+    else GPX_DISPATCH_FAMILY(h->kp.family, GPX_SMALL_LAUNCH(FAM, false));
 #undef GPX_SMALL_LAUNCH
     if (e != cudaSuccess) {
         gpx_set_error("gpx_ivar_greedy_small: %s", cudaGetErrorString(e));
@@ -643,11 +653,12 @@ extern "C" int gpx_ivar_greedy_run(gpx_handle h, const gpx_ivar_state* s, int64_
     int rc;
     for (int64_t n = n_begin; n < n_end; ++n) {
         if (s->cov) {
-            rc = gpx_score_ivar_partials(h, s->workspace, s->nseg, s->ldp, s->varM, s->M, s->varC, s->C, s->noise, s->zero_tol,
-                                         nullptr, s->scores, s->best, s->idx, stream);
+            rc = gpx_score_ivar_partials_w(h, s->workspace, s->nseg, s->ldp, s->varM, s->M, s->varC, s->C, s->noise,
+                                           s->zero_tol, s->wM, nullptr, s->scores, s->best, s->idx, stream);
         } else {
-            rc = gpx_score_ivar(h, s->prologue, s->Wm, s->ldm, s->varM, s->Ma_rows, s->M, s->Wc, s->ldc, s->varC, s->Cb_rows,
-                                s->C, n, s->noise, s->zero_tol, nullptr, s->workspace, s->scores, s->best, s->idx, stream);
+            rc = gpx_score_ivar_w(h, s->prologue, s->Wm, s->ldm, s->varM, s->Ma_rows, s->M, s->Wc, s->ldc, s->varC, s->Cb_rows,
+                                  s->C, n, s->noise, s->zero_tol, s->wM, nullptr, s->workspace, s->scores, s->best, s->idx,
+                                  stream);
         }
         if (rc) return rc;
         rc = launch_gather_store(h, s->Wc, s->ldc, n, s->varC, s->Xc, s->ldc, s->best, s->idx, s->index_offset, s->noise, s->rec,
@@ -662,8 +673,8 @@ extern "C" int gpx_ivar_greedy_run(gpx_handle h, const gpx_ivar_state* s, int64_
         rc = launch_append2(h, win, sc, sm, n, st);
         if (rc) return rc;
         if (s->cov) {
-            rc = gpx_cov_update(h, s->cov, s->ldcov, s->M, s->C, s->Wm + n * s->ldm, s->Wc + n * s->ldc, s->workspace, s->ldp,
-                                stream);
+            rc = gpx_cov_update_w(h, s->cov, s->ldcov, s->M, s->C, s->Wm + n * s->ldm, s->Wc + n * s->ldc, s->wM, s->workspace,
+                                  s->ldp, stream);
             if (rc) return rc;
         }
     }

@@ -533,7 +533,7 @@ class GreedyIVAREngine(_Pivoting):
     ONE_KERNEL_PAIRS = int(os.environ.get("GPX_ONE_KERNEL_PAIRS", ONE_KERNEL_DEFAULT))
 
     def __init__(self, dev: Device, cand: PointSet, mc: PointSet, n_max: int, noise: float, zero_scale: float,
-                 shard=None, index_offset: int = 0, resident: bool = False, cand_noise=None):
+                 shard=None, index_offset: int = 0, resident: bool = False, cand_noise=None, mc_weights=None):
         """resident=True keeps the posterior covariance cov_D(m, c) (8*M*C bytes) in HBM and replaces the per-step
         O(M n C) contraction by one rank-1 update pass (16*M*C bytes of traffic per step, independent of n) -- the
         better algorithm for a greedy LOOP whenever the matrix fits; scoring a GIVEN design still takes the contraction.
@@ -541,12 +541,22 @@ class GreedyIVAREngine(_Pivoting):
         cand_noise: host vector nu of a heteroscedastic noise function at the local candidates (noise must be 0.0 then).
         The candidate running variance is then kept noise-inclusive, varC[c] = var_D(c) + nu(c): every kernel sees the
         noise only as varC + noise, the append's (var + nu) - w^2 is the same update, and the pivot var_D(p) + nu(p)
-        makes U the factor of K_DD + diag(nu(D)).  Integration points carry no noise."""
+        makes U the factor of K_DD + diag(nu(D)).  Integration points carry no noise.
+
+        mc_weights: host vector w of one weight per integration point (used as given, not normalised).  Every reduction
+        over the integration points then carries it: cost(c) = |sum_m w_m var_D(m) - sum_m w_m cov_D(m,c)^2 / (varC + noise)|
+        instead of the plain mean.  The weights are static, so snapshot / restore / rollback need nothing for them."""
         self.cand, self.mc = cand, mc
         self.resident = bool(resident)
         self.noise = float(noise)
         nu = _noise_vector("cand_noise", cand_noise, self.noise, cand.n, "candidates")
         self.cand_noise = None if nu is None else dev.upload(nu)
+        self.mc_weights = None
+        if mc_weights is not None:
+            w = np.asarray(mc_weights, dtype=np.float64).ravel()
+            if w.size != mc.n:
+                raise ValueError(f"mc_weights has {w.size} values for {mc.n} integration points")
+            self.mc_weights = dev.upload(w)
         self.zero_tol = ZERO_VAR_TOL * float(zero_scale)
         ncap = max(int(n_max), 1)
         self._init_pivot(dev, ncap, n_max, shard, index_offset)
@@ -587,8 +597,8 @@ class GreedyIVAREngine(_Pivoting):
 
     def _cov_pass(self, a, b):
         dev, cand, mc = self.dev, self.cand, self.mc
-        check(lib.gpx_cov_update(dev.h, ptr(self.cov), cand.ld, mc.n, cand.n, ptr(a), ptr(b), ptr(self.workspace), self.ldp,
-                                 dev.stream), "gpx_cov_update")
+        check(lib.gpx_cov_update_w(dev.h, ptr(self.cov), cand.ld, mc.n, cand.n, ptr(a), ptr(b), ptr(self.mc_weights),
+                                   ptr(self.workspace), self.ldp, dev.stream), "gpx_cov_update_w")
 
     def prologue(self):
         """(mode, rows of the integration points, rows of the candidates) for the contraction's covariance prologue.
@@ -601,9 +611,10 @@ class GreedyIVAREngine(_Pivoting):
         (cross-check of the two paths on the same state)."""
         dev, cand, mc = self.dev, self.cand, self.mc
         if self.resident and not contraction:
-            check(lib.gpx_score_ivar_partials(dev.h, ptr(self.workspace), self.nseg, self.ldp, ptr(self.varM), mc.n,
-                                              ptr(self.varC), cand.n, self.noise, self.zero_tol, None, ptr(self.scores),
-                                              ptr(self.best), ptr(self.idx), dev.stream), "gpx_score_ivar_partials")
+            check(lib.gpx_score_ivar_partials_w(dev.h, ptr(self.workspace), self.nseg, self.ldp, ptr(self.varM), mc.n,
+                                                ptr(self.varC), cand.n, self.noise, self.zero_tol, ptr(self.mc_weights), None,
+                                                ptr(self.scores), ptr(self.best), ptr(self.idx), dev.stream),
+                  "gpx_score_ivar_partials_w")
             return
         mode, ma_rows, cb_rows = self.prologue()
         ws = self.workspace
@@ -611,9 +622,10 @@ class GreedyIVAREngine(_Pivoting):
             if getattr(self, "_ws2", None) is None:
                 self._ws2 = dev.zeros(self.workspace.numel())
             ws = self._ws2
-        check(lib.gpx_score_ivar(dev.h, mode, ptr(self.Wm), mc.ld, ptr(self.varM), ptr(ma_rows), mc.n, ptr(self.Wc), cand.ld,
-                                 ptr(self.varC), ptr(cb_rows), cand.n, self.n, self.noise, self.zero_tol, None, ptr(ws),
-                                 ptr(self.scores), ptr(self.best), ptr(self.idx), dev.stream), "gpx_score_ivar")
+        check(lib.gpx_score_ivar_w(dev.h, mode, ptr(self.Wm), mc.ld, ptr(self.varM), ptr(ma_rows), mc.n, ptr(self.Wc),
+                                   cand.ld, ptr(self.varC), ptr(cb_rows), cand.n, self.n, self.noise, self.zero_tol,
+                                   ptr(self.mc_weights), None, ptr(ws), ptr(self.scores), ptr(self.best), ptr(self.idx),
+                                   dev.stream), "gpx_score_ivar_w")
 
     def append(self):
         dev, cand, mc = self.dev, self.cand, self.mc
@@ -698,6 +710,7 @@ class GreedyIVAREngine(_Pivoting):
         st.U, st.ldu = ptr(self.U), self.U.shape[1]
         st.picks, st.pick_scores, st.pick_pivots = ptr(self.picks), ptr(self.pick_scores), ptr(self.pick_pivots)
         st.cov, st.ldcov, st.ldp = ptr(self.cov), cand.ld, self.ldp
+        st.wM = ptr(self.mc_weights)
         return st
 
     def run(self, n_points: int, progress=None, chunk: int = 10):

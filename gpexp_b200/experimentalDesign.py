@@ -37,13 +37,24 @@ def _ivar_mc_points(self, dev):
     return cached
 
 
+def _ivar_weights(self):
+    """The cost function's integration weights `mcWeights` (None: the plain Monte-Carlo mean), checked on the host against
+    its integration points: one finite value >= 0 per point and at least one > 0, else ValueError."""
+    w = getattr(self, "mcWeights", None)
+    if w is None:
+        return None
+    return _checked_per_point(w, len(self.mcPoints), "mcWeights has", need_positive=True)
+
+
 def _ivar_evaluate(self, inputPoints):
-    """|mean posterior variance over the MC points| for the design `inputPoints` (:79-117)."""
+    """|mean posterior variance over the MC points| for the design `inputPoints` (:79-117); with weights w
+    (`mcWeights`), |sum_m w_m var(x_m)|."""
     assert inputPoints.shape == (self.numInputs, self.space.dimension), \
         ("inputPoints are the wrong size: ", inputPoints.shape)
     if self.version != 1:
         raise NotImplementedError("IVAR version 0 needs a kernel eigen-basis that no shipped kernel provides "
                                   "(experimentalDesign.py:119-146 is unreachable)")
+    w = _ivar_weights(self)
     gp = self.gaussianProcess
     if self.space.noiseFunc is None:
         gp.addNodesAndComputeCovariance(inputPoints)
@@ -53,6 +64,10 @@ def _ivar_evaluate(self, inputPoints):
     mc = _ivar_mc_points(self, f.dev)
     _, var = f.solve_gram(mc)
     total = f.dev.zeros(1)
+    if w is not None:
+        wd = f.dev.upload(w)
+        check(lib.gpx_sum_w(f.dev.h, ptr(var), ptr(wd), mc.n, ptr(total), f.dev.stream), "gpx_sum_w")
+        return np.abs(float(total.item()))
     check(lib.gpx_sum(f.dev.h, ptr(var), mc.n, ptr(total), f.dev.stream), "gpx_sum")
     return np.abs(float(total.item()) / float(self.nMC))
 
@@ -60,9 +75,11 @@ def _ivar_evaluate(self, inputPoints):
 def _ivar_derivative(self, inputPoints):
     """Gradient of the IVAR cost with respect to the design coordinates, shape (nPoints*dimension,)
     (:148-179, version 1): the row mean over the MC points of GP.evaluateVarianceDerivative, with the noise function's
-    own derivative in the heteroscedastic case.  Squared-exponential kernels."""
+    own derivative in the heteroscedastic case.  Squared-exponential kernels.  With weights w (`mcWeights`) the row
+    reduction is sum_m w_m instead of the mean."""
     gp = self.gaussianProcess
     gp.kernel._require_derivative()
+    w = _ivar_weights(self)
     noise_grad = same = None
     if self.space.noiseFunc is None:
         gp.addNodesAndComputeCovariance(inputPoints)
@@ -76,7 +93,12 @@ def _ivar_derivative(self, inputPoints):
     full = f.variance_gradient(mc, noise_grad, same)
     rows = f.n * gp.kernel.dimension
     out = f.dev.zeros(max(rows, 1))
-    check(lib.gpx_rowsum(f.dev.h, ptr(full), rows, mc.n, mc.ld, 1.0 / float(self.nMC), ptr(out), f.dev.stream), "gpx_rowsum")
+    if w is not None:
+        wd = f.dev.upload(w)
+        check(lib.gpx_rowsum_w(f.dev.h, ptr(full), rows, mc.n, mc.ld, ptr(wd), ptr(out), f.dev.stream), "gpx_rowsum_w")
+    else:
+        check(lib.gpx_rowsum(f.dev.h, ptr(full), rows, mc.n, mc.ld, 1.0 / float(self.nMC), ptr(out), f.dev.stream),
+              "gpx_rowsum")
     return out[:rows].cpu().numpy()
 
 
@@ -86,7 +108,7 @@ def _mi_noise(self):
     each pool point, checked to hold one finite value >= 0 per point."""
     noise = _nugget_arg(self.gaussianProcess.noise)
     if isinstance(noise, np.ndarray):
-        return 0.0, _checked_noise(noise, len(self.mcPoints), "gp.noise has")
+        return 0.0, _checked_per_point(noise, len(self.mcPoints), "gp.noise has")
     return float(noise), None
 
 
@@ -137,7 +159,18 @@ class costFunctionBase(object):
 
 class costFunctionGP_IVAR(costFunctionBase):
     """Integrated posterior variance of a design, Monte-Carlo version: costFunctionGP_IVAR(gp, nInputs, space,
-    version=1, mcPoints=...)  (:60-75).  Holds a shallow copy of the GP; without mcPoints, 10 000 samples of the space."""
+    version=1, mcPoints=..., mcWeights=...)  (:60-75).  Holds a shallow copy of the GP; without mcPoints, 10 000 samples
+    of the space.
+
+    mcWeights (attribute, default None): one float64 weight per integration point (finite, >= 0, at least one > 0),
+    used as given, not normalised.  The cost is then |sum_m w_m var(x_m)| instead of the mean over mcPoints: Gauss-Legendre
+    or other quadrature weights, importance weights p(x_m)/q(x_m) of a density that can be evaluated but not sampled, or a
+    region of interest (weighted IMSE).  w = 1/nMC is the plain cost.  evaluate, derivative and the greedy drivers
+    (beginGreedyIVARExperimentalDesign, performGreedyIVARExperimentalDesign, scoreCandidatesIVAR) read it; bad weights
+    raise ValueError before any device work.  Under install_as_gpExp(path) the reference's own constructor is kept, so
+    there the caller sets `cf.mcWeights = w` after construction."""
+
+    mcWeights = None
 
     def __init__(self, gaussianProcess, nInputs, space, version=1, **kwargs):
         costFunctionBase.__init__(self, nInputs, space)
@@ -145,6 +178,7 @@ class costFunctionGP_IVAR(costFunctionBase):
         if version == 1:
             pts = kwargs['mcPoints'] if 'mcPoints' in kwargs else space.sample((10000, space.dimension))
             self.mcPoints, self.nMC = pts, len(pts)
+            self.mcWeights = kwargs.get('mcWeights')
 
     evaluate = _ivar_evaluate
     derivative = _ivar_derivative
@@ -233,22 +267,25 @@ def performGreedyVarExperimentalDesign(kernel, mcPoints, nPoints, dimension, wei
     return mcPoints[indKeep, :]
 
 
-def _checked_noise(values, n, source):
-    """`values` as one float64 nugget per point for n points; `source` ("noise function returned", "gp.noise has") starts
-    the message of the ValueError raised unless there is exactly one finite value >= 0 per point."""
-    nu = np.asarray(values, dtype=np.float64).ravel()
-    if nu.size != n:
-        raise ValueError(f"{source} {nu.size} values for {n} points (one per point expected)")
-    if not np.all(np.isfinite(nu)):
+def _checked_per_point(values, n, source, need_positive=False):
+    """`values` as one float64 per point for n points (a nugget or an integration weight); `source` ("noise function
+    returned", "gp.noise has", "mcWeights has") starts the message of the ValueError raised unless there is exactly one
+    finite value >= 0 per point -- and, with need_positive, at least one value > 0."""
+    v = np.asarray(values, dtype=np.float64).ravel()
+    if v.size != n:
+        raise ValueError(f"{source} {v.size} values for {n} points (one per point expected)")
+    if not np.all(np.isfinite(v)):
         raise ValueError(f"{source} a value that is not finite")
-    if np.any(nu < 0.0):
+    if np.any(v < 0.0):
         raise ValueError(f"{source} a negative value")
-    return nu
+    if need_positive and not np.any(v > 0.0):
+        raise ValueError(f"{source} no positive value (at least one must be > 0)")
+    return v
 
 
 def _noise_values(noiseFunc, points):
     """noiseFunc(points) as one float64 nugget per point; the noise function is user code, so its output is checked."""
-    return _checked_noise(noiseFunc(points), points.shape[0], "noise function returned")
+    return _checked_per_point(noiseFunc(points), points.shape[0], "noise function returned")
 
 
 def beginGreedyIVARExperimentalDesign(costFuncIVAR, candidates, nPoints, shard=None, resident=None):
@@ -264,8 +301,12 @@ def beginGreedyIVARExperimentalDesign(costFuncIVAR, candidates, nPoints, shard=N
     With a heteroscedastic `costFuncIVAR.space.noiseFunc`, the cost of design + [c] uses the nugget noiseFunc(design + [c])
     as costFunctionGP_IVAR.evaluate does, and gp.noise is not used.  The noise function must be pointwise and
     deterministic: it is evaluated once on this rank's candidates (the reference re-evaluates it on every design + [c]).
-    It must return one finite value >= 0 per point, else ValueError."""
+    It must return one finite value >= 0 per point, else ValueError.
+
+    With `costFuncIVAR.mcWeights` the cost of design + [c] is the weighted sum over the integration points (see
+    costFunctionGP_IVAR); the weights are replicated with the integration points, so every rank passes the same ones."""
     gp = costFuncIVAR.gaussianProcess
+    weights = _ivar_weights(costFuncIVAR)
     lo, hi = 0, candidates.shape[0]
     if shard is not None:
         lo, hi = Shard.split(candidates.shape[0], shard.world, shard.rank)
@@ -289,16 +330,16 @@ def beginGreedyIVARExperimentalDesign(costFuncIVAR, candidates, nPoints, shard=N
             shard.dist.all_reduce(flag, op=shard.dist.ReduceOp.MIN, group=shard.group)
             resident = bool(flag.item())
     return GreedyIVAREngine(dev, cand, mc, nPoints, noise, prior_scale(fam, params), shard=shard, index_offset=lo,
-                            resident=bool(resident), cand_noise=cand_noise)
+                            resident=bool(resident), cand_noise=cand_noise, mc_weights=weights)
 
 
 def performGreedyIVARExperimentalDesign(costFuncIVAR, candidates, nPoints, returnIndices=False, shard=None, resident=None):
     """Discrete greedy IVAR: at every step score `costFuncIVAR.evaluate(design + [c])` for every candidate
     c and add the arg-min -- what a loop over costFunctionGP_IVAR.evaluate (experimentalDesign.py:79-117)
     computes, restated with the Schur identity and run as one FP64 tensor-core contraction per step.
-    Arguments as beginGreedyIVARExperimentalDesign.  Leaves lastIndices, lastScores, lastPivots and illConditionedFrom
-    (first step beyond which 1e-9 agreement with the reference's pinv arithmetic cannot be expected, or None) on the
-    cost function."""
+    Arguments as beginGreedyIVARExperimentalDesign.  Leaves lastIndices, lastScores (weighted costs when the cost function
+    has mcWeights), lastPivots and illConditionedFrom (first step beyond which 1e-9 agreement with the reference's pinv
+    arithmetic cannot be expected, or None) on the cost function."""
     eng = beginGreedyIVARExperimentalDesign(costFuncIVAR, candidates, nPoints, shard=shard, resident=resident)
     idx = eng.run(nPoints)
     costFuncIVAR.lastIndices = idx
@@ -315,8 +356,10 @@ def scoreCandidatesIVAR(costFuncIVAR, design, candidates, shard=None):
     Returns (costs, argmin index).  With `shard` every rank passes the full candidate array, scores its own contiguous
     block and returns (costs of its block, GLOBAL arg-min index).  This is the end-to-end call bench.py times (`e2e`).
     A heteroscedastic `costFuncIVAR.space.noiseFunc` is honoured as in beginGreedyIVARExperimentalDesign: the design
-    Gram gets the nugget noiseFunc(design) and candidate c the noise noiseFunc(c)."""
+    Gram gets the nugget noiseFunc(design) and candidate c the noise noiseFunc(c).  `costFuncIVAR.mcWeights` weights the
+    integration points as in costFunctionGP_IVAR.evaluate."""
     gp = costFuncIVAR.gaussianProcess
+    weights = _ivar_weights(costFuncIVAR)
     noiseFunc = costFuncIVAR.space.noiseFunc
     lo, hi = 0, candidates.shape[0]
     if shard is not None:
@@ -332,7 +375,8 @@ def scoreCandidatesIVAR(costFuncIVAR, design, candidates, shard=None):
     fam, d, params = gp.kernel._gpx_spec()
     cand = dev.points(candidates[lo:hi])
     mc = dev.points(costFuncIVAR.mcPoints)
-    eng = GreedyIVAREngine(dev, cand, mc, max(n, 1), noise, prior_scale(fam, params), cand_noise=cand_noise)
+    eng = GreedyIVAREngine(dev, cand, mc, max(n, 1), noise, prior_scale(fam, params), cand_noise=cand_noise,
+                           mc_weights=weights)
     if n:
         eng.load_design(DesignFactor(dev, dev.points(design), nugget))
     eng.score()

@@ -4,7 +4,7 @@
  * The reference (goroda/GPEXP) is pure Python/numpy and has NO native or FFI layer
  * (SURVEY.md section 8b), so there is no existing binding to mirror: every entry point
  * below cites the reference Python function whose arithmetic it replaces, and
- * INTEGRATION.md shows the ctypes stub a maintainer of the reference would add.
+ * INTEGRATION.md shows the ctypes stub a maintainer of the reference would add.  79 entry points.
  *
  * Conventions
  *   - every pointer is a DEVICE pointer owned by the caller unless the name ends in _host;
@@ -197,6 +197,8 @@ int gpx_argreduce(gpx_handle h, const double* v, const double* weights, const ui
 
 /* Deterministic sum of n doubles (fixed tree order). */
 int gpx_sum(gpx_handle h, const double* v, int64_t n, double* out, void* stream);
+/* Weighted sum  out[0] = sum_j w[j] v[j]  in the tree order of gpx_sum (one fma per term); w = NULL is gpx_sum. */
+int gpx_sum_w(gpx_handle h, const double* v, const double* w, int64_t n, double* out, void* stream);
 
 /* Operand pipeline of the IVAR contraction kernel (A/B measurements; results are bit-identical): 0 = 32-row chunks x 3
  * stages fed by one bulk copy per operand row; 1 = the same ring fed by one 2-D tensor-map TMA load per operand chunk;
@@ -240,6 +242,14 @@ int gpx_score_ivar(gpx_handle h, int prologue, const double* Wm, int64_t ldm, co
                    int64_t M, const double* Wc, int64_t ldc, const double* varC, const double* Cb_rows, int64_t C, int64_t n,
                    double noise, double zero_tol, const uint8_t* mask, double* workspace, double* score_out, double* best,
                    int64_t* idx, void* stream);
+/* The same with weighted integration points wM (nullable, M doubles, used as given):
+ *         r[c]     = sum_m wM[m] ( k(m,c) - sum_{i<n} Wm[i,m] Wc[i,c] )^2      each term fma(wM[m] v, v, .)
+ *         cost[c]  = | sum_m wM[m] varM[m] - r[c] / (varC[c] + noise) |          (no division by M)
+ *     wM = NULL is gpx_score_ivar; wM = 2^-k (M = 2^k) reproduces its costs bit for bit. */
+int gpx_score_ivar_w(gpx_handle h, int prologue, const double* Wm, int64_t ldm, const double* varM, const double* Ma_rows,
+                     int64_t M, const double* Wc, int64_t ldc, const double* varC, const double* Cb_rows, int64_t C, int64_t n,
+                     double noise, double zero_tol, const double* wM, const uint8_t* mask, double* workspace,
+                     double* score_out, double* best, int64_t* idx, void* stream);
 
 /* ---- Resident posterior covariance: the HBM-bound alternative for greedy IVAR loops (SURVEY.md section 7) -----------
  * cov (M x ldcov, row m = integration point, 8*M*C bytes resident) holds cov_D(m,c); each greedy step is ONE pass
@@ -248,6 +258,9 @@ int gpx_score_ivar(gpx_handle h, int prologue, const double* Wm, int64_t ldm, co
 int gpx_cov_segments(int64_t M, int64_t C);
 int gpx_cov_update(gpx_handle h, double* cov, int64_t ldcov, int64_t M, int64_t C, const double* a, const double* b,
                    double* partial, int64_t ldp, void* stream);
+/* The same with weighted integration points: partial[seg][c] = sum_{m in seg} wM[m] cov[m,c]^2 (wM nullable, M doubles). */
+int gpx_cov_update_w(gpx_handle h, double* cov, int64_t ldcov, int64_t M, int64_t C, const double* a, const double* b,
+                     const double* wM, double* partial, int64_t ldp, void* stream);
 /* cov = K(mc, cand) - Wm^T Wc for a given design (DMMA contraction, Gram in the prologue); n = 0 gives K itself. */
 int gpx_cov_from_factors(gpx_handle h, int prologue, const double* Wm, int64_t ldm, const double* Ma_rows, int64_t M,
                          const double* Wc, int64_t ldc, const double* Cb_rows, int64_t C, int64_t n, double* cov, int64_t ldcov,
@@ -256,6 +269,10 @@ int gpx_cov_from_factors(gpx_handle h, int prologue, const double* Wm, int64_t l
 int gpx_score_ivar_partials(gpx_handle h, const double* partial, int nseg, int64_t ldp, const double* varM, int64_t M,
                             const double* varC, int64_t C, double noise, double zero_tol, const uint8_t* mask,
                             double* score_out, double* best, int64_t* idx, void* stream);
+/* ... with weighted integration points (finalisation of gpx_score_ivar_w; the partials come from gpx_cov_update_w). */
+int gpx_score_ivar_partials_w(gpx_handle h, const double* partial, int nseg, int64_t ldp, const double* varM, int64_t M,
+                              const double* varC, int64_t C, double noise, double zero_tol, const double* wM,
+                              const uint8_t* mask, double* score_out, double* best, int64_t* idx, void* stream);
 
 /* K6  MI score = num_var[j] / (1/prec_diag[j] - noise), arg-max over unmasked j
  *     (experimentalDesign.py:259-285 restated: denominator = 1/[(K_SS+noise I)^-1]_yy - noise). */
@@ -354,6 +371,7 @@ typedef struct gpx_ivar_state {
     double* pick_pivots;   /* nullable, ncap */
     double* cov;           /* nullable: resident posterior covariance M x ldcov -> rank-1 update instead of the contraction */
     int64_t ldcov, ldp;
+    const double* wM;      /* nullable: weights of the integration points (M), as in gpx_score_ivar_w */
 } gpx_ivar_state;
 
 /* discrete greedy IVAR (SURVEY.md 3.2: arg-min over c of costFunctionGP_IVAR.evaluate(design + [c]),
@@ -436,6 +454,9 @@ int gpx_coldot(gpx_handle h, const double* A, const double* B, int64_t n, int64_
 /* out[r] = scale * sum_c A[r,c], fixed order (row mean of the gradient matrix = costFunctionGP_IVAR.derivative,
  * experimentalDesign.py:166-169). */
 int gpx_rowsum(gpx_handle h, const double* A, int64_t rows, int64_t cols, int64_t ld, double scale, double* out, void* stream);
+/* out[r] = sum_c w[c] A[r,c] in the order of gpx_rowsum (weighted row reduction: derivative of a weighted IVAR cost). */
+int gpx_rowsum_w(gpx_handle h, const double* A, int64_t rows, int64_t cols, int64_t ld, const double* w, double* out,
+                 void* stream);
 
 /* out[0] = log det(U^T U) = 2 sum log U_ii  (np.linalg.slogdet at gp.py:432 for the marginal log-likelihood). */
 int gpx_logdet_chol(gpx_handle h, const double* U, int64_t n, int64_t ld, double* out, void* stream);

@@ -1,6 +1,6 @@
 """Multi-GPU parity check (run under torch.distributed.run, one rank per GPU):
-sharded greedy IVAR (scalar noise and a heteroscedastic noise function), greedy max-variance and greedy MI (scalar and
-per-point noise) must pick exactly the indices of the single-process CPU oracle."""
+sharded greedy IVAR (scalar noise, a heteroscedastic noise function and weighted integration points), greedy max-variance and
+greedy MI (scalar and per-point noise) must pick exactly the indices of the single-process CPU oracle."""
 import os
 import sys
 
@@ -37,6 +37,18 @@ def main():
         return 1e-4 + 1e-3 * p[:, 0] ** 2
     cfh = ed.costFunctionGP_IVAR(gp.GP(kern, 1e-6), 1, Space(2, None, None, noise=nu), mcPoints=mc)
     hidx = ed.performGreedyIVARExperimentalDesign(cfh, cand, 12, returnIndices=True, shard=shard)
+    # --- the same with weighted integration points: replicated with them, every rank passes the same weights ----------
+    wmc = np.exp(-np.sum(mc * mc, axis=1)) / len(mc)
+    cfw = ed.costFunctionGP_IVAR(gp.GP(kern, 1e-6), 1, Space(2, None, None), mcPoints=mc, mcWeights=wmc)
+    widx = [int(i) for i in ed.performGreedyIVARExperimentalDesign(cfw, cand, 12, returnIndices=True, shard=shard)]
+    from oracle import gpexp_oracle as orc
+    from tests.weighted_oracle import fast_greedy_ivar_w
+    wref, _ = fast_greedy_ivar_w(orc.KernelSpec.se([0.2, 0.3], 1.0, 2), cand, mc, 12, 1e-6, wmc)
+    w_ok = widx == wref   # checked on every rank
+    print("multigpu_check world=%d rank=%d weighted ivar=%s -> %s" % (world, rank, widx[:6], "OK" if w_ok else "MISMATCH"),
+          flush=True)
+    if not w_ok:
+        print("ref weighted ivar", wref, "got", widx)
     # --- greedy max variance, pool sharded ----------------------------------------------------------
     pool = rng.uniform(-1, 1, (10007, 5))
     mk = kernels.KernelIsoMatern(1.0, 1.0, 5)
@@ -97,7 +109,7 @@ def main():
         print("all ranks agree:", same, flush=True)
     dist.barrier()
     dist.destroy_process_group()
-    sys.exit(0 if (ok and same) else 1)
+    sys.exit(0 if (ok and same and w_ok) else 1)
 
 
 if __name__ == "__main__":
