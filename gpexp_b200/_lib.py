@@ -17,7 +17,7 @@ GPX_KROWS = 16
 GPX_I8_MAX_N = 16384  # largest design size the INT8 IVAR core runs
 GPX_PIVOT_HDR = 3 + GPX_MAX_DIM
 GPX_COMM_ID_BYTES = 128
-SE, MATERN32, MEHLER = 0, 1, 2
+SE, MATERN32, MEHLER, MATERN12, MATERN52 = 0, 1, 2, 3, 4
 SIDE_A, SIDE_B = 0, 1
 ROW_KERNEL, ROW_MATRIX = 0, 1
 PRO_EXPANDED, PRO_DIFF = 1, 2

@@ -131,6 +131,12 @@ extern "C" int gpx_set_kernel(gpx_handle h, int family, int d, const double* p, 
         GPX_REQUIRE(p[0] != 0.0, GPX_EINVAL, "rho must be non-zero");
         kp.c0 = sqrt(3.0) / p[0];
         kp.signal = p[1];
+    } else if (family == GPX_MATERN12 || family == GPX_MATERN52) {
+        // c0 = sqrt(2 nu) / rho, the scaling kernels.py:87-89 uses for nu = 3/2
+        GPX_REQUIRE(nparams == 2, GPX_EINVAL, "MATERN12 / MATERN52 expect rho, signalSize");
+        GPX_REQUIRE(p[0] != 0.0, GPX_EINVAL, "rho must be non-zero");
+        kp.c0 = (family == GPX_MATERN12 ? 1.0 : sqrt(5.0)) / p[0];
+        kp.signal = p[1];
     } else if (family == GPX_MEHLER) {
         GPX_REQUIRE(nparams == d, GPX_EINVAL, "MEHLER expects t[d]");
         double pref = 1.0;

@@ -159,6 +159,7 @@ extern "C" int gpx_gram(gpx_handle h, const double* X, int64_t nx, int64_t ldx, 
 // Prepared side for the tensor-core Gram prologue: k = f(e), e = sum over the d+2 rows of  A-row(i) * B-row(j).
 //   SE      e = -1/2 sum a (x-y)^2        rows q<d: (a_q x_q) * y_q ;  alpha = -1/2 sum a x^2 ;  beta = -1/2 sum a y^2
 //   MATERN  e = sum (x-y)^2               rows q<d: (-2 x_q) * y_q   ;  alpha = sum x^2        ;  beta = sum y^2
+//           (every nu; MATERN12 reports maxabs = +inf, as it has no expanded form: see gpx_expanded_form)
 //   MEHLER  e = -sum c (a x^2 - b x y + a y^2)   rows q<d: (c b x_q) * y_q ; alpha = -sum c a x^2 ; beta = -sum c a y^2
 //   row d   : alpha_i on side A, 1 on side B       row d+1 : 1 on side A, beta_j on side B       rows > d+1 : 0
 // For the stationary families the handle's centre is subtracted from every coordinate first (the kernel only sees
@@ -182,11 +183,11 @@ __global__ void __launch_bounds__(256) prep_side_kernel(const __grid_constant__ 
                     x -= ctr.c[i];
                     s = fma(x * x, kp.a[i], s);
                     r = side == GPX_SIDE_A ? x * kp.a[i] : x;
-                } else if (kp.family == GPX_MATERN32) {
+                } else if (gpx_is_matern(kp.family)) {
                     x -= ctr.c[i];
                     s = fma(x, x, s);
                     r = side == GPX_SIDE_A ? -2.0 * x : x;
-                } else {
+                } else if (kp.family == GPX_MEHLER) {
                     s = fma(x * x, kp.c[i] * kp.a[i], s);
                     r = side == GPX_SIDE_A ? kp.c[i] * kp.b[i] * x : x;
                 }
@@ -202,7 +203,7 @@ __global__ void __launch_bounds__(256) prep_side_kernel(const __grid_constant__ 
         for (int i = kp.d + 2; i < GPX_KROWS; ++i) rows[(int64_t)i * ld + j] = 0.0;
     }
     if (maxabs) {
-        double m = fabs(s);
+        double m = gpx_expanded_form(kp.family) ? fabs(s) : INFINITY;
 #pragma unroll
         for (int off = 16; off > 0; off >>= 1) m = fmax(m, __shfl_xor_sync(0xffffffffu, m, off));
         // non-negative doubles order like their bit patterns

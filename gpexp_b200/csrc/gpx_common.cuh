@@ -18,8 +18,8 @@
 struct KParams {
     int family;
     int d;
-    double signal;            // SE / MATERN32: signalSize ; MEHLER: prod_i (1 - t_i^2)^(-1/2)
-    double c0;                // MATERN32: sqrt(3) / rho
+    double signal;            // SE / MATERN*: signalSize ; MEHLER: prod_i (1 - t_i^2)^(-1/2)
+    double c0;                // MATERN12: 1 / rho ; MATERN32: sqrt(3) / rho ; MATERN52: sqrt(5) / rho
     double a[GPX_MAX_DIM];    // SE: cl_i^-2            ; MEHLER: t_i^2
     double b[GPX_MAX_DIM];    // MEHLER: 2 t_i
     double c[GPX_MAX_DIM];    // MEHLER: 1 / (2 (1 - t_i^2))
@@ -84,15 +84,40 @@ static inline bool gpx_aligned16(const void* p) { return (reinterpret_cast<uintp
 // Difference-form covariance evaluation, one dimension at a time (coordinates come from wherever
 // the caller keeps them: registers, shared memory or strided global memory).
 //   SE       kernels.py:121-122   signal * exp(-1/2 sum (x-y)^2 cl^-2)
-//   MATERN32 kernels.py:87-89     signal * (1 + sqrt3 r / rho) exp(-sqrt3 r / rho)
+//   MATERN32 kernels.py:87-89     signal * (1 + t) exp(-t),           t = sqrt3 r / rho
+//   MATERN12                      signal * exp(-t),                   t = r / rho
+//   MATERN52                      signal * (1 + t + t^2/3) exp(-t),   t = sqrt5 r / rho
 //   MEHLER   kernels.py:282-285   prod_i (1-t^2)^(-1/2) exp(-(x^2 t^2 - 2 t x y + y^2 t^2) / (2 (1-t^2)))
+// Every Matern family accumulates e = sum (x-y)^2 and finishes with t = c0 sqrt(e) and its polynomial p(t).
 // ---------------------------------------------------------------------------------------------
+__host__ __device__ constexpr bool gpx_is_matern(int fam) {
+    return fam == GPX_MATERN12 || fam == GPX_MATERN32 || fam == GPX_MATERN52;
+}
+
+// The expanded-form prologue evaluates e = alpha + beta + u.v with an absolute error delta ~ eps (|alpha| + |beta|).
+// k is smooth in e at e = 0 for SE, Mehler and Matern-3/2 and -5/2 (k = s (1 - c0^2 e / 2 + ...), resp. 1 - c0^2 e / 6),
+// so delta costs the same order relative to k.  Matern-1/2 has k = s (1 - c0 sqrt(e) + ...): a near-coincident pair
+// would lose s c0 sqrt(delta), ~3e-6 at delta = 1e-11.  That family runs the difference form only: prologue_rows refuses
+// GPX_PRO_EXPANDED, gpx_prep_side reports maxabs = +inf (so the host picks GPX_PRO_DIFF), and no expanded-form kernel
+// is instantiated for it.
+__host__ __device__ constexpr bool gpx_expanded_form(int fam) { return fam != GPX_MATERN12; }
+
+// p(t) of the Matern families: k = signal * p(t) * exp(-t)
+template <int FAM>
+__device__ __forceinline__ double matern_poly(double t) {
+    static_assert(gpx_is_matern(FAM), "not a Matern family");
+    if (FAM == GPX_MATERN32) return 1.0 + t;
+    if (FAM == GPX_MATERN52) return fma(t, fma(t, 1.0 / 3.0, 1.0), 1.0);
+    return 1.0;
+}
+
 template <int FAM>
 __device__ __forceinline__ void kacc_dim(double& acc, const KParams& kp, int i, double x, double y) {
+    static_assert(FAM == GPX_SE || gpx_is_matern(FAM) || FAM == GPX_MEHLER, "unknown kernel family");
     if (FAM == GPX_SE) {
         const double df = x - y;
         acc = fma(df * df, kp.a[i], acc);
-    } else if (FAM == GPX_MATERN32) {
+    } else if (gpx_is_matern(FAM)) {
         const double df = x - y;
         acc = fma(df, df, acc);
     } else {
@@ -104,9 +129,9 @@ __device__ __forceinline__ void kacc_dim(double& acc, const KParams& kp, int i, 
 template <int FAM>
 __device__ __forceinline__ double kfinish(double acc, const KParams& kp) {
     if (FAM == GPX_SE) return kp.signal * exp(-0.5 * acc);
-    if (FAM == GPX_MATERN32) {
+    if constexpr (gpx_is_matern(FAM)) {
         const double t = kp.c0 * sqrt(acc);
-        return kp.signal * (1.0 + t) * exp(-t);
+        return kp.signal * matern_poly<FAM>(t) * exp(-t);
     }
     return kp.signal * exp(-acc);
 }
@@ -266,9 +291,9 @@ __device__ __forceinline__ double gpx_exp_tab_scaled(double S, const double* __r
 template <int FAM>
 __device__ __forceinline__ double kfinish_tab(double acc, const KParams& kp, const double* __restrict__ tab) {
     if (FAM == GPX_SE) return gpx_exp_tab(-0.5 * acc, tab);
-    if (FAM == GPX_MATERN32) {
+    if constexpr (gpx_is_matern(FAM)) {
         const double t = kp.c0 * sqrt(acc);
-        return (1.0 + t) * gpx_exp_tab(-t, tab);
+        return matern_poly<FAM>(t) * gpx_exp_tab(-t, tab);
     }
     return gpx_exp_tab<true>(-acc, tab);
 }
@@ -276,9 +301,9 @@ __device__ __forceinline__ double kfinish_tab(double acc, const KParams& kp, con
 // Expanded form used by the tensor-core prologue:  k = kexpand(alpha(x) + beta(y) + sum_i u_i(x) v_i(y)).
 template <int FAM>
 __device__ __forceinline__ double kexpand(double e, const KParams& kp) {
-    if (FAM == GPX_MATERN32) {
+    if constexpr (gpx_is_matern(FAM)) {
         const double t = kp.c0 * sqrt(fmax(e, 0.0));
-        return kp.signal * (1.0 + t) * exp(-t);
+        return kp.signal * matern_poly<FAM>(t) * exp(-t);
     }
     return kp.signal * exp(e);
 }
@@ -307,8 +332,14 @@ __device__ __forceinline__ double kexpand(double e, const KParams& kp) {
         } else if ((fam) == GPX_MATERN32) {                   \
             constexpr int FAM = GPX_MATERN32;                 \
             __VA_ARGS__;                                      \
-        } else {                                              \
+        } else if ((fam) == GPX_MEHLER) {                     \
             constexpr int FAM = GPX_MEHLER;                   \
+            __VA_ARGS__;                                      \
+        } else if ((fam) == GPX_MATERN12) {                   \
+            constexpr int FAM = GPX_MATERN12;                 \
+            __VA_ARGS__;                                      \
+        } else if ((fam) == GPX_MATERN52) {                   \
+            constexpr int FAM = GPX_MATERN52;                 \
             __VA_ARGS__;                                      \
         }                                                     \
     } while (0)

@@ -44,9 +44,9 @@ namespace {
 // need (tab[j] = -signal * 2^(j/256)), so these return -k(x,y) without a negation per element.
 template <int FAM>
 __device__ __forceinline__ double neg_kexpand_tab(double e, const KParams& kp, const double* __restrict__ ntab) {
-    if (FAM == GPX_MATERN32) {
+    if constexpr (gpx_is_matern(FAM)) {
         const double t = kp.c0 * sqrt(fmax(e, 0.0));
-        return (1.0 + t) * gpx_exp_tab(-t, ntab);
+        return matern_poly<FAM>(t) * gpx_exp_tab(-t, ntab);
     }
     return gpx_exp_tab<FAM == GPX_MEHLER>(e, ntab);
 }
@@ -974,23 +974,41 @@ int launch_ivar_ws_ring(gpx_handle h, const CoreArgs& a, dim3 grid, cudaStream_t
     return gpx_check_launch("ivar_ws");
 }
 
+// Prologue-evaluating kernels exist for (FAM, PRO) only where the family allows the form (gpx_expanded_form); the
+// launchers below refuse the rest without instantiating them.  prologue_rows has refused such a call before it gets here.
+template <int FAM, int PRO>
+constexpr bool has_prologue = PRO != PRO_EXPANDED || gpx_expanded_form(FAM);
+
+static int no_prologue() {
+    gpx_set_error("dmma core: GPX_PRO_EXPANDED is not available for this kernel family");
+    return GPX_EINVAL;
+}
+
 template <int FAM, int PRO, bool WT>
 int launch_ivar_ws(gpx_handle h, const CoreArgs& a, dim3 grid, cudaStream_t st) {
-    // every prologue fits one chunk of every ring (EXPANDED <= 16 rows, DIFF <= 16 coordinates, chunks >= 24 rows)
-    switch (h->ivar_ring) {
-        case 1: return launch_ivar_ws_ring<FAM, PRO, RingSync, true, WT>(h, a, grid, st);
-        case 2: return launch_ivar_ws_ring<FAM, PRO, RingDeep, true, WT>(h, a, grid, st);
-        default: return launch_ivar_ws_ring<FAM, PRO, RingSync, false, WT>(h, a, grid, st);
+    if constexpr (!has_prologue<FAM, PRO>) {
+        return no_prologue();
+    } else {
+        // every prologue fits one chunk of every ring (EXPANDED <= 16 rows, DIFF <= 16 coordinates, chunks >= 24 rows)
+        switch (h->ivar_ring) {
+            case 1: return launch_ivar_ws_ring<FAM, PRO, RingSync, true, WT>(h, a, grid, st);
+            case 2: return launch_ivar_ws_ring<FAM, PRO, RingDeep, true, WT>(h, a, grid, st);
+            default: return launch_ivar_ws_ring<FAM, PRO, RingSync, false, WT>(h, a, grid, st);
+        }
     }
 }
 
 template <int FAM, int EPI, int PRO, bool WT = false>
 int launch_core(gpx_handle h, const CoreArgs& a, int64_t jt, int64_t it_or_splits, cudaStream_t st) {
-    dim3 grid((unsigned)jt, (unsigned)it_or_splits);
-    int rc = gpx_ensure_smem(h, (const void*)dmma_core_kernel<FAM, EPI, PRO, WT>, Cfg::SMEM_BYTES, "dmma core");
-    if (rc) return rc;
-    dmma_core_kernel<FAM, EPI, PRO, WT><<<grid, Cfg::NT, Cfg::SMEM_BYTES, st>>>(a, h->kp);
-    return gpx_check_launch("dmma core");
+    if constexpr (!has_prologue<FAM, PRO>) {
+        return no_prologue();
+    } else {
+        dim3 grid((unsigned)jt, (unsigned)it_or_splits);
+        int rc = gpx_ensure_smem(h, (const void*)dmma_core_kernel<FAM, EPI, PRO, WT>, Cfg::SMEM_BYTES, "dmma core");
+        if (rc) return rc;
+        dmma_core_kernel<FAM, EPI, PRO, WT><<<grid, Cfg::NT, Cfg::SMEM_BYTES, st>>>(a, h->kp);
+        return gpx_check_launch("dmma core");
+    }
 }
 
 int check_operand(const double* p, int64_t ld, const char* name) {
@@ -1001,11 +1019,15 @@ int check_operand(const double* p, int64_t ld, const char* name) {
     return GPX_OK;
 }
 
-// rows of the prologue chunk for this handle's kernel, or < 0 if the form cannot be used
-int prologue_rows(gpx_handle h, int prologue) {
-    if (prologue == PRO_DIFF) return h->kp.d;
-    if (prologue == PRO_EXPANDED && h->kp.d + 2 <= GPX_KROWS) return (h->kp.d + 2 + 3) & ~3;
-    return -1;
+// rows of the prologue chunk for this handle's kernel in *rows, or an error code if the form cannot be used
+int prologue_rows(gpx_handle h, int prologue, int* rows) {
+    GPX_REQUIRE(prologue != PRO_EXPANDED || gpx_expanded_form(h->kp.family), GPX_EINVAL,
+                "GPX_PRO_EXPANDED is not available for GPX_MATERN12 (k = s exp(-c0 sqrt(e)) is not smooth in e at e = 0): "
+                "use GPX_PRO_DIFF");
+    GPX_REQUIRE(prologue == PRO_DIFF || (prologue == PRO_EXPANDED && h->kp.d + 2 <= GPX_KROWS), GPX_ESIZE,
+                "prologue must be GPX_PRO_DIFF, or GPX_PRO_EXPANDED with d <= GPX_KROWS - 2");
+    *rows = prologue == PRO_DIFF ? h->kp.d : (h->kp.d + 2 + 3) & ~3;
+    return GPX_OK;
 }
 
 // ---------------------------------------------------------------------------------------------
@@ -1432,6 +1454,18 @@ static int ivar_splits_for(gpx_handle h, int64_t M, int64_t C, int bm, int bn = 
 }
 int gpx_ivar_splits(gpx_handle, int64_t, int64_t) { return 32; }  // workspace bound: never more than 32 splits
 
+template <int FAM, int PRO, bool WT>
+static int launch_i8(gpx_handle h, const I8Args& a, const I8Maps& maps, dim3 grid, cudaStream_t st) {
+    if constexpr (!has_prologue<FAM, PRO>) {
+        return no_prologue();
+    } else {
+        int rc = gpx_ensure_smem(h, (const void*)ivar_i8_kernel<FAM, PRO, WT>, I8_SMEM_BYTES, "ivar_i8");
+        if (rc) return rc;
+        ivar_i8_kernel<FAM, PRO, WT><<<grid, I8_THREADS, I8_SMEM_BYTES, st>>>(a, h->kp, maps);
+        return gpx_check_launch("ivar_i8");
+    }
+}
+
 // INT8 core: slice both factors into the handle's scratch, then one ivar_i8_kernel launch (same workspace contract as
 // ivar_ws_kernel: partial column sums per M-split)
 static int launch_ivar_i8(gpx_handle h, int prologue, const double* Wm, int64_t ldm, const double* Ma_rows, int64_t M,
@@ -1474,28 +1508,22 @@ static int launch_ivar_i8(gpx_handle h, int prologue, const double* Wm, int64_t 
     a.wM = wM;
     *nsplit_out = splits;
     const dim3 grid((unsigned)(jt * splits), 1u);
-#define GPX_I8_LAUNCH(F, P, W)                                                                                     \
-    do {                                                                                                           \
-        if ((rc = gpx_ensure_smem(h, (const void*)ivar_i8_kernel<F, P, W>, I8_SMEM_BYTES, "ivar_i8"))) return rc; \
-        ivar_i8_kernel<F, P, W><<<grid, I8_THREADS, I8_SMEM_BYTES, st>>>(a, h->kp, maps);                         \
-    } while (0)
     if (prologue == PRO_DIFF) {
-        if (wM) GPX_DISPATCH_FAMILY(h->kp.family, GPX_I8_LAUNCH(FAM, PRO_DIFF, true));
-        else GPX_DISPATCH_FAMILY(h->kp.family, GPX_I8_LAUNCH(FAM, PRO_DIFF, false));
+        if (wM) GPX_DISPATCH_FAMILY(h->kp.family, rc = (launch_i8<FAM, PRO_DIFF, true>(h, a, maps, grid, st)));
+        else GPX_DISPATCH_FAMILY(h->kp.family, rc = (launch_i8<FAM, PRO_DIFF, false>(h, a, maps, grid, st)));
     } else {
-        if (wM) GPX_DISPATCH_FAMILY(h->kp.family, GPX_I8_LAUNCH(FAM, PRO_EXPANDED, true));
-        else GPX_DISPATCH_FAMILY(h->kp.family, GPX_I8_LAUNCH(FAM, PRO_EXPANDED, false));
+        if (wM) GPX_DISPATCH_FAMILY(h->kp.family, rc = (launch_i8<FAM, PRO_EXPANDED, true>(h, a, maps, grid, st)));
+        else GPX_DISPATCH_FAMILY(h->kp.family, rc = (launch_i8<FAM, PRO_EXPANDED, false>(h, a, maps, grid, st)));
     }
-#undef GPX_I8_LAUNCH
-    return gpx_check_launch("ivar_i8");
+    return rc;
 }
 
 int gpx_launch_core_ivar(gpx_handle h, int prologue, const double* Wm, int64_t ldm, const double* Ma_rows, int64_t M,
                          const double* Wc, int64_t ldc, const double* Cb_rows, int64_t C, int64_t n, const double* wM,
                          double* partial, int64_t ldp, int* nsplit_out, cudaStream_t st) {
     int rc;
-    const int prows = prologue_rows(h, prologue);
-    GPX_REQUIRE(prows >= 0, GPX_ESIZE, "prologue must be GPX_PRO_DIFF, or GPX_PRO_EXPANDED with d <= GPX_KROWS - 2");
+    int prows;
+    if ((rc = prologue_rows(h, prologue, &prows))) return rc;
     if ((rc = check_operand(Ma_rows, ldm, "Ma_rows"))) return rc;
     if ((rc = check_operand(Cb_rows, ldc, "Cb_rows"))) return rc;
     if (n > 0) {
@@ -1569,8 +1597,8 @@ int gpx_launch_core_store(gpx_handle h, int prologue, const double* A, int64_t l
                           const double* B, int64_t ldb, const double* Bp, int64_t J, int64_t K, double* out, int64_t ldo,
                           cudaStream_t st) {
     int rc;
-    const int prows = prologue_rows(h, prologue);
-    GPX_REQUIRE(prows >= 0, GPX_ESIZE, "prologue must be GPX_PRO_DIFF, or GPX_PRO_EXPANDED with d <= GPX_KROWS - 2");
+    int prows;
+    if ((rc = prologue_rows(h, prologue, &prows))) return rc;
     if ((rc = check_operand(Ap, lda, "Ap"))) return rc;
     if ((rc = check_operand(Bp, ldb, "Bp"))) return rc;
     if ((rc = check_operand(out, ldo, "out"))) return rc;

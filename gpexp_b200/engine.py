@@ -94,7 +94,7 @@ def prior_scale(family: int, params) -> float:
     params = np.asarray(params, dtype=np.float64)
     if family == _lib.SE:
         return float(abs(params[-1]))
-    if family == _lib.MATERN32:
+    if family in (_lib.MATERN12, _lib.MATERN32, _lib.MATERN52):
         return float(abs(params[1]))
     return float(np.prod((1.0 - params ** 2.0) ** -0.5))
 

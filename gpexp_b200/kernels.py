@@ -57,10 +57,17 @@ def _evaluateF(self, x1, x2):
     return out[:n].cpu().numpy()
 
 
+# nu -> family.  The reference implements nu = 3/2 only; nu = 1/2 and 5/2 are served here as well (under
+# install_as_gpExp() too, where the unmodified reference would raise).  Its 1e-10 tolerance on nu is kept.
+_MATERN_NU = ((0.5, _lib.MATERN12), (1.5, _lib.MATERN32), (2.5, _lib.MATERN52))
+
+
 def _matern_spec(self):
-    if np.abs(1.5 - self.nu) >= 1e-10:  # the reference leaves `out` unbound for other nu (kernels.py:85-91)
-        raise UnboundLocalError("KernelIsoMatern is implemented for nu = 3/2 only")
-    return _lib.MATERN32, self.dimension, [self.hyperParam['rho'], self.hyperParam['signalSize']]
+    for nu, family in _MATERN_NU:
+        if np.abs(nu - self.nu) < 1e-10:
+            return family, self.dimension, [self.hyperParam['rho'], self.hyperParam['signalSize']]
+    # the reference leaves `out` unbound for any other nu (kernels.py:85-91)
+    raise UnboundLocalError("KernelIsoMatern is implemented for nu = 1/2, 3/2 and 5/2 only")
 
 
 def _se_spec(self):
@@ -138,7 +145,8 @@ class Kernel(object):
 
 @_attach
 class KernelIsoMatern(Kernel):
-    """Isotropic Matern, nu = 3/2; hyper-parameters rho, signalSize (kernels.py:72-91)."""
+    """Isotropic Matern, nu = 1/2, 3/2 or 5/2; hyper-parameters rho, signalSize (kernels.py:72-91, which has nu = 3/2
+    only)."""
 
     def __init__(self, rho, signalSize, dimension, nu=1.5):
         self.nu = nu  # not a hyper-parameter (kernels.py:76)

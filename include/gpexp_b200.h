@@ -42,6 +42,9 @@ extern "C" {
 #define GPX_SE 0       /* KernelSquaredExponential, iso or ARD      kernels.py:100-123     */
 #define GPX_MATERN32 1 /* KernelIsoMatern, nu = 3/2                 kernels.py:72-91       */
 #define GPX_MEHLER 2   /* KernelMehlerND / KernelMehler1D           kernels.py:183-293     */
+#define GPX_MATERN12 3 /* KernelIsoMatern, nu = 1/2 (exponential / Ornstein-Uhlenbeck): s e^-t, t = |x - y| / rho.
+                          Difference-form prologue only: GPX_PRO_EXPANDED is refused (see gpx_prep_side)       */
+#define GPX_MATERN52 4 /* KernelIsoMatern, nu = 5/2: s (1 + t + t^2/3) e^-t, t = sqrt5 |x - y| / rho          */
 
 /* error codes */
 #define GPX_OK 0
@@ -81,7 +84,9 @@ int gpx_destroy(gpx_handle h);
  * i.e. they live in the constant bank (ARD length-scales in constant memory).
  *   GPX_SE       params_host = cl[0..d) , signalSize           (nparams = d+1)  kernels.py:103-111
  *   GPX_MATERN32 params_host = rho, signalSize                 (nparams = 2)    kernels.py:74-78
- *   GPX_MEHLER   params_host = t[0..d)                          (nparams = d)    kernels.py:185-189 */
+ *   GPX_MEHLER   params_host = t[0..d)                          (nparams = d)    kernels.py:185-189
+ *   GPX_MATERN12 params_host = rho, signalSize                 (nparams = 2)    as GPX_MATERN32, nu = 1/2
+ *   GPX_MATERN52 params_host = rho, signalSize                 (nparams = 2)    as GPX_MATERN32, nu = 5/2 */
 int gpx_set_kernel(gpx_handle h, int family, int d, const double* params_host, int nparams);
 
 /* a1  Kernel.evaluate (kernels.py:49-65): out[j] = k(X[j], Y[j]); nx == ny, or one of them 1
@@ -118,7 +123,9 @@ int gpx_set_center(gpx_handle h, const double* center_host);
 /* Prepared side of a point set for the GPX_PRO_EXPANDED prologue: k(x,y) = f(sum_r rowsA[r][i] * rowsB[r][j]) with
  *     rows  : GPX_KROWS x ld = d scaled coordinates, then (alpha_i | 1) and (1 | beta_j) for side A | B, then zeros;
  *     maxabs (nullable, device): max |alpha| resp. |beta| -- the expanded form loses eps * (max|alpha| + max|beta|) to
- *     cancellation, so the caller switches to GPX_PRO_DIFF when that exceeds its tolerance (1e-11 in gpexp_b200). */
+ *     cancellation, so the caller switches to GPX_PRO_DIFF when that exceeds its tolerance (1e-11 in gpexp_b200).
+ *     GPX_MATERN12 reports +inf: k = s e^-t has an infinite slope in e = |x - y|^2 at e = 0, so an absolute error
+ *     delta of e costs a near-coincident pair ~ s c0 sqrt(delta), and the tensor-core routines refuse the form. */
 int gpx_prep_side(gpx_handle h, int side, const double* X, int64_t n, int64_t ldx, double* rows, int64_t ld,
                   double* maxabs, void* stream);
 
