@@ -22,6 +22,22 @@ Pinning: the reference ships no tests or golden vectors
 pinned against outputs of the *unmodified reference itself*, imported in the
 build container by ``tests/golden/make_golden.py`` and frozen in
 ``tests/golden/*.npz`` (indices, per-step scores, variances, Gram matrices).
+
+Each criterion also takes the variants the CUDA path supports, as optional
+arguments whose defaults give the plain forms above:
+
+* per-point noise -- ``ref_ivar_cost`` takes a nugget vector, ``ref_greedy_ivar``
+  a ``noise_func`` giving the nugget of design+{c}, ``fast_ivar_scores`` /
+  ``fast_greedy_ivar`` a per-candidate vector nu, and the three MI functions a
+  per-point vector nu (K_AA + diag nu_A, K_SS + diag nu_S);
+* weighted integration points -- ``mc_weights`` w makes the IVAR cost
+  |sum_m w_m var(x_m)| instead of the Monte-Carlo mean.  Every weighted square
+  is formed as (w v) v, the form the kernels use, so that w = 2^-k scales each
+  term exactly: with M = 2^k and w = 1/M it reproduces the unweighted cost bit
+  for bit;
+* Matern nu = 1/2 and nu = 5/2 kernels -- ``KernelSpec.matern12`` /
+  ``matern52``, k = s p(t) exp(-t) with t = sqrt(2 nu) |x - y| / rho, the
+  scaling the reference uses for nu = 3/2 (kernels.py:87-89).
 """
 from __future__ import annotations
 
@@ -33,8 +49,21 @@ import numpy as np
 SE = 0
 MATERN32 = 1
 MEHLER = 2
+MATERN12 = 3
+MATERN52 = 4
 
-FAMILY_NAMES = {SE: "se", MATERN32: "matern32", MEHLER: "mehler"}
+FAMILY_NAMES = {SE: "se", MATERN32: "matern32", MEHLER: "mehler", MATERN12: "matern12", MATERN52: "matern52"}
+MATERN_NU = {MATERN12: 0.5, MATERN32: 1.5, MATERN52: 2.5}
+
+
+def matern_closed_form(nu, r, rho, s):
+    """s p(t) exp(-t), t = sqrt(2 nu) r / rho, for nu in {1/2, 3/2, 5/2}; r an array of distances.
+        nu = 1/2   p = 1
+        nu = 3/2   p = 1 + t
+        nu = 5/2   p = 1 + t + t^2 / 3"""
+    t = np.sqrt(2.0 * nu) * np.asarray(r, dtype=np.float64) / rho
+    p = {0.5: 1.0, 1.5: 1.0 + t, 2.5: 1.0 + t + t * t / 3.0}[nu]
+    return s * p * np.exp(-t)
 
 
 # --------------------------------------------------------------------------
@@ -47,6 +76,7 @@ class KernelSpec:
     family SE        params: cl[d] (correlation lengths), signal   kernels.py:103-123
     family MATERN32  params: rho, signal                           kernels.py:74-91
     family MEHLER    params: t[d]                                  kernels.py:183-228, :250-293
+    family MATERN12, MATERN52  params: rho, signal                 matern_closed_form
     """
 
     family: int
@@ -68,6 +98,14 @@ class KernelSpec:
     @staticmethod
     def matern32(rho, signal, dim):
         return KernelSpec(MATERN32, dim, rho=float(rho), signal=float(signal))
+
+    @staticmethod
+    def matern12(rho, signal, dim):
+        return KernelSpec(MATERN12, dim, rho=float(rho), signal=float(signal))
+
+    @staticmethod
+    def matern52(rho, signal, dim):
+        return KernelSpec(MATERN52, dim, rho=float(rho), signal=float(signal))
 
     @staticmethod
     def mehler(t, dim):
@@ -95,6 +133,9 @@ class KernelSpec:
                     -(a ** 2.0 * t ** 2.0 - 2.0 * t * a * b + b ** 2.0 * t ** 2.0)
                     / (2.0 * (1.0 - t ** 2.0))))
             return out
+        if self.family in (MATERN12, MATERN52):
+            d = np.sqrt(np.sum((x1 - x2) ** 2.0, axis=1))
+            return matern_closed_form(MATERN_NU[self.family], d, self.rho, self.signal)
         raise ValueError("unknown kernel family")
 
     # ---- evaluate: pairwise with (1,d) broadcast        kernels.py:49-65 --
@@ -136,6 +177,12 @@ class KernelSpec:
                     -(a ** 2.0 * t ** 2.0 - 2.0 * t * a * b + b ** 2.0 * t ** 2.0)
                     / (2.0 * (1.0 - t ** 2.0))))
             return out
+        if self.family in (MATERN12, MATERN52):
+            acc = np.zeros((X.shape[0], Y.shape[0]))
+            for i in range(self.dim):
+                diff = X[:, i:i + 1] - Y[None, :, i]
+                acc += diff ** 2.0
+            return matern_closed_form(MATERN_NU[self.family], np.sqrt(acc), self.rho, self.signal)
         raise ValueError("unknown kernel family")
 
     def prior(self, X):
@@ -146,7 +193,7 @@ class KernelSpec:
         """Flat parameter vector in the order the C ABI expects (include/gpexp_b200.h)."""
         if self.family == SE:
             return np.concatenate([self.cl, [self.signal]])
-        if self.family == MATERN32:
+        if self.family in (MATERN32, MATERN12, MATERN52):
             return np.array([self.rho, self.signal])
         return self.t.copy()
 
@@ -188,15 +235,18 @@ def ref_evaluate_variance(kern, nodes, precision, newpt):
     return var
 
 
-def ref_ivar_cost(kern, design, mc, noise):
+def ref_ivar_cost(kern, design, mc, noise, mc_weights=None):
     """experimentalDesign.py:105-117 -- |mean posterior variance over the MC points|.
 
     ``noise`` is a float (homoscedastic gp.noise) or an ndarray of per-point
-    nuggets (the space.noiseFunc branch, :110-114).
+    nuggets (the space.noiseFunc branch, :110-114).  With ``mc_weights`` w the
+    cost is |sum_m w_m var(x_m)|.
     """
     _, prec = ref_add_nodes(kern, design, noise)
     var_mc = ref_evaluate_variance(kern, design, prec, mc)
-    return abs(1.0 / float(mc.shape[0]) * np.sum(var_mc))
+    if mc_weights is None:
+        return abs(1.0 / float(mc.shape[0]) * np.sum(var_mc))
+    return abs(np.sum(mc_weights * var_mc))
 
 
 def ref_greedy_var(kern, pool, n_points, weights=None, ind_keep_start=()):
@@ -231,11 +281,13 @@ def ref_greedy_var(kern, pool, n_points, weights=None, ind_keep_start=()):
     return ind, scores
 
 
-def ref_greedy_ivar(kern, cand, mc, n_points, noise, cand_subset=None):
+def ref_greedy_ivar(kern, cand, mc, n_points, noise, cand_subset=None, *, mc_weights=None, noise_func=None):
     """Discrete greedy IVAR as SURVEY.md section 8(c) defines it (the reference has the
     cost function, experimentalDesign.py:79-117, but no discrete driver): at each step
     evaluate the reference IVAR cost of design+{c} for every candidate c and take
-    np.argmin.  Returns (indices, per-step cost vectors)."""
+    np.argmin.  With ``noise_func`` the nugget of design+{c} is noise_func(design+{c})
+    (the reference's heteroscedastic branch, :110-114) and ``noise`` is not used.
+    Returns (indices, per-step cost vectors)."""
     ind = []
     costs = []
     cs = range(cand.shape[0]) if cand_subset is None else cand_subset
@@ -243,33 +295,38 @@ def ref_greedy_ivar(kern, cand, mc, n_points, noise, cand_subset=None):
         cost = np.full(cand.shape[0], np.inf)
         for c in cs:
             pts = np.vstack([cand[ind, :], cand[c:c + 1, :]])
-            cost[c] = ref_ivar_cost(kern, pts, mc, noise)
+            nugget = noise if noise_func is None else noise_func(pts)
+            cost[c] = ref_ivar_cost(kern, pts, mc, nugget, mc_weights)
         costs.append(cost)
         ind.append(int(np.argmin(cost)))
     return ind, costs
 
 
 def ref_mi_cost(kern, pool, noise, index, index_added):
-    """experimentalDesign.py:252-285 -- var(y|A) / var(y|V minus A minus y), two pinv's."""
+    """experimentalDesign.py:252-285 -- var(y|A) / var(y|V minus A minus y), two pinv's.
+
+    ``noise`` is a float or a per-point vector nu, which each subset's Gram takes on
+    that subset: K_AA + diag nu_A and K_SS + diag nu_S, S = V minus A minus y."""
+    vec = np.ndim(noise) > 0
     dim = pool.shape[1]
     point = pool[index, :].reshape(1, dim)
     var = kern.evaluate(point, point)
     added = pool[index_added, :].reshape(len(index_added), dim)
     kva = kern.evaluate(added, point)
-    cov_num = ref_covariance_matrix(kern, added, noise)
+    cov_num = ref_covariance_matrix(kern, added, noise[index_added] if vec else noise)
     numerator = var - np.dot(kva.T, np.dot(np.linalg.pinv(cov_num), kva))
     left = np.setdiff1d(np.arange(pool.shape[0]), index_added)
     left = np.setdiff1d(left, [index])
     pts_left = pool[left, :]
     kvl = kern.evaluate(pts_left, point)
-    cov_den = ref_covariance_matrix(kern, pts_left, noise)
+    cov_den = ref_covariance_matrix(kern, pts_left, noise[left] if vec else noise)
     denominator = var - np.dot(kvl.T, np.dot(np.linalg.pinv(cov_den), kvl))
     return numerator / denominator
 
 
 def ref_greedy_mi(kern, pool, noise, n_points, start=0):
-    """experimentalDesign.py:753-785.  Returns (indices, per-step score vectors over the
-    remaining options, per-step option index arrays)."""
+    """experimentalDesign.py:753-785; ``noise`` as in ref_mi_cost.  Returns (indices, per-step
+    score vectors over the remaining options, per-step option index arrays)."""
     ind = [start]
     options = np.setdiff1d(np.arange(pool.shape[0]), ind)
     scores, opts = [], []
@@ -328,24 +385,30 @@ def fast_greedy_var(kern, pool, n_points, weights=None, ind_keep_start=()):
     return ind, scores
 
 
-def fast_ivar_scores(kern, cand, mc, w_m, var_m, w_c, var_c, noise, block=4096):
+def fast_ivar_scores(kern, cand, mc, w_m, var_m, w_c, var_c, noise, block=4096, *, mc_weights=None):
     """IVAR cost of design+{c} for every candidate c via the Schur identity (SURVEY.md 3.2):
 
         cost[c] = | mean_m var_D(m) - (1/M) sum_m cov_D(m,c)^2 / (var_D(c) + noise) |
         cov_D(m,c) = k(m,c) - W_M[:,m] . W_C[:,c]
 
+    ``noise`` is a scalar or a per-candidate vector nu.  With ``mc_weights`` w the mean and
+    (1/M) sum_m cov^2 become sum_m w_m var_D(m) and sum_m (w_m cov) cov.
     The reduction is 0 where var_D(c)+noise is numerically zero (SURVEY.md section 7,
     duplicate-candidate rule: pinv drops the null direction)."""
     m = mc.shape[0]
     c = cand.shape[0]
-    base = np.sum(var_m) / m
+    base = np.sum(var_m) / m if mc_weights is None else np.sum(mc_weights * var_m)
     r = np.zeros(c)
     for c0 in range(0, c, block):
         cov = kern.gram(mc, cand[c0:c0 + block]) - w_m.T @ w_c[:, c0:c0 + block]
-        r[c0:c0 + block] = np.sum(cov * cov, axis=0)
+        wcov = cov if mc_weights is None else mc_weights[:, None] * cov
+        r[c0:c0 + block] = np.sum(wcov * cov, axis=0)
     den = var_c + noise
     tiny = den <= ZERO_VAR_TOL * kern_scale(kern, cand)
-    red = np.where(tiny, 0.0, r / np.where(tiny, 1.0, den) / m)
+    red = r / np.where(tiny, 1.0, den)
+    if mc_weights is None:
+        red = red / m
+    red = np.where(tiny, 0.0, red)
     return np.abs(base - red)
 
 
@@ -359,20 +422,23 @@ def kern_scale(kern, pts=None):
     return abs(kern.signal)
 
 
-def fast_greedy_ivar(kern, cand, mc, n_points, noise):
+def fast_greedy_ivar(kern, cand, mc, n_points, noise, *, mc_weights=None):
     """Incremental greedy IVAR (SURVEY.md 3.2): append one row to W_M and W_C per step with
-    divisor sqrt(var_D(p)+noise), running var updates.  Returns (indices, per-step costs)."""
+    divisor sqrt(var_D(p)+nu[p]), running var updates.  ``noise`` is a scalar or a
+    per-candidate vector nu; integration points carry no noise.  ``mc_weights`` as in
+    fast_ivar_scores.  Returns (indices, per-step costs)."""
     c, m = cand.shape[0], mc.shape[0]
+    nu = np.broadcast_to(noise, (c,))
     w_c = np.zeros((n_points, c))
     w_m = np.zeros((n_points, m))
     var_c = kern.prior(cand).copy()
     var_m = kern.prior(mc).copy()
     ind, costs = [], []
     for n in range(n_points):
-        cost = fast_ivar_scores(kern, cand, mc, w_m[:n], var_m, w_c[:n], var_c, noise)
+        cost = fast_ivar_scores(kern, cand, mc, w_m[:n], var_m, w_c[:n], var_c, nu, mc_weights=mc_weights)
         costs.append(cost)
         p = int(np.argmin(cost))
-        lnn = math.sqrt(var_c[p] + noise)
+        lnn = math.sqrt(var_c[p] + nu[p])
         col = w_c[:n, p].copy()
         row_c = (kern.gram(cand[p:p + 1], cand)[0] - col @ w_c[:n, :]) / lnn
         row_m = (kern.gram(cand[p:p + 1], mc)[0] - col @ w_m[:n, :]) / lnn
@@ -384,22 +450,26 @@ def fast_greedy_ivar(kern, cand, mc, n_points, noise):
     return ind, costs
 
 
-def fast_greedy_mi(kern, pool, noise, n_points, start=0):
+def fast_greedy_mi(kern, pool, noise, n_points, start=0, *, with_pivots=False):
     """Greedy MI with the exact restatement of SURVEY.md 3.3:
 
         numerator(y)   = var(y | A)                 (incremental pivoted-Cholesky rows, nugget=noise)
         denominator(y) = 1 / [(K_SS + noise I)^-1]_yy - noise,   S = V minus A  (y in S)
 
-    and a rank-1 downdate of the precision when a point leaves S.  Returns
-    (indices, per-step score vectors of length |V| with selected entries = -inf)."""
+    and a rank-1 downdate of the precision when a point leaves S.  ``noise`` is a scalar or
+    a per-point vector nu: the precision is (K_VV + diag nu)^-1, the appended rows are divided
+    by sqrt(num[p] + nu[p]) and the denominator is 1/pd[y] - nu[y].  Returns (indices, per-step
+    score vectors of length |V| with selected entries = -inf), and with ``with_pivots`` the
+    per-step pivots num[p] + nu[p] as a third value."""
     v = pool.shape[0]
-    kvv = kern.gram(pool, pool) + noise * np.eye(v)
+    nu = np.broadcast_to(noise, (v,))
+    kvv = kern.gram(pool, pool) + np.diag(nu)
     prec = np.linalg.inv(kvv)
     prior = kern.prior(pool)
     num = prior.copy()
     w = np.zeros((n_points, v))
     selected = np.zeros(v, dtype=bool)
-    ind, scores = [], []
+    ind, scores, pivots = [], [], []
     pd = np.diag(prec).copy()
     us = []
 
@@ -412,7 +482,8 @@ def fast_greedy_mi(kern, pool, noise, n_points, start=0):
     def take(p):
         nonlocal pd
         n = len(ind)
-        lnn = math.sqrt(num[p] + noise)
+        pivots.append(num[p] + nu[p])
+        lnn = math.sqrt(pivots[-1])
         row = (kern.gram(pool[p:p + 1], pool)[0] - w[:n, p] @ w[:n, :]) / lnn
         w[n, :] = row
         num[:] = num - row * row
@@ -425,11 +496,11 @@ def fast_greedy_mi(kern, pool, noise, n_points, start=0):
 
     take(start)
     while len(ind) < n_points:
-        den = 1.0 / np.where(selected, 1.0, pd) - noise
+        den = 1.0 / np.where(selected, 1.0, pd) - nu
         s = np.where(selected, -np.inf, num / den)
         scores.append(s)
         take(int(np.argmax(s)))
-    return ind, scores
+    return (ind, scores, pivots) if with_pivots else (ind, scores)
 
 
 # --------------------------------------------------------------------------

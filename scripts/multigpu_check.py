@@ -42,8 +42,7 @@ def main():
     cfw = ed.costFunctionGP_IVAR(gp.GP(kern, 1e-6), 1, Space(2, None, None), mcPoints=mc, mcWeights=wmc)
     widx = [int(i) for i in ed.performGreedyIVARExperimentalDesign(cfw, cand, 12, returnIndices=True, shard=shard)]
     from oracle import gpexp_oracle as orc
-    from tests.weighted_oracle import fast_greedy_ivar_w
-    wref, _ = fast_greedy_ivar_w(orc.KernelSpec.se([0.2, 0.3], 1.0, 2), cand, mc, 12, 1e-6, wmc)
+    wref, _ = orc.fast_greedy_ivar(orc.KernelSpec.se([0.2, 0.3], 1.0, 2), cand, mc, 12, 1e-6, mc_weights=wmc)
     w_ok = widx == wref   # checked on every rank
     print("multigpu_check world=%d rank=%d weighted ivar=%s -> %s" % (world, rank, widx[:6], "OK" if w_ok else "MISMATCH"),
           flush=True)
@@ -70,14 +69,12 @@ def main():
     hmidx, hminfo = [int(i) for i in cfm.lastIndices], int(cfm.lastEngine.info.item())
     torch.cuda.synchronize()
     if rank == 0:
-        from oracle import gpexp_oracle as orc
-        from tests.hetero_mi_oracle import fast_greedy_mi_nu
         mref, _ = orc.fast_greedy_mi(orc.KernelSpec.mehler([0.9, 0.9, 0.9], 3), vpool, 1e-2, 14, start=0)
         mi_ok = [int(i) for i in midx] == mref and minfo == 0
         print("multigpu_check world=%d mi=%s -> %s" % (world, [int(i) for i in midx][:8], "OK" if mi_ok else "MISMATCH"), flush=True)
         if not mi_ok:
             print("ref mi", mref, "got", [int(i) for i in midx], "info", minfo)
-        hmref, _, _ = fast_greedy_mi_nu(orc.KernelSpec.mehler([0.9, 0.9, 0.9], 3), vpool, vnu, 14, start=0)
+        hmref, _ = orc.fast_greedy_mi(orc.KernelSpec.mehler([0.9, 0.9, 0.9], 3), vpool, vnu, 14, start=0)
         ed.performGreedyMIExperimentalDesign(cfm, 14, start=0)   # the same design on this GPU alone
         hm_one = [int(i) for i in cfm.lastIndices]
         hm_ok = hmidx == hmref == hm_one and hminfo == 0
@@ -87,8 +84,7 @@ def main():
         mi_ok = mi_ok and hm_ok
         ref, _ = orc.fast_greedy_ivar(orc.KernelSpec.se([0.2, 0.3], 1.0, 2), cand, mc, 12, 1e-6)
         vref, _ = orc.fast_greedy_var(orc.KernelSpec.matern32(1.0, 1.0, 5), pool, 25)
-        from tests.hetero_oracle import fast_greedy_ivar_nu
-        href, _ = fast_greedy_ivar_nu(orc.KernelSpec.se([0.2, 0.3], 1.0, 2), cand, mc, 12, nu(cand))
+        href, _ = orc.fast_greedy_ivar(orc.KernelSpec.se([0.2, 0.3], 1.0, 2), cand, mc, 12, nu(cand))
         h_ok = [int(i) for i in hidx] == href
         print("multigpu_check world=%d hetero ivar=%s -> %s" % (world, [int(i) for i in hidx][:6], "OK" if h_ok else "MISMATCH"),
               flush=True)

@@ -3,7 +3,7 @@ nugget nu(design + [c]), the reference's branch of costFunctionGP_IVAR.evaluate 
 device engine keeps its candidate running variance noise-inclusive, var_D(c) + nu(c), and runs the unchanged kernels
 with scalar noise 0.
 
-The oracles are tests/hetero_oracle.py.
+The oracles are oracle/gpexp_oracle.py's ref_greedy_ivar with noise_func and fast_greedy_ivar with a nu vector.
 CPU: the vectorised oracle with a nu vector against the reference's loop with the callable; both oracles with a constant
 nu against the float-noise oracles; the candidate-sharding protocol (gloo) with nu(p) travelling in the pivot record;
 rejected noise functions.
@@ -19,7 +19,6 @@ import pytest
 
 from oracle import gpexp_oracle as orc
 from tests.cases import product_kernel, spec
-from tests.hetero_oracle import fast_greedy_ivar_nu, ref_greedy_ivar_nu
 
 DMMA, I8 = 1, 2
 HDR = 3 + 16
@@ -76,23 +75,24 @@ def test_fast_oracle_with_noise_vector_equals_reference_loop(name, nu):
     cand, mc = _sample(name, rng, 60, 400)
     cand[41] = cand[7]   # a duplicated candidate: once one copy is picked the other is scored against a repeated node
     ks = spec(name)
-    ref_idx, ref_costs = ref_greedy_ivar_nu(ks, cand, mc, 8, nu)
-    idx, costs = fast_greedy_ivar_nu(ks, cand, mc, 8, nu(cand))
+    ref_idx, ref_costs = orc.ref_greedy_ivar(ks, cand, mc, 8, None, noise_func=nu)
+    idx, costs = orc.fast_greedy_ivar(ks, cand, mc, 8, nu(cand))
     assert idx == ref_idx
     for s in range(8):
         assert _rel(costs[s], ref_costs[s]) <= 1e-9, s
 
 
 def test_constant_noise_oracles_are_the_float_oracles():
-    """With nu = s2 everywhere, both heteroscedastic oracles reproduce the float-noise oracles bit for bit."""
+    """With nu = s2 everywhere, the noise-function and noise-vector forms of both oracles reproduce their float-noise
+    forms bit for bit."""
     rng = np.random.default_rng(32)
     cand, mc = _sample("matern_5d", rng, 40, 300)
     ks, s2 = spec("matern_5d"), 1e-4
     a_idx, a_costs = orc.ref_greedy_ivar(ks, cand, mc, 6, s2)
-    b_idx, b_costs = ref_greedy_ivar_nu(ks, cand, mc, 6, lambda p: np.full(p.shape[0], s2))
+    b_idx, b_costs = orc.ref_greedy_ivar(ks, cand, mc, 6, None, noise_func=lambda p: np.full(p.shape[0], s2))
     assert a_idx == b_idx and all(np.array_equal(a, b) for a, b in zip(a_costs, b_costs))
     f_idx, f_costs = orc.fast_greedy_ivar(ks, cand, mc, 6, s2)
-    g_idx, g_costs = fast_greedy_ivar_nu(ks, cand, mc, 6, np.full(cand.shape[0], s2))
+    g_idx, g_costs = orc.fast_greedy_ivar(ks, cand, mc, 6, np.full(cand.shape[0], s2))
     assert f_idx == g_idx == a_idx and all(np.array_equal(a, b) for a, b in zip(f_costs, g_costs))
 
 
@@ -153,8 +153,8 @@ def test_sharded_protocol_carries_the_pick_noise():
     n_points, world = 9, 2
     nu = nu_span(cand)
     ks = orc.KernelSpec.se([0.3, 0.45], 1.7, 2)
-    ref, _ = fast_greedy_ivar_nu(ks, cand, mc, n_points, nu)
-    assert ref == ref_greedy_ivar_nu(ks, cand, mc, n_points, nu_span)[0]
+    ref, _ = orc.fast_greedy_ivar(ks, cand, mc, n_points, nu)
+    assert ref == orc.ref_greedy_ivar(ks, cand, mc, n_points, None, noise_func=nu_span)[0]
     ctx = mp.get_context("spawn")
     q = ctx.Queue()
     port = _free_port()
@@ -239,7 +239,7 @@ def _reference_run(name):
     """C = 200 candidates, M = 2 000 integration points, 12 steps of the reference's loop (about 10 s each)."""
     nu = dict(GPU_CASES)[name]
     cand, mc = _sample(name, np.random.default_rng(36), 200, 2000)
-    idx, costs = ref_greedy_ivar_nu(spec(name), cand, mc, N_GPU, nu)
+    idx, costs = orc.ref_greedy_ivar(spec(name), cand, mc, N_GPU, None, noise_func=nu)
     return cand, mc, idx, costs
 
 
@@ -334,7 +334,7 @@ def test_varying_noise_changes_the_design(env):
     cf_s = ed.costFunctionGP_IVAR(env.gp.GP(k, mean), 1, env.Space(2, None, None), mcPoints=mc)
     h = [int(i) for i in ed.performGreedyIVARExperimentalDesign(cf_h, cand, N, returnIndices=True)]
     s = [int(i) for i in ed.performGreedyIVARExperimentalDesign(cf_s, cand, N, returnIndices=True)]
-    assert h == fast_greedy_ivar_nu(ks, cand, mc, N, nu(cand))[0]
+    assert h == orc.fast_greedy_ivar(ks, cand, mc, N, nu(cand))[0]
     assert s == orc.fast_greedy_ivar(ks, cand, mc, N, mean)[0]
     assert h != s
 
@@ -347,7 +347,7 @@ def test_zero_noise_half_domain_follows_the_pinv_rule(env):
     rng = np.random.default_rng(39)
     cand, mc = rng.uniform(-1, 1, (60, 2)), rng.uniform(-1, 1, (400, 2))
     ks, k, N = spec("se_ard_2d_wide"), product_kernel("se_ard_2d_wide"), 10
-    ref_idx, ref_costs = ref_greedy_ivar_nu(ks, cand, mc, N, nu_half_zero)
+    ref_idx, ref_costs = orc.ref_greedy_ivar(ks, cand, mc, N, None, noise_func=nu_half_zero)
     cf = ed.costFunctionGP_IVAR(env.gp.GP(k, 1e-6), 1, env.Space(2, None, None, noise=nu_half_zero), mcPoints=mc)
     eng = ed.beginGreedyIVARExperimentalDesign(cf, cand, N, resident=False)
     eng.score_trace = []
@@ -402,7 +402,7 @@ def test_mid_size_matches_fast_oracle(env):
     C, M, N = 20_000, 1500, 64
     cand, mc = rng.uniform(-1, 1, (C, 2)), rng.uniform(-1, 1, (M, 2))
     ks, k = spec("se_ard_2d"), product_kernel("se_ard_2d")
-    ref, costs = fast_greedy_ivar_nu(ks, cand, mc, N, nu_golden(cand))
+    ref, costs = orc.fast_greedy_ivar(ks, cand, mc, N, nu_golden(cand))
     want = np.array([c[i] for c, i in zip(costs, ref)])
     cf = ed.costFunctionGP_IVAR(env.gp.GP(k, 1e-6), 1, env.Space(2, None, None, noise=nu_golden), mcPoints=mc)
     for resident in (False, True):

@@ -1,6 +1,6 @@
 """Greedy IVAR with weighted integration points (costFunctionGP_IVAR.mcWeights): cost_w(D) = |sum_m w_m var_D(x_m)|.
 
-The oracles are tests/weighted_oracle.py.
+The oracles are oracle/gpexp_oracle.py's ref_greedy_ivar and fast_greedy_ivar with mc_weights.
 CPU: the vectorised weighted oracle against the reference's pinv loop (SE, Matern, Mehler; random, half-zero and
 Gauss-Legendre weights; with and without a noise function); w = 1/M (M = 2^k) reproduces the unweighted oracles bit for bit;
 integer weights equal replicated points; rejected weights.
@@ -13,7 +13,6 @@ import pytest
 from oracle import gpexp_oracle as orc
 from tests.cases import product_kernel, spec
 from tests.test_ivar_contraction_exact import gx  # noqa: F401  (the exact-contraction harness's device fixture)
-from tests.weighted_oracle import fast_greedy_ivar_w, fast_ivar_scores_w, gauss_legendre_grid, ref_greedy_ivar_w
 
 DMMA, I8 = 1, 2
 
@@ -31,6 +30,17 @@ def _sample(name, rng, *shapes):
 
 def nu_smooth(p):
     return 1e-4 + 1e-3 * p[:, 0] ** 2
+
+
+def gauss_legendre_grid(n, d, lo=-1.0, hi=1.0):
+    """Tensor Gauss-Legendre rule of n^d nodes on [lo, hi]^d: (points (n^d, d), weights summing to the box volume)."""
+    x, w = np.polynomial.legendre.leggauss(n)
+    x = lo + (x + 1.0) * (hi - lo) / 2.0
+    w = w * (hi - lo) / 2.0
+    grids = np.meshgrid(*([x] * d), indexing="ij")
+    wgrid = np.meshgrid(*([w] * d), indexing="ij")
+    pts = np.stack([g.ravel() for g in grids], axis=1)
+    return pts, np.prod(np.stack([g.ravel() for g in wgrid], axis=1), axis=1)
 
 
 def _weights(profile, mc, rng):
@@ -61,23 +71,24 @@ def test_fast_weighted_oracle_equals_reference_loop(name, profile, with_nf):
         w = _weights(profile, mc, rng)
     noise = 1e-2 if name.startswith("mehler") else 1e-5
     nf = (lambda p: 10.0 * noise * (1.0 + p[:, 0] ** 2)) if with_nf else None
-    ref_idx, ref_costs = ref_greedy_ivar_w(ks, cand, mc, 6, noise, w, noise_func=nf)
-    idx, costs = fast_greedy_ivar_w(ks, cand, mc, 6, noise, w, nu=None if nf is None else nf(cand))
+    ref_idx, ref_costs = orc.ref_greedy_ivar(ks, cand, mc, 6, noise, mc_weights=w, noise_func=nf)
+    idx, costs = orc.fast_greedy_ivar(ks, cand, mc, 6, noise if nf is None else nf(cand), mc_weights=w)
     assert idx == ref_idx
     for s in range(6):
         assert _rel(costs[s], ref_costs[s]) <= 1e-9, s
 
 
 def test_uniform_power_of_two_weights_are_the_unweighted_oracles():
-    """M = 256, w = 1/M: both weighted oracles reproduce orc.ref_greedy_ivar / orc.fast_greedy_ivar bit for bit."""
+    """M = 256, w = 1/M: the weighted forms of ref_greedy_ivar and fast_greedy_ivar reproduce their unweighted forms bit
+    for bit."""
     rng = np.random.default_rng(52)
     cand, mc = rng.uniform(-1, 1, (30, 2)), rng.uniform(-1, 1, (256, 2))
     ks, s2, w = spec("se_ard_2d_wide"), 1e-4, np.full(256, 1.0 / 256)
     a_idx, a_costs = orc.ref_greedy_ivar(ks, cand, mc, 5, s2)
-    b_idx, b_costs = ref_greedy_ivar_w(ks, cand, mc, 5, s2, w)
+    b_idx, b_costs = orc.ref_greedy_ivar(ks, cand, mc, 5, s2, mc_weights=w)
     assert a_idx == b_idx and all(np.array_equal(x, y) for x, y in zip(a_costs, b_costs))
     f_idx, f_costs = orc.fast_greedy_ivar(ks, cand, mc, 5, s2)
-    g_idx, g_costs = fast_greedy_ivar_w(ks, cand, mc, 5, s2, w)
+    g_idx, g_costs = orc.fast_greedy_ivar(ks, cand, mc, 5, s2, mc_weights=w)
     assert f_idx == g_idx == a_idx and all(np.array_equal(x, y) for x, y in zip(f_costs, g_costs))
 
 
@@ -87,8 +98,8 @@ def test_integer_weights_equal_replicated_points():
     ks, s2 = spec("se_ard_2d_wide"), 1e-5
     k = rng.integers(1, 5, mc.shape[0])
     rep = np.repeat(mc, k, axis=0)
-    a_idx, a_costs = fast_greedy_ivar_w(ks, cand, mc, 10, s2, k.astype(np.float64))
-    b_idx, b_costs = fast_greedy_ivar_w(ks, cand, rep, 10, s2, np.ones(rep.shape[0]))
+    a_idx, a_costs = orc.fast_greedy_ivar(ks, cand, mc, 10, s2, mc_weights=k.astype(np.float64))
+    b_idx, b_costs = orc.fast_greedy_ivar(ks, cand, rep, 10, s2, mc_weights=np.ones(rep.shape[0]))
     assert a_idx == b_idx == orc.fast_greedy_ivar(ks, cand, rep, 10, s2)[0]
     for s in range(10):
         assert _rel(a_costs[s], b_costs[s]) <= 1e-12, s
@@ -300,7 +311,7 @@ def test_nonuniform_weights_match_reference_loop(env, name):
     k, ks, N = product_kernel(name), spec(name), 8
     noise = 1e-2 if name.startswith("mehler") else 1e-5
     for nf in (None, lambda p: 10.0 * noise * (1.0 + p[:, 0] ** 2)):
-        ref_idx, ref_costs = ref_greedy_ivar_w(ks, cand, mc, N, noise, w, noise_func=nf)
+        ref_idx, ref_costs = orc.ref_greedy_ivar(ks, cand, mc, N, noise, mc_weights=w, noise_func=nf)
         want = np.array([c[i] for c, i in zip(ref_costs, ref_idx)])
         cf = ed.costFunctionGP_IVAR(env.gp.GP(k, noise), 1, env.Space(ks.dim, None, None, noise=nf), mcPoints=mc,
                                     mcWeights=w)
@@ -327,7 +338,7 @@ def test_nonuniform_weights_mid_size_every_loop_mode(env):
     w = _weights("smooth", mc, rng)
     ks, k, N = spec("se_ard_2d"), product_kernel("se_ard_2d"), 16
     for nf in (None, nu_smooth):
-        ref, costs = fast_greedy_ivar_w(ks, cand, mc, N, 1e-6, w, nu=None if nf is None else nf(cand))
+        ref, costs = orc.fast_greedy_ivar(ks, cand, mc, N, 1e-6 if nf is None else nf(cand), mc_weights=w)
         want = np.array([c[i] for c, i in zip(costs, ref)])
         cf = ed.costFunctionGP_IVAR(env.gp.GP(k, 1e-6), 1, env.Space(2, None, None, noise=nf), mcPoints=mc, mcWeights=w)
         for mode in LOOP_MODES:
@@ -351,7 +362,7 @@ def test_score_candidates_evaluate_and_derivative(env):
         low = np.linalg.cholesky(ks.gram(design, design) + np.diag(np.broadcast_to(nug, (20,))))
         w_m, w_c = solve_triangular(low, ks.gram(design, mc), lower=True), solve_triangular(low, ks.gram(design, cand), lower=True)
         var_m, var_c = ks.prior(mc) - np.sum(w_m ** 2, axis=0), ks.prior(cand) - np.sum(w_c ** 2, axis=0)
-        fast = fast_ivar_scores_w(ks, cand, mc, w_m, var_m, w_c, var_c, 1e-5 if nf is None else nf(cand), w)
+        fast = orc.fast_ivar_scores(ks, cand, mc, w_m, var_m, w_c, var_c, 1e-5 if nf is None else nf(cand), mc_weights=w)
         assert best == int(np.argmin(fast)) and _rel(costs, fast) <= 1e-9
         var = orc.fast_posterior_variance(ks, design, mc, nug)
         assert abs(cf.evaluate(design) - abs(np.sum(w * var))) <= 1e-9 * abs(np.sum(w * var))

@@ -15,14 +15,11 @@ import numpy as np
 import pytest
 
 from oracle import gpexp_oracle as orc
-from tests.hetero_oracle import fast_greedy_ivar_nu
-from tests.matern_oracle import MATERN12, MATERN52, MaternSpec, matern_closed_form
-from tests.weighted_oracle import fast_greedy_ivar_w
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 DMMA, I8 = 1, 2
 EINVAL = -1
-NEW = {"matern12": MATERN12, "matern52": MATERN52}
+NEW = {"matern12": orc.MATERN12, "matern52": orc.MATERN52}
 
 
 def _rel(a, b):
@@ -38,8 +35,8 @@ def test_closed_forms_equal_the_bessel_expression(nu):
     """s 2^(1-nu) / Gamma(nu) (c0 r)^nu K_nu(c0 r), c0 = sqrt(2 nu) / rho, from r = 1e-6 to 40 rho; r = 0 gives s."""
     from scipy.special import gamma, kv
     rho, s = 0.37, 1.7
-    spec = {0.5: MaternSpec.matern12(rho, s, 2), 1.5: orc.KernelSpec.matern32(rho, s, 2),
-            2.5: MaternSpec.matern52(rho, s, 2)}[nu]
+    spec = {0.5: orc.KernelSpec.matern12(rho, s, 2), 1.5: orc.KernelSpec.matern32(rho, s, 2),
+            2.5: orc.KernelSpec.matern52(rho, s, 2)}[nu]
     r = np.concatenate([np.geomspace(1e-6, 40 * rho, 400), [0.5 * rho, rho, 2 * rho]])
     x1 = np.zeros((r.size, 2))
     x2 = np.stack([0.6 * r, 0.8 * r], axis=1)
@@ -49,14 +46,15 @@ def test_closed_forms_equal_the_bessel_expression(nu):
     assert _rel(got, want) <= 1e-13
     assert np.array_equal(spec.gram(x1[:5], x2[:5]).diagonal(), got[:5])
     assert np.all(spec.evaluateF(np.ones((3, 2)), np.ones((3, 2))) == s)
-    assert np.all(matern_closed_form(nu, np.zeros(2), rho, s) == s)
+    assert np.all(orc.matern_closed_form(nu, np.zeros(2), rho, s) == s)
 
 
 def test_header_constants_equal_the_binding():
     from gpexp_b200 import _lib
     text = open(os.path.join(ROOT, "include", "gpexp_b200.h")).read()
     defs = dict(re.findall(r"#define\s+(GPX_\w+)\s+(-?\d+)\b", text))
-    assert (int(defs["GPX_MATERN12"]), int(defs["GPX_MATERN52"])) == (_lib.MATERN12, _lib.MATERN52) == (MATERN12, MATERN52)
+    assert (int(defs["GPX_MATERN12"]), int(defs["GPX_MATERN52"])) == (_lib.MATERN12, _lib.MATERN52) == \
+        (orc.MATERN12, orc.MATERN52)
     fams = [int(defs[k]) for k in ("GPX_SE", "GPX_MATERN32", "GPX_MEHLER", "GPX_MATERN12", "GPX_MATERN52")]
     assert len(set(fams)) == 5 and fams[:3] == [0, 1, 2]
 
@@ -247,13 +245,13 @@ def test_expanded_form_is_refused_for_nu_half(gx):
     gx.check(lib.gpx_cov_from_factors(dev.h, L.PRO_DIFF, None, a.ld, ptr(a.X), M, None, b.ld, ptr(b.X), C, 0, ptr(out),
                                       b.ld, dev.stream))
     dev.sync()
-    ks = MaternSpec.matern12(0.4, 1.0, 2)
+    ks = orc.KernelSpec.matern12(0.4, 1.0, 2)
     assert np.max(np.abs(out[:, :C].cpu().numpy() - ks.gram(pts[:200], pts[200:]))) <= 1e-14
 
 
 # far pairs: the test_ivar_contraction_exact geometry (d = 1, integration points at +50, candidates at -50), with rho
 # putting every t = c0 |x - y| between ~2400 and ~4600, far past the table exp's flush point
-FAR = {"matern12": (MATERN12, [0.04, 1.0], 50.0), "matern52": (MATERN52, [0.05, 1.0], 50.0)}
+FAR = {"matern12": (orc.MATERN12, [0.04, 1.0], 50.0), "matern52": (orc.MATERN52, [0.05, 1.0], 50.0)}
 
 
 @pytest.mark.gpu
@@ -286,7 +284,7 @@ NOISE = 1e-4
 
 def _kernels(gx, family, signal=1.3, d=3):
     nu = 0.5 if family == "matern12" else 2.5
-    ks = (MaternSpec.matern12 if family == "matern12" else MaternSpec.matern52)(RHO[family], signal, d)
+    ks = (orc.KernelSpec.matern12 if family == "matern12" else orc.KernelSpec.matern52)(RHO[family], signal, d)
     return ks, gx.kernels.KernelIsoMatern(RHO[family], signal, d, nu=nu)
 
 
@@ -396,13 +394,13 @@ def test_noise_function_and_mc_weights(gx, family):
     rng = np.random.default_rng(44)
     cand, mc = rng.uniform(-1, 1, (600, 3)), rng.uniform(-1, 1, (800, 3))
     ks, k = _kernels(gx, family)
-    ref_idx, ref_costs = fast_greedy_ivar_nu(ks, cand, mc, 12, nu_span(cand))
+    ref_idx, ref_costs = orc.fast_greedy_ivar(ks, cand, mc, 12, nu_span(cand))
     cf = ed.costFunctionGP_IVAR(gx.gp.GP(k, 0.5), 1, gx.Space(3, None, None, noise=nu_span), mcPoints=mc)
     idx = ed.performGreedyIVARExperimentalDesign(cf, cand, 12, returnIndices=True)
     assert [int(i) for i in idx] == ref_idx
     assert _rel(cf.lastScores, [c[i] for c, i in zip(ref_costs, ref_idx)]) <= 1e-9
     w = rng.uniform(0.0, 2.0, mc.shape[0]) / mc.shape[0]
-    ref_idx, ref_costs = fast_greedy_ivar_w(ks, cand, mc, 12, NOISE, w)
+    ref_idx, ref_costs = orc.fast_greedy_ivar(ks, cand, mc, 12, NOISE, mc_weights=w)
     cf = ed.costFunctionGP_IVAR(gx.gp.GP(k, NOISE), 1, gx.Space(3, None, None), mcPoints=mc, mcWeights=w)
     idx = ed.performGreedyIVARExperimentalDesign(cf, cand, 12, returnIndices=True)
     assert [int(i) for i in idx] == ref_idx

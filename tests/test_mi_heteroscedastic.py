@@ -3,7 +3,7 @@ Gram takes diag(nu) on that subset, so the numerator is var(y | A) with K_AA + d
 1/[(K_SS + diag nu_S)^-1]_yy - nu_y.  The engines factor K_VV + diag nu, divide the append by sqrt(num_p + nu_p) and
 score with 1/pd_j - nu_j.
 
-The oracles are tests/hetero_mi_oracle.py.
+The oracles are oracle/gpexp_oracle.py's ref_greedy_mi, ref_mi_cost and fast_greedy_mi with a nu vector.
 CPU: the vectorised oracle against the reference's pinv loop with nu on each subset; both oracles with a constant nu
 against the float-noise oracles, bit for bit; rejected noise vectors.
 GPU: a constant nu reproduces the scalar run bit for bit on the golden cases; a varying nu against the reference's loop
@@ -20,7 +20,6 @@ import pytest
 
 from oracle import gpexp_oracle as orc
 from tests.cases import product_kernel, spec
-from tests.hetero_mi_oracle import fast_greedy_mi_nu, ref_greedy_mi_nu, ref_mi_cost_nu
 
 SCORE_RTOL = 2e-8
 SE_CL, SE_SIGNAL = [0.15, 0.2], 1.0   # the noise-free half of a 100-point pool has cond(K) ~ 3e4 (DESIGN section 2: <~ 1e6)
@@ -90,7 +89,7 @@ V_REF, N_REF, START = 100, 8, 3
 def _reference_run(name, nu):
     """|V| = 100, 8 picks of the reference's pinv loop (a few seconds each)."""
     pool = _pool(name, np.random.default_rng(41), V_REF)
-    idx, scores, opts = ref_greedy_mi_nu(kernel_spec(name), pool, nu(pool), N_REF, start=START)
+    idx, scores, opts = orc.ref_greedy_mi(kernel_spec(name), pool, nu(pool), N_REF, start=START)
     return pool, idx, scores, opts
 
 
@@ -100,7 +99,7 @@ def _reference_run(name, nu):
 @pytest.mark.parametrize("name,nu", CPU_CASES, ids=[f"{n}-{f.__name__}" for n, f in CPU_CASES])
 def test_fast_oracle_with_noise_vector_equals_reference_loop(name, nu):
     pool, ref_idx, ref_scores, opts = _reference_run(name, nu)
-    idx, scores, pivots = fast_greedy_mi_nu(kernel_spec(name), pool, nu(pool), N_REF, start=START)
+    idx, scores, pivots = orc.fast_greedy_mi(kernel_spec(name), pool, nu(pool), N_REF, start=START, with_pivots=True)
     assert idx == ref_idx
     for s in range(N_REF - 1):
         assert _rel(scores[s][opts[s]], ref_scores[s]) <= SCORE_RTOL, s
@@ -108,16 +107,16 @@ def test_fast_oracle_with_noise_vector_equals_reference_loop(name, nu):
 
 
 def test_constant_noise_oracles_are_the_float_oracles():
-    """With nu = s2 everywhere, both heteroscedastic MI oracles reproduce the float-noise oracles bit for bit."""
+    """With nu = s2 everywhere, the noise-vector forms of both MI oracles reproduce their float-noise forms bit for bit."""
     ks, s2 = spec("matern_5d"), 1e-3
     pool = np.random.default_rng(42).uniform(-1, 1, (60, 5))
     nu = np.full(60, s2)
     a_idx, a_scores, a_opts = orc.ref_greedy_mi(ks, pool, s2, 6, start=2)
-    b_idx, b_scores, b_opts = ref_greedy_mi_nu(ks, pool, nu, 6, start=2)
+    b_idx, b_scores, b_opts = orc.ref_greedy_mi(ks, pool, nu, 6, start=2)
     assert a_idx == b_idx and all(np.array_equal(a, b) for a, b in zip(a_scores, b_scores))
     assert all(np.array_equal(a, b) for a, b in zip(a_opts, b_opts))
     f_idx, f_scores = orc.fast_greedy_mi(ks, pool, s2, 6, start=2)
-    g_idx, g_scores, _ = fast_greedy_mi_nu(ks, pool, nu, 6, start=2)
+    g_idx, g_scores = orc.fast_greedy_mi(ks, pool, nu, 6, start=2)
     assert f_idx == g_idx == a_idx and all(np.array_equal(a, b) for a, b in zip(f_scores, g_scores))
 
 
@@ -246,7 +245,7 @@ def test_varying_noise_matches_reference_loop(env, name, nu):
         assert _rel(sc[opts[s]], ref_scores[s]) <= SCORE_RTOL, s
     # the single-candidate call against the restated reference cost
     for j in opts[3][::17]:
-        want = ref_mi_cost_nu(ks, pool, nuv, int(j), ref_idx[:3])[0]
+        want = orc.ref_mi_cost(ks, pool, nuv, int(j), ref_idx[:3])[0]
         got = cf.evaluate(int(j), ref_idx[:3])
         assert got.shape == (1,) and abs(got[0] - want) <= SCORE_RTOL * abs(want), j
 
@@ -257,7 +256,7 @@ def test_cfg4_kernel_matches_fast_oracle(env, v, n):
     """cfg-4's kernel (3-D Mehler t = 0.9, N(0, I) pool) with nu(x) = 1e-2 (1 + |x|^2 / 3)."""
     pool = np.random.default_rng(4).standard_normal((v, 3))
     nu = nu_cfg4(pool)
-    ref, _, ref_piv = fast_greedy_mi_nu(spec("mehler_3d"), pool, nu, n, start=0)
+    ref, _, ref_piv = orc.fast_greedy_mi(spec("mehler_3d"), pool, nu, n, start=0, with_pivots=True)
     cf = _cost_function(env, "mehler_3d", pool, nu)
     env.ed.performGreedyMIExperimentalDesign(cf, n, start=0)
     assert [int(i) for i in cf.lastIndices] == ref
@@ -269,7 +268,7 @@ def test_cfg4_kernel_matches_fast_oracle(env, v, n):
 def test_noise_profile_changes_the_design(env):
     pool = _pool("se_mid", np.random.default_rng(41), V_REF)
     nu = nu_steep(pool)
-    ref, _, _ = fast_greedy_mi_nu(kernel_spec("se_mid"), pool, nu, N_REF, start=START)
+    ref, _ = orc.fast_greedy_mi(kernel_spec("se_mid"), pool, nu, N_REF, start=START)
     scalar = _cost_function(env, "se_mid", pool, 1e-3)
     hetero = _cost_function(env, "se_mid", pool, nu)
     env.ed.performGreedyMIExperimentalDesign(scalar, N_REF, start=START)
@@ -289,7 +288,7 @@ def test_changing_noise_rebuilds_the_factorisation(env):
 
     def check(nu):
         got = np.array([cf.evaluate(j, added)[0] for j in js])
-        want = np.array([ref_mi_cost_nu(ks, pool, nu, j, added)[0] for j in js])
+        want = np.array([orc.ref_mi_cost(ks, pool, nu, j, added)[0] for j in js])
         assert _rel(got, want) <= SCORE_RTOL
         return got, cf._mi_cache["engine"]   # the object, not its id(): a freed engine's id can be reused
 
@@ -312,7 +311,7 @@ def test_dense_and_sharded_engines_agree(env, monkeypatch, v, blk):
     name, n = "mehler_3d", 10
     pool = _pool(name, np.random.default_rng(46), v)
     nu = nu_mehler_span(pool)
-    ref, ref_scores, ref_piv = fast_greedy_mi_nu(spec(name), pool, nu, n, start=2)
+    ref, ref_scores, ref_piv = orc.fast_greedy_mi(spec(name), pool, nu, n, start=2, with_pivots=True)
     kernel_obj(name)._bind(env.dev)
     sharded = env.engine.ShardedMIEngine(env.dev, pool, n, 0.0, pool_noise=nu)
     dense = env.engine.GreedyMIEngine(env.dev, env.dev.points(pool), n, 0.0, pool_noise=nu)
