@@ -28,7 +28,8 @@ def patch_reference(ref):
       gpExp.gp.GP              train, evaluate, addNodesAndComputeCovariance, evaluateVariance,
                                evaluateVarianceDerivative, computeLogLike, loglikeParams, covarianceMatrix / precisionMatrix
       gpExp.experimentalDesign costFunctionGP_IVAR.evaluate / derivative, costFunctionGP_MI.evaluate,
-                               performGreedyVar / MI ExperimentalDesign (+ the new greedy-IVAR drivers)
+                               performGreedyVar / MI ExperimentalDesign (+ the new greedy-IVAR drivers: begin / perform /
+                               refineGreedyIVARExperimentalDesign, scoreCandidatesIVAR)
     Returns `ref`."""
     from . import experimentalDesign as ed, gp, gp_kernel_utilities as gku, kernels
     rk = importlib.import_module(ref.__name__ + ".kernels")

@@ -117,6 +117,10 @@ SIGNATURES = {
     "gpx_transpose": [_p, _p, _i64, _i64, _i64, _p, _i64, _p],
     "gpx_set_mask": [_p, _p, _p, C.c_uint8, _p],
     "gpx_store_pivot": [_p, _p, _i64, _p, _i64, _p, _p, _p, _p],
+    "gpx_design_delete_factor": [_p, _p, _i64, _i64, _i64, _p, _p, _p, _p, _p],
+    "gpx_design_delete_rows": [_p, _p, _i64, _i64, _p, _i64, _i64, _p, _p],
+    "gpx_exchange_keep": [_p, _p, _i64, _i64, _p, _dbl, _p, _p, _p, _p],
+    "gpx_exchange_record": [_p, _p, _p, _i64, _p, _p, _p, _p, _p],
     "gpx_comm_unique_id": [_p, _int],
     "gpx_comm_init": [_p, _p, _int, _int],
     "gpx_comm_destroy": [_p],

@@ -579,6 +579,8 @@ class GreedyIVAREngine(_Pivoting):
         self.score_trace = None
         self.cov = None
         self.zero_scale = float(zero_scale)
+        self.removals = 0          # remove() calls so far (a snapshot is valid only for the count it was taken at)
+        self._rot = None           # exchange buffers, allocated by the first remove()
         if self.resident:
             self.cov = dev.empty(mc.n, cand.ld)
             # cov_0 = K(mc, cand), then the column sums of squares for the first scoring
@@ -648,9 +650,12 @@ class GreedyIVAREngine(_Pivoting):
         """Cheap save point (running variances + design size); rows >= n of W are never read.
         Not available in resident mode (the covariance matrix is updated in place)."""
         assert not self.resident, "resident mode cannot be rolled back"
-        return (self.n, self.varC.clone(), self.varM.clone())
+        return (self.n, self.varC.clone(), self.varM.clone(), self.removals)
 
     def restore(self, snap):
+        if snap[3] != self.removals:
+            # remove() rotates rows 0..n-1 of W in place: the rows a snapshot would reuse are gone
+            raise ValueError("restore: the snapshot was taken before a remove()")
         self.n = snap[0]
         self.varC.copy_(snap[1])
         self.varM.copy_(snap[2])
@@ -694,6 +699,75 @@ class GreedyIVAREngine(_Pivoting):
         if self.score_trace is not None:
             self.score_trace.append(self.scores[: self.cand.n].cpu().numpy().copy())
         self.append()
+
+    def remove(self, position: int):
+        """Delete design point `position` (0 <= position < n) without refactoring: Givens rotations turn U into the
+        factor of the remaining n-1 points (gpx_design_delete_factor), the same rotations bring W_M and W_C along and add
+        the residual row's squares to varM / varC (gpx_design_delete_rows), and in resident mode one covariance pass adds
+        r_M r_C^T back (and refreshes the column sums the scoring reads).  picks / pick_scores / pick_pivots close the
+        gap; pick_pivots[i] becomes U'[i,i]^2.  The removed point's global index is left in `self.removed` (device)."""
+        n = self.n
+        if not 0 <= int(position) < n:
+            raise IndexError(f"remove: position {position} outside the design of {n} points")
+        j = int(position)
+        dev, cand, mc = self.dev, self.cand, self.mc
+        if self._rot is None:
+            self._rot = dev.zeros(max(2 * self.ncap, 2))
+            self.removed = dev.zeros(1, dtype=torch.int64)
+            self.inc_score = dev.zeros(1)
+            self._rneg = dev.zeros(cand.ld) if self.resident else None
+        self.removed.copy_(self.picks[j: j + 1])
+        check(lib.gpx_design_delete_factor(dev.h, ptr(self.U), n, self.U.shape[1], j, ptr(self._rot), ptr(self.picks),
+                                           ptr(self.pick_scores), ptr(self.pick_pivots), dev.stream), "gpx_design_delete_factor")
+        check(lib.gpx_design_delete_rows(dev.h, ptr(self._rot), j, n, ptr(self.Wm), mc.ld, mc.n, ptr(self.varM), dev.stream),
+              "gpx_design_delete_rows")
+        check(lib.gpx_design_delete_rows(dev.h, ptr(self._rot), j, n, ptr(self.Wc), cand.ld, cand.n, ptr(self.varC),
+                                         dev.stream), "gpx_design_delete_rows")
+        if self.resident:
+            # cov_{D \ j} = cov_D + r_M r_C^T = cov_D - r_M (-r_C)^T: the append's update pass with one side negated
+            check(lib.gpx_axpby(dev.h, cand.n, -1.0, ptr(self.Wc[n - 1]), 0.0, ptr(self._rneg), dev.stream), "gpx_axpby")
+            self._cov_pass(self.Wm[n - 1], self._rneg)
+        self.n = n - 1
+        self.removals += 1
+
+    def exchange(self, max_sweeps: int, rtol: float):
+        """Fedorov-type exchange pass over the current design, run as a queue: each step removes position 0 (the point
+        that has waited longest), scores every candidate against the other n-1 points, and appends the winner at the
+        end -- the removed point itself unless a challenger scores below (1 - rtol) x the removed point's own score
+        (gpx_exchange_keep; among challengers the arg-min with the lowest index).  One sweep = n steps, so every point
+        present at the start of a sweep is decided once.  Stops after a sweep without a swap or after max_sweeps.
+        Nothing is read back inside a sweep; one read per sweep decides whether to go on.
+        Returns the accepted swaps per sweep; `self.exchange_costs` (device) holds the design cost after every step."""
+        n = self.n
+        if max_sweeps <= 0 or n == 0:
+            self.exchange_costs = self.dev.zeros(0)
+            return []
+        swaps = self.dev.zeros(max_sweeps, dtype=torch.int64)
+        costs = self.dev.zeros(max_sweeps * n)
+        out = []
+        for sweep in range(max_sweeps):
+            for t in range(n):
+                self.exchange_step(rtol, swaps[sweep:], costs[sweep * n + t:])
+            out.append(int(swaps[sweep].item()))
+            if out[-1] == 0:
+                break
+        self.exchange_costs = costs[: len(out) * n]
+        return out
+
+    def exchange_step(self, rtol: float, swaps=None, cost=None):
+        """One step of exchange(): remove position 0, score, keep-or-swap, append.  swaps / cost (device, nullable):
+        int64 counter incremented on a swap, and the slot that receives the design cost after the step."""
+        dev, st = self.dev, self.dev.stream
+        n = self.n
+        self.remove(0)
+        self.score()
+        check(lib.gpx_exchange_keep(dev.h, ptr(self.removed), self.index_offset, self.cand.n, ptr(self.scores), float(rtol),
+                                    ptr(self.best), ptr(self.idx), ptr(self.inc_score), st), "gpx_exchange_keep")
+        if self.shard is not None and self.shard.world > 1:  # the owner's score of the removed point, for every rank
+            self.shard.dist.all_reduce(self.inc_score, group=self.shard.group)
+        self.append()
+        check(lib.gpx_exchange_record(dev.h, ptr(self.removed), ptr(self.inc_score), n - 1, ptr(self.picks),
+                                      ptr(self.pick_scores), ptr(swaps), ptr(cost), st), "gpx_exchange_record")
 
     def _state(self):
         st = _lib.IvarState()

@@ -7,6 +7,7 @@ the device-resident engines of gpexp_b200.engine.
     performGreedyMIExperimentalDesign           experimentalDesign.py:753-785
     performGreedyIVARExperimentalDesign,        NEW: the discrete greedy-IVAR driver the north star asks for; the
     beginGreedyIVARExperimentalDesign,          reference only has the per-design cost function (SURVEY.md 3.2 / 8c)
+    refineGreedyIVARExperimentalDesign,         NEW: exchange passes that improve a discrete IVAR design on the candidates
     scoreCandidatesIVAR
 
 The continuous optimisers that CALL these cost functions (ExperimentalDesignDerivative / NoDerivative and the batch-greedy
@@ -351,6 +352,60 @@ def performGreedyIVARExperimentalDesign(costFuncIVAR, candidates, nPoints, retur
     return candidates[idx, :]
 
 
+def refineGreedyIVARExperimentalDesign(costFuncIVAR, candidates, indices, maxSweeps=10, rtol=1e-8, returnIndices=False,
+                                       shard=None, resident=None):
+    """Improve a discrete IVAR design by exchange (Fedorov-type) passes over the candidate set.
+
+    `indices` are candidate indices of the design (e.g. performGreedyIVARExperimentalDesign(..., returnIndices=True) or
+    cf.lastIndices); duplicates are allowed as greedy allows them.  The engine is built as in
+    beginGreedyIVARExperimentalDesign (noise function, mcWeights, every kernel family, both contraction cores, resident and
+    sharded runs apply unchanged) and the given points are forced in order.  Then, as a queue, each step takes the oldest
+    point out, scores every candidate c as the design of the other n-1 points plus c, and puts back the arg-min
+    challenger (lowest index on ties) only if its cost is below (1 - rtol) x the removed point's own cost from the same
+    pass; otherwise the removed point returns.  One sweep re-decides every point once; the pass stops after a sweep without
+    a swap or after maxSweeps.  The cost never increases, and the result is 1-swap optimal up to rtol when the pass stops
+    by itself.  rtol = 1e-8 lies well above the rounding of the scores, so the pass cannot cycle on ties.
+
+    Returns the refined points (or indices with returnIndices) in factor order, the oldest first.  Leaves on the cost
+    function: lastIndices, lastScores (design cost after every exchange step), lastSwaps (accepted swaps per sweep),
+    lastCost (cost of the returned design: the mean posterior variance over mcPoints, or sum_m w_m var(x_m) with
+    mcWeights) and illConditionedFrom (as performGreedyIVARExperimentalDesign, for the returned design).
+    ValueError for indices that are not integers or lie outside the candidates, rtol < 0, maxSweeps < 0, and for a
+    design whose factor has a non-finite entry (e.g. a repeated point under zero noise).  maxSweeps = 0 returns the
+    input design."""
+    idx = np.asarray(indices)
+    if idx.ndim != 1 or idx.size == 0 or not np.issubdtype(idx.dtype, np.integer):
+        raise ValueError("indices must be a non-empty 1-D sequence of integer candidate indices")
+    if np.any(idx < 0) or np.any(idx >= candidates.shape[0]):
+        raise ValueError(f"indices must lie in [0, {candidates.shape[0]})")
+    if not rtol >= 0.0:
+        raise ValueError(f"rtol must be >= 0, got {rtol}")
+    if isinstance(maxSweeps, (bool, np.bool_)) or not isinstance(maxSweeps, (int, np.integer)) or maxSweeps < 0:
+        raise ValueError(f"maxSweeps must be an integer >= 0, got {maxSweeps!r}")
+    n = idx.size
+    eng = beginGreedyIVARExperimentalDesign(costFuncIVAR, candidates, n, shard=shard, resident=resident)
+    for i in idx:
+        eng.force(int(i))
+    import torch
+    if not bool(torch.isfinite(eng.U[:n, :n]).all()):
+        raise ValueError("the design's Cholesky factor has a non-finite entry (a repeated or numerically dependent "
+                         "point without noise): it cannot be refined")
+    swaps = eng.exchange(int(maxSweeps), float(rtol))
+    dev, mc = eng.dev, eng.mc
+    total = dev.zeros(1)
+    check(lib.gpx_sum_w(dev.h, ptr(eng.varM), ptr(eng.mc_weights), mc.n, ptr(total), dev.stream), "gpx_sum_w")
+    cost = float(total.item())
+    out = eng.indices()
+    costFuncIVAR.lastIndices = out
+    costFuncIVAR.lastScores = eng.exchange_costs.cpu().numpy()
+    costFuncIVAR.lastSwaps = swaps
+    costFuncIVAR.lastCost = abs(cost) if eng.mc_weights is not None else abs(cost / float(mc.n))
+    costFuncIVAR.illConditionedFrom = eng.ill_conditioned_from(eng.zero_scale)
+    if returnIndices:
+        return out
+    return candidates[out, :]
+
+
 def scoreCandidatesIVAR(costFuncIVAR, design, candidates, shard=None):
     """One stateless IVAR scoring pass from HOST buffers: cost of design + [c] for every candidate c.
     Returns (costs, argmin index).  With `shard` every rank passes the full candidate array, scores its own contiguous
@@ -402,5 +457,6 @@ DEVICE_FUNCTIONS = {
     "performGreedyMIExperimentalDesign": performGreedyMIExperimentalDesign,
     "performGreedyIVARExperimentalDesign": performGreedyIVARExperimentalDesign,
     "beginGreedyIVARExperimentalDesign": beginGreedyIVARExperimentalDesign,
+    "refineGreedyIVARExperimentalDesign": refineGreedyIVARExperimentalDesign,
     "scoreCandidatesIVAR": scoreCandidatesIVAR,
 }

@@ -4,7 +4,7 @@
  * The reference (goroda/GPEXP) is pure Python/numpy and has NO native or FFI layer
  * (SURVEY.md section 8b), so there is no existing binding to mirror: every entry point
  * below cites the reference Python function whose arithmetic it replaces, and
- * INTEGRATION.md shows the ctypes stub a maintainer of the reference would add.  79 entry points.
+ * INTEGRATION.md shows the ctypes stub a maintainer of the reference would add.  83 entry points.
  *
  * Conventions
  *   - every pointer is a DEVICE pointer owned by the caller unless the name ends in _host;
@@ -330,6 +330,32 @@ int gpx_set_mask(gpx_handle h, uint8_t* mask, const int64_t* idx_dev, uint8_t va
  * number whose smallness flags an ill-conditioned design), column n of the design factor U (each nullable) */
 int gpx_store_pivot(gpx_handle h, const double* rec, int64_t n, double* U, int64_t ldu, int64_t* picks,
                     double* scores, double* pivots, void* stream);
+
+/* ---- Exchange refinement of a greedy IVAR design: deleting design position j (0 <= j < n) in place ------------------
+ * gpx_design_delete_factor: U (n x n within ldu, upper triangular, K_DD + diag(noise) = U^T U) becomes the (n-1) x (n-1)
+ *     factor of the design without point j: column j is dropped and Givens rotations G_i on rows (i, i+1), i = j .. n-2,
+ *     zero the subdiagonal (c = a/rho, s = b/rho, rho = hypot(a, b) >= 0 the new diagonal; the identity when a = b = 0).
+ *     rot receives the pairs (c, s), 2 (n-1-j) doubles (16-byte aligned; NULL allowed when j = n-1).  Row and column
+ *     n-1 are cleared.  picks / scores / pivots (each nullable): the greedy history; entries j+1 .. n-1 move down by one and
+ *     pivots[i] = U'[i,i]^2 for i >= j.  One block, n - 1 - j <= 8192.
+ * gpx_design_delete_rows: the same rotations on rows j .. n-1 of a factor W = U^-T K(D, X) (ncols columns, ldw even):
+ *     rows j .. n-2 become those of the reduced design, row n-1 receives the residual row r (the part of K(D, x) that only
+ *     the deleted point explained) and var[x] += r[x]^2.  Rows 0 .. j-1 are not touched.  HBM-bound: 16 (n-j) ncols bytes.
+ *     A resident covariance follows with gpx_cov_update_w(a = r_M, b = -r_C). */
+int gpx_design_delete_factor(gpx_handle h, double* U, int64_t n, int64_t ldu, int64_t j, double* rot, int64_t* picks,
+                             double* scores, double* pivots, void* stream);
+int gpx_design_delete_rows(gpx_handle h, const double* rot, int64_t j, int64_t n, double* W, int64_t ldw, int64_t ncols,
+                           double* var, void* stream);
+/* Keep-or-swap rule of one exchange step, between scoring and the pivot gather.  *inc = GLOBAL index of the removed point;
+ * on the rank that holds it (0 <= *inc - index_offset < C): inc_score[0] = its score s, and if (1 - rtol) s <= best[0]
+ * then best[0] = (1 - rtol) s, idx[0] = its local index, so a challenger wins only below (1 - rtol) s (ties keep it).
+ * Other ranks write inc_score[0] = 0 (a sum over the ranks gives s everywhere).  rtol >= 0. */
+int gpx_exchange_keep(gpx_handle h, const int64_t* inc, int64_t index_offset, int64_t C, const double* scores, double rtol,
+                      double* best, int64_t* idx, double* inc_score, void* stream);
+/* After the append of step n: if picks[n] == *inc (the removed point came back) pick_scores[n] = inc_score[0] (its true
+ * cost instead of the discounted one), else swaps[0] += 1; trace[0] = pick_scores[n].  swaps, trace nullable. */
+int gpx_exchange_record(gpx_handle h, const int64_t* inc, const double* inc_score, int64_t n, const int64_t* picks,
+                        double* pick_scores, int64_t* swaps, double* trace, void* stream);
 
 /* ---- N1  collectives (SURVEY.md 8b).  NCCL is resolved at run time (dlopen of libnccl.so.2, preferring the copy the
  * process already loaded); a caller that never shards never needs it.  One communicator per handle. --------------------- */
