@@ -29,7 +29,8 @@ def patch_reference(ref):
                                evaluateVarianceDerivative, computeLogLike, loglikeParams, covarianceMatrix / precisionMatrix
       gpExp.experimentalDesign costFunctionGP_IVAR.evaluate / derivative, costFunctionGP_MI.evaluate,
                                performGreedyVar / MI ExperimentalDesign (+ the new greedy-IVAR drivers: begin / perform /
-                               refineGreedyIVARExperimentalDesign, scoreCandidatesIVAR)
+                               refineGreedyIVARExperimentalDesign, scoreCandidatesIVAR; the exchange refinements
+                               refineGreedyMI / Var ExperimentalDesign)
     Returns `ref`."""
     from . import experimentalDesign as ed, gp, gp_kernel_utilities as gku, kernels
     rk = importlib.import_module(ref.__name__ + ".kernels")

@@ -120,6 +120,9 @@ SIGNATURES = {
     "gpx_design_delete_factor": [_p, _p, _i64, _i64, _i64, _p, _p, _p, _p, _p],
     "gpx_design_delete_rows": [_p, _p, _i64, _i64, _p, _i64, _i64, _p, _p],
     "gpx_exchange_keep": [_p, _p, _i64, _i64, _p, _dbl, _p, _p, _p, _p],
+    "gpx_design_delete_factors": [_p, _i64, _i64, _p, _i64, _p, _p, _p, _p, _p, _i64, _p, _p],
+    "gpx_exchange_keep_max": [_p, _p, _i64, _i64, _i64, _i64, _i64, _p, _p, _dbl, _p, _p, _p, _p],
+    "gpx_exchange_unmask": [_p, _p, _i64, _i64, _i64, _i64, _i64, _p, _p],
     "gpx_exchange_record": [_p, _p, _p, _i64, _p, _p, _p, _p, _p],
     "gpx_comm_unique_id": [_p, _int],
     "gpx_comm_init": [_p, _p, _int, _int],

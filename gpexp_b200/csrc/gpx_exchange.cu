@@ -1,4 +1,5 @@
-// Deleting a point from the middle of a greedy IVAR design, and the keep-or-swap rule of the exchange pass.
+// Deleting a point from the middle of a greedy design (IVAR, MI, maximum variance), and the keep-or-swap rule of the
+// exchange pass.
 //
 // Engine state: K_DD + diag(noise) = U^T U (U upper triangular, column i = W[0..i-1, p_i] and sqrt(pivot_i), as
 // gpx_store_pivot writes it) and W_X = U^-T K(D, X).  Deleting design position j:
@@ -24,9 +25,24 @@ namespace {
 constexpr int DF_NT = 1024;
 constexpr int DF_CPT = 8;   // columns per thread: at most DF_NT * DF_CPT rotations
 
-__global__ void __launch_bounds__(DF_NT, 1) delete_factor_kernel(double* __restrict__ U, int64_t ldu, int n, int j,
-                                                                  double* __restrict__ rot, int64_t* __restrict__ picks,
-                                                                  double* __restrict__ scores, double* __restrict__ pivots) {
+struct DeleteFactorArgs {
+    double* U;
+    int64_t ldu;
+    double* rot;
+    int64_t* picks;
+    double* scores;
+    double* pivots;
+};
+
+// Block b downdates factor b: independent factors of one design (MI keeps two) go in one launch of two blocks.
+__global__ void __launch_bounds__(DF_NT, 1) delete_factor_kernel(DeleteFactorArgs f0, DeleteFactorArgs f1, int n, int j) {
+    const bool b0 = blockIdx.x == 0;
+    double* __restrict__ U = b0 ? f0.U : f1.U;
+    const int64_t ldu = b0 ? f0.ldu : f1.ldu;
+    double* __restrict__ rot = b0 ? f0.rot : f1.rot;
+    int64_t* __restrict__ picks = b0 ? f0.picks : f1.picks;
+    double* __restrict__ scores = b0 ? f0.scores : f1.scores;
+    double* __restrict__ pivots = b0 ? f0.pivots : f1.pivots;
     extern __shared__ double sdiag[];          // sdiag[k - j] = U[k+1, k+1], k = j .. n-2
     __shared__ double srot[2][3];              // (c, s, rho) of the current and the next rotation
     const int tid = threadIdx.x;
@@ -199,21 +215,41 @@ __global__ void __launch_bounds__(DR_NT) delete_rows_kernel(const double* __rest
     }
 }
 
-// keep-or-swap: the removed point (global index *inc) stays unless a challenger beats (1 - rtol) x its own score
-__global__ void exchange_keep_kernel(const int64_t* __restrict__ inc, int64_t offset, int64_t C, const double* __restrict__ scores,
-                                     double rtol, double* __restrict__ best, int64_t* __restrict__ idx, double* __restrict__ inc_score) {
-    const int64_t p = inc[0] - offset;
-    if (p < 0 || p >= C) {
+// local column of global index g on this rank, or -1: the contiguous block [offset, offset + C) when blk == 0, else the
+// block-cyclic map of gpx_local_index_cyclic (global block g / blk lives on rank (g / blk) % world as local block
+// (g / blk) / world)
+__device__ __forceinline__ int64_t exchange_local(int64_t g, int64_t offset, int64_t blk, int64_t world, int64_t rank,
+                                                  int64_t C) {
+    int64_t p = g - offset;
+    if (blk > 0) p = (g >= 0 && (g / blk) % world == rank) ? ((g / blk) / world) * blk + g % blk : -1;
+    return (p >= 0 && p < C) ? p : -1;
+}
+
+// keep-or-swap: the removed point (global index *inc) stays unless a challenger beats its own score s, discounted to
+// (1 - rtol) s when scores are minimised and inflated to (1 + rtol) s when they are maximised; it wins ties
+template <bool MAXIMISE>
+__global__ void exchange_keep_kernel(const int64_t* __restrict__ inc, int64_t offset, int64_t blk, int64_t world, int64_t rank,
+                                     int64_t C, const double* __restrict__ scores, const double* __restrict__ weights,
+                                     double rtol, double* __restrict__ best, int64_t* __restrict__ idx,
+                                     double* __restrict__ inc_score) {
+    const int64_t p = exchange_local(inc[0], offset, blk, world, rank, C);
+    if (p < 0) {
         inc_score[0] = 0.0;
         return;
     }
-    const double s = scores[p];
+    const double s = weights ? scores[p] * weights[p] : scores[p];   // the arg-reduce's own product
     inc_score[0] = s;
-    const double d = (1.0 - rtol) * s;
-    if (idx[0] < 0 || d <= best[0]) {
+    const double d = MAXIMISE ? (1.0 + rtol) * s : (1.0 - rtol) * s;
+    if (idx[0] < 0 || (MAXIMISE ? d >= best[0] : d <= best[0])) {
         best[0] = d;
         idx[0] = p;
     }
+}
+
+__global__ void exchange_unmask_kernel(const int64_t* __restrict__ inc, int64_t offset, int64_t blk, int64_t world,
+                                       int64_t rank, int64_t C, uint8_t* __restrict__ mask) {
+    const int64_t p = exchange_local(inc[0], offset, blk, world, rank, C);
+    if (p >= 0) mask[p] = 0;
 }
 
 __global__ void exchange_record_kernel(const int64_t* __restrict__ inc, const double* __restrict__ inc_score, int64_t n,
@@ -242,8 +278,31 @@ extern "C" int gpx_design_delete_factor(gpx_handle h, double* U, int64_t n, int6
                                        "delete_factor");
         if (rc) return rc;
     }
-    delete_factor_kernel<<<1, DF_NT, smem, (cudaStream_t)stream>>>(U, ldu, (int)n, (int)j, rot, picks, scores, pivots);
+    const DeleteFactorArgs f{U, ldu, rot, picks, scores, pivots};
+    delete_factor_kernel<<<1, DF_NT, smem, (cudaStream_t)stream>>>(f, f, (int)n, (int)j);
     return gpx_check_launch("gpx_design_delete_factor");
+}
+
+extern "C" int gpx_design_delete_factors(gpx_handle h, int64_t n, int64_t j, double* U0, int64_t ldu0, double* rot0,
+                                         int64_t* picks, double* scores, double* pivots, double* U1, int64_t ldu1,
+                                         double* rot1, void* stream) {
+    GPX_REQUIRE(h && U0 && U1, GPX_EINVAL, "bad arguments");
+    GPX_REQUIRE(n >= 1 && j >= 0 && j < n, GPX_EINVAL, "position j must satisfy 0 <= j < n");
+    GPX_REQUIRE(ldu0 >= n && ldu1 >= n, GPX_EINVAL, "ldu < n");
+    GPX_REQUIRE(n - 1 - j <= (int64_t)DF_NT * DF_CPT, GPX_ESIZE, "more than 8192 rotations (n - 1 - j)");
+    GPX_REQUIRE((rot0 != nullptr && rot1 != nullptr && rot0 != rot1) || j == n - 1, GPX_EINVAL,
+                "rot0 and rot1 must be two separate buffers");
+    GPX_REQUIRE(U0 != U1, GPX_EINVAL, "U0 and U1 must be two separate factors");
+    const size_t smem = (size_t)(n - 1 - j > 0 ? n - 1 - j : 1) * sizeof(double);
+    if (smem > 48 * 1024) {
+        const int rc = gpx_ensure_smem(h, (const void*)delete_factor_kernel, (size_t)DF_NT * DF_CPT * sizeof(double),
+                                       "delete_factor");
+        if (rc) return rc;
+    }
+    const DeleteFactorArgs f0{U0, ldu0, rot0, picks, scores, pivots};
+    const DeleteFactorArgs f1{U1, ldu1, rot1, nullptr, nullptr, nullptr};
+    delete_factor_kernel<<<2, DF_NT, smem, (cudaStream_t)stream>>>(f0, f1, (int)n, (int)j);
+    return gpx_check_launch("gpx_design_delete_factors");
 }
 
 extern "C" int gpx_design_delete_rows(gpx_handle h, const double* rot, int64_t j, int64_t n, double* W, int64_t ldw,
@@ -263,8 +322,28 @@ extern "C" int gpx_exchange_keep(gpx_handle h, const int64_t* inc, int64_t index
                                  double rtol, double* best, int64_t* idx, double* inc_score, void* stream) {
     GPX_REQUIRE(h && inc && scores && best && idx && inc_score && C >= 0, GPX_EINVAL, "bad arguments");
     GPX_REQUIRE(rtol >= 0.0, GPX_EINVAL, "rtol must be >= 0");
-    exchange_keep_kernel<<<1, 1, 0, (cudaStream_t)stream>>>(inc, index_offset, C, scores, rtol, best, idx, inc_score);
+    exchange_keep_kernel<false><<<1, 1, 0, (cudaStream_t)stream>>>(inc, index_offset, 0, 1, 0, C, scores, nullptr, rtol, best,
+                                                                    idx, inc_score);
     return gpx_check_launch("gpx_exchange_keep");
+}
+
+extern "C" int gpx_exchange_keep_max(gpx_handle h, const int64_t* inc, int64_t index_offset, int64_t blk, int64_t world,
+                                     int64_t rank, int64_t C, const double* scores, const double* weights, double rtol,
+                                     double* best, int64_t* idx, double* inc_score, void* stream) {
+    GPX_REQUIRE(h && inc && scores && best && idx && inc_score && C >= 0, GPX_EINVAL, "bad arguments");
+    GPX_REQUIRE(blk >= 0 && world >= 1 && rank >= 0 && rank < world, GPX_EINVAL, "blk >= 0, 0 <= rank < world");
+    GPX_REQUIRE(rtol >= 0.0, GPX_EINVAL, "rtol must be >= 0");
+    exchange_keep_kernel<true><<<1, 1, 0, (cudaStream_t)stream>>>(inc, index_offset, blk, world, rank, C, scores, weights,
+                                                                   rtol, best, idx, inc_score);
+    return gpx_check_launch("gpx_exchange_keep_max");
+}
+
+extern "C" int gpx_exchange_unmask(gpx_handle h, const int64_t* inc, int64_t index_offset, int64_t blk, int64_t world,
+                                   int64_t rank, int64_t C, uint8_t* mask, void* stream) {
+    GPX_REQUIRE(h && inc && mask && C >= 0, GPX_EINVAL, "bad arguments");
+    GPX_REQUIRE(blk >= 0 && world >= 1 && rank >= 0 && rank < world, GPX_EINVAL, "blk >= 0, 0 <= rank < world");
+    exchange_unmask_kernel<<<1, 1, 0, (cudaStream_t)stream>>>(inc, index_offset, blk, world, rank, C, mask);
+    return gpx_check_launch("gpx_exchange_unmask");
 }
 
 extern "C" int gpx_exchange_record(gpx_handle h, const int64_t* inc, const double* inc_score, int64_t n, const int64_t* picks,

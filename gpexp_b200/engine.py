@@ -168,6 +168,48 @@ class _Pivoting:
                       f"evaluation from this step on (add noise or shorten the design)", GpxConditionWarning, stacklevel=3)
         return step
 
+    def exchange(self, max_sweeps: int, rtol: float, first: int = 0):
+        """Fedorov-type exchange pass over the current design, run as a queue: each step removes position `first` (the
+        exchangeable point that has waited longest; positions before it are fixed), scores every candidate against the
+        other n-1 points, and appends the winner at the end -- the removed point itself unless a challenger beats its own
+        score by the factor rtol (the engine's exchange_step applies the rule of its criterion).  One sweep = n - first
+        steps, so every exchangeable point present at the start of a sweep is decided once.  Stops after a sweep without
+        a swap or after max_sweeps.  Nothing is read back inside a sweep; one read per sweep decides whether to go on.
+        Returns the accepted swaps per sweep; `self.exchange_costs` (device) holds the score of the point put back at
+        every step (for IVAR the design cost after the step)."""
+        steps = self.n - int(first)
+        if max_sweeps <= 0 or steps <= 0:
+            self.exchange_costs = self.dev.zeros(0)
+            return []
+        swaps = self.dev.zeros(max_sweeps, dtype=torch.int64)
+        costs = self.dev.zeros(max_sweeps * steps)
+        out = []
+        for sweep in range(max_sweeps):
+            for t in range(steps):
+                self.exchange_step(rtol, swaps[sweep:], costs[sweep * steps + t:], int(first))
+            out.append(int(swaps[sweep].item()))
+            if out[-1] == 0:
+                break
+        self.exchange_costs = costs[: len(out) * steps]
+        return out
+
+    def _exchange_buffers(self):
+        """Device buffers of remove() / exchange_step(), allocated by the first remove()."""
+        if getattr(self, "removed", None) is None:
+            self.removed = self.dev.zeros(1, dtype=torch.int64)
+            self.inc_score = self.dev.zeros(1)
+            self._rot = self.dev.zeros(max(2 * self.ncap, 2))
+
+    def _exchange_record(self, n: int, swaps, cost):
+        """After the append of an exchange step on a design of n points: the removed point's own score into the history
+        when it came back, else one more swap; the step's trace entry."""
+        check(lib.gpx_exchange_record(self.dev.h, ptr(self.removed), ptr(self.inc_score), n - 1, ptr(self.picks),
+                                      ptr(self.pick_scores), ptr(swaps), ptr(cost), self.dev.stream), "gpx_exchange_record")
+
+    def _share_inc_score(self):
+        if self.shard is not None and self.shard.world > 1:  # the owner's score of the removed point, for every rank
+            self.shard.dist.all_reduce(self.inc_score, group=self.shard.group)
+
     def _native_ready(self) -> bool:
         """The C-side loop can run this engine: single rank, or an NCCL shard whose ranks all hold candidates."""
         if self.shard is None or self.shard.world == 1:
@@ -185,7 +227,9 @@ class GreedyVarEngine(_Pivoting):
     incremental diagonally-pivoted Cholesky of K_CC: per step one arg-max and one HBM-bound row append."""
 
     def __init__(self, dev: Device, pool: PointSet, n_max: int, weights=None, noise: float = 0.0, shard=None,
-                 index_offset: int = 0):
+                 index_offset: int = 0, keep_factors: bool = False):
+        """keep_factors=True also grows the design factor U (K_AA + noise I = U^T U, ncap x roundup(ncap), replicated on
+        every rank) from the pivot records, which remove() and exchange() need; the steps are then issued from Python."""
         self.pool = pool
         self.noise = float(noise)
         ncap = max(int(n_max), 1)
@@ -195,6 +239,7 @@ class GreedyVarEngine(_Pivoting):
         check(lib.gpx_prior_diag(dev.h, ptr(pool.X), pool.n, pool.ld, ptr(self.var), dev.stream), "gpx_prior_diag")
         self.weights = None if weights is None else dev.upload(np.asarray(weights, dtype=np.float64))
         self.score_trace = None
+        self.U = dev.zeros(ncap, roundup(ncap)) if keep_factors else None
 
     def _local_count(self):
         return self.pool.n
@@ -209,12 +254,47 @@ class GreedyVarEngine(_Pivoting):
         self._gather(self.W, pool.ld, self.var, pool, self.noise, minimize=False)
         check(lib.gpx_append_row(dev.h, _lib.ROW_KERNEL, ptr(self.rec_win), None, ptr(pool.X), pool.n, pool.ld,
                                  ptr(self.W), pool.ld, self.n, ptr(self.var), dev.stream), "gpx_append_row")
-        self._record()
+        self._record(self.U, 0 if self.U is None else self.U.shape[1])
         self.n += 1
 
     def force(self, global_index: int):
         self._force_local(int(global_index))
         self.append()
+
+    def remove(self, position: int):
+        """Delete design point `position` (0 <= position < n) without refactoring (keep_factors=True): Givens rotations
+        turn U into the factor of the remaining n-1 points and bring W along, var += r^2 with the residual row r, and the
+        history closes the gap (pick_pivots[i] = U'[i,i]^2).  Every rank rotates its own columns with the same
+        rotations, computed from the replicated U.  The removed point's global index is left in `self.removed`."""
+        if self.U is None:
+            raise RuntimeError("remove() needs an engine built with keep_factors=True")
+        n = self.n
+        if not 0 <= int(position) < n:
+            raise IndexError(f"remove: position {position} outside the design of {n} points")
+        j = int(position)
+        dev, pool = self.dev, self.pool
+        self._exchange_buffers()
+        self.removed.copy_(self.picks[j: j + 1])
+        check(lib.gpx_design_delete_factor(dev.h, ptr(self.U), n, self.U.shape[1], j, ptr(self._rot), ptr(self.picks),
+                                           ptr(self.pick_scores), ptr(self.pick_pivots), dev.stream), "gpx_design_delete_factor")
+        check(lib.gpx_design_delete_rows(dev.h, ptr(self._rot), j, n, ptr(self.W), pool.ld, pool.n, ptr(self.var),
+                                         dev.stream), "gpx_design_delete_rows")
+        self.n = n - 1
+
+    def exchange_step(self, rtol: float, swaps=None, cost=None, position: int = 0):
+        """One step of exchange(): remove `position`, arg-max of var * weights, keep-or-swap (gpx_exchange_keep_max: a
+        challenger must score above (1 + rtol) x the removed point's score), append.  swaps / cost as in
+        GreedyIVAREngine.exchange_step."""
+        dev, pool = self.dev, self.pool
+        n = self.n
+        self.remove(position)
+        self.select()
+        check(lib.gpx_exchange_keep_max(dev.h, ptr(self.removed), self.index_offset, 0, 1, 0, pool.n, ptr(self.var),
+                                        ptr(self.weights), float(rtol), ptr(self.best), ptr(self.idx), ptr(self.inc_score),
+                                        dev.stream), "gpx_exchange_keep_max")
+        self._share_inc_score()
+        self.append()
+        self._exchange_record(n, swaps, cost)
 
     def step(self):
         if self.score_trace is not None:
@@ -237,8 +317,9 @@ class GreedyVarEngine(_Pivoting):
     def run(self, n_points: int, progress=None, chunk: int = 10):
         """Grow the design to n_points.  Without a score trace the steps are issued by the C-side loop
         (gpx_var_greedy_run) in chunks of `chunk`, between which `progress(n)` is called (the reference prints every
-        10 points, experimentalDesign.py:812-813)."""
-        if self.score_trace is not None or not self._native_ready():
+        10 points, experimentalDesign.py:812-813).  An engine that keeps its factor steps from Python (the C-side loop
+        does not grow U)."""
+        if self.score_trace is not None or self.U is not None or not self._native_ready():
             while self.n < n_points:
                 if progress is not None:
                     progress(self.n)
@@ -580,7 +661,7 @@ class GreedyIVAREngine(_Pivoting):
         self.cov = None
         self.zero_scale = float(zero_scale)
         self.removals = 0          # remove() calls so far (a snapshot is valid only for the count it was taken at)
-        self._rot = None           # exchange buffers, allocated by the first remove()
+        self._rneg = None          # -r_C of a resident remove(), allocated by the first one
         if self.resident:
             self.cov = dev.empty(mc.n, cand.ld)
             # cov_0 = K(mc, cand), then the column sums of squares for the first scoring
@@ -711,11 +792,9 @@ class GreedyIVAREngine(_Pivoting):
             raise IndexError(f"remove: position {position} outside the design of {n} points")
         j = int(position)
         dev, cand, mc = self.dev, self.cand, self.mc
-        if self._rot is None:
-            self._rot = dev.zeros(max(2 * self.ncap, 2))
-            self.removed = dev.zeros(1, dtype=torch.int64)
-            self.inc_score = dev.zeros(1)
-            self._rneg = dev.zeros(cand.ld) if self.resident else None
+        self._exchange_buffers()
+        if self.resident and self._rneg is None:
+            self._rneg = dev.zeros(cand.ld)
         self.removed.copy_(self.picks[j: j + 1])
         check(lib.gpx_design_delete_factor(dev.h, ptr(self.U), n, self.U.shape[1], j, ptr(self._rot), ptr(self.picks),
                                            ptr(self.pick_scores), ptr(self.pick_pivots), dev.stream), "gpx_design_delete_factor")
@@ -730,44 +809,20 @@ class GreedyIVAREngine(_Pivoting):
         self.n = n - 1
         self.removals += 1
 
-    def exchange(self, max_sweeps: int, rtol: float):
-        """Fedorov-type exchange pass over the current design, run as a queue: each step removes position 0 (the point
-        that has waited longest), scores every candidate against the other n-1 points, and appends the winner at the
-        end -- the removed point itself unless a challenger scores below (1 - rtol) x the removed point's own score
-        (gpx_exchange_keep; among challengers the arg-min with the lowest index).  One sweep = n steps, so every point
-        present at the start of a sweep is decided once.  Stops after a sweep without a swap or after max_sweeps.
-        Nothing is read back inside a sweep; one read per sweep decides whether to go on.
-        Returns the accepted swaps per sweep; `self.exchange_costs` (device) holds the design cost after every step."""
-        n = self.n
-        if max_sweeps <= 0 or n == 0:
-            self.exchange_costs = self.dev.zeros(0)
-            return []
-        swaps = self.dev.zeros(max_sweeps, dtype=torch.int64)
-        costs = self.dev.zeros(max_sweeps * n)
-        out = []
-        for sweep in range(max_sweeps):
-            for t in range(n):
-                self.exchange_step(rtol, swaps[sweep:], costs[sweep * n + t:])
-            out.append(int(swaps[sweep].item()))
-            if out[-1] == 0:
-                break
-        self.exchange_costs = costs[: len(out) * n]
-        return out
-
-    def exchange_step(self, rtol: float, swaps=None, cost=None):
-        """One step of exchange(): remove position 0, score, keep-or-swap, append.  swaps / cost (device, nullable):
-        int64 counter incremented on a swap, and the slot that receives the design cost after the step."""
+    def exchange_step(self, rtol: float, swaps=None, cost=None, position: int = 0):
+        """One step of exchange(): remove `position`, score, keep-or-swap (gpx_exchange_keep: a challenger must score
+        below (1 - rtol) x the removed point's own score; among challengers the arg-min with the lowest index), append.
+        swaps / cost (device, nullable): int64 counter incremented on a swap, and the slot that receives the design cost
+        after the step."""
         dev, st = self.dev, self.dev.stream
         n = self.n
-        self.remove(0)
+        self.remove(position)
         self.score()
         check(lib.gpx_exchange_keep(dev.h, ptr(self.removed), self.index_offset, self.cand.n, ptr(self.scores), float(rtol),
                                     ptr(self.best), ptr(self.idx), ptr(self.inc_score), st), "gpx_exchange_keep")
-        if self.shard is not None and self.shard.world > 1:  # the owner's score of the removed point, for every rank
-            self.shard.dist.all_reduce(self.inc_score, group=self.shard.group)
+        self._share_inc_score()
         self.append()
-        check(lib.gpx_exchange_record(dev.h, ptr(self.removed), ptr(self.inc_score), n - 1, ptr(self.picks),
-                                      ptr(self.pick_scores), ptr(swaps), ptr(cost), st), "gpx_exchange_record")
+        self._exchange_record(n, swaps, cost)
 
     def _state(self):
         st = _lib.IvarState()
@@ -916,10 +971,17 @@ class ShardedMIEngine(_Pivoting):
     # 2 GPUs, |V| = 80 000: 512 -> 5.81 s, 1024 -> 5.64 s (round 1, contiguous ranges, no zero skipping: 10.65 s)
     BLK = 1024
 
-    def __init__(self, dev: Device, pool_host: np.ndarray, n_max: int, noise: float, shard=None, pool_noise=None):
+    def __init__(self, dev: Device, pool_host: np.ndarray, n_max: int, noise: float, shard=None, pool_noise=None,
+                 keep_factors: bool = False):
         """pool_noise: host vector nu of a per-point noise at ALL |V| pool points (noise must be 0.0 then), as in
         GreedyMIEngine.  Each rank keeps nu at its own columns; the owner of a pivot p sends num_p + nu_p to the other
-        ranks in the pivot record's divisor rec[2]."""
+        ranks in the pivot record's divisor rec[2].
+
+        keep_factors=True also grows the two design factors that remove() and exchange() need, both ncap x roundup(ncap)
+        and replicated on every rank: U_A (K_AA + diag nu_A = U_A^T U_A) from the numerator's pivot records and U_Q
+        (Q_AA = U_Q^T U_Q, Q = (K_VV + diag nu)^-1) from the records of the precision downdates, so that W = U_A^-T K(A, V)
+        and Us = U_Q^-T Q(A, V)."""
+        self.keep_factors = bool(keep_factors)
         import os
         self.BLK = int(os.environ.get("GPX_MI_BLK", self.BLK))
         if self.BLK < 256 or self.BLK & (self.BLK - 1):
@@ -1047,6 +1109,12 @@ class ShardedMIEngine(_Pivoting):
         self.mask = dev.zeros(ld, dtype=torch.uint8)
         self.scores = dev.zeros(ld)
         self.score_trace = None
+        self.UA = self.UQ = None
+        self.removed = None
+        if self.keep_factors:
+            self.UA = dev.zeros(ncap, roundup(ncap))
+            self.UQ = dev.zeros(ncap, roundup(ncap))
+            self._rotQ = dev.zeros(max(2 * ncap, 2))
 
     def reset(self, n_max: int):
         """Forget the chosen points but keep the O(|V|^3) factorisation (costFunctionGP_MI.evaluate is called once per
@@ -1099,8 +1167,65 @@ class ShardedMIEngine(_Pivoting):
             check(lib.gpx_append_row(dev.h, _lib.ROW_MATRIX, ptr(bufU), ptr(self.pcol), None, nloc, ld, ptr(self.Us), ld,
                                      self.n, ptr(self.pd), st), "gpx_append_row")
             check(lib.gpx_set_mask(dev.h, ptr(self.mask), ptr(self.loc2), 1, st), "gpx_set_mask")
-        self._record()
+        if self.UA is None:
+            self._record()
+        else:
+            ldu = self.UA.shape[1]
+            self._record(self.UA, ldu)
+            # bufU (every rank's copy after the sum) holds pd_p and Us[0:n, p]: column n of U_Q
+            check(lib.gpx_store_pivot(dev.h, ptr(bufU), self.n, ptr(self.UQ), ldu, None, None, None, st), "gpx_store_pivot")
         self.n += 1
+
+    def remove(self, position: int):
+        """Delete design point `position` (0 <= position < n) without refactoring (keep_factors=True): one launch
+        downdates U_A (with the history) and U_Q, each with its own Givens rotations; the rotations of U_A carry W along
+        (num += r^2) and those of U_Q carry Us along (pd += r^2), and the removed point returns to the pool (its mask entry
+        is cleared on the rank that owns it).  Every rank computes the same rotations from the replicated factors and
+        rotates its own columns: no communication.  The removed point's global index is left in `self.removed`."""
+        if self.UA is None:
+            raise RuntimeError("remove() needs an engine built with keep_factors=True")
+        n = self.n
+        if not 0 <= int(position) < n:
+            raise IndexError(f"remove: position {position} outside the design of {n} points")
+        j = int(position)
+        dev, ld, nloc, st = self.dev, self.ld, self.nloc, self.dev.stream
+        self._exchange_buffers()
+        self.removed.copy_(self.picks[j: j + 1])
+        ldu = self.UA.shape[1]
+        check(lib.gpx_design_delete_factors(dev.h, n, j, ptr(self.UA), ldu, ptr(self._rot), ptr(self.picks),
+                                            ptr(self.pick_scores), ptr(self.pick_pivots), ptr(self.UQ), ldu, ptr(self._rotQ),
+                                            st), "gpx_design_delete_factors")
+        check(lib.gpx_design_delete_rows(dev.h, ptr(self._rot), j, n, ptr(self.W), ld, nloc, ptr(self.num), st),
+              "gpx_design_delete_rows")
+        check(lib.gpx_design_delete_rows(dev.h, ptr(self._rotQ), j, n, ptr(self.Us), ld, nloc, ptr(self.pd), st),
+              "gpx_design_delete_rows")
+        check(lib.gpx_exchange_unmask(dev.h, ptr(self.removed), 0, self.BLK, self.world, self.rank, nloc, ptr(self.mask), st),
+              "gpx_exchange_unmask")
+        self.n = n - 1
+
+    def exchange_step(self, rtol: float, swaps=None, cost=None, position: int = 0):
+        """One step of exchange(): remove `position`, score, keep-or-swap (gpx_exchange_keep_max: a challenger must score
+        above (1 + rtol) x the removed point's own score; among challengers the arg-max with the lowest index), take.
+        swaps / cost as in GreedyIVAREngine.exchange_step."""
+        dev = self.dev
+        n = self.n
+        self.remove(position)
+        self.score()
+        check(lib.gpx_exchange_keep_max(dev.h, ptr(self.removed), 0, self.BLK, self.world, self.rank, self.nloc,
+                                        ptr(self.scores), None, float(rtol), ptr(self.best), ptr(self.idx),
+                                        ptr(self.inc_score), dev.stream), "gpx_exchange_keep_max")
+        self._share_inc_score()
+        self.take()
+        self._exchange_record(n, swaps, cost)
+
+    def mutual_information(self) -> float:
+        """I(y_A; y_{V minus A}) in nats = sum_i log U_A[i,i] + sum_i log U_Q[i,i] (det Q_AA = det K_SS / det K_VV with
+        the noise on both diagonals, S = V minus A): half the sum of the two factors' log-determinants."""
+        dev = self.dev
+        out = dev.zeros(2)
+        for k, U in enumerate((self.UA, self.UQ)):
+            check(lib.gpx_logdet_chol(dev.h, ptr(U), self.n, U.shape[1], ptr(out[k:]), dev.stream), "gpx_logdet_chol")
+        return 0.5 * float(out.sum().item())
 
     def force(self, index: int):
         self._force_local(int(index))

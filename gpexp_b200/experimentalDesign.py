@@ -8,6 +8,8 @@ the device-resident engines of gpexp_b200.engine.
     performGreedyIVARExperimentalDesign,        NEW: the discrete greedy-IVAR driver the north star asks for; the
     beginGreedyIVARExperimentalDesign,          reference only has the per-design cost function (SURVEY.md 3.2 / 8c)
     refineGreedyIVARExperimentalDesign,         NEW: exchange passes that improve a discrete IVAR design on the candidates
+    refineGreedyMIExperimentalDesign,           NEW: the same for greedy MI designs on the pool
+    refineGreedyVarExperimentalDesign           NEW: the same for greedy maximum-variance designs
     scoreCandidatesIVAR
 
 The continuous optimisers that CALL these cost functions (ExperimentalDesignDerivative / NoDerivative and the batch-greedy
@@ -113,12 +115,13 @@ def _mi_noise(self):
     return float(noise), None
 
 
-def _mi_new_engine(self, n_max, shard=None):
+def _mi_new_engine(self, n_max, shard=None, keep_factors=False):
     gp = self.gaussianProcess
     noise, nu = _mi_noise(self)
     # left-looking blocked set-up (measured faster than a right-looking dense engine on one GPU as well:
     # |V| = 40 000: 2.33 s vs 2.97 s)
-    return ShardedMIEngine(gp.kernel._bind(), self.mcPoints, n_max, noise, shard=shard, pool_noise=nu)
+    return ShardedMIEngine(gp.kernel._bind(), self.mcPoints, n_max, noise, shard=shard, pool_noise=nu,
+                           keep_factors=keep_factors)
 
 
 def _mi_evaluate(self, index, indexAdded):
@@ -373,23 +376,12 @@ def refineGreedyIVARExperimentalDesign(costFuncIVAR, candidates, indices, maxSwe
     ValueError for indices that are not integers or lie outside the candidates, rtol < 0, maxSweeps < 0, and for a
     design whose factor has a non-finite entry (e.g. a repeated point under zero noise).  maxSweeps = 0 returns the
     input design."""
-    idx = np.asarray(indices)
-    if idx.ndim != 1 or idx.size == 0 or not np.issubdtype(idx.dtype, np.integer):
-        raise ValueError("indices must be a non-empty 1-D sequence of integer candidate indices")
-    if np.any(idx < 0) or np.any(idx >= candidates.shape[0]):
-        raise ValueError(f"indices must lie in [0, {candidates.shape[0]})")
-    if not rtol >= 0.0:
-        raise ValueError(f"rtol must be >= 0, got {rtol}")
-    if isinstance(maxSweeps, (bool, np.bool_)) or not isinstance(maxSweeps, (int, np.integer)) or maxSweeps < 0:
-        raise ValueError(f"maxSweeps must be an integer >= 0, got {maxSweeps!r}")
+    idx = _checked_exchange_args(indices, candidates.shape[0], maxSweeps, rtol, "candidate")
     n = idx.size
     eng = beginGreedyIVARExperimentalDesign(costFuncIVAR, candidates, n, shard=shard, resident=resident)
     for i in idx:
         eng.force(int(i))
-    import torch
-    if not bool(torch.isfinite(eng.U[:n, :n]).all()):
-        raise ValueError("the design's Cholesky factor has a non-finite entry (a repeated or numerically dependent "
-                         "point without noise): it cannot be refined")
+    _require_finite_factor(eng.U, n)
     swaps = eng.exchange(int(maxSweeps), float(rtol))
     dev, mc = eng.dev, eng.mc
     total = dev.zeros(1)
@@ -404,6 +396,120 @@ def refineGreedyIVARExperimentalDesign(costFuncIVAR, candidates, indices, maxSwe
     if returnIndices:
         return out
     return candidates[out, :]
+
+
+def _checked_exchange_args(indices, n_total, maxSweeps, rtol, what, unique=False):
+    """The design of an exchange refinement as an int64 array, after the checks every refine driver makes (ValueError)."""
+    idx = np.asarray(indices)
+    if idx.ndim != 1 or idx.size == 0 or not np.issubdtype(idx.dtype, np.integer):
+        raise ValueError(f"indices must be a non-empty 1-D sequence of integer {what} indices")
+    if np.any(idx < 0) or np.any(idx >= n_total):
+        raise ValueError(f"indices must lie in [0, {n_total})")
+    if unique and np.unique(idx).size != idx.size:
+        raise ValueError("indices must be distinct: a chosen point leaves the pool")
+    if not rtol >= 0.0:
+        raise ValueError(f"rtol must be >= 0, got {rtol}")
+    if isinstance(maxSweeps, (bool, np.bool_)) or not isinstance(maxSweeps, (int, np.integer)) or maxSweeps < 0:
+        raise ValueError(f"maxSweeps must be an integer >= 0, got {maxSweeps!r}")
+    return idx.astype(np.int64)
+
+
+def _require_finite_factor(U, n, strict=False):
+    """ValueError unless the leading n x n block of the design factor U is finite (and, with strict, its diagonal > 0: the
+    objectives take its logarithm)."""
+    import torch
+    u = U[:n, :n]
+    ok = bool(torch.isfinite(u).all()) and (not strict or bool((torch.diagonal(u) > 0).all()))
+    if not ok:
+        raise ValueError("the design's Cholesky factor has a non-finite entry (a repeated or numerically dependent "
+                         "point without noise): it cannot be refined")
+
+
+def refineGreedyMIExperimentalDesign(costFuncMI, indices, maxSweeps=10, rtol=1e-8, returnIndices=False, shard=None):
+    """Improve a discrete mutual-information design by exchange (Fedorov-type) passes over the cost function's pool.
+
+    `indices` are distinct pool indices of the design (e.g. costFuncMI.lastIndices after
+    performGreedyMIExperimentalDesign).  The engine is built as performGreedyMIExperimentalDesign builds it (scalar noise,
+    per-point gp.noise and `shard` apply unchanged; the pool is factored once) and the given points are forced in order.
+    Then, as a queue, each step takes the oldest point out of A (it returns to the pool S), scores every pool point y with
+    the greedy's own score var(y | A) / var(y | S minus y) against the other n-1 points, and puts back the arg-max
+    challenger (lowest index on ties) only if its score exceeds (1 + rtol) x the removed point's own score from the same
+    pass; otherwise the removed point returns.  One sweep re-decides every point once; the pass stops after a sweep
+    without a swap or after maxSweeps.
+
+    The keep rule uses the greedy's score.  With zero noise a swap of j for c changes I(y_A; y_{V minus A}) by exactly
+    1/2 log(score_c / score_j), so every accepted swap raises the mutual information.  With a nugget (scalar or per point)
+    the score is not the exact gain and no monotone objective is claimed; maxSweeps bounds the pass.
+
+    Returns the refined points (or indices with returnIndices) in factor order, the oldest first.  Leaves on the cost
+    function: lastIndices, lastScores (the score of the point put back at every step), lastSwaps (accepted swaps per
+    sweep) and lastMI (I(y_A; y_{V minus A}) in nats of the returned design, from its two Cholesky factors).
+    ValueError for repeated, out-of-range or non-integer indices, rtol < 0, maxSweeps < 0 and a factor with a non-finite
+    entry.  maxSweeps = 0 returns the input design."""
+    idx = _checked_exchange_args(indices, len(costFuncMI.mcPoints), maxSweeps, rtol, "pool", unique=True)
+    n = idx.size
+    eng = _mi_new_engine(costFuncMI, n, shard=shard, keep_factors=True)
+    for i in idx:
+        eng.force(int(i))
+    _require_finite_factor(eng.UA, n, strict=True)
+    _require_finite_factor(eng.UQ, n, strict=True)
+    swaps = eng.exchange(int(maxSweeps), float(rtol))
+    out = eng.indices()
+    costFuncMI.lastIndices = out
+    costFuncMI.lastScores = eng.exchange_costs.cpu().numpy()
+    costFuncMI.lastSwaps = swaps
+    costFuncMI.lastMI = eng.mutual_information()
+    if returnIndices:
+        return out
+    return costFuncMI.mcPoints[out, :]
+
+
+def refineGreedyVarExperimentalDesign(kernel, mcPoints, indices, weights=None, nFixed=0, maxSweeps=10, rtol=1e-8,
+                                      returnIndices=False, returnInfo=False, shard=None):
+    """Improve a discrete maximum-variance (conditional entropy) design by exchange passes over the pool mcPoints.
+
+    The nugget is 0.0 and `weights` (one finite value >= 0 per pool point, at least one > 0) scales the variances, as in
+    performGreedyVarExperimentalDesign.  The first `nFixed` indices are fixed seeds (what indKeepStart holds there): they
+    keep their place and are never removed.  The others are exchanged as a queue: each step takes the oldest exchangeable
+    point out (position nFixed), scores every pool point by its posterior variance x weight given the other n-1 points,
+    and appends the arg-max challenger (lowest index on ties) only if its score exceeds (1 + rtol) x the removed point's
+    own score from the same pass; otherwise the removed point returns.  One sweep re-decides every exchangeable point
+    once; the pass stops after a sweep without a swap or after maxSweeps.  Every accepted swap raises
+    log det K_AA + sum_{i in A} log w_i by log(score_c / score_j) (without weights, log det K_AA: the D-optimal /
+    maximum-entropy exchange).  With `shard` every rank passes the full pool and works on its own contiguous block.
+
+    Returns the refined points (or indices with returnIndices) in factor order: the seeds, then the oldest first.  With
+    returnInfo, (result, info) with info = {"indices", "scores" (score of the point put back at every step), "swaps"
+    (accepted swaps per sweep), "logdet" (the objective above, of the returned design)}.  ValueError for repeated (their
+    Gram without a nugget is singular), out-of-range or non-integer indices, nFixed outside [0, len(indices)], bad
+    weights, rtol < 0, maxSweeps < 0 and a factor with a non-finite entry or a zero pivot.  maxSweeps = 0 returns the
+    input design."""
+    N = mcPoints.shape[0]
+    idx = _checked_exchange_args(indices, N, maxSweeps, rtol, "pool", unique=True)
+    n = idx.size
+    if isinstance(nFixed, (bool, np.bool_)) or not isinstance(nFixed, (int, np.integer)) or not 0 <= nFixed <= n:
+        raise ValueError(f"nFixed must be an integer in [0, {n}], got {nFixed!r}")
+    w = None if weights is None else _checked_per_point(weights, N, "weights has", need_positive=True)
+    dev = kernel._bind()
+    lo, hi = 0, N
+    if shard is not None:
+        lo, hi = Shard.split(N, shard.world, shard.rank)
+    eng = GreedyVarEngine(dev, dev.points(mcPoints[lo:hi]), n, weights=None if w is None else w[lo:hi], noise=0.0,
+                          shard=shard, index_offset=lo, keep_factors=True)
+    for i in idx:
+        eng.force(int(i))
+    _require_finite_factor(eng.U, n, strict=True)
+    swaps = eng.exchange(int(maxSweeps), float(rtol), first=int(nFixed))
+    out = eng.indices()
+    total = dev.zeros(1)
+    check(lib.gpx_logdet_chol(dev.h, ptr(eng.U), n, eng.U.shape[1], ptr(total), dev.stream), "gpx_logdet_chol")
+    logdet = float(total.item())
+    if w is not None:
+        logdet += float(np.sum(np.log(w[out])))
+    result = out if returnIndices else mcPoints[out, :]
+    if returnInfo:
+        return result, {"indices": out, "scores": eng.exchange_costs.cpu().numpy(), "swaps": swaps, "logdet": logdet}
+    return result
 
 
 def scoreCandidatesIVAR(costFuncIVAR, design, candidates, shard=None):
@@ -458,5 +564,7 @@ DEVICE_FUNCTIONS = {
     "performGreedyIVARExperimentalDesign": performGreedyIVARExperimentalDesign,
     "beginGreedyIVARExperimentalDesign": beginGreedyIVARExperimentalDesign,
     "refineGreedyIVARExperimentalDesign": refineGreedyIVARExperimentalDesign,
+    "refineGreedyMIExperimentalDesign": refineGreedyMIExperimentalDesign,
+    "refineGreedyVarExperimentalDesign": refineGreedyVarExperimentalDesign,
     "scoreCandidatesIVAR": scoreCandidatesIVAR,
 }

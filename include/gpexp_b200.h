@@ -4,7 +4,7 @@
  * The reference (goroda/GPEXP) is pure Python/numpy and has NO native or FFI layer
  * (SURVEY.md section 8b), so there is no existing binding to mirror: every entry point
  * below cites the reference Python function whose arithmetic it replaces, and
- * INTEGRATION.md shows the ctypes stub a maintainer of the reference would add.  83 entry points.
+ * INTEGRATION.md shows the ctypes stub a maintainer of the reference would add.  86 entry points.
  *
  * Conventions
  *   - every pointer is a DEVICE pointer owned by the caller unless the name ends in _host;
@@ -331,7 +331,7 @@ int gpx_set_mask(gpx_handle h, uint8_t* mask, const int64_t* idx_dev, uint8_t va
 int gpx_store_pivot(gpx_handle h, const double* rec, int64_t n, double* U, int64_t ldu, int64_t* picks,
                     double* scores, double* pivots, void* stream);
 
-/* ---- Exchange refinement of a greedy IVAR design: deleting design position j (0 <= j < n) in place ------------------
+/* ---- Exchange refinement of a greedy design: deleting design position j (0 <= j < n) in place ----------------------
  * gpx_design_delete_factor: U (n x n within ldu, upper triangular, K_DD + diag(noise) = U^T U) becomes the (n-1) x (n-1)
  *     factor of the design without point j: column j is dropped and Givens rotations G_i on rows (i, i+1), i = j .. n-2,
  *     zero the subdiagonal (c = a/rho, s = b/rho, rho = hypot(a, b) >= 0 the new diagonal; the identity when a = b = 0).
@@ -346,12 +346,28 @@ int gpx_design_delete_factor(gpx_handle h, double* U, int64_t n, int64_t ldu, in
                              double* scores, double* pivots, void* stream);
 int gpx_design_delete_rows(gpx_handle h, const double* rot, int64_t j, int64_t n, double* W, int64_t ldw, int64_t ncols,
                            double* var, void* stream);
+/* gpx_design_delete_factor for two independent factors of the same design in one launch of two blocks (the MI exchange
+ * keeps U_A, K_AA + diag nu_A = U_A^T U_A, and U_Q, Q_AA = U_Q^T U_Q with Q = (K_VV + diag nu)^-1): U0 with the history
+ * picks / scores / pivots (nullable) and rotations rot0, U1 with rotations rot1 and no history.  rot0 != rot1. */
+int gpx_design_delete_factors(gpx_handle h, int64_t n, int64_t j, double* U0, int64_t ldu0, double* rot0, int64_t* picks,
+                              double* scores, double* pivots, double* U1, int64_t ldu1, double* rot1, void* stream);
 /* Keep-or-swap rule of one exchange step, between scoring and the pivot gather.  *inc = GLOBAL index of the removed point;
  * on the rank that holds it (0 <= *inc - index_offset < C): inc_score[0] = its score s, and if (1 - rtol) s <= best[0]
  * then best[0] = (1 - rtol) s, idx[0] = its local index, so a challenger wins only below (1 - rtol) s (ties keep it).
  * Other ranks write inc_score[0] = 0 (a sum over the ranks gives s everywhere).  rtol >= 0. */
 int gpx_exchange_keep(gpx_handle h, const int64_t* inc, int64_t index_offset, int64_t C, const double* scores, double rtol,
                       double* best, int64_t* idx, double* inc_score, void* stream);
+/* The same rule for maximised scores (MI, maximum variance): s = scores[p] * (weights ? weights[p] : 1), the arg-reduce's
+ * product; if (1 + rtol) s >= best[0] then best[0] = (1 + rtol) s, idx[0] = p, so a challenger wins only above
+ * (1 + rtol) s (ties keep it).  The local column p of *inc: *inc - index_offset in [0, C) when blk == 0, else the
+ * block-cyclic map of gpx_local_index_cyclic (blk, world, rank).  Ranks that do not own *inc write inc_score[0] = 0. */
+int gpx_exchange_keep_max(gpx_handle h, const int64_t* inc, int64_t index_offset, int64_t blk, int64_t world, int64_t rank,
+                          int64_t C, const double* scores, const double* weights, double rtol, double* best, int64_t* idx,
+                          double* inc_score, void* stream);
+/* mask[p] = 0 for the local column p of *inc (mapped as in gpx_exchange_keep_max) on the rank that owns it: a point
+ * deleted from an MI design returns to the pool. */
+int gpx_exchange_unmask(gpx_handle h, const int64_t* inc, int64_t index_offset, int64_t blk, int64_t world, int64_t rank,
+                        int64_t C, uint8_t* mask, void* stream);
 /* After the append of step n: if picks[n] == *inc (the removed point came back) pick_scores[n] = inc_score[0] (its true
  * cost instead of the discounted one), else swaps[0] += 1; trace[0] = pick_scores[n].  swaps, trace nullable. */
 int gpx_exchange_record(gpx_handle h, const int64_t* inc, const double* inc_score, int64_t n, const int64_t* picks,
