@@ -21,6 +21,7 @@ SE, MATERN32, MEHLER, MATERN12, MATERN52 = 0, 1, 2, 3, 4
 SIDE_A, SIDE_B = 0, 1
 ROW_KERNEL, ROW_MATRIX = 0, 1
 PRO_EXPANDED, PRO_DIFF = 1, 2
+MEASURE_BOX, MEASURE_GAUSS = 1, 2
 
 
 class GpxError(RuntimeError):
@@ -97,6 +98,12 @@ SIGNATURES = {
     "gpx_score_ivar": [_p, _int, _p, _i64, _p, _p, _i64, _p, _i64, _p, _p, _i64, _i64, _dbl, _dbl, _p, _p, _p, _p, _p, _p],
     "gpx_score_ivar_w": [_p, _int, _p, _i64, _p, _p, _i64, _p, _i64, _p, _p, _i64, _i64, _dbl, _dbl, _p, _p, _p, _p, _p, _p,
                          _p],
+    "gpx_set_measure": [_p, _int, _int, C.POINTER(_dbl), C.POINTER(_dbl)],
+    "gpx_phi_gram": [_p, _p, _i64, _i64, _p, _i64, _i64, _p, _i64, _p],
+    "gpx_phi_diag": [_p, _p, _i64, _i64, _p, _p],
+    "gpx_phi_append_row": [_p, _p, _p, _i64, _i64, _p, _i64, _i64, _p],
+    "gpx_psi_row": [_p, _p, _i64, _p, _i64, _p, _i64, _i64, _p, _i64, _p],
+    "gpx_ivar_measure_score": [_p, _p, _p, _p, _i64, _p, _p, _i64, _i64, _int, _p, _i64, _dbl, _dbl, _p, _p, _p, _p, _p],
     "gpx_cov_segments": [_i64, _i64],
     "gpx_cov_update": [_p, _p, _i64, _i64, _i64, _p, _p, _p, _i64, _p],
     "gpx_cov_update_w": [_p, _p, _i64, _i64, _i64, _p, _p, _p, _p, _i64, _p],

@@ -154,6 +154,7 @@ extern "C" int gpx_set_kernel(gpx_handle h, int family, int d, const double* p, 
     }
     h->kp = kp;
     h->has_kernel = true;
+    h->has_measure = false;  // a measure's constants belong to one kernel
     memset(h->center, 0, sizeof(h->center));  // a centre belongs to one kernel / data set
     return GPX_OK;
 }

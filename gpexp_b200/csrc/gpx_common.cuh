@@ -31,6 +31,22 @@ struct KCenter {
     double c[GPX_MAX_DIM];
 };
 
+// Integration measure of the closed-form IVAR path (gpx_set_measure), for the handle's SE kernel:
+//   Phi(x, y) = pref * exp(sum_q [-a4_q (x_q - y_q)^2 + E_q(m_q)]) * prod_q F_q(m_q),   m = (x + y) / 2
+// with E_q F_q the per-dimension factor I_q(m_q) of include/gpexp_b200.h split into an exponent and a bounded rest.
+//   BOX    p0 = lo_q / cl_q, p1 = hi_q / cl_q, rs_q = 1 / cl_q, width_q = (hi_q - lo_q) / cl_q ; pref = s^2 / prod width_q
+//   GAUSS  p0 = mean_q, rs_q = 1 / sqrt(cl_q^2 + 2 std_q^2)                                  ; pref = s^2 prod (1 + 2 std_q^2 / cl_q^2)^-1/2
+struct MParams {
+    int kind;
+    int d;
+    double pref;
+    double a4[GPX_MAX_DIM];
+    double rs[GPX_MAX_DIM];
+    double p0[GPX_MAX_DIM];
+    double p1[GPX_MAX_DIM];
+    double width[GPX_MAX_DIM];
+};
+
 struct gpx_context {
     int device;
     int sm_count;
@@ -55,6 +71,8 @@ struct gpx_context {
     int ivar_core;            // GPX_CORE_DMMA | GPX_CORE_I8 (gpx_set_ivar_core)
     void* i8_scratch;         // caller memory for the INT8 core's operand slices (gpx_set_ivar_scratch)
     int64_t i8_scratch_bytes;
+    bool has_measure;         // gpx_set_measure since the last gpx_set_kernel (the constants depend on the kernel)
+    MParams mp;
 };
 
 #ifndef GPX_DEFAULT_IVAR_RING

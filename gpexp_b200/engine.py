@@ -865,6 +865,137 @@ class GreedyIVAREngine(_Pivoting):
         return self.indices()
 
 
+class MeasureIVAREngine(_Pivoting):
+    """Discrete greedy IVAR with the integral over a box or Gaussian measure in closed form (squared-exponential kernels):
+    no integration points and no contraction.  With K_DD + diag(noise) = U^T U it keeps, for the candidates,
+        W_C = U^-T K(D, C),  Z_C = U^-T Phi(D, C),  Y_C = Psi W_C,  Phi_cc,  varC
+    and Psi = U^-T Phi_DD U^-1 (n x n), Phi(a, b) = int k(x, a) k(x, b) dmu(x).  The cost of design + {c} is
+        |s - tr Psi - q_c / (varC_c + noise)|,   q_c = Phi_cc - 2 w_c.z_c + w_c.y_c,
+    the M -> infinity limit of GreedyIVAREngine's score.  A step appends one row to W_C and Z_C, one row and column to
+    Psi, and the scoring pass updates Y_C by one rank-1 term and one new row: O(n C) memory traffic.
+
+    measure: (kind, p0, p1) with kind = _lib.MEASURE_BOX (p0 = lower, p1 = upper bounds) or _lib.MEASURE_GAUSS (p0 =
+    means, p1 = standard deviations), d doubles each.  cand_noise as in GreedyIVAREngine (noise-inclusive varC).
+    Single rank only."""
+
+    def __init__(self, dev: Device, cand: PointSet, n_max: int, noise: float, kernel_spec, measure, cand_noise=None):
+        fam, d, params = kernel_spec
+        if fam != _lib.SE:
+            raise NotImplementedError("the closed-form measure integral is implemented for squared-exponential kernels only")
+        self.cand = cand
+        self.kernel_spec = (fam, d, np.asarray(params, dtype=np.float64))
+        kind, p0, p1 = measure
+        self.measure = (int(kind), np.ascontiguousarray(p0, dtype=np.float64).ravel(),
+                        np.ascontiguousarray(p1, dtype=np.float64).ravel())
+        self.noise = float(noise)
+        nu = _noise_vector("cand_noise", cand_noise, self.noise, cand.n, "candidates")
+        self.cand_noise = None if nu is None else dev.upload(nu)
+        self.zero_scale = prior_scale(fam, params)
+        self.zero_tol = ZERO_VAR_TOL * self.zero_scale
+        ncap = max(int(n_max), 1)
+        self._init_pivot(dev, ncap, n_max, None, 0)
+        self._bind()
+        self.Wc = dev.zeros(ncap, cand.ld)
+        self.Zc = dev.zeros(ncap, cand.ld)
+        self.Yc = dev.zeros(ncap, cand.ld)
+        self.U = dev.zeros(ncap, roundup(ncap))
+        self.Psi = dev.zeros(ncap, roundup(ncap))
+        self.varC = dev.zeros(cand.ld)
+        self.phic = dev.zeros(cand.ld)
+        self.scores = dev.zeros(cand.ld)
+        self.cost = dev.zeros(1)   # s - tr Psi of the current design, written by score()
+        self.ny = 0                # rows of Y_C that are current (n - 1 right after an append)
+        check(lib.gpx_prior_diag(dev.h, ptr(cand.X), cand.n, cand.ld, ptr(self.varC), dev.stream), "gpx_prior_diag")
+        if self.cand_noise is not None:
+            check(lib.gpx_axpby(dev.h, cand.n, 1.0, ptr(self.cand_noise), 1.0, ptr(self.varC), dev.stream), "gpx_axpby")
+        check(lib.gpx_phi_diag(dev.h, ptr(cand.X), cand.n, cand.ld, ptr(self.phic), dev.stream), "gpx_phi_diag")
+        self.score_trace = None
+
+    def _local_count(self):
+        return self.cand.n
+
+    def _bind(self):
+        """Make this engine's kernel and measure the handle's (another engine or kernel may have rebound the handle)."""
+        fam, d, params = self.kernel_spec
+        self.dev.set_kernel(fam, d, params)
+        kind, p0, p1 = self.measure
+        dbl = C.POINTER(C.c_double)
+        check(lib.gpx_set_measure(self.dev.h, kind, d, p0.ctypes.data_as(dbl), p1.ctypes.data_as(dbl)), "gpx_set_measure")
+
+    def score(self):
+        """Score every candidate and arg-min (bringing Y_C up to date with the last append on the way)."""
+        self._bind()
+        dev, cand = self.dev, self.cand
+        update = 1 if self.ny < self.n else 0
+        check(lib.gpx_ivar_measure_score(dev.h, ptr(self.Wc), ptr(self.Zc), ptr(self.Yc), cand.ld, ptr(self.phic),
+                                         ptr(self.varC), cand.n, self.n, update, ptr(self.Psi), self.Psi.shape[1],
+                                         self.noise, self.zero_tol, ptr(self.cost), ptr(self.scores), ptr(self.best),
+                                         ptr(self.idx), dev.stream), "gpx_ivar_measure_score")
+        self.ny = self.n
+
+    def append(self):
+        assert self.ny == self.n, "append() needs Y_C current: score() first"
+        self._bind()
+        dev, cand, n = self.dev, self.cand, self.n
+        self._gather(self.Wc, cand.ld, self.varC, cand, self.noise, minimize=True)
+        check(lib.gpx_append_row(dev.h, _lib.ROW_KERNEL, ptr(self.rec_win), None, ptr(cand.X), cand.n, cand.ld,
+                                 ptr(self.Wc), cand.ld, n, ptr(self.varC), dev.stream), "gpx_append_row")
+        check(lib.gpx_phi_append_row(dev.h, ptr(self.rec_win), ptr(cand.X), cand.n, cand.ld, ptr(self.Zc), cand.ld, n,
+                                     dev.stream), "gpx_phi_append_row")
+        self._record(self.U, self.U.shape[1])
+        check(lib.gpx_psi_row(dev.h, ptr(self.U), self.U.shape[1], ptr(self.Zc), cand.ld, ptr(self.picks), 0, n,
+                              ptr(self.Psi), self.Psi.shape[1], dev.stream), "gpx_psi_row")
+        self.n = n + 1
+
+    def force(self, global_index: int):
+        if self.ny < self.n:
+            self.score()
+        self._force_local(int(global_index))
+        self.append()
+
+    def step(self):
+        self.score()
+        if self.score_trace is not None:
+            self.score_trace.append(self.scores[: self.cand.n].cpu().numpy().copy())
+        self.append()
+
+    def run(self, n_points: int, progress=None):
+        while self.n < n_points:
+            if progress is not None:
+                progress(self.n)
+            self.step()
+        return self.indices()
+
+    def load_design(self, factor: DesignFactor):
+        """State for a GIVEN design (not grown greedily): W_C and varC through the fused Gram + TRSM, Z_C = U^-T Phi(D, C),
+        Psi = U^-T (U^-T Phi_DD)^T, Y_C = Psi W_C by the DMMA update."""
+        assert factor.n <= self.ncap
+        self._bind()
+        dev, cand, D = self.dev, self.cand, factor.design
+        n = factor.n
+        self.n = self.ny = n
+        _, vC = factor.solve_gram(cand, W=self.Wc)
+        self.varC.copy_(vC)
+        if self.cand_noise is not None:
+            check(lib.gpx_axpby(dev.h, cand.n, 1.0, ptr(self.cand_noise), 1.0, ptr(self.varC), dev.stream), "gpx_axpby")
+        if n == 0:
+            return
+        st, ldu, ldp = dev.stream, factor.ldu, self.Psi.shape[1]
+        check(lib.gpx_phi_gram(dev.h, ptr(D.X), n, D.ld, ptr(cand.X), cand.n, cand.ld, ptr(self.Zc), cand.ld, st), "gpx_phi_gram")
+        check(lib.gpx_trsm(dev.h, ptr(factor.U), n, ldu, ptr(self.Zc), cand.n, cand.ld, st), "gpx_trsm")
+        T = dev.zeros(n, ldp)
+        check(lib.gpx_phi_gram(dev.h, ptr(D.X), n, D.ld, ptr(D.X), n, D.ld, ptr(T), ldp, st), "gpx_phi_gram")
+        check(lib.gpx_trsm(dev.h, ptr(factor.U), n, ldu, ptr(T), n, ldp, st), "gpx_trsm")           # U^-T Phi_DD
+        self.Psi.zero_()
+        check(lib.gpx_transpose(dev.h, ptr(T), n, n, ldp, ptr(self.Psi), ldp, st), "gpx_transpose")  # Phi_DD U^-1
+        check(lib.gpx_trsm(dev.h, ptr(factor.U), n, ldu, ptr(self.Psi), n, ldp, st), "gpx_trsm")    # U^-T Phi_DD U^-1
+        self.Yc[:n].zero_()
+        check(lib.gpx_dgemm_tn_sub(dev.h, ptr(self.Psi), ldp, ptr(self.Wc), cand.ld, ptr(self.Yc), cand.ld, n, cand.n, n, 0,
+                                   st), "gpx_dgemm_tn_sub")                                          # -Psi W_C
+        check(lib.gpx_scale_rows_cols(dev.h, ptr(self.Yc), n, cand.n, cand.ld, None, None, -1.0, ptr(self.Yc), cand.ld, st),
+              "gpx_scale_rows_cols")
+
+
 class GreedyMIEngine(_Pivoting):
     """Greedy mutual information (experimentalDesign.py:753-785 with :252-285 restated):
     numerator = running posterior variance given A (nugget = noise); denominator from the diagonal of

@@ -23,9 +23,12 @@ import itertools
 
 import numpy as np
 
+from . import _lib
 from ._lib import check, lib
+from .approximation import UniformMeasure
 from .device import ptr
-from .engine import (DesignFactor, GreedyIVAREngine, GreedyVarEngine, Shard, ShardedMIEngine, prior_scale)
+from .engine import (DesignFactor, GreedyIVAREngine, GreedyVarEngine, MeasureIVAREngine, Shard, ShardedMIEngine,
+                     prior_scale)
 from .gp_kernel_utilities import _nugget_arg
 
 VERBOSE = True  # the reference prints its progress unconditionally (experimentalDesign.py:812-813)
@@ -49,21 +52,49 @@ def _ivar_weights(self):
     return _checked_per_point(w, len(self.mcPoints), "mcWeights has", need_positive=True)
 
 
+def _ivar_measure(self, what=None):
+    """The cost function's `measure` as (kind, lower-or-mean, upper-or-std) for its kernel's dimension, or None.
+    ValueError with mcWeights set as well; NotImplementedError for a kernel other than squared-exponential and for `what`
+    (the name of a feature the closed form does not support), each naming the measure."""
+    m = getattr(self, "measure", None)
+    if m is None:
+        return None
+    if getattr(self, "mcWeights", None) is not None:
+        raise ValueError(f"{m!r} integrates exactly and mcWeights weights integration points: set one of the two")
+    if what is not None:
+        raise NotImplementedError(f"{m!r}: {what} is not implemented for the closed-form measure integral")
+    fam, d, _ = self.gaussianProcess.kernel._gpx_spec()
+    if fam != _lib.SE:
+        raise NotImplementedError(f"{m!r}: the closed-form measure integral is implemented for squared-exponential "
+                                  f"kernels only")
+    p0, p1 = m.params(d)
+    return (_lib.MEASURE_BOX if isinstance(m, UniformMeasure) else _lib.MEASURE_GAUSS), p0, p1
+
+
 def _ivar_evaluate(self, inputPoints):
     """|mean posterior variance over the MC points| for the design `inputPoints` (:79-117); with weights w
-    (`mcWeights`), |sum_m w_m var(x_m)|."""
+    (`mcWeights`), |sum_m w_m var(x_m)|; with a `measure`, the exact |int var(x) dmu(x)|."""
     assert inputPoints.shape == (self.numInputs, self.space.dimension), \
         ("inputPoints are the wrong size: ", inputPoints.shape)
     if self.version != 1:
         raise NotImplementedError("IVAR version 0 needs a kernel eigen-basis that no shipped kernel provides "
                                   "(experimentalDesign.py:119-146 is unreachable)")
-    w = _ivar_weights(self)
+    meas = _ivar_measure(self)
+    w = None if meas is not None else _ivar_weights(self)
     gp = self.gaussianProcess
     if self.space.noiseFunc is None:
         gp.addNodesAndComputeCovariance(inputPoints)
     else:
         gp.addNodesAndComputeCovariance(inputPoints, self.space.noiseFunc(inputPoints))
     f = gp._factor
+    if meas is not None:
+        if not isinstance(f, DesignFactor):
+            raise NotImplementedError(f"{self.measure!r}: the closed-form measure integral needs a full GP, not FITC")
+        # the design's own points serve as the engine's candidates: only its cost s - tr Psi is read
+        eng = MeasureIVAREngine(f.dev, f.design, f.n, 0.0, gp.kernel._gpx_spec(), meas)
+        eng.load_design(f)
+        eng.score()
+        return np.abs(float(eng.cost.item()))
     mc = _ivar_mc_points(self, f.dev)
     _, var = f.solve_gram(mc)
     total = f.dev.zeros(1)
@@ -81,6 +112,7 @@ def _ivar_derivative(self, inputPoints):
     own derivative in the heteroscedastic case.  Squared-exponential kernels.  With weights w (`mcWeights`) the row
     reduction is sum_m w_m instead of the mean."""
     gp = self.gaussianProcess
+    _ivar_measure(self, "the derivative")
     gp.kernel._require_derivative()
     w = _ivar_weights(self)
     noise_grad = same = None
@@ -172,16 +204,27 @@ class costFunctionGP_IVAR(costFunctionBase):
     region of interest (weighted IMSE).  w = 1/nMC is the plain cost.  evaluate, derivative and the greedy drivers
     (beginGreedyIVARExperimentalDesign, performGreedyIVARExperimentalDesign, scoreCandidatesIVAR) read it; bad weights
     raise ValueError before any device work.  Under install_as_gpExp(path) the reference's own constructor is kept, so
-    there the caller sets `cf.mcWeights = w` after construction."""
+    there the caller sets `cf.mcWeights = w` after construction.
+
+    measure (attribute or keyword, default None): a gpexp_b200.approximation.UniformMeasure or GaussianMeasure.  The cost
+    is then the exact |int var(x) dmu(x)| for a squared-exponential kernel, with no integration points and no sampling
+    error; evaluate, the greedy drivers and scoreCandidatesIVAR use it (a heteroscedastic space.noiseFunc applies as in
+    the Monte-Carlo path).  With a measure, mcPoints is not sampled when not given.  ValueError together with mcWeights;
+    NotImplementedError for other kernels, derivative, refineGreedyIVARExperimentalDesign, shard= and resident=True."""
 
     mcWeights = None
+    measure = None
 
     def __init__(self, gaussianProcess, nInputs, space, version=1, **kwargs):
         costFunctionBase.__init__(self, nInputs, space)
         self.gaussianProcess, self.version = copy.copy(gaussianProcess), version
         if version == 1:
-            pts = kwargs['mcPoints'] if 'mcPoints' in kwargs else space.sample((10000, space.dimension))
-            self.mcPoints, self.nMC = pts, len(pts)
+            self.measure = kwargs.get('measure')
+            if 'mcPoints' in kwargs:
+                pts = kwargs['mcPoints']
+            else:
+                pts = space.sample((10000, space.dimension)) if self.measure is None else None
+            self.mcPoints, self.nMC = pts, 0 if pts is None else len(pts)
             self.mcWeights = kwargs.get('mcWeights')
 
     evaluate = _ivar_evaluate
@@ -308,9 +351,13 @@ def beginGreedyIVARExperimentalDesign(costFuncIVAR, candidates, nPoints, shard=N
     It must return one finite value >= 0 per point, else ValueError.
 
     With `costFuncIVAR.mcWeights` the cost of design + [c] is the weighted sum over the integration points (see
-    costFunctionGP_IVAR); the weights are replicated with the integration points, so every rank passes the same ones."""
+    costFunctionGP_IVAR); the weights are replicated with the integration points, so every rank passes the same ones.
+
+    With `costFuncIVAR.measure` the engine is a gpexp_b200.engine.MeasureIVAREngine (exact integral, `.run(n)`,
+    `.indices()`, `.pick_scores`); shard and resident=True raise NotImplementedError there."""
     gp = costFuncIVAR.gaussianProcess
-    weights = _ivar_weights(costFuncIVAR)
+    meas = _ivar_measure(costFuncIVAR, "shard=" if shard is not None else "resident=True" if resident else None)
+    weights = None if meas is not None else _ivar_weights(costFuncIVAR)
     lo, hi = 0, candidates.shape[0]
     if shard is not None:
         lo, hi = Shard.split(candidates.shape[0], shard.world, shard.rank)
@@ -324,6 +371,8 @@ def beginGreedyIVARExperimentalDesign(costFuncIVAR, candidates, nPoints, shard=N
     dev = gp.kernel._bind()
     fam, d, params = gp.kernel._gpx_spec()
     cand = dev.points(candidates[lo:hi])
+    if meas is not None:
+        return MeasureIVAREngine(dev, cand, nPoints, noise, (fam, d, params), meas, cand_noise=cand_noise)
     mc = _ivar_mc_points(costFuncIVAR, dev)
     if resident is None:
         import torch
@@ -375,7 +424,8 @@ def refineGreedyIVARExperimentalDesign(costFuncIVAR, candidates, indices, maxSwe
     mcWeights) and illConditionedFrom (as performGreedyIVARExperimentalDesign, for the returned design).
     ValueError for indices that are not integers or lie outside the candidates, rtol < 0, maxSweeps < 0, and for a
     design whose factor has a non-finite entry (e.g. a repeated point under zero noise).  maxSweeps = 0 returns the
-    input design."""
+    input design.  NotImplementedError for a cost function with a `measure`."""
+    _ivar_measure(costFuncIVAR, "exchange refinement")
     idx = _checked_exchange_args(indices, candidates.shape[0], maxSweeps, rtol, "candidate")
     n = idx.size
     eng = beginGreedyIVARExperimentalDesign(costFuncIVAR, candidates, n, shard=shard, resident=resident)
@@ -518,9 +568,11 @@ def scoreCandidatesIVAR(costFuncIVAR, design, candidates, shard=None):
     block and returns (costs of its block, GLOBAL arg-min index).  This is the end-to-end call bench.py times (`e2e`).
     A heteroscedastic `costFuncIVAR.space.noiseFunc` is honoured as in beginGreedyIVARExperimentalDesign: the design
     Gram gets the nugget noiseFunc(design) and candidate c the noise noiseFunc(c).  `costFuncIVAR.mcWeights` weights the
-    integration points as in costFunctionGP_IVAR.evaluate."""
+    integration points as in costFunctionGP_IVAR.evaluate; `costFuncIVAR.measure` makes the costs the exact integrals
+    (shard= then raises NotImplementedError)."""
     gp = costFuncIVAR.gaussianProcess
-    weights = _ivar_weights(costFuncIVAR)
+    meas = _ivar_measure(costFuncIVAR, "shard=" if shard is not None else None)
+    weights = None if meas is not None else _ivar_weights(costFuncIVAR)
     noiseFunc = costFuncIVAR.space.noiseFunc
     lo, hi = 0, candidates.shape[0]
     if shard is not None:
@@ -535,9 +587,12 @@ def scoreCandidatesIVAR(costFuncIVAR, design, candidates, shard=None):
     dev = gp.kernel._bind()
     fam, d, params = gp.kernel._gpx_spec()
     cand = dev.points(candidates[lo:hi])
-    mc = dev.points(costFuncIVAR.mcPoints)
-    eng = GreedyIVAREngine(dev, cand, mc, max(n, 1), noise, prior_scale(fam, params), cand_noise=cand_noise,
-                           mc_weights=weights)
+    if meas is not None:
+        eng = MeasureIVAREngine(dev, cand, max(n, 1), noise, (fam, d, params), meas, cand_noise=cand_noise)
+    else:
+        mc = dev.points(costFuncIVAR.mcPoints)
+        eng = GreedyIVAREngine(dev, cand, mc, max(n, 1), noise, prior_scale(fam, params), cand_noise=cand_noise,
+                               mc_weights=weights)
     if n:
         eng.load_design(DesignFactor(dev, dev.points(design), nugget))
     eng.score()

@@ -258,6 +258,51 @@ int gpx_score_ivar_w(gpx_handle h, int prologue, const double* Wm, int64_t ldm, 
                      double noise, double zero_tol, const double* wM, const uint8_t* mask, double* workspace,
                      double* score_out, double* best, int64_t* idx, void* stream);
 
+/* ---- Closed-form IVAR over a measure (squared-exponential kernels) ---------------------------------------------------
+ * Replaces the Monte-Carlo estimate of int var_D(x) dmu(x) (the mean over mcPoints, experimentalDesign.py:105-117, and
+ * the M x n x C contraction of gpx_score_ivar) by its exact value for a product measure mu:
+ *     Phi(a, b) = int k(x, a) k(x, b) dmu(x) = s^2 prod_q exp(-(a_q - b_q)^2 / (4 cl_q^2)) I_q((a_q + b_q) / 2)
+ *     GPX_MEASURE_BOX    uniform on [lo_q, hi_q]:  I_q(m) = cl_q sqrt(pi) / (2 (hi_q - lo_q)) (erf((hi_q - m)/cl_q) - erf((lo_q - m)/cl_q))
+ *     GPX_MEASURE_GAUSS  N(mean_q, std_q^2):        I_q(m) = (1 + 2 std_q^2/cl_q^2)^-1/2 exp(-(m - mean_q)^2 / (cl_q^2 + 2 std_q^2))
+ * With K_DD + diag(noise) = U^T U, W_C = U^-T K(D, C), Z_C = U^-T Phi(D, C), Psi = U^-T Phi_DD U^-1 and Y_C = Psi W_C:
+ *     int var_D dmu = s - tr Psi ,   int cov_D(x, c)^2 dmu = q_c = Phi_cc - 2 w_c.z_c + w_c.y_c
+ * and the cost of design+{c} is |s - tr Psi - q_c / (var_D(c) + noise_c)|, the M -> infinity limit of gpx_score_ivar. */
+#define GPX_MEASURE_BOX 1   /* p0 = lower bounds, p1 = upper bounds (p0 < p1)                                */
+#define GPX_MEASURE_GAUSS 2 /* p0 = means, p1 = standard deviations (> 0)                                     */
+
+/* Per-dimension constants of the measure for the handle's current kernel (d doubles each, host).  GPX_EINVAL for a
+ * non-SE kernel, a d other than the kernel's, lower >= upper, std <= 0 or a non-finite value.  gpx_set_kernel clears
+ * the measure; the calls below return GPX_ENOKERNEL without one. */
+int gpx_set_measure(gpx_handle h, int kind, int d, const double* p0, const double* p1);
+
+/* out[i*ld + j] = Phi(X[i], Y[j]) (the measure's analogue of gpx_gram, no nugget); gpx_phi_diag: out[j] = Phi(X[j], X[j]).
+ * One exp of the summed exponent per element; a result below 2^-1022 is returned as 0, as gpx_gram flushes k. */
+int gpx_phi_gram(gpx_handle h, const double* X, int64_t nx, int64_t ldx, const double* Y, int64_t ny, int64_t ldy,
+                 double* out, int64_t ld, void* stream);
+int gpx_phi_diag(gpx_handle h, const double* X, int64_t n, int64_t ldx, double* out, void* stream);
+
+/* Row n of Z for every column j < ncols, the recurrence of gpx_append_row with Phi as the source term:
+ *     Z[n, j] = (Phi(x_p, Y[j]) - sum_{i<n} rec.col[i] Z[i, j]) / sqrt(rec[2])      (no running variance)
+ * rec: the pivot record of the same step (gpx_gather_pivot).  ldz even, Z 16-byte aligned.  Reads 8*n*ncols bytes. */
+int gpx_phi_append_row(gpx_handle h, const double* rec, const double* Y, int64_t ncols, int64_t ldy, double* Z,
+                       int64_t ldz, int64_t n, void* stream);
+
+/* Row and column n of Psi after the append of design point n: U^T x = b with b_k = Z[n, cols[k] - index_offset]
+ * (k <= n; cols = the design's candidate indices, e.g. the engine's picks), Psi[n, k] = Psi[k, n] = x_k.  One block;
+ * U (ldu > n) as grown by gpx_store_pivot. */
+int gpx_psi_row(gpx_handle h, const double* U, int64_t ldu, const double* Z, int64_t ldz, const int64_t* cols,
+                int64_t index_offset, int64_t n, double* Psi, int64_t ldpsi, void* stream);
+
+/* Cost of design+{c} for every candidate c from the stored rows (W, Z, Y share the leading dimension ld):
+ *     score[c] = |s - tr Psi - q_c / (varC[c] + noise)|,  q_c = phic[c] - 2 sum_{i<n} W[i,c] Z[i,c] + sum_{i<n} W[i,c] Y[i,c]
+ * (reduction 0 where varC[c] + noise <= zero_tol, as gpx_score_ivar), then the arg-min into best/idx.  update != 0 first
+ * brings Y up to date with the last append: Y[i,c] += Psi[i,n-1] W[n-1,c] (i < n-1), Y[n-1,c] = sum_j Psi[n-1,j] W[j,c].
+ * cost (nullable, device) receives s - tr Psi.  One pass: reads 3n doubles per candidate, writes n with update. */
+int gpx_ivar_measure_score(gpx_handle h, const double* W, const double* Z, double* Y, int64_t ld, const double* phic,
+                           const double* varC, int64_t C, int64_t n, int update, const double* Psi, int64_t ldpsi,
+                           double noise, double zero_tol, double* cost, double* score_out, double* best, int64_t* idx,
+                           void* stream);
+
 /* ---- Resident posterior covariance: the HBM-bound alternative for greedy IVAR loops (SURVEY.md section 7) -----------
  * cov (M x ldcov, row m = integration point, 8*M*C bytes resident) holds cov_D(m,c); each greedy step is ONE pass
  *     cov -= a b^T ,  partial[seg][c] = sum_{m in seg} cov[m,c]^2          (16 B of HBM traffic per pair, any n)
