@@ -3,7 +3,8 @@
 
 UniformMeasure and GaussianMeasure are not in the reference: set as `costFunctionGP_IVAR.measure`, they make the IVAR
 cost the exact integral of the posterior variance over that measure instead of its Monte-Carlo mean over mcPoints
-(squared-exponential kernels)."""
+(squared-exponential and Mehler kernels; a Mehler kernel needs std_q^2 < (1 + t_q) / (2 t_q) in a GaussianMeasure, or
+the integral of its prior variance is infinite)."""
 from typing import Callable, Optional
 
 import numpy as np

@@ -31,20 +31,31 @@ struct KCenter {
     double c[GPX_MAX_DIM];
 };
 
-// Integration measure of the closed-form IVAR path (gpx_set_measure), for the handle's SE kernel:
+// Integration measure of the closed-form IVAR path (gpx_set_measure), for the handle's SE or Mehler kernel:
 //   Phi(x, y) = pref * exp(sum_q [-a4_q (x_q - y_q)^2 + E_q(m_q)]) * prod_q F_q(m_q),   m = (x + y) / 2
-// with E_q F_q the per-dimension factor I_q(m_q) of include/gpexp_b200.h split into an exponent and a bounded rest.
-//   BOX    p0 = lo_q / cl_q, p1 = hi_q / cl_q, rs_q = 1 / cl_q, width_q = (hi_q - lo_q) / cl_q ; pref = s^2 / prod width_q
-//   GAUSS  p0 = mean_q, rs_q = 1 / sqrt(cl_q^2 + 2 std_q^2)                                  ; pref = s^2 prod (1 + 2 std_q^2 / cl_q^2)^-1/2
+// with E_q F_q the per-dimension factor of include/gpexp_b200.h split into an exponent and a bounded rest.
+// SE (a4_q = 1 / (4 cl_q^2)):
+//   BOX    p0 = lo_q, p1 = hi_q, rs_q = 1 / cl_q, width_q = (hi_q - lo_q) / cl_q      ; pref = s^2 / prod width_q
+//   GAUSS  p0 = mean_q, rs_q = 1 / sqrt(cl_q^2 + 2 std_q^2)                           ; pref = s^2 prod (1 + 2 std_q^2 / cl_q^2)^-1/2
+// MEHLER (r_q = 1 - t_q^2, a4_q = t_q^2 / (4 r_q)):
+//   BOX    p0, p1 = sorted(t_q lo_q, t_q hi_q), rs_q = r_q^-1/2, width_q = |t_q| (hi_q - lo_q) / sqrt(r_q); E_q includes m^2
+//          and F_q is the mean J / width_q                                             ; pref = prod 1 / r_q
+//   GAUSS  E_q(m) = g2_q m^2 + g1_q m + g0_q, g = r + 2 t^2 std^2:  g2 = t^2 (2 std^2 - 1) / g, g1 = 2 t mean / g,
+//          g0 = -t^2 mean^2 / g                                                        ; pref = prod (r_q g_q)^-1/2
+// prior = s = int k(x, x) dmu(x): the SE signal, or the Mehler product of gpx_set_measure's per-dimension integrals.
 struct MParams {
     int kind;
     int d;
     double pref;
+    double prior;
     double a4[GPX_MAX_DIM];
     double rs[GPX_MAX_DIM];
     double p0[GPX_MAX_DIM];
     double p1[GPX_MAX_DIM];
     double width[GPX_MAX_DIM];
+    double g2[GPX_MAX_DIM];
+    double g1[GPX_MAX_DIM];
+    double g0[GPX_MAX_DIM];
 };
 
 struct gpx_context {

@@ -1,7 +1,7 @@
-// Closed-form IVAR over a box or Gaussian measure for squared-exponential kernels: the measure's constants, the kernel
-// products Phi(x, y) = int k(t, x) k(t, y) dmu(t), the Z-row append, the Psi-row forward substitution and the scoring
-// pass.  The Monte-Carlo contraction of the other IVAR path is not used: every greedy step here is append-only or rank-1
-// and moves O(n C) doubles.
+// Closed-form IVAR over a box or Gaussian measure for squared-exponential and Mehler kernels: the measure's constants, the
+// kernel products Phi(x, y) = int k(t, x) k(t, y) dmu(t), the Z-row append, the Psi-row forward substitution and the
+// scoring pass.  The Monte-Carlo contraction of the other IVAR path is not used: every greedy step here is append-only or
+// rank-1 and moves O(n C) doubles.
 #include <float.h>
 #include <math.h>
 #include <string.h>
@@ -20,7 +20,10 @@
 //             a < 1/2: sqrt(pi)/2 (erf(b) - erf(a)); here b - a > 1 (else "narrow"), so erf(b) >= 2.2 (erf(b) - erf(a)).
 //             a >= 1/2: sqrt(pi)/2 e^{-a^2} (erfcx(a) - e^{-(b - a)(b + a)} erfcx(b)), the erfc difference without its
 //             tails; (b - a)(b + a) > 2 outside "narrow", so the bracket keeps more than 1 - e^-2 of erfcx(a).
+// MEAN returns J / (v - u) instead, for a width that may be 0 (Mehler with t = 0): "narrow" then gives the Gauss-Legendre
+// mean itself, never 0 / 0, and every other branch has width > 0.
 // ---------------------------------------------------------------------------------------------
+template <bool MEAN>
 __device__ __forceinline__ double box_tail_j(double u, double v, double width, double& E) {
     const double SQRTPI_2 = 0.88622692545275801365;
     const double c = 0.5 * (u + v);
@@ -37,29 +40,46 @@ __device__ __forceinline__ double box_tail_j(double u, double v, double width, d
             sum = fma(w[k], exp(-(2.0 * c + s) * s) + exp((2.0 * c - s) * s), sum);
         }
         E = -c * c;
-        return h * sum;
+        return MEAN ? 0.5 * sum : h * sum;
     }
     E = 0.0;
-    if (u <= 0.0 && v >= 0.0) return SQRTPI_2 * (erf(v) + erf(-u));
+    double j;
     const double a = fmin(fabs(u), fabs(v)), b = fmax(fabs(u), fabs(v));
-    if (a < 0.5) return SQRTPI_2 * (erf(b) - erf(a));
-    E = -a * a;
-    return SQRTPI_2 * (erfcx(a) - exp(-width * (a + b)) * erfcx(b));
+    if (u <= 0.0 && v >= 0.0) {
+        j = SQRTPI_2 * (erf(v) + erf(-u));
+    } else if (a < 0.5) {
+        j = SQRTPI_2 * (erf(b) - erf(a));
+    } else {
+        E = -a * a;
+        j = SQRTPI_2 * (erfcx(a) - exp(-width * (a + b)) * erfcx(b));
+    }
+    return MEAN ? j / width : j;
 }
 
-// one dimension of Phi(x, y): exponent sum S and bounded factor F
-template <int KIND>
+// one dimension of Phi(x, y): exponent sum S and bounded factor F.  Mehler, with t = t_q, r = 1 - t^2:
+//     k(z, x) k(z, y) = r^-1 exp(m^2 - t^2 (x - y)^2 / (4 r)) exp(-(t z - m)^2 / r)
+// so the box factor is J((t lo - m) / sqrt(r), (t hi - m) / sqrt(r)) / width with m^2 joining the exponent, and the Gaussian
+// one is the closed-form quadratic g2 m^2 + g1 m + g0 (MParams), whose arrangement avoids cancelling m^2 against
+// (m - t mean)^2 / g.
+template <int FAM, int KIND>
 __device__ __forceinline__ void phi_dim(const MParams& mp, int q, double x, double y, double& S, double& F) {
+    static_assert(FAM == GPX_SE || FAM == GPX_MEHLER, "the closed-form measure is for SE and Mehler kernels");
     const double df = x - y;
     S = fma(-df * df, mp.a4[q], S);
     const double m = 0.5 * (x + y);
-    if (KIND == GPX_MEASURE_GAUSS) {
+    if (FAM == GPX_SE && KIND == GPX_MEASURE_GAUSS) {
         const double t = (m - mp.p0[q]) * mp.rs[q];
         S = fma(-t, t, S);
+    } else if (FAM == GPX_SE) {
+        double E;
+        F *= box_tail_j<false>((mp.p0[q] - m) * mp.rs[q], (mp.p1[q] - m) * mp.rs[q], mp.width[q], E);
+        S += E;
+    } else if (KIND == GPX_MEASURE_GAUSS) {
+        S += fma(fma(mp.g2[q], m, mp.g1[q]), m, mp.g0[q]);
     } else {
         double E;
-        F *= box_tail_j((mp.p0[q] - m) * mp.rs[q], (mp.p1[q] - m) * mp.rs[q], mp.width[q], E);
-        S += E;
+        F *= box_tail_j<true>((mp.p0[q] - m) * mp.rs[q], (mp.p1[q] - m) * mp.rs[q], mp.width[q], E);
+        S += fma(m, m, E);
     }
 }
 
@@ -69,12 +89,12 @@ __device__ __forceinline__ double phi_finish(const MParams& mp, double S, double
     return fabs(v) < DBL_MIN ? 0.0 : v;
 }
 
-template <int KIND>
+template <int FAM, int KIND>
 __device__ __forceinline__ double phi_eval(const MParams& mp, const double* __restrict__ X, int64_t ldx, int64_t i,
                                            const double* __restrict__ Y, int64_t ldy, int64_t j) {
     double S = 0.0, F = 1.0;
 #pragma unroll 1
-    for (int q = 0; q < mp.d; ++q) phi_dim<KIND>(mp, q, X[q * ldx + i], Y[q * ldy + j], S, F);
+    for (int q = 0; q < mp.d; ++q) phi_dim<FAM, KIND>(mp, q, X[q * ldx + i], Y[q * ldy + j], S, F);
     return phi_finish(mp, S, F);
 }
 
@@ -89,15 +109,96 @@ __device__ __forceinline__ double phi_eval(const MParams& mp, const double* __re
         }                                              \
     } while (0)
 
+// the kernel families gpx_set_measure accepts (it rejects every other one)
+#define GPX_DISPATCH_MEASURE_FAMILY(fam, kind, ...)                \
+    do {                                                           \
+        if ((fam) == GPX_MEHLER) {                                 \
+            constexpr int FAM = GPX_MEHLER;                        \
+            GPX_DISPATCH_MEASURE(kind, __VA_ARGS__);               \
+        } else {                                                   \
+            constexpr int FAM = GPX_SE;                            \
+            GPX_DISPATCH_MEASURE(kind, __VA_ARGS__);               \
+        }                                                          \
+    } while (0)
+
 #define GPX_NEED_MEASURE(h)                                                                                 \
     do {                                                                                                    \
         GPX_NEED_KERNEL(h);                                                                                 \
         GPX_REQUIRE((h)->has_measure, GPX_ENOKERNEL, "gpx_set_measure has not been called for this kernel"); \
     } while (0)
 
+// int_lo^hi exp(c x^2) dx = e^K G for the box prior of a Mehler kernel (c = t / (1 + t), an erf for c < 0 and a
+// Dawson / erfi form for c > 0), as one composite 10-point Gauss-Legendre rule of the positive integrand
+// e^{c x^2 - K} = e^{c d (d + 2 xr)}, d = x - xr, K = c xr^2 its largest exponent on [lo, hi] (xr = +-max|x| for c > 0,
+// the point nearest 0 for c < 0).  Nodes are placed in d, so that their rounding is relative to the distance from the
+// peak, not to |x|.  Only the part of [lo, hi] where the exponent exceeds -50 is integrated: the rest adds less than
+// e^-50 relative.  Panels of half-width <= 1/2 min(|c|^-1/2, 1 / (|c| max |x|)) keep the exponent's slope within 1 and
+// its curvature within 1/4 per panel, where the rule is exact to rounding; the panel sums are added with Neumaier
+// compensation.  NaN when the panel count is not finite and below 2^20 (an overflowing box).
+static double mehler_box_integral(double c, double lo, double hi, double& K) {
+    static const double X[5] = {0x1.30e507891e27ap-3, 0x1.bbcc009016adcp-2, 0x1.5bdb9228de198p-1, 0x1.bae995e9cb2f3p-1,
+                                0x1.f2a3e062af2d8p-1};
+    static const double W[5] = {0x1.2e9de7014d6eep-2, 0x1.13baa7a559c01p-2, 0x1.c0b059d00bc30p-3, 0x1.32138c878efdep-3,
+                                0x1.1115f8b62dc1fp-4};
+    const double T = 50.0;
+    K = 0.0;
+    if (c == 0.0) return hi - lo;
+    double xk, xr[2], a[2], b[2];
+    int pieces = 0;
+    if (c > 0.0) {
+        xk = fmax(fabs(lo), fabs(hi));
+        const double xt = sqrt(fmax(0.0, xk * xk - T / c));
+        if (lo < -xt) {
+            xr[pieces] = -xk;
+            a[pieces] = lo;
+            b[pieces++] = fmin(hi, -xt);
+        }
+        if (hi > xt) {
+            xr[pieces] = xk;
+            a[pieces] = fmax(lo, xt);
+            b[pieces++] = hi;
+        }
+    } else {
+        xk = lo > 0.0 ? lo : (hi < 0.0 ? hi : 0.0);
+        const double xt = sqrt(xk * xk - T / c);
+        xr[0] = xk;
+        a[0] = fmax(lo, -xt);
+        b[0] = fmin(hi, xt);
+        pieces = 1;
+    }
+    // K = c xr^2 rounded, and its rounding error (exact products by fma) folded into G: e^K is then off by at most the
+    // rounding of exp, not by |K| ulp
+    const double cx = c * xk;
+    K = cx * xk;
+    const double Klo = fma(fma(c, xk, -cx), xk, fma(cx, xk, -K));
+    double sum = 0.0, comp = 0.0;
+    for (int p = 0; p < pieces; ++p) {
+        const double xm = fmax(fabs(a[p]), fabs(b[p]));
+        const double h = 0.5 * fmin(1.0 / sqrt(fabs(c)), 1.0 / (fabs(c) * xm));
+        const double panels = ceil((b[p] - a[p]) / (2.0 * h));
+        if (!(panels <= 1048576.0)) return NAN;
+        const int np = panels < 1.0 ? 1 : (int)panels;
+        const double da = a[p] - xr[p], hp = (b[p] - a[p]) / (2.0 * np), x2 = 2.0 * xr[p];
+        for (int k = 0; k < np; ++k) {
+            const double mid = da + (2 * k + 1) * hp;
+            double panel = 0.0;
+            for (int i = 0; i < 5; ++i) {
+                const double d0 = mid - hp * X[i], d1 = mid + hp * X[i];
+                panel += W[i] * (exp(c * (d0 * (d0 + x2))) + exp(c * (d1 * (d1 + x2))));
+            }
+            const double term = hp * panel, t = sum + term;
+            comp += fabs(sum) >= fabs(term) ? (sum - t) + term : (term - t) + sum;
+            sum = t;
+        }
+    }
+    return (sum + comp) * exp(Klo);
+}
+
 extern "C" int gpx_set_measure(gpx_handle h, int kind, int d, const double* p0, const double* p1) {
     GPX_NEED_KERNEL(h);
-    GPX_REQUIRE(h->kp.family == GPX_SE, GPX_EINVAL, "a closed-form measure needs a squared-exponential kernel");
+    const int fam = h->kp.family;
+    GPX_REQUIRE(fam == GPX_SE || fam == GPX_MEHLER, GPX_EINVAL,
+                "a closed-form measure needs a squared-exponential or Mehler kernel");
     GPX_REQUIRE(kind == GPX_MEASURE_BOX || kind == GPX_MEASURE_GAUSS, GPX_EINVAL, "unknown measure kind");
     GPX_REQUIRE(d == h->kp.d, GPX_EINVAL, "measure dimension differs from the kernel's");
     GPX_REQUIRE(p0 != nullptr && p1 != nullptr, GPX_EINVAL, "NULL parameter array");
@@ -106,13 +207,51 @@ extern "C" int gpx_set_measure(gpx_handle h, int kind, int d, const double* p0, 
     mp.kind = kind;
     mp.d = d;
     const double s = h->kp.signal;
-    double pref = s * s;
+    double pref = fam == GPX_SE ? s * s : 1.0;
+    double prior = fam == GPX_SE ? s : 1.0;
     for (int q = 0; q < d; ++q) {
         GPX_REQUIRE(isfinite(p0[q]) && isfinite(p1[q]), GPX_EINVAL, "measure parameters must be finite");
+        if (kind == GPX_MEASURE_BOX) {
+            GPX_REQUIRE(p0[q] < p1[q], GPX_EINVAL, "box needs lower < upper in every dimension");
+        } else {
+            GPX_REQUIRE(p1[q] > 0.0, GPX_EINVAL, "Gaussian measure needs std > 0 in every dimension");
+        }
+        if (fam == GPX_MEHLER) {
+            // t = kp.b / 2 exactly; r = 1 - t^2 as (1 - t)(1 + t), within 2 ulp also for t near 1
+            const double t = 0.5 * h->kp.b[q], r = (1.0 - t) * (1.0 + t);
+            mp.a4[q] = 0.25 * t * t / r;
+            if (kind == GPX_MEASURE_BOX) {
+                const double len = p1[q] - p0[q];
+                GPX_REQUIRE(isfinite(len), GPX_EINVAL, "box width overflows");
+                mp.rs[q] = 1.0 / sqrt(r);
+                mp.p0[q] = t >= 0.0 ? t * p0[q] : t * p1[q];
+                mp.p1[q] = t >= 0.0 ? t * p1[q] : t * p0[q];
+                mp.width[q] = fabs(t) * len * mp.rs[q];
+                pref /= r;
+                // s_q = r^-1/2 / (hi - lo) int_lo^hi e^{c x^2} dx
+                double K;
+                const double G = mehler_box_integral(t / (1.0 + t), p0[q], p1[q], K);
+                prior *= G / (len * sqrt(r)) * exp(K);
+            } else {
+                const double sd2 = p1[q] * p1[q], mu = p0[q];
+                const double g = fma(2.0 * t * t, sd2, r);
+                mp.g2[q] = t * t * fma(2.0, sd2, -1.0) / g;
+                mp.g1[q] = 2.0 * t * mu / g;
+                mp.g0[q] = -(t * t) * (mu * mu) / g;
+                pref /= sqrt(r * g);
+                // s_q = r^-1/2 (1 - 2 c std^2)^-1/2 exp(c mean^2 / (1 - 2 c std^2)), c = t / (1 + t), written through
+                // num = (1 + t)(1 - 2 c std^2) = 1 + t - 2 t std^2
+                const double num = fma(-2.0 * t, sd2, 1.0 + t);
+                GPX_REQUIRE(num > 0.0, GPX_EINVAL,
+                            "Gaussian measure too wide for the Mehler kernel: int k(x, x) dmu is infinite unless "
+                            "std^2 < (1 + t) / (2 t) in every dimension");
+                prior *= exp(t * mu * mu / num) / sqrt((1.0 - t) * num);
+            }
+            continue;
+        }
         const double a = h->kp.a[q];  // cl_q^-2
         mp.a4[q] = 0.25 * a;
         if (kind == GPX_MEASURE_BOX) {
-            GPX_REQUIRE(p0[q] < p1[q], GPX_EINVAL, "box needs lower < upper in every dimension");
             mp.rs[q] = sqrt(a);
             mp.p0[q] = p0[q];
             mp.p1[q] = p1[q];
@@ -120,7 +259,6 @@ extern "C" int gpx_set_measure(gpx_handle h, int kind, int d, const double* p0, 
             GPX_REQUIRE(isfinite(mp.width[q]), GPX_EINVAL, "box width overflows");
             pref /= mp.width[q];
         } else {
-            GPX_REQUIRE(p1[q] > 0.0, GPX_EINVAL, "Gaussian measure needs std > 0 in every dimension");
             const double g = fma(2.0 * p1[q] * p1[q], a, 1.0);  // 1 + 2 std^2 / cl^2
             GPX_REQUIRE(isfinite(g), GPX_EINVAL, "Gaussian std overflows");
             mp.rs[q] = sqrt(a / g);                              // 1 / sqrt(cl^2 + 2 std^2)
@@ -129,7 +267,10 @@ extern "C" int gpx_set_measure(gpx_handle h, int kind, int d, const double* p0, 
             pref /= sqrt(g);
         }
     }
+    GPX_REQUIRE(isfinite(pref) && isfinite(prior) && prior > 0.0, GPX_EINVAL,
+                "int k(x, x) dmu or the Phi prefactor is not a finite positive double for this kernel and measure");
     mp.pref = pref;
+    mp.prior = prior;
     h->mp = mp;
     h->has_measure = true;
     return GPX_OK;
@@ -139,13 +280,13 @@ extern "C" int gpx_set_measure(gpx_handle h, int kind, int d, const double* p0, 
 // Phi(X_i, Y_j) cross block and diagonal.  Per element: d evaluations of erf / erfcx (box) or one FMA chain (Gaussian)
 // and one exp; the coordinates are re-read from L1 for every row rather than kept in a per-dimension register array.
 // ---------------------------------------------------------------------------------------------
-template <int KIND>
+template <int FAM, int KIND>
 __global__ void __launch_bounds__(256) phi_gram_kernel(const __grid_constant__ MParams mp, const double* __restrict__ X,
                                                        int64_t nx, int64_t ldx, const double* __restrict__ Y, int64_t ny,
                                                        int64_t ldy, double* __restrict__ out, int64_t ld) {
     const int64_t j = (int64_t)blockIdx.x * 256 + threadIdx.x;
     if (j >= ny) return;
-    for (int64_t i = blockIdx.y; i < nx; i += gridDim.y) out[i * ld + j] = phi_eval<KIND>(mp, X, ldx, i, Y, ldy, j);
+    for (int64_t i = blockIdx.y; i < nx; i += gridDim.y) out[i * ld + j] = phi_eval<FAM, KIND>(mp, X, ldx, i, Y, ldy, j);
 }
 
 extern "C" int gpx_phi_gram(gpx_handle h, const double* X, int64_t nx, int64_t ldx, const double* Y, int64_t ny,
@@ -155,16 +296,16 @@ extern "C" int gpx_phi_gram(gpx_handle h, const double* X, int64_t nx, int64_t l
     if (nx == 0 || ny == 0) return GPX_OK;
     GPX_REQUIRE(X && Y && out, GPX_EINVAL, "NULL pointer");
     const dim3 grid((unsigned)((ny + 255) / 256), (unsigned)(nx < 65535 ? nx : 65535));
-    GPX_DISPATCH_MEASURE(h->mp.kind, (phi_gram_kernel<KIND><<<grid, 256, 0, (cudaStream_t)stream>>>(h->mp, X, nx, ldx, Y, ny,
+    GPX_DISPATCH_MEASURE_FAMILY(h->kp.family, h->mp.kind, (phi_gram_kernel<FAM, KIND><<<grid, 256, 0, (cudaStream_t)stream>>>(h->mp, X, nx, ldx, Y, ny,
                                                                                                      ldy, out, ld)));
     return gpx_check_launch("gpx_phi_gram");
 }
 
-template <int KIND>
+template <int FAM, int KIND>
 __global__ void __launch_bounds__(256) phi_diag_kernel(const __grid_constant__ MParams mp, const double* __restrict__ X,
                                                        int64_t n, int64_t ldx, double* __restrict__ out) {
     const int64_t j = (int64_t)blockIdx.x * 256 + threadIdx.x;
-    if (j < n) out[j] = phi_eval<KIND>(mp, X, ldx, j, X, ldx, j);
+    if (j < n) out[j] = phi_eval<FAM, KIND>(mp, X, ldx, j, X, ldx, j);
 }
 
 extern "C" int gpx_phi_diag(gpx_handle h, const double* X, int64_t n, int64_t ldx, double* out, void* stream) {
@@ -172,7 +313,7 @@ extern "C" int gpx_phi_diag(gpx_handle h, const double* X, int64_t n, int64_t ld
     GPX_REQUIRE(n >= 0, GPX_EINVAL, "negative size");
     if (n == 0) return GPX_OK;
     GPX_REQUIRE(X && out, GPX_EINVAL, "NULL pointer");
-    GPX_DISPATCH_MEASURE(h->mp.kind, (phi_diag_kernel<KIND><<<(unsigned)((n + 255) / 256), 256, 0, (cudaStream_t)stream>>>(
+    GPX_DISPATCH_MEASURE_FAMILY(h->kp.family, h->mp.kind, (phi_diag_kernel<FAM, KIND><<<(unsigned)((n + 255) / 256), 256, 0, (cudaStream_t)stream>>>(
                                           h->mp, X, n, ldx, out)));
     return gpx_check_launch("gpx_phi_diag");
 }
@@ -183,7 +324,7 @@ extern "C" int gpx_phi_diag(gpx_handle h, const double* X, int64_t n, int64_t ld
 // streaming loads), the pivot's W column in shared memory.  Reads 8 n ncols bytes.  A non-positive pivot appends a zero
 // row, as gpx_append_row does.
 // ---------------------------------------------------------------------------------------------
-template <int KIND>
+template <int FAM, int KIND>
 __global__ void __launch_bounds__(128) phi_append_kernel(const __grid_constant__ MParams mp, const double* __restrict__ rec,
                                                          const double* __restrict__ Y, int64_t ncols, int64_t ldy,
                                                          double* __restrict__ Z, int64_t ldz, int n) {
@@ -193,8 +334,8 @@ __global__ void __launch_bounds__(128) phi_append_kernel(const __grid_constant__
     const bool active = j < ncols, two = j + 1 < ncols;
     double s0 = 0.0, s1 = 0.0;
     // the pivot's coordinates are rec[3 .. 3+d), read as a one-column coordinate array
-    if (active) s0 = phi_eval<KIND>(mp, rec + 3, 1, 0, Y, ldy, j);
-    if (two) s1 = phi_eval<KIND>(mp, rec + 3, 1, 0, Y, ldy, j + 1);
+    if (active) s0 = phi_eval<FAM, KIND>(mp, rec + 3, 1, 0, Y, ldy, j);
+    if (two) s1 = phi_eval<FAM, KIND>(mp, rec + 3, 1, 0, Y, ldy, j + 1);
     const double lnn = rec[2] > 0.0 ? sqrt(rec[2]) : INFINITY;
     __syncthreads();
     if (!active) return;
@@ -223,12 +364,12 @@ extern "C" int gpx_phi_append_row(gpx_handle h, const double* rec, const double*
     GPX_REQUIRE(smem <= 200 * 1024, GPX_ESIZE, "design size exceeds the shared-memory column buffer (25600)");
     cudaStream_t st = (cudaStream_t)stream;
     const unsigned grid = (unsigned)((ncols + 255) / 256);
-    GPX_DISPATCH_MEASURE(h->mp.kind, {
+    GPX_DISPATCH_MEASURE_FAMILY(h->kp.family, h->mp.kind, {
         if (smem > 48 * 1024) {
-            const int rc = gpx_ensure_smem(h, (const void*)phi_append_kernel<KIND>, 200 * 1024, "phi_append_row");
+            const int rc = gpx_ensure_smem(h, (const void*)phi_append_kernel<FAM, KIND>, 200 * 1024, "phi_append_row");
             if (rc) return rc;
         }
-        phi_append_kernel<KIND><<<grid, 128, smem, st>>>(h->mp, rec, Y, ncols, ldy, Z, ldz, (int)n);
+        phi_append_kernel<FAM, KIND><<<grid, 128, smem, st>>>(h->mp, rec, Y, ncols, ldy, Z, ldz, (int)n);
     });
     return gpx_check_launch("gpx_phi_append_row");
 }
@@ -445,11 +586,11 @@ extern "C" int gpx_ivar_measure_score(gpx_handle h, const double* W, const doubl
             if (rc) return rc;
         }
         ivar_measure_score_kernel<true><<<(unsigned)blocks, 256, smem, st>>>(W, Z, Y, ld, phic, varC, C, (int)n, Psi, ldpsi,
-                                                                            h->kp.signal, noise, zero_tol, cost, score_out,
+                                                                            h->mp.prior, noise, zero_tol, cost, score_out,
                                                                             h->red_val, h->red_idx, h->red_counter, best, idx);
     } else {
         ivar_measure_score_kernel<false><<<(unsigned)blocks, 256, 0, st>>>(W, Z, Y, ld, phic, varC, C, (int)n, Psi, ldpsi,
-                                                                          h->kp.signal, noise, zero_tol, cost, score_out,
+                                                                          h->mp.prior, noise, zero_tol, cost, score_out,
                                                                           h->red_val, h->red_idx, h->red_counter, best, idx);
     }
     return gpx_check_launch("gpx_ivar_measure_score");

@@ -866,13 +866,15 @@ class GreedyIVAREngine(_Pivoting):
 
 
 class MeasureIVAREngine(_Pivoting):
-    """Discrete greedy IVAR with the integral over a box or Gaussian measure in closed form (squared-exponential kernels):
-    no integration points and no contraction.  With K_DD + diag(noise) = U^T U it keeps, for the candidates,
+    """Discrete greedy IVAR with the integral over a box or Gaussian measure in closed form (squared-exponential and
+    Mehler kernels): no integration points and no contraction.  With K_DD + diag(noise) = U^T U it keeps, for the
+    candidates,
         W_C = U^-T K(D, C),  Z_C = U^-T Phi(D, C),  Y_C = Psi W_C,  Phi_cc,  varC
     and Psi = U^-T Phi_DD U^-1 (n x n), Phi(a, b) = int k(x, a) k(x, b) dmu(x).  The cost of design + {c} is
         |s - tr Psi - q_c / (varC_c + noise)|,   q_c = Phi_cc - 2 w_c.z_c + w_c.y_c,
-    the M -> infinity limit of GreedyIVAREngine's score.  A step appends one row to W_C and Z_C, one row and column to
-    Psi, and the scoring pass updates Y_C by one rank-1 term and one new row: O(n C) memory traffic.
+    the M -> infinity limit of GreedyIVAREngine's score.  s = int k(x, x) dmu(x) is the signal for SE kernels and a
+    per-(kernel, measure) constant computed by gpx_set_measure for Mehler kernels.  A step appends one row to W_C and
+    Z_C, one row and column to Psi, and the scoring pass updates Y_C by one rank-1 term and one new row: O(n C) memory traffic.
 
     measure: (kind, p0, p1) with kind = _lib.MEASURE_BOX (p0 = lower, p1 = upper bounds) or _lib.MEASURE_GAUSS (p0 =
     means, p1 = standard deviations), d doubles each.  cand_noise as in GreedyIVAREngine (noise-inclusive varC).
@@ -880,8 +882,9 @@ class MeasureIVAREngine(_Pivoting):
 
     def __init__(self, dev: Device, cand: PointSet, n_max: int, noise: float, kernel_spec, measure, cand_noise=None):
         fam, d, params = kernel_spec
-        if fam != _lib.SE:
-            raise NotImplementedError("the closed-form measure integral is implemented for squared-exponential kernels only")
+        if fam not in (_lib.SE, _lib.MEHLER):
+            raise NotImplementedError("the closed-form measure integral is implemented for squared-exponential and Mehler "
+                                      "kernels only")
         self.cand = cand
         self.kernel_spec = (fam, d, np.asarray(params, dtype=np.float64))
         kind, p0, p1 = measure

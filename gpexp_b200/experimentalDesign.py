@@ -20,6 +20,7 @@ module, and its optimiser loops then drive the device path unchanged.
 import copy
 import hashlib
 import itertools
+import math
 
 import numpy as np
 
@@ -54,8 +55,9 @@ def _ivar_weights(self):
 
 def _ivar_measure(self, what=None):
     """The cost function's `measure` as (kind, lower-or-mean, upper-or-std) for its kernel's dimension, or None.
-    ValueError with mcWeights set as well; NotImplementedError for a kernel other than squared-exponential and for `what`
-    (the name of a feature the closed form does not support), each naming the measure."""
+    ValueError with mcWeights set as well, and for a Gaussian measure too wide for a Mehler kernel (int k(x, x) dmu is
+    infinite unless std_q^2 < (1 + t_q) / (2 t_q)); NotImplementedError for a kernel other than squared-exponential or
+    Mehler and for `what` (the name of a feature the closed form does not support), each naming the measure."""
     m = getattr(self, "measure", None)
     if m is None:
         return None
@@ -63,12 +65,19 @@ def _ivar_measure(self, what=None):
         raise ValueError(f"{m!r} integrates exactly and mcWeights weights integration points: set one of the two")
     if what is not None:
         raise NotImplementedError(f"{m!r}: {what} is not implemented for the closed-form measure integral")
-    fam, d, _ = self.gaussianProcess.kernel._gpx_spec()
-    if fam != _lib.SE:
+    fam, d, params = self.gaussianProcess.kernel._gpx_spec()
+    if fam not in (_lib.SE, _lib.MEHLER):
         raise NotImplementedError(f"{m!r}: the closed-form measure integral is implemented for squared-exponential "
-                                  f"kernels only")
+                                  f"and Mehler kernels only")
     p0, p1 = m.params(d)
-    return (_lib.MEASURE_BOX if isinstance(m, UniformMeasure) else _lib.MEASURE_GAUSS), p0, p1
+    gauss = not isinstance(m, UniformMeasure)
+    if gauss and fam == _lib.MEHLER:
+        t = np.asarray(params, dtype=np.float64)
+        for q in range(d):
+            if t[q] > 0.0 and not p1[q] * p1[q] < (1.0 + t[q]) / (2.0 * t[q]):
+                raise ValueError(f"{m!r} is too wide for the Mehler kernel in dimension {q} (t = {t[q]!r}): "
+                                 f"int k(x, x) dmu is infinite there unless std < {math.sqrt((1.0 + t[q]) / (2.0 * t[q]))!r}")
+    return (_lib.MEASURE_GAUSS if gauss else _lib.MEASURE_BOX), p0, p1
 
 
 def _ivar_evaluate(self, inputPoints):
@@ -207,10 +216,13 @@ class costFunctionGP_IVAR(costFunctionBase):
     there the caller sets `cf.mcWeights = w` after construction.
 
     measure (attribute or keyword, default None): a gpexp_b200.approximation.UniformMeasure or GaussianMeasure.  The cost
-    is then the exact |int var(x) dmu(x)| for a squared-exponential kernel, with no integration points and no sampling
-    error; evaluate, the greedy drivers and scoreCandidatesIVAR use it (a heteroscedastic space.noiseFunc applies as in
-    the Monte-Carlo path).  With a measure, mcPoints is not sampled when not given.  ValueError together with mcWeights;
-    NotImplementedError for other kernels, derivative, refineGreedyIVARExperimentalDesign, shard= and resident=True."""
+    is then the exact |int var(x) dmu(x)| for a squared-exponential or Mehler kernel, with no integration points and no
+    sampling error; evaluate, the greedy drivers and scoreCandidatesIVAR use it (a heteroscedastic space.noiseFunc
+    applies as in the Monte-Carlo path).  With a measure, mcPoints is not sampled when not given.  A Mehler kernel's
+    prior variance grows like exp(x^2 t / (1 + t)), so its Monte-Carlo estimate under N(0, 1) has infinite variance for
+    t >= 1/3; the closed form has none.  ValueError together with mcWeights, and for a GaussianMeasure with
+    std_q^2 >= (1 + t_q) / (2 t_q) under a Mehler kernel (the integral is infinite); NotImplementedError for Matern
+    kernels, derivative, refineGreedyIVARExperimentalDesign, shard= and resident=True."""
 
     mcWeights = None
     measure = None
@@ -353,8 +365,9 @@ def beginGreedyIVARExperimentalDesign(costFuncIVAR, candidates, nPoints, shard=N
     With `costFuncIVAR.mcWeights` the cost of design + [c] is the weighted sum over the integration points (see
     costFunctionGP_IVAR); the weights are replicated with the integration points, so every rank passes the same ones.
 
-    With `costFuncIVAR.measure` the engine is a gpexp_b200.engine.MeasureIVAREngine (exact integral, `.run(n)`,
-    `.indices()`, `.pick_scores`); shard and resident=True raise NotImplementedError there."""
+    With `costFuncIVAR.measure` the engine is a gpexp_b200.engine.MeasureIVAREngine (exact integral for a
+    squared-exponential or Mehler kernel, `.run(n)`, `.indices()`, `.pick_scores`); shard and resident=True raise
+    NotImplementedError there."""
     gp = costFuncIVAR.gaussianProcess
     meas = _ivar_measure(costFuncIVAR, "shard=" if shard is not None else "resident=True" if resident else None)
     weights = None if meas is not None else _ivar_weights(costFuncIVAR)

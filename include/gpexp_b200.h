@@ -258,21 +258,32 @@ int gpx_score_ivar_w(gpx_handle h, int prologue, const double* Wm, int64_t ldm, 
                      double noise, double zero_tol, const double* wM, const uint8_t* mask, double* workspace,
                      double* score_out, double* best, int64_t* idx, void* stream);
 
-/* ---- Closed-form IVAR over a measure (squared-exponential kernels) ---------------------------------------------------
+/* ---- Closed-form IVAR over a measure (squared-exponential and Mehler kernels) ----------------------------------------
  * Replaces the Monte-Carlo estimate of int var_D(x) dmu(x) (the mean over mcPoints, experimentalDesign.py:105-117, and
  * the M x n x C contraction of gpx_score_ivar) by its exact value for a product measure mu:
- *     Phi(a, b) = int k(x, a) k(x, b) dmu(x) = s^2 prod_q exp(-(a_q - b_q)^2 / (4 cl_q^2)) I_q((a_q + b_q) / 2)
+ * SE:     Phi(a, b) = int k(x, a) k(x, b) dmu(x) = s^2 prod_q exp(-(a_q - b_q)^2 / (4 cl_q^2)) I_q((a_q + b_q) / 2)
  *     GPX_MEASURE_BOX    uniform on [lo_q, hi_q]:  I_q(m) = cl_q sqrt(pi) / (2 (hi_q - lo_q)) (erf((hi_q - m)/cl_q) - erf((lo_q - m)/cl_q))
  *     GPX_MEASURE_GAUSS  N(mean_q, std_q^2):        I_q(m) = (1 + 2 std_q^2/cl_q^2)^-1/2 exp(-(m - mean_q)^2 / (cl_q^2 + 2 std_q^2))
+ *         s = int k(x, x) dmu = signalSize
+ * MEHLER: Phi(a, b) = prod_q Phi_q(a_q, b_q); with t = t_q, r = 1 - t^2, m = (a + b) / 2:
+ *     GPX_MEASURE_BOX    Phi_q = r^-1 exp(m^2 - t^2 (a - b)^2 / (4 r)) J(u, v) / w,  J(u, v) = int_u^v e^{-s^2} ds,
+ *                        u, v = sorted((t lo - m) / sqrt(r), (t hi - m) / sqrt(r)), w = |t| (hi - lo) / sqrt(r)
+ *                        (J / w = e^{-u^2} at t = 0)
+ *     GPX_MEASURE_GAUSS  Phi_q = (r g)^-1/2 exp(-t^2 (a - b)^2 / (4 r) + [t^2 (2 std^2 - 1) m^2 + 2 t mean m - t^2 mean^2] / g),
+ *                        g = r + 2 t^2 std^2  (under N(0, 1): Phi = the Mehler kernel with parameter t^2)
+ *         s = prod_q s_q, c = t / (1 + t):  box  s_q = r^-1/2 / (hi - lo) int_lo^hi e^{c x^2} dx ;
+ *                                            Gaussian  s_q = r^-1/2 (1 - 2 c std^2)^-1/2 exp(c mean^2 / (1 - 2 c std^2)),
+ *                                            finite only for 2 c std^2 < 1
  * With K_DD + diag(noise) = U^T U, W_C = U^-T K(D, C), Z_C = U^-T Phi(D, C), Psi = U^-T Phi_DD U^-1 and Y_C = Psi W_C:
  *     int var_D dmu = s - tr Psi ,   int cov_D(x, c)^2 dmu = q_c = Phi_cc - 2 w_c.z_c + w_c.y_c
  * and the cost of design+{c} is |s - tr Psi - q_c / (var_D(c) + noise_c)|, the M -> infinity limit of gpx_score_ivar. */
 #define GPX_MEASURE_BOX 1   /* p0 = lower bounds, p1 = upper bounds (p0 < p1)                                */
 #define GPX_MEASURE_GAUSS 2 /* p0 = means, p1 = standard deviations (> 0)                                     */
 
-/* Per-dimension constants of the measure for the handle's current kernel (d doubles each, host).  GPX_EINVAL for a
- * non-SE kernel, a d other than the kernel's, lower >= upper, std <= 0 or a non-finite value.  gpx_set_kernel clears
- * the measure; the calls below return GPX_ENOKERNEL without one. */
+/* Per-dimension constants of the measure, and s, for the handle's current kernel (d doubles each, host).  GPX_EINVAL for
+ * a kernel other than SE or Mehler, a d other than the kernel's, lower >= upper, std <= 0, a non-finite value, or an s
+ * that is not a finite positive double (a Gaussian too wide for a Mehler kernel, an overflowing box).  gpx_set_kernel
+ * clears the measure; the calls below return GPX_ENOKERNEL without one. */
 int gpx_set_measure(gpx_handle h, int kind, int d, const double* p0, const double* p1);
 
 /* out[i*ld + j] = Phi(X[i], Y[j]) (the measure's analogue of gpx_gram, no nugget); gpx_phi_diag: out[j] = Phi(X[j], X[j]).
